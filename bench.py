@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          (N > 1: launched under torchrun)
   python bench.py --impl reference ...                    (CPU oracle port, rank 0 only)
+  python bench.py ... --dump-outputs DIR                  (also write what the last timed step computed)
 
 Workload: BASELINE.json configs[2] = synthetic 4096x3000 (12 MP) scans, vertical + horizontal,
 8-step phase shift + 10-bit Gray code (56 u8 frames per scan).  A "step" is one pass of the hot
@@ -27,6 +28,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (no __pycache__ in it)
 
 import numpy as np
 
@@ -133,6 +135,49 @@ class ClockSampler:
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": mx,
                 "reasons": sorted(reasons), "samples": len(sm), "window": window,
                 "power_w": float(np.median(pw)) if pw else None}
+
+
+DUMP_SEED = 0x3D5CA9
+DUMP_SAMPLES = 1 << 18      # pixels of every plane and rows of the point cloud written per scan
+DUMP_SCANS = 4              # scans written at most: 4 x 2^18 x 40 B = 42 MB
+
+
+def scan_outputs(s3, ctx, dirs):
+    """What a caller of the timed path reads back after a context's last scan (include/scan3d.h results)."""
+    out = {"unwrapped_v": ctx.plane(s3.PLANE_UNWRAPPED_V), "code_v": ctx.code_i32(0), "valid": ctx.plane(s3.PLANE_VALID)}
+    if dirs == 2:
+        out.update(unwrapped_h=ctx.plane(s3.PLANE_UNWRAPPED_H), code_h=ctx.code_i32(1),
+                   cpmap=ctx.plane(s3.PLANE_CPMAP), points=ctx.points())
+    return out
+
+
+def oracle_outputs(r, dirs):
+    """The same arrays from one oracle reconstruction (--impl reference)."""
+    out = {"unwrapped_v": r.unwrapped_v, "code_v": r.code_v, "valid": r.valid_v if dirs == 1 else r.valid}
+    if dirs == 2:
+        out.update(unwrapped_h=r.unwrapped_h, code_h=r.code_h, cpmap=r.cpmap, points=r.pts)
+    return out
+
+
+def dump_outputs(out_dir, scans, H, W):
+    """--dump-outputs: scans = {ring member k: () -> {name: array}} -> out_dir/ring<k>_<name>.npy, float32 (the point
+    count float64).  Every per-pixel plane is sampled at one seeded set of DUMP_SAMPLES pixels and the point cloud at
+    a seeded set of DUMP_SAMPLES rows (the same for every scan and both arms), so that the files stay below 64 MB."""
+    assert len(scans) <= DUMP_SCANS
+    os.makedirs(out_dir, exist_ok=True)
+    n = DUMP_SAMPLES
+    npix = H * W
+    pix = np.arange(npix) if npix <= n else np.sort(np.random.default_rng(DUMP_SEED).choice(npix, n, replace=False))
+    for k, fetch in sorted(scans.items()):
+        for name, a in fetch().items():
+            if name == "points":
+                np.save(os.path.join(out_dir, "ring%d_point_count.npy" % k), np.array([len(a)], np.float64))
+                if len(a) > n:
+                    a = a[np.sort(np.random.default_rng(DUMP_SEED + 1).choice(len(a), n, replace=False))]
+            else:
+                a = np.asarray(a).reshape(npix, -1)[pix]
+                a = a[:, 0] if a.shape[1] == 1 else a
+            np.save(os.path.join(out_dir, "ring%d_%s.npy" % (k, name)), np.ascontiguousarray(a, np.float32))
 
 
 def oracle_scan_seconds(cfg, ocal, stack, roi, threads, min_seconds, max_runs):
@@ -298,7 +343,14 @@ def main():
     ap.add_argument("--contexts", type=int, default=4, help="contexts (each on its own stream) the batch alternates over")
     ap.add_argument("--cta-limit", type=int, default=1, help="CTA slots per SM each context's kernel may take (0 = all)")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"], help="row-shard workload, N>1: how the points reach rank 0")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/ring<k>_<name>.npy (rank 0: "
+                         "the last scans of up to 4 ring members; seeded samples of planes and points, < 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload.startswith("c5_"):
+        ap.error("--dump-outputs covers the frame-parallel workloads, not the row-sharded one")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -341,8 +393,10 @@ def main():
             run_oracle(cfg, ocal, stack, roi, threads=threads)
         t0 = time.time()
         for _ in range(args.steps):
-            run_oracle(cfg, ocal, stack, roi, threads=threads)
+            r = run_oracle(cfg, ocal, stack, roi, threads=threads)
         dt = time.time() - t0
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {0: lambda: oracle_outputs(r, dirs)}, H, W)     # ring member 0 = this stack
         val = args.steps * npix / dt / 1e6
         config["scans_per_gpu_per_step"] = 1
         line = {"impl": "reference", "metric": METRIC, "value": val, "unit": "Mpix/s", "n_gpus": args.gpus,
@@ -471,6 +525,14 @@ def main():
     launches = sum(c.launch_count() for c in ctxs) - l0
     clocks = sampler.stop(t_wall0, t_wall1)
     count = ctx.point_count() if dirs == 2 else 0
+    if args.dump_outputs and rank == 0:
+        # each context still holds the results of its last scan of the last step (the e2e leg below reuses ctx):
+        # the last DUMP_SCANS of them, named by the ring member they read
+        last = {}
+        for b in range(args.batch):
+            last[b % len(ctxs)] = b
+        scans = {b % args.ring: ctxs[c] for c, b in sorted(last.items(), key=lambda cb: cb[1])[-DUMP_SCANS:]}
+        dump_outputs(args.dump_outputs, {k: (lambda c=c: scan_outputs(s3, c, dirs)) for k, c in scans.items()}, H, W)
     tms = torch.tensor([ms], device="cuda", dtype=torch.float64)
     if world > 1:
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)

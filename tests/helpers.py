@@ -1,15 +1,10 @@
-"""Shared test helpers: golden fixtures, calibration, reference-tree access."""
+"""Shared test helpers: golden fixtures, calibration."""
 import json
 import os
 
 import numpy as np
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-REF = "/root/reference/M_tech_project_console/"
-
-
-def have_reference():
-    return os.path.isdir(REF)
 
 
 def load_calib_c1():
@@ -35,14 +30,3 @@ def load_c1_crop():
 def load_c1_full():
     """The reference's whole captured scan (tools/make_golden.py c1full)."""
     return dict(np.load(os.path.join(GOLDEN, "c1_full.npz")))
-
-
-def read_bmp8(path):
-    b = open(path, "rb").read()
-    off = int.from_bytes(b[10:14], "little")
-    W = int.from_bytes(b[18:22], "little", signed=True)
-    H = int.from_bytes(b[22:26], "little", signed=True)
-    assert int.from_bytes(b[28:30], "little") == 8
-    stride = (W + 3) & ~3
-    a = np.frombuffer(b[off:off + stride * abs(H)], np.uint8).reshape(abs(H), stride)[:, :W]
-    return a[::-1].copy() if H > 0 else a.copy()

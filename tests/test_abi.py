@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 import oracle_ffi as o
-from helpers import GOLDEN, REF, have_reference, load_calib_c1
+from helpers import GOLDEN, load_c1_full, load_calib_c1
 
 s3 = importlib.import_module("3dscan_b200")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -77,27 +77,6 @@ def test_pattern_rows_match_reference_generated_patterns():
     assert np.array_equal(s3.synth_pattern_row(0, 5, 32, 4, 768), k["fringe5_k4_h_col0"])
 
 
-@pytest.mark.skipif(not have_reference(), reason="reference tree not mounted")
-def test_reference_pattern_images_are_their_profiles():
-    """The device generator expands 1-D profiles: every stored pattern image of the reference is
-    constant along its stripes and equals the profile of its configuration, full frame."""
-    from helpers import read_bmp8
-    g = REF + "Generated_patterns/"
-    cases = [(f"Fringe_patterns/{d}/Pattern_{k}.bmp", 0, 3, 32, k, d) for d in ("Vertical", "Horizontal") for k in range(3)]
-    cases += [(f"Fringe_patterns/{d}/Pattern_3.bmp", 0, 4, 16, 3, d) for d in ("Vertical", "Horizontal")]
-    cases += [(f"Fringe_patterns/{d}/Pattern_4.bmp", 0, 5, 32, 4, d) for d in ("Vertical", "Horizontal")]
-    for d, M in (("Vertical", 6), ("Horizontal", 5)):
-        for j in range(M):
-            cases.append((f"Coded_patterns/Gray_coded/{d}/Pattern_{j}.bmp", 1, M, 32, j, d))
-            cases.append((f"Coded_patterns/Gray_coded/{d}/inverse_Pattern_{j}.bmp", 2, M, 32, j, d))
-    for path, kind, n_or_m, fw, k, d in cases:
-        img = read_bmp8(g + path)
-        length = img.shape[1] if d == "Vertical" else img.shape[0]
-        r = s3.synth_pattern_row(kind, n_or_m, fw, k, length)
-        want = np.broadcast_to(r[None, :] if d == "Vertical" else r[:, None], img.shape)
-        assert np.array_equal(img, want), path
-
-
 def _cal():
     c = load_calib_c1()
     args = [c[k] for k in ("Kc", "dc", "Kp", "dp", "rc", "tc", "rp", "tp")]
@@ -134,18 +113,66 @@ def test_synth_is_deterministic_and_row_shardable():
     assert 0.6 < roi.mean() < 0.8
 
 
-@pytest.mark.skipif(not have_reference(), reason="reference tree not mounted")
-def test_reference_tree_loaders():
-    cal = s3.load_calibration(REF)
+def _cv_xml(path, name, arr):
+    """A matrix file as OpenCV's cvSave writes it (opencv_storage, doubles as %.16e)."""
+    arr = np.asarray(arr, np.float64)
+    rows, cols = (arr.shape[0], 1) if arr.ndim == 1 else arr.shape
+    os.makedirs(os.path.dirname(path), exist_ok=True)
+    data = " ".join("%.16e" % v for v in arr.ravel())
+    with open(path, "w") as f:
+        f.write(f'<?xml version="1.0"?>\n<opencv_storage>\n<{name} type_id="opencv-matrix">\n  <rows>{rows}</rows>\n'
+                f"  <cols>{cols}</cols>\n  <dt>d</dt>\n  <data>\n    {data}</data></{name}>\n</opencv_storage>\n")
+
+
+def _cv_bmp8(path, img):
+    """An 8-bit grey BMP as cvSaveImage writes it: 256-entry grey palette, bottom-up rows padded to 4 bytes."""
+    H, W = img.shape
+    stride = (W + 3) & ~3
+    rows = np.zeros((H, stride), np.uint8)
+    rows[:, :W] = img[::-1]
+    pal = np.repeat(np.arange(256, dtype=np.uint8), 4).reshape(256, 4)
+    pal[:, 3] = 0
+    off = 14 + 40 + 1024
+    hdr = b"BM" + (off + rows.size).to_bytes(4, "little") + bytes(4) + off.to_bytes(4, "little")
+    info = b"".join(v.to_bytes(n, "little") for v, n in ((40, 4), (W, 4), (H, 4), (1, 2), (8, 2), (0, 4), (rows.size, 4),
+                                                          (0, 4), (0, 4), (0, 4), (0, 4)))
+    os.makedirs(os.path.dirname(path), exist_ok=True)
+    with open(path, "wb") as f:
+        f.write(hdr + info + pal.tobytes() + rows.tobytes())
+
+
+def test_reference_tree_loaders(tmp_path):
+    """load_calibration / load_captured_set on a tree laid out like the reference's: its calibration matrices
+    (tests/golden/calib_c1.json) and its whole captured scan (tests/golden/c1_full.npz) in the files and formats the
+    reference stores them in."""
+    root =str(tmp_path / "M_tech_project_console")
     c = load_calib_c1()
+    for path, name, key in (("/Camera_calibration/Matrices/cam_intrinsic_mat.xml", "cam_intrinsic_mat", "Kc"),
+                            ("/Camera_calibration/Matrices/cam_distortion_vect.xml", "cam_distortion_vect", "dc"),
+                            ("/Projector_calibration/Matrices/proj_intrinsic_mat.xml", "proj_intrinsic_mat", "Kp"),
+                            ("/Projector_calibration/Matrices/proj_distortion_vect.xml", "proj_distortion_vect", "dp"),
+                            ("/Triangulation/Camera_extrinsic_parametrs/world_to_cam_rot_vect.xml", "world_to_cam_rot_vect", "rc"),
+                            ("/Triangulation/Camera_extrinsic_parametrs/world_to_cam_trans_vect.xml", "world_to_cam_trans_vect", "tc"),
+                            ("/Triangulation/Projector_extrinsic_parametrs/world_to_proj_rot_vect.xml", "world_to_proj_rot_vect", "rp"),
+                            ("/Triangulation/Projector_extrinsic_parametrs/world_to_proj_trans_vect.xml", "world_to_proj_trans_vect", "tp")):
+        _cv_xml(root + path, name, c[key].reshape(3, 3) if key in ("Kc", "Kp") else c[key])
+    d = load_c1_full()
+    want = []
+    for name, key in (("Vertical", "v"), ("Horizontal", "h")):
+        fr = f"{root}/Captured_patterns/Fringe_patterns/{name}/Undistorted/"
+        gc = f"{root}/Captured_patterns/Coded_patterns/Gray_coded/{name}/Undistorted/"
+        for prefix, folder, frames in (("", fr, d[f"fringe_{key}"]), ("", gc, d[f"gray_{key}"]), ("inverse_", gc, d[f"inv_{key}"])):
+            for i, img in enumerate(frames):
+                _cv_bmp8(f"{folder}{prefix}Gray_captured_image_{i}.bmp", img)
+            want.append(frames)
+
+    cal = s3.load_calibration(root)
     for k in ("Kc", "dc", "Kp", "dp", "rc", "tc", "rp", "tp"):
         assert np.array_equal(np.array(list(getattr(cal, k))), c[k])
     cfg = s3.make_config(1600, 1200, 1280, 720, 3, 6, 5, 32, 32, 2)
-    stack = s3.load_captured_set(REF, cfg)
+    stack = s3.load_captured_set(root, cfg)
     assert stack.shape == (28, 1200, 1600)
-    from helpers import read_bmp8
-    want = read_bmp8(REF + "Captured_patterns/Coded_patterns/Gray_coded/Horizontal/Undistorted/inverse_Gray_captured_image_4.bmp")
-    assert np.array_equal(stack[-1], want)
+    assert np.array_equal(stack, np.concatenate(want))
 
 
 def test_bmp_and_ply_roundtrip(tmp_path):

@@ -11,7 +11,7 @@ import pytest
 
 import oracle_ffi as o
 from gpu_common import calibs, run_oracle, s3
-from helpers import load_c1_crop, load_calib_c1
+from helpers import load_c1_crop, load_c1_full, load_calib_c1
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CUDA_INC = "/usr/local/cuda/include"
@@ -130,24 +130,20 @@ def test_atan2_on_every_3_and_4_step_argument_pair(shim):
     assert np.array_equal(out.view(np.uint32), want.view(np.uint32))
 
 
-from helpers import REF, have_reference, read_bmp8  # noqa: E402
-
-
-@pytest.mark.skipif(not have_reference(), reason="reference tree not mounted")
 def test_reference_scan_full_frame_through_the_kernel_arithmetic(shim):
     """configs[0]: the reference's own 1600x1200 capture (3-step, 6/5 Gray bits, fw 32, its calibration files),
-    whole frame: the stored wrapped-phase image gives the mask, the stored unwrapped-phase images must come out of
-    the kernel arithmetic bit for bit (358 580 pixels x 2 directions), and c_p_map / validity / points equal the oracle."""
-    base = REF + "Captured_patterns/"
+    whole frame (tests/golden/c1_full.npz): the stored wrapped-phase image gives the mask, the stored unwrapped-phase
+    images must come out of the kernel arithmetic bit for bit (358 580 pixels x 2 directions), and c_p_map /
+    validity / points equal the oracle."""
+    d = load_c1_full()
     planes = []
     gold = {}
     for name, M in (("Vertical", 6), ("Horizontal", 5)):
-        planes += [read_bmp8(f"{base}Fringe_patterns/{name}/Undistorted/Gray_captured_image_{i}.bmp") for i in range(3)]
-        planes += [read_bmp8(f"{base}Coded_patterns/Gray_coded/{name}/Undistorted/Gray_captured_image_{i}.bmp") for i in range(M)]
-        planes += [read_bmp8(f"{base}Coded_patterns/Gray_coded/{name}/Undistorted/inverse_Gray_captured_image_{i}.bmp") for i in range(M)]
-        gold[name] = (read_bmp8(REF + f"Wrapped_phase_images/{name}/Wrapped_phase_image.bmp"),
-                      read_bmp8(REF + f"Unwrapped_phase_images/Gray_coded/{name}/Unwrapped_phase_{name.lower()}.bmp"))
-    stack = np.stack(planes)
+        key = name[0].lower()
+        assert len(d[f"gray_{key}"]) == len(d[f"inv_{key}"]) == M
+        planes += [d[f"fringe_{key}"], d[f"gray_{key}"], d[f"inv_{key}"]]
+        gold[name] = (d[f"golden_wrapped_{key}"], d[f"golden_unwrapped_{key}"])
+    stack = np.concatenate(planes)
     roi = (gold["Vertical"][0] != 0).astype(np.uint8)
     assert int(roi.sum()) == 358580
     c = load_calib_c1()

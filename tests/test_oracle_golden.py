@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import oracle_ffi as o
-from helpers import GOLDEN, REF, have_reference, load_c1_crop, load_calib_c1, read_bmp8, scaled_calib
+from helpers import GOLDEN, load_c1_crop, load_c1_full, load_calib_c1, scaled_calib
 
 
 def _stage34(fr, g, gi, gw, direction):
@@ -38,15 +38,14 @@ def test_c1_crop_matches_reference_images(key, direction, codes):
     assert (code[~m] == -1).all() and (code[m] >= 0).all()
 
 
-@pytest.mark.skipif(not have_reference(), reason="reference tree not mounted")
 @pytest.mark.parametrize("name,M,direction,codes", [("Vertical", 6, 0, 40), ("Horizontal", 5, 1, 23)])
 def test_full_frame_matches_reference_images(name, M, direction, codes):
-    base = REF + "Captured_patterns/"
-    fr = np.stack([read_bmp8(f"{base}Fringe_patterns/{name}/Undistorted/Gray_captured_image_{i}.bmp") for i in range(3)])
-    g = np.stack([read_bmp8(f"{base}Coded_patterns/Gray_coded/{name}/Undistorted/Gray_captured_image_{i}.bmp") for i in range(M)])
-    gi = np.stack([read_bmp8(f"{base}Coded_patterns/Gray_coded/{name}/Undistorted/inverse_Gray_captured_image_{i}.bmp") for i in range(M)])
-    gw = read_bmp8(REF + f"Wrapped_phase_images/{name}/Wrapped_phase_image.bmp")
-    gu = read_bmp8(REF + f"Unwrapped_phase_images/Gray_coded/{name}/Unwrapped_phase_{name.lower()}.bmp")
+    """The reference's whole 1600x1200 scan and its stored stage-3/4 images (tests/golden/c1_full.npz)."""
+    d = load_c1_full()
+    key = name[0].lower()
+    fr, g, gi = d[f"fringe_{key}"], d[f"gray_{key}"], d[f"inv_{key}"]
+    assert len(g) == len(gi) == M
+    gw, gu = d[f"golden_wrapped_{key}"], d[f"golden_unwrapped_{key}"]
     valid, w, dbg, code, w2, unw = _stage34(fr, g, gi, gw, direction)
     assert int(valid.sum()) == 358580
     m = valid == 1
