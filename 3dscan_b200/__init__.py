@@ -165,6 +165,13 @@ def cuda_lib():
         getattr(L, fn).argtypes = [vp]
         getattr(L, fn).restype = vp
     L.scan3d_write_mesh_ply.argtypes = [vp, C.c_char_p, i32]
+    L.scan3d_voxel_begin.argtypes = [vp, C.c_float, i64]
+    L.scan3d_voxel_add_points.argtypes = [vp]
+    L.scan3d_voxel_add_points_dev.argtypes = [vp, vp, vp, vp, i64]
+    L.scan3d_voxel_finish.argtypes = [vp]
+    L.scan3d_voxel_count.argtypes = [vp, C.POINTER(i64), C.POINTER(i64)]
+    L.scan3d_get_voxels.argtypes = [vp, vp, vp, vp, vp, i64]
+    L.scan3d_write_voxel_ply.argtypes = [vp, C.c_char_p, i32]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -531,6 +538,44 @@ class Scan3D:
 
     def write_mesh_ply(self, path, binary=False):
         self._ck(self.L.scan3d_write_mesh_ply(self.h, path.encode(), 1 if binary else 0))
+
+    # -- voxel-grid merge of registered views (include/scan3d.h has the exact rules)
+    def voxel_begin(self, voxel_size, max_voxels):
+        """Reset the ctx's merge accumulator: voxels of edge voxel_size, up to max_voxels of them."""
+        self._ck(self.L.scan3d_voxel_begin(self.h, voxel_size, int(max_voxels)))
+
+    def voxel_add(self):
+        """Add the ctx's current points (with the fresh mesh's normals and the texture's colours); asynchronous."""
+        self._ck(self.L.scan3d_voxel_add_points(self.h))
+
+    def voxel_add_dev(self, xyz, normals=None, rgb=None, n=None):
+        """Add n points from device memory on the ctx's GPU: torch tensors or raw pointers (then n is required);
+        normals / rgb None mean zeros.  Asynchronous on the ctx stream."""
+        def dptr(a):
+            return None if a is None else C.c_void_p(a if isinstance(a, int) else a.data_ptr())
+        if n is None:
+            n = xyz.shape[0]
+        self._ck(self.L.scan3d_voxel_add_points_dev(self.h, dptr(xyz), dptr(normals), dptr(rgb), int(n)))
+
+    def voxel_finish(self):
+        self._ck(self.L.scan3d_voxel_finish(self.h))
+
+    def voxel_count(self):
+        """(voxels, dropped points) of the last voxel_finish (synchronises)."""
+        v, d = C.c_int64(), C.c_int64()
+        self._ck(self.L.scan3d_voxel_count(self.h, C.byref(v), C.byref(d)))
+        return v.value, d.value
+
+    def voxels(self):
+        """(xyz float32 [v][3], normals float32 [v][3], rgb uint8 [v][3], counts uint32 [v]) in first-point order."""
+        v, _ = self.voxel_count()
+        out = (np.empty((v, 3), np.float32), np.empty((v, 3), np.float32), np.empty((v, 3), np.uint8),
+               np.empty(v, np.uint32))
+        self._ck(self.L.scan3d_get_voxels(self.h, *[_ptr(a) for a in out], v))
+        return out
+
+    def write_voxel_ply(self, path, binary=False):
+        self._ck(self.L.scan3d_write_voxel_ply(self.h, path.encode(), 1 if binary else 0))
 
     def set_points_buffer(self, dev_ptr, capacity_points):
         """Compacted points go to this device pointer (may be another GPU's memory mapped here); 0/None restores."""

@@ -30,7 +30,8 @@ if os.environ.get("SCAN3D_BUILD_TRACE") == "1":
 # their own SCAN3D_LIBDIR; the default build defines none of them)
 NVCC_FLAGS += [d for d in os.environ.get("SCAN3D_BUILD_DEFS", "").split() if d.startswith("-D")]
 CU_SOURCES = ["scan3d_api.cu", "scan3d_stage_kernels.cu", "scan3d_worklist.cu", "scan3d_fused_kernel7.cu",
-              "scan3d_aux_kernels.cu", "scan3d_aux_api.cu", "scan3d_shard.cu", "scan3d_mesh_kernels.cu"]
+              "scan3d_aux_kernels.cu", "scan3d_aux_api.cu", "scan3d_shard.cu", "scan3d_mesh_kernels.cu",
+              "scan3d_voxel_kernels.cu"]
 # SCAN3D_BUILD_V8=1 also compiles the warp-autonomous cut of the single-pass kernel (scan3d_fused_kernel8.cu: parity
 # green, one launch per scan, but slower than k_fused7 on the 12 MP workload -- profiles/r2_optimisation_log.md);
 # it is then selected with SCAN3D_FUSED_IMPL=8

@@ -209,7 +209,9 @@ void scan3d_destroy(scan3d_ctx* ctx)
                     ctx->mask[1], ctx->valid, ctx->cpmap, ctx->xyz, ctx->pts, ctx->pix, ctx->rgb,
                     ctx->texture, ctx->d_count, ctx->block_counts, ctx->tile_state, ctx->sched_ctr, ctx->stage_pts, ctx->stage_vb, ctx->tile_flags, ctx->tile_list, ctx->trace, ctx->d_stack, ctx->d_roi, ctx->d_undist, ctx->roi_eff, ctx->roi_eff_h, ctx->roi_strict, ctx->pattern_profiles,
                     ctx->undist_xy[0], ctx->undist_xy[1], ctx->undist_frac[0], ctx->undist_frac[1],
-                    ctx->mesh_idx, ctx->mesh_counts, ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals};
+                    ctx->mesh_idx, ctx->mesh_counts, ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals,
+                    ctx->vox.keys, ctx->vox.acc, ctx->vox.ordinal, ctx->vox.ord2slot, ctx->vox.state,
+                    ctx->vox_point_slot, ctx->vox_flags, ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb, ctx->vox_cnt};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
@@ -900,6 +902,31 @@ int scan3d_write_ply(scan3d_ctx* ctx, const char* path, int binary)
     return ok ? SCAN3D_OK : fail(ctx, SCAN3D_ERR_IO, "PLY write failed");
 }
 
+// The vertex element "x y z nx ny nz red green blue" of scan3d_write_mesh_ply and scan3d_write_voxel_ply: the header
+// (extra_header, e.g. a face element, goes before end_header) and the n vertex records, ascii (%.9g) or binary.
+static void write_ply_with_normals(FILE* f, int binary, int64_t n, const float* xyz, const float* nrm, const uint8_t* rgb,
+                                   const char* extra_header)
+{
+    fprintf(f, "ply\nformat %s 1.0\ncomment scan3d-b200\nelement vertex %lld\n"
+               "property float x\nproperty float y\nproperty float z\n"
+               "property float nx\nproperty float ny\nproperty float nz\n"
+               "property uchar red\nproperty uchar green\nproperty uchar blue\n%send_header\n",
+            binary ? "binary_little_endian" : "ascii", (long long)n, extra_header);
+    if (binary) {
+        std::vector<uint8_t> rec((size_t)n * 27);
+        for (int64_t i = 0; i < n; i++) {
+            memcpy(&rec[(size_t)i * 27], &xyz[(size_t)i * 3], 12);
+            memcpy(&rec[(size_t)i * 27 + 12], &nrm[(size_t)i * 3], 12);
+            memcpy(&rec[(size_t)i * 27 + 24], &rgb[(size_t)i * 3], 3);
+        }
+        fwrite(rec.data(), 1, rec.size(), f);
+    } else {
+        for (int64_t i = 0; i < n; i++)
+            fprintf(f, "%.9g %.9g %.9g %.9g %.9g %.9g %u %u %u\n", xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2], nrm[3 * i],
+                    nrm[3 * i + 1], nrm[3 * i + 2], rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2]);
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // camera-grid mesh of the compacted points (common/scan3d_mesh_math.h has the exact rules)
 // ------------------------------------------------------------------------------------------
@@ -979,20 +1006,10 @@ int scan3d_write_mesh_ply(scan3d_ctx* ctx, const char* path, int binary)
     if (rc) return rc;
     FILE* f = fopen(path, "wb");
     if (!f) return fail(ctx, SCAN3D_ERR_IO, "cannot open PLY for writing");
-    fprintf(f, "ply\nformat %s 1.0\ncomment scan3d-b200\nelement vertex %lld\n"
-               "property float x\nproperty float y\nproperty float z\n"
-               "property float nx\nproperty float ny\nproperty float nz\n"
-               "property uchar red\nproperty uchar green\nproperty uchar blue\n"
-               "element face %lld\nproperty list uchar int vertex_indices\nend_header\n",
-            binary ? "binary_little_endian" : "ascii", (long long)np, (long long)nf);
+    char face_header[96];
+    snprintf(face_header, sizeof(face_header), "element face %lld\nproperty list uchar int vertex_indices\n", (long long)nf);
+    write_ply_with_normals(f, binary, np, xyz.data(), nrm.data(), rgb.data(), face_header);
     if (binary) {
-        std::vector<uint8_t> rec((size_t)np * 27);
-        for (int64_t i = 0; i < np; i++) {
-            memcpy(&rec[(size_t)i * 27], &xyz[(size_t)i * 3], 12);
-            memcpy(&rec[(size_t)i * 27 + 12], &nrm[(size_t)i * 3], 12);
-            memcpy(&rec[(size_t)i * 27 + 24], &rgb[(size_t)i * 3], 3);
-        }
-        fwrite(rec.data(), 1, rec.size(), f);
         std::vector<uint8_t> frec((size_t)nf * 13);
         for (int64_t i = 0; i < nf; i++) {
             frec[(size_t)i * 13] = 3;
@@ -1000,11 +1017,179 @@ int scan3d_write_mesh_ply(scan3d_ctx* ctx, const char* path, int binary)
         }
         fwrite(frec.data(), 1, frec.size(), f);
     } else {
-        for (int64_t i = 0; i < np; i++)
-            fprintf(f, "%.9g %.9g %.9g %.9g %.9g %.9g %u %u %u\n", xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2], nrm[3 * i],
-                    nrm[3 * i + 1], nrm[3 * i + 2], rgb[3 * i], rgb[3 * i + 1], rgb[3 * i + 2]);
         for (int64_t i = 0; i < nf; i++) fprintf(f, "3 %d %d %d\n", faces[3 * i], faces[3 * i + 1], faces[3 * i + 2]);
     }
+    const bool ok = fclose(f) == 0;
+    return ok ? SCAN3D_OK : fail(ctx, SCAN3D_ERR_IO, "PLY write failed");
+}
+
+// ------------------------------------------------------------------------------------------
+// voxel-grid merge of registered views (include/scan3d.h and common/scan3d_voxel_math.h have the exact rules)
+// ------------------------------------------------------------------------------------------
+static void free_ptr(void* p)
+{
+    if (p) cudaFree(p);
+}
+
+int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!(voxel_size > 0.0f && voxel_size - voxel_size == 0.0f))
+        return fail(ctx, SCAN3D_ERR_ARG, "voxel_size must be finite and > 0");
+    if (max_voxels < 1 || max_voxels >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_ARG, "max_voxels must be in [1, 2^31)");
+    CK(cudaSetDevice(ctx->device));
+    ctx->vox_begun = ctx->vox_fresh = false;
+    VoxelTable& t = ctx->vox;
+    const uint32_t cap = voxel_table_capacity((uint32_t)max_voxels, ctx->sm_count);
+    if (cap > ctx->vox_alloc_cap) {
+        free_ptr(t.keys); free_ptr(t.acc); free_ptr(t.ordinal);
+        t.keys = nullptr; t.acc = nullptr; t.ordinal = nullptr;
+        ctx->vox_alloc_cap = 0;
+        CK(dalloc(&t.keys, cap));
+        CK(dalloc(&t.acc, cap));
+        CK(dalloc(&t.ordinal, cap));
+        ctx->vox_alloc_cap = cap;
+    }
+    if ((uint32_t)max_voxels > ctx->vox_alloc_max) {
+        free_ptr(t.ord2slot); free_ptr(ctx->vox_xyz); free_ptr(ctx->vox_nrm); free_ptr(ctx->vox_rgb); free_ptr(ctx->vox_cnt);
+        t.ord2slot = nullptr; ctx->vox_xyz = ctx->vox_nrm = nullptr; ctx->vox_rgb = nullptr; ctx->vox_cnt = nullptr;
+        ctx->vox_alloc_max = 0;
+        const size_t m = (size_t)max_voxels;
+        CK(dalloc(&t.ord2slot, m));
+        CK(dalloc(&ctx->vox_xyz, 3 * m));
+        CK(dalloc(&ctx->vox_nrm, 3 * m));
+        CK(dalloc(&ctx->vox_rgb, 3 * m));
+        CK(dalloc(&ctx->vox_cnt, m));
+        ctx->vox_alloc_max = (uint32_t)max_voxels;
+    }
+    const size_t n = npix(ctx);
+    if (!t.state) CK(dalloc(&t.state, 1));
+    if (!ctx->vox_point_slot) CK(dalloc(&ctx->vox_point_slot, n));
+    if (!ctx->vox_flags) CK(dalloc(&ctx->vox_flags, n));
+    if (!ctx->block_counts) CK(dalloc(&ctx->block_counts, (n + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+    CK(cudaMemsetAsync(t.keys, 0xff, (size_t)cap * sizeof(*t.keys), ctx->stream));
+    CK(cudaMemsetAsync(t.acc, 0, (size_t)cap * sizeof(*t.acc), ctx->stream));
+    CK(cudaMemsetAsync(t.ordinal, 0xff, (size_t)cap * sizeof(*t.ordinal), ctx->stream));
+    CK(cudaMemsetAsync(t.state, 0, sizeof(*t.state), ctx->stream));
+    t.cap = cap;
+    t.max_voxels = (uint32_t)max_voxels;
+    t.S = (double)voxel_size;
+    ctx->vox_bound = 0;
+    ctx->vox_chunks = 0;
+    ctx->vox_begun = true;
+    return SCAN3D_OK;
+}
+
+// one add of <= W*H points (n_dev: the count is on the device)
+static int voxel_add(scan3d_ctx* ctx, const float* xyz, const float* nrm, const uint8_t* rgb, const uint32_t* n_dev,
+                     uint32_t plane)
+{
+    CK(launch_voxel_add(ctx->vox, xyz, nrm, rgb, n_dev, plane, ctx->vox_point_slot, ctx->vox_flags, ctx->block_counts,
+                        (int)(ctx->vox_chunks & 1), ctx->stream));
+    ctx->vox_chunks++;
+    ctx->launches += VOXEL_ADD_LAUNCHES;
+    return SCAN3D_OK;
+}
+
+static const uint64_t VOXEL_MAX_POINTS = 0xffffffffull;   // point indices since begin are uint32
+
+int scan3d_voxel_add_points(scan3d_ctx* ctx)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!ctx->vox_begun) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before scan3d_voxel_begin");
+    if (ctx->cfg.dirs != 2) return fail(ctx, SCAN3D_ERR_STATE, "no point cloud in a one-direction configuration");
+    if (!ctx->have_points) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before the points are computed");
+    const uint64_t ub = npix(ctx);
+    if (ctx->vox_bound + ub > VOXEL_MAX_POINTS)
+        return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^32 - 1 points since scan3d_voxel_begin (W*H counted per ctx add)");
+    CK(cudaSetDevice(ctx->device));
+    ctx->vox_bound += ub;
+    ctx->vox_fresh = false;
+    return voxel_add(ctx, points_of(ctx), ctx->have_mesh ? ctx->mesh_normals : nullptr,
+                     ctx->texture && ctx->rgb ? ctx->rgb : nullptr, ctx->d_count, (uint32_t)ub);
+}
+
+int scan3d_voxel_add_points_dev(scan3d_ctx* ctx, const float* xyz_dev, const float* normals_dev, const uint8_t* rgb_dev,
+                                int64_t n)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (n < 0) return fail(ctx, SCAN3D_ERR_ARG, "n < 0");
+    if (!xyz_dev && n > 0) return fail(ctx, SCAN3D_ERR_ARG, "null xyz_dev");
+    if (((uintptr_t)xyz_dev & 3) || ((uintptr_t)normals_dev & 3))
+        return fail(ctx, SCAN3D_ERR_ARG, "xyz_dev and normals_dev must be 4-byte aligned");
+    if (!ctx->vox_begun) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before scan3d_voxel_begin");
+    if (ctx->vox_bound + (uint64_t)n > VOXEL_MAX_POINTS)
+        return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^32 - 1 points since scan3d_voxel_begin");
+    CK(cudaSetDevice(ctx->device));
+    ctx->vox_bound += (uint64_t)n;
+    ctx->vox_fresh = false;
+    const int64_t chunk = (int64_t)npix(ctx);   // the per-point scratch holds W*H points
+    for (int64_t off = 0; off < n; off += chunk) {
+        const int64_t k = std::min(chunk, n - off);
+        const int rc = voxel_add(ctx, xyz_dev + 3 * off, normals_dev ? normals_dev + 3 * off : nullptr,
+                                 rgb_dev ? rgb_dev + 3 * off : nullptr, nullptr, (uint32_t)k);
+        if (rc) return rc;
+    }
+    return SCAN3D_OK;
+}
+
+int scan3d_voxel_finish(scan3d_ctx* ctx)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!ctx->vox_begun) return fail(ctx, SCAN3D_ERR_STATE, "voxel finish before scan3d_voxel_begin");
+    CK(cudaSetDevice(ctx->device));
+    CK(launch_voxel_finish(ctx->vox, (int)(ctx->vox_chunks & 1), ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb, ctx->vox_cnt,
+                           ctx->sm_count, ctx->stream));
+    ctx->launches += 1;
+    ctx->vox_fresh = true;
+    return SCAN3D_OK;
+}
+
+int scan3d_voxel_count(scan3d_ctx* ctx, int64_t* voxels_out, int64_t* dropped_out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!ctx->vox_begun || !ctx->vox_fresh)
+        return fail(ctx, SCAN3D_ERR_STATE, "no voxel outputs of the current adds: call scan3d_voxel_finish");
+    CK(cudaSetDevice(ctx->device));
+    VoxelState st;
+    CK(cudaMemcpyAsync(&st, ctx->vox.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st.overflow || st.occupied > ctx->vox.max_voxels)
+        return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct voxels than max_voxels: begin again with a larger max_voxels");
+    if (voxels_out) *voxels_out = st.total[ctx->vox_chunks & 1];
+    if (dropped_out) *dropped_out = (int64_t)st.dropped;
+    return SCAN3D_OK;
+}
+
+int scan3d_get_voxels(scan3d_ctx* ctx, float* xyz_host, float* normals_host, uint8_t* rgb_host, uint32_t* counts_host,
+                      int64_t max_voxels)
+{
+    int64_t n = 0;
+    int rc = scan3d_voxel_count(ctx, &n, nullptr);
+    if (rc) return rc;
+    if (n > max_voxels) n = max_voxels;
+    if (n <= 0) return SCAN3D_OK;
+    if (xyz_host) CK(cudaMemcpyAsync(xyz_host, ctx->vox_xyz, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    if (normals_host) CK(cudaMemcpyAsync(normals_host, ctx->vox_nrm, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    if (rgb_host) CK(cudaMemcpyAsync(rgb_host, ctx->vox_rgb, (size_t)n * 3, cudaMemcpyDeviceToHost, ctx->stream));
+    if (counts_host) CK(cudaMemcpyAsync(counts_host, ctx->vox_cnt, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return SCAN3D_OK;
+}
+
+int scan3d_write_voxel_ply(scan3d_ctx* ctx, const char* path, int binary)
+{
+    if (!ctx || !path) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    int64_t n = 0;
+    int rc = scan3d_voxel_count(ctx, &n, nullptr);
+    if (rc) return rc;
+    std::vector<float> xyz((size_t)n * 3), nrm((size_t)n * 3);
+    std::vector<uint8_t> rgb((size_t)n * 3);
+    rc = scan3d_get_voxels(ctx, xyz.data(), nrm.data(), rgb.data(), nullptr, n);
+    if (rc) return rc;
+    FILE* f = fopen(path, "wb");
+    if (!f) return fail(ctx, SCAN3D_ERR_IO, "cannot open PLY for writing");
+    write_ply_with_normals(f, binary, n, xyz.data(), nrm.data(), rgb.data(), "");
     const bool ok = fclose(f) == 0;
     return ok ? SCAN3D_OK : fail(ctx, SCAN3D_ERR_IO, "PLY write failed");
 }

@@ -21,6 +21,33 @@ struct TensorMapCache {
     int next = 0;
 };
 typedef TensorMapCache Fused8Cache;
+
+// the voxel-grid merge's hash table (scan3d_voxel_kernels.cu)
+constexpr uint32_t VOXEL_NO_SLOT = 0xffffffffu;   // no slot / no ordinal yet
+// the integer sums of one voxel (zero-initialised); first_inv = ~(index of the first point within the current add)
+struct VoxelSlot {
+    unsigned long long q[3];   // positions inside the voxel, Q steps
+    unsigned long long m[3];   // normals, Q steps, two's complement
+    unsigned long long c[3];   // colours
+    uint32_t n, first_inv;
+};
+struct VoxelState {
+    unsigned long long dropped;
+    uint32_t occupied;         // slots taken = distinct voxels inserted
+    uint32_t overflow;         // an ordinal >= max_voxels was assigned
+    uint32_t total[2];         // voxels with an ordinal, after an even / odd number of adds (chunks)
+    uint32_t chunk_new;        // new voxels of the current add (chunk)
+    uint32_t pad;
+};
+struct VoxelTable {
+    unsigned long long* keys;  // [cap], s3v::EMPTY_KEY = free
+    VoxelSlot* acc;            // [cap]
+    uint32_t* ordinal;         // [cap], VOXEL_NO_SLOT until assigned
+    uint32_t* ord2slot;        // [max_voxels]
+    VoxelState* state;
+    uint32_t cap, max_voxels;
+    double S;                  // (double)voxel_size
+};
 }  // namespace s3d
 
 struct scan3d_ctx {
@@ -88,6 +115,20 @@ struct scan3d_ctx {
     uint32_t* mesh_totals = nullptr;      // [2] points, faces
     int32_t* mesh_faces = nullptr;        // [2(W-1)(H-1)][3]
     float* mesh_normals = nullptr;        // [H*W][3]
+
+    // scan3d_voxel_begin: the merge accumulator (independent of the points; reallocated when a begin asks for more)
+    s3d::VoxelTable vox{};
+    bool vox_begun = false;        // a begin has run
+    bool vox_fresh = false;        // the outputs are those of the adds since begin (a finish ran after the last add)
+    uint64_t vox_bound = 0;        // upper bound of the points added since begin (W*H per ctx add, n per dev add)
+    uint32_t vox_chunks = 0;       // adds (chunks of <= W*H points) since begin
+    uint32_t vox_alloc_cap = 0, vox_alloc_max = 0;   // what the buffers hold
+    uint32_t* vox_point_slot = nullptr;   // [H*W] per-point scratch of an add
+    uint8_t* vox_flags = nullptr;         // [H*W]
+    float* vox_xyz = nullptr;             // [max_voxels][3] outputs of scan3d_voxel_finish
+    float* vox_nrm = nullptr;             // [max_voxels][3]
+    uint8_t* vox_rgb = nullptr;           // [max_voxels][3]
+    uint32_t* vox_cnt = nullptr;          // [max_voxels]
 
     int cta_limit = 0;             // scan3d_set_cta_limit
 
@@ -221,6 +262,20 @@ constexpr int MESH_LAUNCHES = 6;
 cudaError_t launch_mesh(const uint8_t* valid, const float* pts, int W, int H, float max_edge, int32_t* idx,
                         uint32_t* block_counts, uint32_t* face_counts, uint32_t* totals, int32_t* faces, float* normals,
                         cudaStream_t st);
+
+// ---- voxel-grid merge (scan3d_voxel_kernels.cu; common/scan3d_voxel_math.h has the arithmetic) ----
+// VOXEL_ADD_LAUNCHES launches for `plane` points (the ctx add reads the point count from n_dev, <= plane): insert,
+// flag, k_count + k_scan over the flags, assign.  point_slot and flags [plane], block_counts [cdiv(plane,
+// POINT_BLOCK)]; par = number of adds (chunks) since begin, mod 2.  nrm / rgb may be null (zeros).
+constexpr int VOXEL_ADD_LAUNCHES = 5;
+cudaError_t launch_voxel_add(const VoxelTable& t, const float* xyz, const float* nrm, const uint8_t* rgb,
+                             const uint32_t* n_dev, uint32_t plane, uint32_t* point_slot, uint8_t* flags,
+                             uint32_t* block_counts, int par, cudaStream_t st);
+// slots of the table for max_voxels: at most half of them are ever taken (scan3d_voxel_kernels.cu)
+uint32_t voxel_table_capacity(uint32_t max_voxels, int sm_count);
+// 1 launch: the merged voxels in first-point order into xyz / nrm [max_voxels][3], rgb [max_voxels][3], cnt
+cudaError_t launch_voxel_finish(const VoxelTable& t, int par, float* xyz, float* nrm, uint8_t* rgb, uint32_t* cnt,
+                                int sm_count, cudaStream_t st);
 
 // ---- debug / self-test ----
 cudaError_t launch_debug_atan2(const double* y, const double* x, float* out, int n, int mode,

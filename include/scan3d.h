@@ -254,6 +254,59 @@ void *scan3d_device_point_normals(scan3d_ctx *ctx);
  * "property list uchar int vertex_indices"; ascii (%.9g, faces "3 i j k") or binary_little_endian */
 int scan3d_write_mesh_ply(scan3d_ctx *ctx, const char *path, int binary);
 
+/* ---- voxel-grid merge of registered views (the reference concatenated them: 9/register_point_clouds.cpp) ---------
+ * One output point per occupied voxel of edge s = voxel_size, averaged over every point that fell into it, from every
+ * add since scan3d_voxel_begin.  Per point and axis t = (double)x / (double)s, i = floor(t), q = the position inside
+ * the voxel in 2^24 steps; a point is dropped (counted, contributes nothing) when a coordinate is not finite or some
+ * i is outside [-2^20, 2^20).  A normal with a non-finite component counts as (0,0,0); otherwise each component is
+ * clamped to [-1, 1] and rounded to 2^24 steps.  The sums per voxel are integers, so the outputs do not depend on the
+ * hash function, the table layout, thread scheduling or how a cloud is split into adds:
+ *   coordinate (float)(((double)i + (double)sum_q / (2^24 (double)n)) * (double)s)
+ *   normal     the sum of the fixed-point normals divided by its length (double), (0,0,0) if the sum is 0, so views
+ *              without normals do not bias the direction
+ *   colour     (sum + n/2) / n per channel (integer division), count n (uint32)
+ * The exact arithmetic is in 3dscan_b200/common/scan3d_voxel_math.h.
+ *
+ * Output order: voxels come in order of their first point.  Points are numbered across all adds since begin, first by
+ * add, then by position within the add; dropped points take no place.  Adding A then B gives the same per-voxel
+ * values as B then A, only the order differs.
+ *
+ * scan3d_voxel_begin: resets the ctx's accumulator and sizes it for up to max_voxels distinct voxels (device memory of
+ * about 190 B per voxel plus 31 B per voxel of outputs, reused by later begins that ask for no more).  The
+ * accumulator is independent of the ctx's points: a later reconstruct does not touch it.  No kernel launch.
+ * scan3d_voxel_add_points: the ctx's current points, wherever they are (scan3d_set_points_buffer included, row-sharded
+ * contexts included); each brings its normal from the mesh when the mesh of the current points is fresh
+ * (scan3d_build_mesh), else (0,0,0), and its colour when a texture is set, else (0,0,0), as scan3d_write_ply does.
+ * Always 5 kernel launches.
+ * scan3d_voxel_add_points_dev: n points from caller device memory on the ctx's GPU (xyz f32[n][3], normals f32[n][3]
+ * or NULL, rgb u8[n][3] or NULL; NULL means zeros), ordered on the ctx stream.  Runs in chunks of W*H points, 5 kernel
+ * launches per chunk (none for n = 0); the order rule holds across chunks.
+ * Both adds are asynchronous and never synchronise.
+ * scan3d_voxel_finish: computes the outputs, asynchronously, 1 kernel launch.  A begin or an add after it makes the
+ * outputs stale: the getters below return SCAN3D_ERR_STATE before the first finish and while the outputs are stale.
+ *
+ * Errors: SCAN3D_ERR_ARG for voxel_size not finite or <= 0, max_voxels < 1 or >= 2^31, a null xyz_dev with n > 0,
+ * n < 0, xyz_dev / normals_dev not 4-byte aligned, a null path.  SCAN3D_ERR_STATE for an add before begin, a ctx add
+ * without points or with dirs == 1.  SCAN3D_ERR_CONFIG, before any launch, for an add whose upper bound (W*H for the
+ * ctx add, n for the dev add) would push the points since begin past 2^32 - 1.
+ * More distinct voxels than max_voxels is detected on the device; the adds stop inserting new voxels, so they neither
+ * hang nor write outside their buffers.  The condition is sticky: scan3d_voxel_count, scan3d_get_voxels and
+ * scan3d_write_voxel_ply return SCAN3D_ERR_CONFIG with a message until the next begin. */
+int scan3d_voxel_begin(scan3d_ctx *ctx, float voxel_size, int64_t max_voxels);
+int scan3d_voxel_add_points(scan3d_ctx *ctx);                       /* the ctx's current points */
+int scan3d_voxel_add_points_dev(scan3d_ctx *ctx, const float *xyz_dev, const float *normals_dev,
+                                const uint8_t *rgb_dev, int64_t n);
+int scan3d_voxel_finish(scan3d_ctx *ctx);                           /* async */
+/* syncs; either pointer may be NULL */
+int scan3d_voxel_count(scan3d_ctx *ctx, int64_t *voxels_out, int64_t *dropped_out);
+/* xyz f32[n][3], normals f32[n][3], rgb u8[n][3], counts u32[n] of the first n = min(voxels, max_voxels) voxels;
+ * any pointer may be NULL */
+int scan3d_get_voxels(scan3d_ctx *ctx, float *xyz_host, float *normals_host, uint8_t *rgb_host,
+                      uint32_t *counts_host, int64_t max_voxels);
+/* the vertex element of scan3d_write_mesh_ply ("x y z nx ny nz red green blue"), no face element; ascii (%.9g) or
+ * binary_little_endian */
+int scan3d_write_voxel_ply(scan3d_ctx *ctx, const char *path, int binary);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,
