@@ -26,18 +26,9 @@ NVCC_FLAGS = [
 # they cost ~2 % of the kernel's instructions, so the default build leaves them out.
 if os.environ.get("SCAN3D_BUILD_TRACE") == "1":
     NVCC_FLAGS.append("-DS3D_TRACE=1")
-# SCAN3D_BUILD_DEFS="-DS3D_VAR_X=1 ...": experimental kernel variants (tools/build_variants.py builds them into
-# their own SCAN3D_LIBDIR; the default build defines none of them)
-NVCC_FLAGS += [d for d in os.environ.get("SCAN3D_BUILD_DEFS", "").split() if d.startswith("-D")]
 CU_SOURCES = ["scan3d_api.cu", "scan3d_stage_kernels.cu", "scan3d_worklist.cu", "scan3d_fused_kernel7.cu",
               "scan3d_aux_kernels.cu", "scan3d_aux_api.cu", "scan3d_shard.cu", "scan3d_mesh_kernels.cu",
               "scan3d_voxel_kernels.cu"]
-# SCAN3D_BUILD_V8=1 also compiles the warp-autonomous cut of the single-pass kernel (scan3d_fused_kernel8.cu: parity
-# green, one launch per scan, but slower than k_fused7 on the 12 MP workload -- profiles/r2_optimisation_log.md);
-# it is then selected with SCAN3D_FUSED_IMPL=8
-if os.environ.get("SCAN3D_BUILD_V8") == "1":
-    CU_SOURCES.append("scan3d_fused_kernel8.cu")
-    NVCC_FLAGS.append("-DS3D_BUILD_V8=1")
 HOST_SOURCES = ["scan3d_io.cpp", "scan3d_synth.cpp"]
 COMPAT_SOURCES = ["scan3d_stages.cpp"]
 

@@ -156,8 +156,6 @@ int scan3d_create(const scan3d_config* cfg, int device, scan3d_ctx** out)
             CK(dalloc(&ctx->trace, (size_t)1024 * 64 * 8));
             CK(cudaMemsetAsync(ctx->trace, 0, (size_t)1024 * 64 * 8 * 8, ctx->stream));
         }
-        CK(dalloc(&ctx->sched_ctr, 4));
-        CK(cudaMemsetAsync(ctx->sched_ctr, 0, 16, ctx->stream));
         CK(dalloc(&ctx->tile_flags, (size_t)ntiles + 16));
         CK(dalloc(&ctx->tile_list, (size_t)ntiles + 16));
         CK(dalloc(&ctx->atan_tab, (size_t)ATAN_TAB_DOUBLES));
@@ -207,7 +205,7 @@ void scan3d_destroy(scan3d_ctx* ctx)
     void* ptrs[] = {ctx->cam_lut, ctx->proj_lut, ctx->atan_tab, ctx->nstep_w, ctx->wrapped[0], ctx->wrapped[1],
                     ctx->unwrapped[0], ctx->unwrapped[1], ctx->code[0], ctx->code[1], ctx->mask[0],
                     ctx->mask[1], ctx->valid, ctx->cpmap, ctx->xyz, ctx->pts, ctx->pix, ctx->rgb,
-                    ctx->texture, ctx->d_count, ctx->block_counts, ctx->tile_state, ctx->sched_ctr, ctx->stage_pts, ctx->stage_vb, ctx->tile_flags, ctx->tile_list, ctx->trace, ctx->d_stack, ctx->d_roi, ctx->d_undist, ctx->roi_eff, ctx->roi_eff_h, ctx->roi_strict, ctx->pattern_profiles,
+                    ctx->texture, ctx->d_count, ctx->block_counts, ctx->tile_state, ctx->tile_flags, ctx->tile_list, ctx->trace, ctx->d_stack, ctx->d_roi, ctx->d_undist, ctx->roi_eff, ctx->roi_eff_h, ctx->roi_strict, ctx->pattern_profiles,
                     ctx->undist_xy[0], ctx->undist_xy[1], ctx->undist_frac[0], ctx->undist_frac[1],
                     ctx->mesh_idx, ctx->mesh_counts, ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals,
                     ctx->vox.keys, ctx->vox.acc, ctx->vox.ordinal, ctx->vox.ord2slot, ctx->vox.state,
@@ -575,27 +573,8 @@ int scan3d_reconstruct_dev(scan3d_ctx* ctx, const uint8_t* stack_dev, const uint
     a.W = c.W; a.H = c.H; a.row0 = c.row0; a.H_total = c.H_total; a.PW = c.PW; a.PH = c.PH;
     a.N = c.N; a.M_v = c.M_v; a.M_h = c.M_h; a.fw_v = c.fw_v; a.fw_h = c.fw_h;
     a.fw_v_d = (double)c.fw_v; a.fw_h_d = (double)c.fw_h;
-#if S3D_BUILD_V8
-    static const int impl = getenv("SCAN3D_FUSED_IMPL") ? atoi(getenv("SCAN3D_FUSED_IMPL")) : 7;
-    if (impl >= 8 && fused8_supported(c)) {
-        a.sched_ctr = ctx->sched_ctr;
-        a.pos_base = ctx->sched_base;
-        if (c.dirs == 2 && !ctx->stage_pts) {
-            CK(dalloc(&ctx->stage_pts, fused8_stage_floats(ctx->sm_count)));
-            CK(dalloc(&ctx->stage_vb, fused8_stage_vb_words(ctx->sm_count)));
-        }
-        a.stage_pts = ctx->stage_pts;
-        a.stage_vb = ctx->stage_vb;
-        uint32_t advance = 0;
-        CK(launch_fused8(c, a, ctx->dcal, ctx->sm_count, &ctx->tmaps, &advance, ctx->stream));
-        ctx->sched_base += advance;
-        ctx->launches += 1;   // the one persistent kernel
-    } else
-#endif
-    {
-        CK(launch_fused7(c, a, ctx->dcal, ctx->sm_count, ctx->stream));
-        ctx->launches += 3;   // work-list flags, work-list scan, persistent fused kernel
-    }
+    CK(launch_fused7(c, a, ctx->dcal, ctx->sm_count, ctx->stream));
+    ctx->launches += 3;   // work-list flags, work-list scan, persistent fused kernel
     if (ctx->reg_on && !fold_reg && c.dirs == 2) {
         // shapes without the folding variant: the same transform as one more pass over the compacted points
         CK(launch_register_points(points_of(ctx), points_of(ctx), (long long)npix(ctx), ctx->reg_R, ctx->reg_t[0], ctx->reg_t[1],

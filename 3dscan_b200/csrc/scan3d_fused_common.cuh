@@ -37,39 +37,8 @@ __device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity)
         : "memory");
     return done != 0;
 }
-// non-blocking probe: for a warp whose lanes look at DIFFERENT barriers (try_wait would suspend the whole warp
-// on the slowest lane's barrier)
-__device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity)
-{
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return done != 0;
-}
 // (A non-blocking mbarrier.test_wait probe in the IO warp's event loop measured 4-10 % SLOWER than
 // try_wait, whose hardware suspend keeps the polling warp out of the issue slots.)
-// poll with back-off so that a waiting warp does not steal issue slots from the computing ones
-// (one copy per warp role so that profiles attribute the waiting to the right role)
-#define S3D_WAIT_BODY                                        \
-    if (mbar_try(bar, parity)) return;                      \
-    while (!mbar_try(bar, parity)) __nanosleep(128);
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
-{
-    S3D_WAIT_BODY
-}
-__device__ __forceinline__ void mbar_wait_consumer(uint32_t bar, uint32_t parity)
-{
-    S3D_WAIT_BODY
-}
-__device__ __forceinline__ void mbar_wait_epilogue(uint32_t bar, uint32_t parity)
-{
-    S3D_WAIT_BODY
-}
 __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar)
 {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
@@ -84,14 +53,6 @@ __device__ __forceinline__ void tensor_g2s_2d(uint32_t dst, const void* tmap, in
         ::"r"(dst), "l"(tmap), "r"(c0), "r"(c1), "r"(bar)
         : "memory");
 }
-__device__ __forceinline__ void bulk_s2g(void* dst, uint32_t src, uint32_t bytes)
-{
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src), "r"(bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 __device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
@@ -122,7 +83,7 @@ __device__ __forceinline__ void trace(unsigned long long* t, int it, int ev)
 }
 
 
-// work-list kernels (scan3d_fused_kernel.cu)
+// work-list kernels (scan3d_worklist.cu)
 cudaError_t launch_worklist(const FusedArgs& a, int T, int dirs, cudaStream_t st);
 
 }  // namespace s3d

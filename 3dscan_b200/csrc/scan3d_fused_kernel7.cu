@@ -67,24 +67,15 @@ static bool plan7(const scan3d_config& c, Plan7* out)
     if (mod7(c) && c.N != 3) return false;
     // Shapes are bounded by the register file of an SM sub-partition (16 K registers): warps are
     // dealt round-robin to the 4 sub-partitions, so ceil(warps per SM / 4) * 32 * regs <= 16384:
-    // 20 warps at 96 registers, 16 at 128, 24 at 80.
-    int cw = 7, minb = 3;
-    if (const char* e = getenv("SCAN3D_FUSED_CFG")) {
-        int a = 0, b = 0, s = 0;
-        if (sscanf(e, "%d,%d,%d", &a, &b, &s) >= 2) { cw = a; minb = b; }
-    }
-    const int shapes[7][2] = {{cw, minb}, {7, 3}, {9, 2}, {7, 2}, {4, 4}, {6, 2}, {5, 4}};
-    for (int i = 0; i < 7; i++) {
-        const int w = shapes[i][0], b = shapes[i][1];
-        if (!((w == 7 && b == 2) || (w == 7 && b == 3) || (w == 9 && b == 2) || (w == 4 && b == 4) || (w == 6 && b == 2) || (w == 5 && b == 4))) continue;
-        if (mod7(c) && !(w == 7 && (b == 2 || b == 3))) continue;      // (the modulation variant is built for these two shapes)
+    // 24 warps at 80 registers (7, 3), 20 at 96 (9, 2), 16 at 128 (7, 2).  The first shape that fits
+    // the shared memory wins; (7, 2) fits every configuration accepted above (at most 76 frames).
+    auto fits = [&](int w, int b) {
         const size_t sm = smem7(c, w);
-        if ((sm + 1024) * b <= (size_t)SMEM_MAX + 1024) {
-            out->cw = w; out->minb = b; out->smem = sm;
-            return true;
-        }
-    }
-    return false;
+        if ((sm + 1024) * b > (size_t)SMEM_MAX + 1024) return false;
+        out->cw = w; out->minb = b; out->smem = sm;
+        return true;
+    };
+    return fits(7, 3) || (!mod7(c) && fits(9, 2)) || fits(7, 2);
 }
 
 bool fused7_supported(const scan3d_config& c)
@@ -97,7 +88,7 @@ bool fused7_supported(const scan3d_config& c)
 bool fused7_folds_registration(const scan3d_config& c)
 {
     Plan7 p;
-    return plan7(c, &p) && c.dirs == 2 && !mod7(c) && p.cw == 7 && (p.minb == 2 || p.minb == 3);
+    return plan7(c, &p) && c.dirs == 2 && !mod7(c) && p.cw == 7;
 }
 
 constexpr int regs7(int cw, int minb)
@@ -166,13 +157,11 @@ k_fused7(const __grid_constant__ FusedArgs a, const __grid_constant__ DeviceCali
     for (int i = tid; i < ATAN_TAB_DOUBLES; i += (CW + 1) * 32) tab[i] = a.atan_tab[i];
     __syncthreads();
 
-    // Work-list positions are handed out in order.  Static mode: CTA b takes b, b + G, b + 2G, ...
-    // Dynamic mode: the IO warp draws the next position from a global counter whenever its slot
-    // frees.  The CTAs of an SM do not run at the same speed (the warp schedulers favour the
-    // lower warp slots: measured 14k / 15k / 19k cycles per tile for the 1st / 2nd / 3rd CTA of an
-    // SM), so equal shares leave the fast CTAs waiting for the slow one's counts.
+    // Work-list positions are handed out in order: the IO warp draws the next position from a global
+    // counter whenever its slot frees.  The CTAs of an SM do not run at the same speed (the warp
+    // schedulers favour the lower warp slots: measured 14k / 15k / 19k cycles per tile for the 1st /
+    // 2nd / 3rd CTA of an SM), so equal static shares leave the fast CTAs waiting for the slow one's counts.
     const int n_work = *a.n_list;
-    const int Gsz = (int)gridDim.x, bid = (int)blockIdx.x;
     int* const next_pos = a.n_list + a.n_tiles + 8;      // zeroed by k_tile_list
 
     if (warp == CW) {
@@ -196,11 +185,9 @@ k_fused7(const __grid_constant__ FusedArgs a, const __grid_constant__ DeviceCali
             // ---- (1) the slot is free again: issue the next tile's loads (or the end marker) ----
             if (!ended && __any_sync(0xffffffffu, mbar_try(bar_free, (load_it & 1) ^ 1))) {
                 progressed = true;
-                int pos = load_it * Gsz + bid;
-                if (a.dynamic) {
-                    if (lane == 0) pos = atomicAdd(next_pos, 1);
-                    pos = __shfl_sync(0xffffffffu, pos, 0);
-                }
+                int pos = 0;
+                if (lane == 0) pos = atomicAdd(next_pos, 1);
+                pos = __shfl_sync(0xffffffffu, pos, 0);
                 if (pos < n_work) {
                     const int tile = a.tile_list[pos];
                     const int p0 = tile * T, wt = min(T, plane - p0);
@@ -220,19 +207,13 @@ k_fused7(const __grid_constant__ FusedArgs a, const __grid_constant__ DeviceCali
                         trace(a.trace, load_it, 0);
                         ctl[0] = pos;
                         posr[load_it & 7] = pos;
-                        mbar_expect_tx(bar_full, (uint32_t)NF * (a.use_tmap ? T : wt) + NROI * roi_sum);
+                        mbar_expect_tx(bar_full, (uint32_t)NF * T + NROI * roi_sum);
                     }
                     __syncwarp();
-                    const uint32_t dst = smem_u32(slot);
-                    if (a.use_tmap) {
-                        // the whole [NF frames] x [T bytes] tile is ONE 2-D tensor copy (64-bit elements;
-                        // bytes past the end of a frame are zero-filled).  56 per-frame bulk copies took the
-                        // warp ~5k cycles to issue, squarely on the slot-free -> data-ready path.
-                        if (lane == 0) tensor_g2s_2d(dst, &stack_map, p0 >> 3, 0, bar_full);
-                    } else {
-                        const uint8_t* src = a.stack + p0;
-                        for (int f = lane; f < NF; f += 32) bulk_g2s(dst + f * T, src + (size_t)f * plane, (uint32_t)wt, bar_full);
-                    }
+                    // the whole [NF frames] x [T bytes] tile is ONE 2-D tensor copy (64-bit elements;
+                    // bytes past the end of a frame are zero-filled).  56 per-frame bulk copies took the
+                    // warp ~5k cycles to issue, squarely on the slot-free -> data-ready path.
+                    if (lane == 0) tensor_g2s_2d(smem_u32(slot), &stack_map, p0 >> 3, 0, bar_full);
                     if (roi_tx) {
                         bulk_g2s(smem_u32(sroi) + lane * G.roi_row + (uint32_t)(seg0 - (gbase + (long long)(lane - 2) * W)),
                                  a.roi + seg0, roi_tx, bar_full);
@@ -627,29 +608,30 @@ k_fused7(const __grid_constant__ FusedArgs a, const __grid_constant__ DeviceCali
 
 // 2-D view of the capture stack for the tile loads: inner dimension = one frame as 64-bit words,
 // outer = the frames; box = [T/8 words] x [NF frames], landing in shared memory as [NF][T] bytes.
-static bool stack_tensor_map(CUtensorMap* map, const uint8_t* stack, size_t plane, int NF, int T)
+static cudaError_t stack_tensor_map(CUtensorMap* map, const uint8_t* stack, size_t plane, int NF, int T)
 {
     typedef CUresult (*encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static encode_fn encode = nullptr;
-    static bool looked_up = false;
-    if (!looked_up) {
-        looked_up = true;
+    // looked up once per process (a function-local static is initialised once even when several host threads launch)
+    static const encode_fn encode = []() -> encode_fn {
         void* fn = nullptr;
         cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            encode = (encode_fn)fn;
-    }
-    if (!encode || NF > 256 || T / 8 > 256 || (plane & 15) || ((uintptr_t)stack & 15)) return false;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess ||
+            q != cudaDriverEntryPointSuccess)
+            return nullptr;
+        return (encode_fn)fn;
+    }();
+    if (!encode) return cudaErrorNotSupported;
     const cuuint64_t gdim[2] = {(cuuint64_t)(plane / 8), (cuuint64_t)NF};
     const cuuint64_t gstride[1] = {(cuuint64_t)plane};
     const cuuint32_t box[2] = {(cuuint32_t)(T / 8), (cuuint32_t)NF};
     const cuuint32_t estr[2] = {1, 1};
     return encode(map, CU_TENSOR_MAP_DATA_TYPE_UINT64, 2, const_cast<uint8_t*>(stack), gdim, gstride, box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS
+               ? cudaSuccess
+               : cudaErrorInvalidValue;
 }
 
 template <int N, int DIRS, int CW, int MINB, bool EXACT, bool MOD = false, bool REG = false, int MV = 0, int MH = 0, int LUTS = -1>
@@ -683,47 +665,37 @@ static cudaError_t launch7_t(const FusedArgs& a, const DeviceCalib& cal, int sm_
     // fill and drain overlap the other scans' steady state
     const int per_sm = a.ctas_per_sm > 0 && a.ctas_per_sm < per_sm_cached ? a.ctas_per_sm : per_sm_cached;
     const int grid = a.n_tiles < sm_count * per_sm ? a.n_tiles : sm_count * per_sm;   // all CTAs resident
+    // the tensor map depends on the stack's address and the tile size only: the context keeps the last few
+    TensorMapCache& cache = *a.tmap_cache;
+    const CUtensorMap* map = nullptr;
+    for (int i = 0; i < TensorMapCache::SLOTS; i++)
+        if (cache.stack[i] == a.stack && cache.box[i] == 128 * CW) map = &cache.map[i];
+    if (!map) {
+        const int slot = cache.next++ % TensorMapCache::SLOTS;
+        cache.stack[slot] = nullptr;
+        const int NF = DIRS == 2 ? 2 * N + 2 * (a.M_v + a.M_h) : N + 2 * a.M_v;
+        e = stack_tensor_map(&cache.map[slot], a.stack, (size_t)a.W * a.H, NF, 128 * CW);
+        if (e != cudaSuccess) return e;
+        cache.stack[slot] = a.stack;
+        cache.box[slot] = 128 * CW;
+        map = &cache.map[slot];
+    }
     e = launch_worklist(a, 128 * CW, DIRS, st);
     if (e != cudaSuccess) return e;
-    FusedArgs a2 = a;
-    const int NF = DIRS == 2 ? 2 * N + 2 * (a.M_v + a.M_h) : N + 2 * a.M_v;
-    // the tensor map depends on the stack's address only: the context keeps the last few
-    static const bool no_tmap = getenv("SCAN3D_NO_TMAP") != nullptr;
-    const CUtensorMap* map = nullptr;
-    alignas(64) CUtensorMap local;
-    TensorMapCache* cache = a.tmap_cache;
-    if (!no_tmap) {
-        if (cache)
-            for (int i = 0; i < TensorMapCache::SLOTS; i++)
-                if (cache->stack[i] == a.stack && cache->box[i] == 128 * CW) map = &cache->map[i];
-        if (!map) {
-            CUtensorMap* dst = &local;
-            int slot = -1;
-            if (cache) { slot = cache->next++ % TensorMapCache::SLOTS; cache->stack[slot] = nullptr; dst = &cache->map[slot]; }
-            if (stack_tensor_map(dst, a.stack, (size_t)a.W * a.H, NF, 128 * CW)) {
-                map = dst;
-                if (cache) { cache->stack[slot] = a.stack; cache->box[slot] = 128 * CW; }
-            }
-        }
-    }
-    if (!map) { memset(&local, 0, sizeof(local)); map = &local; a2.use_tmap = 0; }
-    else a2.use_tmap = 1;
-    kern<<<grid, (CW + 1) * 32, p.smem, st>>>(a2, cal, *map);
+    kern<<<grid, (CW + 1) * 32, p.smem, st>>>(a, cal, *map);
     return cudaGetLastError();
 }
 
+// One instantiation per (shape, N, DIRS, variant) that plan7 and fused7_folds_registration can select: one direction
+// runs at (7, 3) only (at most 38 frames); (9, 2) serves two directions without the folded transform; (7, 2) without
+// the modulation mask is reached by 8-step scans only (72-76 frames; every other N stays below 72).
 template <int N, int DIRS>
 static cudaError_t launch7_nd(const FusedArgs& a, const DeviceCalib& cal, int sm_count, const Plan7& p, bool exact,
                               cudaStream_t st)
 {
-#define S3D_CASE7(CWV, MB)                                                                        \
-    if (p.cw == CWV && p.minb == MB) {                                                            \
-        if (exact || DIRS == 1) return launch7_t<N, DIRS, CWV, MB, true>(a, cal, sm_count, p, st); \
-        return launch7_t<N, DIRS, CWV, MB, (DIRS == 1)>(a, cal, sm_count, p, st);                  \
-    }
-    // The named configurations in the default shape get their Gray depths as compile-time constants:
-    // C3 / C4 / C5 (8-step, 10 + 10 bits), C1 (3-step, 6 + 5 bits), C2 (3-step, 8 bits, one direction).
     if (p.cw == 7 && p.minb == 3) {
+        // The named configurations in the default shape get their Gray depths as compile-time constants:
+        // C3 / C4 / C5 (8-step, 10 + 10 bits), C1 (3-step, 6 + 5 bits), C2 (3-step, 8 bits, one direction).
         // ... and with them the reference's calibration class (distorted camera, distortion-free projector: LUTS = 1)
         const bool ref_class = a.cam_lut != nullptr && a.proj_lut == nullptr;
         if (N == 8 && DIRS == 2 && a.M_v == 10 && a.M_h == 10) {
@@ -741,31 +713,36 @@ static cudaError_t launch7_nd(const FusedArgs& a, const DeviceCalib& cal, int sm
                          : launch7_t<3, 2, 7, 3, false, false, false, 6, 5>(a, cal, sm_count, p, st);
         }
         if (N == 3 && DIRS == 1 && a.M_v == 8) return launch7_t<3, 1, 7, 3, true, false, false, 8, 0>(a, cal, sm_count, p, st);
+        if (DIRS == 2 && a.reg_on) return exact ? launch7_t<N, 2, 7, 3, true, false, true>(a, cal, sm_count, p, st)
+                                                : launch7_t<N, 2, 7, 3, false, false, true>(a, cal, sm_count, p, st);
+        if (exact || DIRS == 1) return launch7_t<N, DIRS, 7, 3, true>(a, cal, sm_count, p, st);
+        return launch7_t<N, DIRS, 7, 3, (DIRS == 1)>(a, cal, sm_count, p, st);
     }
-    // the variant that folds the turntable transform into the point store exists for the two default shapes
-    if (DIRS == 2 && a.reg_on && p.cw == 7) {
-        if (p.minb == 3) return exact ? launch7_t<N, 2, 7, 3, true, false, true>(a, cal, sm_count, p, st)
-                                      : launch7_t<N, 2, 7, 3, false, false, true>(a, cal, sm_count, p, st);
-        if (p.minb == 2) return exact ? launch7_t<N, 2, 7, 2, true, false, true>(a, cal, sm_count, p, st)
-                                      : launch7_t<N, 2, 7, 2, false, false, true>(a, cal, sm_count, p, st);
+    if constexpr (DIRS == 2) {
+        if (p.cw == 9 && p.minb == 2)
+            return exact ? launch7_t<N, 2, 9, 2, true>(a, cal, sm_count, p, st) : launch7_t<N, 2, 9, 2, false>(a, cal, sm_count, p, st);
+        if constexpr (N == 8) {
+            if (p.cw == 7 && p.minb == 2) {
+                if (a.reg_on) return exact ? launch7_t<8, 2, 7, 2, true, false, true>(a, cal, sm_count, p, st)
+                                           : launch7_t<8, 2, 7, 2, false, false, true>(a, cal, sm_count, p, st);
+                return exact ? launch7_t<8, 2, 7, 2, true>(a, cal, sm_count, p, st) : launch7_t<8, 2, 7, 2, false>(a, cal, sm_count, p, st);
+            }
+        }
     }
-    S3D_CASE7(7, 2) S3D_CASE7(7, 3) S3D_CASE7(9, 2) S3D_CASE7(4, 4) S3D_CASE7(6, 2) S3D_CASE7(5, 4)
-#undef S3D_CASE7
     return cudaErrorInvalidValue;
 }
 
-// the modulation-criterion variant (3-step only, two launch shapes)
+// the modulation-criterion variant (3-step only): (7, 3), and (7, 2) for two directions from 54 frames on
 template <int DIRS>
 static cudaError_t launch7_mod(const FusedArgs& a, const DeviceCalib& cal, int sm_count, const Plan7& p, bool exact, cudaStream_t st)
 {
-    if (p.cw != 7) return cudaErrorInvalidValue;
-    if (p.minb == 3) {
+    if (p.cw == 7 && p.minb == 3) {
         if (exact || DIRS == 1) return launch7_t<3, DIRS, 7, 3, true, true>(a, cal, sm_count, p, st);
         return launch7_t<3, DIRS, 7, 3, (DIRS == 1), true>(a, cal, sm_count, p, st);
     }
-    if (p.minb == 2) {
-        if (exact || DIRS == 1) return launch7_t<3, DIRS, 7, 2, true, true>(a, cal, sm_count, p, st);
-        return launch7_t<3, DIRS, 7, 2, (DIRS == 1), true>(a, cal, sm_count, p, st);
+    if constexpr (DIRS == 2) {
+        if (p.cw == 7 && p.minb == 2)
+            return exact ? launch7_t<3, 2, 7, 2, true, true>(a, cal, sm_count, p, st) : launch7_t<3, 2, 7, 2, false, true>(a, cal, sm_count, p, st);
     }
     return cudaErrorInvalidValue;
 }
@@ -778,10 +755,7 @@ cudaError_t launch_fused7(const scan3d_config& c, const FusedArgs& a_in, const D
     if (((uintptr_t)a_in.stack & 15) || ((uintptr_t)a_in.roi & 15)) return cudaErrorMisalignedAddress;
     FusedArgs a = a_in;
     const int T = 128 * p.cw;
-    a.tiles_per_row = 0;
     a.n_tiles = (int)(((size_t)c.W * c.H + T - 1) / T);
-    a.dynamic = 1;
-    if (const char* e = getenv("SCAN3D_FUSED_DYN")) a.dynamic = atoi(e) != 0;
     const bool exact = !(c.flags & SCAN3D_FLAG_FAST_TRIANGULATION);
     if (mod7(c)) {
         if (!a.roi2 || !a.roi_list) return cudaErrorInvalidValue;

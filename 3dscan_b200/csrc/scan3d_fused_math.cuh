@@ -17,7 +17,6 @@ __device__ __forceinline__ uint32_t ge_bytes_raw(uint32_t a, uint32_t b)
     const uint32_t d = (a | 0x80808080u) - (b & 0x7f7f7f7fu);
     return (a & ~b) | (~(a ^ b) & d);
 }
-__device__ __forceinline__ uint32_t ge_bytes(uint32_t a, uint32_t b) { return ge_bytes_raw(a, b) & 0x80808080u; }
 // bytes (b0,b1,b2,b3) -> 16-bit lanes (b0,b1) and (b2,b3)
 __device__ __forceinline__ uint32_t lanes_lo(uint32_t w) { return __byte_perm(w, 0, 0x4140); }
 __device__ __forceinline__ uint32_t lanes_hi(uint32_t w) { return __byte_perm(w, 0, 0x4342); }
@@ -54,11 +53,6 @@ __device__ __forceinline__ void fringe_terms(const uint32_t* __restrict__ sw, in
             T.t[3][h] = L[1][h] + L[7 % N][h] + 0x04000400u - L[3 % N][h] - L[5 % N][h];
         }
     }
-}
-__device__ __forceinline__ int term_of(const Terms& T, int k, int j, int bias)
-{
-    const uint32_t r = (j & 2) ? T.t[k][1] : T.t[k][0];
-    return (int)((r >> ((j & 1) * 16)) & 0xffffu) - bias;
 }
 
 // Gray -> binary (B0 = G0, Bi = B(i-1) xor Gi, 4/phase_unwrap.cpp:187-191) for the 4 pixels at
@@ -113,11 +107,6 @@ __device__ __forceinline__ double lane_f64(uint32_t u, int bias)
 {
     return __hiloint2double(0x43300000, (int)u) - (bias == 512 ? K_2P52_512 : K_2P52_1024);
 }
-__device__ __forceinline__ double term_f64(const Terms& T, int k, int j, int bias)
-{
-    const uint32_t r = (j & 2) ? T.t[k][1] : T.t[k][0];
-    return lane_f64((j & 1) ? (r >> 16) : (r & 0xffffu), bias);
-}
 
 // The pair of pixels (2h, 2h + 1) of a thread shares its term registers: selecting them once per pair (by h, which
 // is a run-time value in the rolled pass loop) leaves only compile-time lane extractions per pixel.
@@ -152,34 +141,11 @@ __device__ __forceinline__ float phase_of_pair(const TermsPair& P, int u, const 
     }
 }
 
-template <int N>
-__device__ __forceinline__ float phase_of(const Terms& T, int j, const double* tab)
-{
-    if (N == 8) {
-        const double a1 = term_f64(T, 0, j, 512), b1 = term_f64(T, 1, j, 1024);
-        const double a2 = term_f64(T, 2, j, 512), b2 = term_f64(T, 3, j, 1024);
-        const double r = 0.70710678118654752440;
-        const double d1 = dadd(a1, dmul(b1, r));
-        const double d2 = dadd(a2, dmul(b2, r));
-        return atan2_to_float(d1, d2, 0.0f, 0.0f, tab);
-    } else {
-        const int t1 = term_of(T, 0, j, N == 5 ? 1024 : 512);
-        const int t2 = term_of(T, 1, j, N == 4 ? 512 : 1024);
-        if (N == 5) return atan2f_fdlibm((float)t1, (float)t2);   // 3/wrapped_phase.cpp:220 (float atan2f)
-        return atan2_to_float((double)t1, (double)t2, 0.0f, 0.0f, tab);
-    }
-}
-
 // fringe order of pixel u (0 / 1, compile time) of a pair whose accumulators have been shifted down by 16 * h
 __device__ __forceinline__ int code_of_pair(uint32_t binA_h, uint32_t binB_h, int u, int M)
 {
     const uint32_t a = (binA_h >> (8 * u)) & 0xffu, b = (binB_h >> (8 * u)) & 0xffu;
     return (int)(((a << 8) | b) >> (16 - M));
-}
-
-__device__ __forceinline__ int sat32(long long v)
-{
-    return (int)max(min(v, 2147483647LL), -2147483648LL);
 }
 
 }  // namespace s3d

@@ -20,7 +20,6 @@ struct TensorMapCache {
     alignas(64) CUtensorMap map[SLOTS];
     int next = 0;
 };
-typedef TensorMapCache Fused8Cache;
 
 // the voxel-grid merge's hash table (scan3d_voxel_kernels.cu)
 constexpr uint32_t VOXEL_NO_SLOT = 0xffffffffu;   // no slot / no ordinal yet
@@ -98,11 +97,7 @@ struct scan3d_ctx {
     int* tile_list = nullptr;
     unsigned long long* trace = nullptr;       // SCAN3D_TRACE=1: per-CTA pipeline timeline
     uint32_t epoch = 0;
-    uint32_t* sched_ctr = nullptr;             // k_fused8: work-position counter, never reset ...
-    uint32_t sched_base = 0;                   // ... its value at the next launch (advances by n_tiles + grid per launch)
-    s3d::Fused8Cache tmaps;
-    float* stage_pts = nullptr;                // k_fused8: staging rings (allocated on first use)
-    uint32_t* stage_vb = nullptr;
+    s3d::TensorMapCache tmaps;
 
     // staging for the host-buffer entries
     uint8_t* d_stack = nullptr;
@@ -208,15 +203,9 @@ struct FusedArgs {
     unsigned long long* tile_state;
     uint8_t* tile_flags;          // [n_tiles] tile holds at least one ROI pixel
     int* tile_list;               // [n_tiles] ids of those tiles, raster order
-    int* n_list;                  // [1]; n_list[n_tiles + 8] is the dynamic scheduler's counter
-    int dynamic;                  // v7: draw work-list positions from that counter instead of b, b+G, ...
-    uint32_t* sched_ctr;          // v8: work-position counter (monotonic across launches)
-    uint32_t pos_base;            // v8: the counter's value when this launch starts
+    int* n_list;                  // [1]; n_list[n_tiles + 8] is the counter the CTAs draw work-list positions from
     int reg_on;                   // fold register_point_clouds' transform into the point store (scan3d_set_registration)
     float reg_R[16], reg_t[3];
-    float* stage_pts;             // v8: per-warp rings of staging slots for triangulated points (L2 resident)
-    uint32_t* stage_vb;           // v8: ... and for the ballots of their valid bits (pixel indices / colours)
-    int use_tmap;                 // v7: tile loads are one 2-D tensor copy (set by the launcher)
     int ctas_per_sm;              // 0 = all the kernel can have; else the launch takes at most this many CTA slots per SM
     TensorMapCache* tmap_cache;   // host pointer (the launcher's cache of tensor maps; unused on the device)
     unsigned long long* trace;    // optional timeline buffer (SCAN3D_TRACE), else null
@@ -226,7 +215,7 @@ struct FusedArgs {
     int W, H, row0, H_total, PW, PH;
     int N, M_v, M_h, fw_v, fw_h;
     double fw_v_d, fw_h_d;        // the fringe widths as doubles (5/compute_correspondance.cpp:648: fw * (Phi / 2Pi) in double)
-    int n_tiles, tiles_per_row;
+    int n_tiles;
 };
 int fused_num_tiles(const scan3d_config& c);
 
@@ -235,15 +224,6 @@ bool fused7_supported(const scan3d_config& c);
 bool fused7_folds_registration(const scan3d_config& c);
 cudaError_t launch_fused7(const scan3d_config& c, const FusedArgs& a, const DeviceCalib& cal,
                           int sm_count, cudaStream_t st);
-
-// third cut (scan3d_fused_kernel8.cu, the default): one launch per scan, no consumer barrier.  *advance = how far
-// the launch moves the context's work-position counter
-bool fused8_supported(const scan3d_config& c);
-int fused8_num_chunks(const scan3d_config& c);
-size_t fused8_stage_floats(int sm_count);
-size_t fused8_stage_vb_words(int sm_count);
-cudaError_t launch_fused8(const scan3d_config& c, const FusedArgs& a, const DeviceCalib& cal, int sm_count,
-                          Fused8Cache* cache, uint32_t* advance, cudaStream_t st);
 
 // ---- either side of the path (scan3d_aux_kernels.cu) ----
 cudaError_t launch_undistort_map(const double K[9], const double d[5], int W, int H, short2* map_xy, uint16_t* map_frac,

@@ -100,17 +100,6 @@ __device__ __forceinline__ double rcp_seed(double x)
 #endif
 }
 
-__device__ __forceinline__ float rcp_seed_f32(float x)
-{
-#if defined(__CUDA_ARCH__)
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-    return r;
-#else
-    return 1.0f / x;
-#endif
-}
-
 __device__ __forceinline__ double fast_div(double num, double den)
 {
     double r = rcp_seed(den);                                  // ~20 good bits

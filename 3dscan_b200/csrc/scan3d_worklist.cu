@@ -7,7 +7,7 @@ namespace s3d {
 
 int fused_num_tiles(const scan3d_config& c)
 {
-    // upper bound over every work unit the single-pass kernels use (smallest: 128 pixels)
+    // upper bound of the single-pass kernel's tile count (its tiles hold at least 128 pixels)
     return (int)(((size_t)c.W * c.H + 127) / 128) + 1;
 }
 
@@ -80,7 +80,7 @@ __global__ void k_tile_list(const uint8_t* __restrict__ flags, int n_tiles, int*
         if (flags[i]) list[pos++] = i;
     if (threadIdx.x == 0) {
         *n_list = wsum[31];
-        n_list[n_tiles + 8] = 0;   // v7 dynamic scheduler: next work-list position
+        n_list[n_tiles + 8] = 0;   // the fused kernel's counter: next work-list position
         *d_count = 0;   // overwritten by the fused kernel's last tile when there is any work
     }
 }

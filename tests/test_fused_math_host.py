@@ -23,11 +23,9 @@ pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(CUDA_INC, "cuda_
 @pytest.fixture(scope="module")
 def shim(tmp_path_factory):
     so = str(tmp_path_factory.mktemp("fusedhost") / "libfused_math_host.so")
-    # S3D_HOST_DEFS="-DS3D_VAR_ROWSEL_RCP=1 ...": the same checks for an experimental variant (tools/build_variants.py)
-    defs = [d for d in os.environ.get("S3D_HOST_DEFS", "").split() if d.startswith("-D")]
     subprocess.check_call(["/usr/bin/g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-Wall", "-Wno-unknown-pragmas",
-                           "-Wno-unused-function", "-ffp-contract=off", "-I", CUDA_INC] + defs +
-                          ["-o", so, os.path.join(HERE, "fused_math_host.cpp")])
+                           "-Wno-unused-function", "-ffp-contract=off", "-I", CUDA_INC,
+                           "-o", so, os.path.join(HERE, "fused_math_host.cpp")])
     return C.CDLL(so)
 
 

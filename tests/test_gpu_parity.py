@@ -121,6 +121,8 @@ FUSED_CASES = [
     (512, 300, 640, 480, 4, 7, 6, 5, 8, 2),
     (256, 128, 512, 512, 5, 6, 6, 8, 8, 2),
     (16, 3, 64, 64, 3, 4, 4, 4, 4, 2),               # degenerate tiny frame
+    (256, 64, 2048, 2048, 8, 12, 12, 1, 1, 2),       # 64 frames: launch shape (9 consumer warps, 2 CTAs per SM)
+    (256, 64, 8192, 8192, 8, 14, 14, 1, 1, 2),       # 72 frames: launch shape (7, 2)
 ]
 
 
@@ -147,7 +149,7 @@ def test_fused_matches_oracle(case):
     ctx.close()
 
 
-@pytest.mark.parametrize("case", FUSED_CASES[:1] + FUSED_CASES[2:5])
+@pytest.mark.parametrize("case", FUSED_CASES[:1] + FUSED_CASES[2:5] + FUSED_CASES[7:8])
 def test_fused_fast_triangulation_within_tolerance(case):
     """SCAN3D_FLAG_FAST_TRIANGULATION: everything up to c_p_map stays bit-exact; the points are
     the same least-squares solution with a different rounding order (bar: 1e-5 relative)."""
@@ -423,6 +425,20 @@ def test_modulation_mask_flag_matches_oracle():
     assert (ref.valid_v != ref.valid_h).any() and 0 < ref.count == n
     st = compare(cfg, ref, ctx, fused=True)
     assert st["pts_nonidentical"] == 0
+    # 54 frames (12 + 12 Gray bits): the variant at launch shape (7 consumer warps, 2 CTAs per SM)
+    cfg54 = s3.make_config(256, 64, 2048, 2048, 3, 12, 12, 1, 1, 2, flags=s3.FLAG_MODULATION_MASK)
+    cal54, ocal54, _ = calibs(256 / 1600.0, 2048 / 1280.0)
+    stack54, roi54 = s3.synth_stack(cfg54, cal54)
+    stack54 = stack54.copy()
+    stack54[0:3, 20:40, 80:160] = 90                                                    # flat in V only
+    ctx54 = _ctx(cfg54, cal54)
+    l0 = ctx54.launch_count()
+    n54 = ctx54.reconstruct(stack54, roi54)
+    assert ctx54.launch_count() - l0 == 5
+    ref54 = run_oracle(cfg54, ocal54, stack54, roi54, modulation=True)
+    assert (ref54.valid_v != ref54.valid_h).any() and 0 < ref54.count == n54
+    assert compare(cfg54, ref54, ctx54, fused=True)["pts_nonidentical"] == 0
+    ctx54.close()
     # fast triangulation + one direction through the same variant
     cfg1 = s3.make_config(W, H, PW, PH, 3, 7, 7, 8, 8, 1, flags=s3.FLAG_MODULATION_MASK)
     ctx1 = _ctx(cfg1, cal)
@@ -544,7 +560,7 @@ def test_c1_full_capture_through_gpu_matches_reference_images():
     ref = run_oracle(cfg, ocal, stack, roi)
     l0 = ctx.launch_count()
     n = ctx.reconstruct(stack, roi)
-    assert ctx.launch_count() - l0 in (1, 3)      # the single-pass kernel (v7: + its two work-list launches), not the stage chain
+    assert ctx.launch_count() - l0 == 3           # the single-pass kernel and its two work-list launches, not the stage chain
     st = compare(cfg, ref, ctx)
     assert st["unw_v_nonidentical"] == 0 and st["unw_h_nonidentical"] == 0 and st["pts_nonidentical"] == 0
     assert n == ref.count and n > 300000

@@ -176,16 +176,17 @@ def test_register_point_clouds_call(tmp_path):
     getattr(L, "_Z22scan3d_compat_shutdownv")()
 
 
-@pytest.mark.parametrize("shape", [(640, 480), (1000, 40)])
+@pytest.mark.parametrize("shape", [(640, 480, 512, 288, 3, 7, 6, 4, 5), (1000, 40, 512, 288, 3, 7, 6, 4, 5),
+                                   (256, 64, 8192, 8192, 8, 14, 14, 1, 1)])
 def test_raw_entry_and_folded_registration_equal_the_separate_calls(shape):
     """SURVEY 8 f4: scan3d_reconstruct_raw (capture-side cvUndistort2 of every frame + the single-pass kernel, one call)
     with scan3d_set_registration (register_point_clouds' transform in the kernel's point store) gives, bit for bit,
     what scan3d_undistort_frames -> scan3d_reconstruct -> scan3d_register_points give (2/project_pattern.cpp:220-234,
-    9/register_point_clouds.cpp:83-148).  The second shape takes the shape-generic stage route (W % 16 != 0)."""
-    W, H = shape
-    PW, PH = 512, 288
+    9/register_point_clouds.cpp:83-148).  The second shape takes the shape-generic stage route (W % 16 != 0); the
+    third one's 72 frames take the single-pass kernel's launch shape with 2 CTAs per SM."""
+    W, H, PW, PH, N, Mv, Mh, fwv, fwh = shape
     cal, ocal, _ = calibs(W / 1600.0, PW / 1280.0)
-    cfg = s3.make_config(W, H, PW, PH, 3, 7, 6, 4, 5, 2)
+    cfg = s3.make_config(W, H, PW, PH, N, Mv, Mh, fwv, fwh, 2)
     raw, roi = s3.synth_stack(cfg, cal)
     theta, t = 36.0, (12.5, -3.25, 903.1)
     a = s3.Scan3D(cfg, 0, cal)

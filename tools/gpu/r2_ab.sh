@@ -1,4 +1,7 @@
-# A/B of kernel build variants inside ONE box (box-to-box variance is ~3 %): usage  r2_ab.sh <libdir-suffix>...
+# A/B of library builds inside ONE box (box-to-box variance is ~3 %): usage  r2_ab.sh <name>...
+# Each <name> is a library directory 3dscan_b200/lib_var_<name>; build one from another commit by running
+#   SCAN3D_LIBDIR=$PWD/3dscan_b200/lib_var_<name> python 3dscan_b200/build.py
+# in a checkout of that commit, and copy lib_var_<name> into this tree if that checkout is elsewhere.
 D=gpurun_out/ab; rm -rf $D; mkdir -p $D
 # AB_ARGS overrides the short single-context run, e.g. AB_ARGS="" for the driver-style default (1.4 s under the power cap)
 B="python bench.py --no-e2e --no-cpu-baseline --no-rowshard ${AB_ARGS---steps 20 --batch 16 --contexts 1 --cta-limit 0}"
