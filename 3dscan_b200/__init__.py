@@ -55,6 +55,33 @@ class SynthParams(C.Structure):
                 ("projector_pixelated", C.c_int32), ("seed", C.c_uint64)]
 
 
+class AlignParams(C.Structure):
+    _fields_ = [("T_init", C.c_double * 16), ("max_distance", C.c_float), ("max_iterations", C.c_int32),
+                ("stride", C.c_int32), ("stop_rotation", C.c_double), ("stop_translation", C.c_double),
+                ("apply", C.c_int32)]
+
+
+class AlignResultC(C.Structure):
+    _fields_ = [("T", C.c_double * 16), ("iterations", C.c_int32), ("status", C.c_int32),
+                ("pairs_first", C.c_int64), ("pairs_last", C.c_int64), ("rms_first", C.c_double),
+                ("rms_last", C.c_double)]
+
+
+class AlignResult:
+    """scan3d_align_result: T (4x4 float64, p_model = T p_source), iterations, status (0 converged, 1 iteration
+    limit, 2 too few pairs / singular system), pairs_first / pairs_last, rms_first / rms_last."""
+
+    def __init__(self, r):
+        self.T = np.array(list(r.T), np.float64).reshape(4, 4)
+        self.iterations, self.status = r.iterations, r.status
+        self.pairs_first, self.pairs_last = r.pairs_first, r.pairs_last
+        self.rms_first, self.rms_last = r.rms_first, r.rms_last
+
+    def __repr__(self):
+        return (f"AlignResult(status={self.status}, iterations={self.iterations}, pairs={self.pairs_first}->"
+                f"{self.pairs_last}, rms={self.rms_first:.6g}->{self.rms_last:.6g})")
+
+
 class Scan3DError(RuntimeError):
     pass
 
@@ -172,6 +199,8 @@ def cuda_lib():
     L.scan3d_voxel_count.argtypes = [vp, C.POINTER(i64), C.POINTER(i64)]
     L.scan3d_get_voxels.argtypes = [vp, vp, vp, vp, vp, i64]
     L.scan3d_write_voxel_ply.argtypes = [vp, C.c_char_p, i32]
+    L.scan3d_align_to_voxels.argtypes = [vp, C.POINTER(AlignParams), C.POINTER(AlignResultC)]
+    L.scan3d_align_to_voxels_dev.argtypes = [vp, vp, i64, C.POINTER(AlignParams), C.POINTER(AlignResultC)]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -576,6 +605,42 @@ class Scan3D:
 
     def write_voxel_ply(self, path, binary=False):
         self._ck(self.L.scan3d_write_voxel_ply(self.h, path.encode(), 1 if binary else 0))
+
+    # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
+    @staticmethod
+    def _align_params(max_distance, max_iterations, stride, T_init, apply, stop_rotation, stop_translation):
+        p = AlignParams()
+        T = np.eye(4) if T_init is None else np.asarray(T_init, np.float64).reshape(4, 4)
+        p.T_init[:] = T.reshape(-1).tolist()
+        p.max_distance = max_distance
+        p.max_iterations = int(max_iterations)
+        p.stride = int(stride)
+        p.stop_rotation = stop_rotation
+        p.stop_translation = 1e-4 * float(C.c_float(max_distance).value) if stop_translation is None else stop_translation
+        p.apply = int(bool(apply))
+        return p
+
+    def align(self, max_distance, max_iterations=30, stride=1, T_init=None, apply=True, stop_rotation=1e-6,
+              stop_translation=None):
+        """Point-to-plane ICP of the ctx's current points against the outputs of the last voxel_finish; with apply the
+        points are transformed in place (the mesh goes stale).  stop_translation None = 1e-4 * max_distance.
+        Synchronises once; returns an AlignResult."""
+        p = self._align_params(max_distance, max_iterations, stride, T_init, apply, stop_rotation, stop_translation)
+        r = AlignResultC()
+        self._ck(self.L.scan3d_align_to_voxels(self.h, C.byref(p), C.byref(r)))
+        return AlignResult(r)
+
+    def align_dev(self, xyz, max_distance, max_iterations=30, stride=1, T_init=None, apply=True, stop_rotation=1e-6,
+                  stop_translation=None, n=None):
+        """align() for n points in device memory on the ctx's GPU: a torch tensor [n][3] float32, or a raw pointer
+        (then n is required); with apply they are transformed in place."""
+        if n is None:
+            n = xyz.shape[0]
+        ptr = C.c_void_p(xyz if isinstance(xyz, int) else xyz.data_ptr())
+        p = self._align_params(max_distance, max_iterations, stride, T_init, apply, stop_rotation, stop_translation)
+        r = AlignResultC()
+        self._ck(self.L.scan3d_align_to_voxels_dev(self.h, ptr, int(n), C.byref(p), C.byref(r)))
+        return AlignResult(r)
 
     def set_points_buffer(self, dev_ptr, capacity_points):
         """Compacted points go to this device pointer (may be another GPU's memory mapped here); 0/None restores."""

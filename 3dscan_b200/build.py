@@ -28,7 +28,7 @@ if os.environ.get("SCAN3D_BUILD_TRACE") == "1":
     NVCC_FLAGS.append("-DS3D_TRACE=1")
 CU_SOURCES = ["scan3d_api.cu", "scan3d_stage_kernels.cu", "scan3d_worklist.cu", "scan3d_fused_kernel7.cu",
               "scan3d_aux_kernels.cu", "scan3d_aux_api.cu", "scan3d_shard.cu", "scan3d_mesh_kernels.cu",
-              "scan3d_voxel_kernels.cu"]
+              "scan3d_voxel_kernels.cu", "scan3d_align_kernels.cu"]
 HOST_SOURCES = ["scan3d_io.cpp", "scan3d_synth.cpp"]
 COMPAT_SOURCES = ["scan3d_stages.cpp"]
 

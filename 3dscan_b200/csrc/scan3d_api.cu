@@ -13,6 +13,7 @@
 #include "scan3d_internal.h"
 #include "../common/scan3d_pattern_profile.h"
 #include "../common/scan3d_aux_math.h"
+#include "../common/scan3d_align_math.h"
 
 using namespace s3d;
 
@@ -209,7 +210,9 @@ void scan3d_destroy(scan3d_ctx* ctx)
                     ctx->undist_xy[0], ctx->undist_xy[1], ctx->undist_frac[0], ctx->undist_frac[1],
                     ctx->mesh_idx, ctx->mesh_counts, ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals,
                     ctx->vox.keys, ctx->vox.acc, ctx->vox.ordinal, ctx->vox.ord2slot, ctx->vox.state,
-                    ctx->vox_point_slot, ctx->vox_flags, ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb, ctx->vox_cnt};
+                    ctx->vox_point_slot, ctx->vox_flags, ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb, ctx->vox_cnt,
+                    ctx->aln.keys, ctx->aln.cells, ctx->aln.model_slot, ctx->aln.entries, ctx->aln.cursor,
+                    ctx->aln_partials, ctx->aln_state};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
@@ -1171,6 +1174,137 @@ int scan3d_write_voxel_ply(scan3d_ctx* ctx, const char* path, int binary)
     write_ply_with_normals(f, binary, n, xyz.data(), nrm.data(), rgb.data(), "");
     const bool ok = fclose(f) == 0;
     return ok ? SCAN3D_OK : fail(ctx, SCAN3D_ERR_IO, "PLY write failed");
+}
+
+// ------------------------------------------------------------------------------------------
+// scan-to-model alignment (include/scan3d.h and common/scan3d_align_math.h have the exact rules)
+// ------------------------------------------------------------------------------------------
+static bool finite_d(double v) { return v - v == 0.0; }
+
+// T_init: finite, last row (0, 0, 0, 1), R^T R - I and det R - 1 within 1e-6
+static bool rigid_4x4(const double* T)
+{
+    for (int k = 0; k < 16; k++)
+        if (!finite_d(T[k])) return false;
+    if (T[12] != 0.0 || T[13] != 0.0 || T[14] != 0.0 || T[15] != 1.0) return false;
+    for (int i = 0; i < 3; i++)
+        for (int j = 0; j < 3; j++) {
+            const double d = T[i] * T[j] + T[4 + i] * T[4 + j] + T[8 + i] * T[8 + j] - (i == j ? 1.0 : 0.0);
+            if (!(fabs(d) <= 1e-6)) return false;
+        }
+    const double det = T[0] * (T[5] * T[10] - T[6] * T[9]) - T[1] * (T[4] * T[10] - T[6] * T[8]) +
+                       T[2] * (T[4] * T[9] - T[5] * T[8]);
+    return fabs(det - 1.0) <= 1e-6;
+}
+
+static int check_align_args(scan3d_ctx* ctx, const scan3d_align_params* p, scan3d_align_result* out)
+{
+    if (!p || !out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (!(p->max_distance > 0.0f && p->max_distance - p->max_distance == 0.0f))
+        return fail(ctx, SCAN3D_ERR_ARG, "max_distance must be finite and > 0");
+    if (p->max_iterations < 1 || p->max_iterations > 64) return fail(ctx, SCAN3D_ERR_ARG, "max_iterations must be in 1..64");
+    if (p->stride < 1) return fail(ctx, SCAN3D_ERR_ARG, "stride must be >= 1");
+    if (!(p->stop_rotation >= 0.0) || !(p->stop_translation >= 0.0))
+        return fail(ctx, SCAN3D_ERR_ARG, "stop thresholds must be >= 0");
+    if (!rigid_4x4(p->T_init)) return fail(ctx, SCAN3D_ERR_ARG, "T_init must be a finite rigid transform (rotation within 1e-6)");
+    if (!ctx->vox_begun || !ctx->vox_fresh)
+        return fail(ctx, SCAN3D_ERR_STATE, "no voxel outputs of the current adds to align to: call scan3d_voxel_finish");
+    return SCAN3D_OK;
+}
+
+// the whole run on the source xyz (n_dev: its count is on the device, <= n_max)
+static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long long n_max, const scan3d_align_params* p,
+                     scan3d_align_result* out)
+{
+    CK(cudaSetDevice(ctx->device));
+    const uint32_t maxv = ctx->vox.max_voxels;
+    AlignIndex& ix = ctx->aln;
+    if (maxv > ctx->aln_alloc_max) {
+        free_ptr(ix.keys); free_ptr(ix.cells); free_ptr(ix.model_slot); free_ptr(ix.entries);
+        ix.keys = nullptr; ix.cells = nullptr; ix.model_slot = nullptr; ix.entries = nullptr;
+        ctx->aln_alloc_max = 0;
+        const size_t cap = (size_t)ALIGN_CELLS_PER_VOXEL * maxv;
+        CK(dalloc(&ix.keys, cap));
+        CK(dalloc(&ix.cells, cap));
+        CK(dalloc(&ix.model_slot, (size_t)maxv));
+        CK(dalloc(&ix.entries, 2 * (size_t)maxv));
+        ctx->aln_alloc_max = maxv;
+    }
+    if (!ctx->aln_state) CK(dalloc(&ctx->aln_state, 1));
+    if (!ix.cursor) CK(dalloc(&ix.cursor, 1));
+    const uint32_t blocks = align_match_blocks(n_max, p->stride);
+    if (blocks > ctx->aln_alloc_blocks) {
+        free_ptr(ctx->aln_partials);
+        ctx->aln_partials = nullptr;
+        ctx->aln_alloc_blocks = 0;
+        CK(dalloc(&ctx->aln_partials, (size_t)(ALIGN_NSUM + 1) * blocks));
+        ctx->aln_alloc_blocks = blocks;
+    }
+    ix.cap = ALIGN_CELLS_PER_VOXEL * maxv;
+    CK(cudaMemsetAsync(ix.keys, 0xff, (size_t)ix.cap * sizeof(*ix.keys), ctx->stream));
+    CK(cudaMemsetAsync(ix.cells, 0, (size_t)ix.cap * sizeof(*ix.cells), ctx->stream));
+    CK(cudaMemsetAsync(ix.cursor, 0, sizeof(*ix.cursor), ctx->stream));
+    AlignRun run;
+    for (int k = 0; k < 12; k++) run.T0[k] = p->T_init[k];
+    run.S = s3l::cell_edge(p->max_distance);
+    run.r2 = (double)p->max_distance * (double)p->max_distance;   // host TU: -ffp-contract=off
+    run.stop_rotation = p->stop_rotation;
+    run.stop_translation = p->stop_translation;
+    run.max_iterations = p->max_iterations;
+    const int par = (int)(ctx->vox_chunks & 1);
+    CK(launch_align_index(ix, ctx->vox, par, ctx->vox_xyz, ctx->vox_nrm, run.S, ctx->aln_state, run, n_dev,
+                          ctx->sm_count, ctx->stream));
+    ctx->launches += ALIGN_INDEX_LAUNCHES;
+    for (int it = 0; it < p->max_iterations; it++) {
+        CK(launch_align_iteration(ix, ctx->aln_state, run, xyz, n_dev, n_max, p->stride, ctx->aln_partials, ctx->stream));
+        ctx->launches += 2;
+    }
+    AlignState st;
+    CK(cudaMemcpyAsync(&st, ctx->aln_state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st.overflow)
+        return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct voxels than max_voxels: begin again with a larger max_voxels");
+    for (int k = 0; k < 12; k++) out->T[k] = st.T[k];
+    out->T[12] = out->T[13] = out->T[14] = 0.0;
+    out->T[15] = 1.0;
+    out->iterations = st.iterations;
+    out->status = st.status;
+    out->pairs_first = st.pairs_first;
+    out->pairs_last = st.pairs_last;
+    out->rms_first = st.rms_first;
+    out->rms_last = st.rms_last;
+    const long long n = n_dev ? std::min((long long)st.n_src, n_max) : n_max;
+    if (p->apply && n > 0) {
+        float R[16];
+        for (int k = 0; k < 16; k++) R[k] = (float)out->T[k];
+        CK(launch_register_points(xyz, xyz, n, R, 0.0f, 0.0f, 0.0f, ctx->sm_count, ctx->stream));
+        ctx->launches += 1;
+    }
+    return SCAN3D_OK;
+}
+
+int scan3d_align_to_voxels(scan3d_ctx* ctx, const scan3d_align_params* p, scan3d_align_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    int rc = check_align_args(ctx, p, out);
+    if (rc) return rc;
+    if (ctx->cfg.dirs != 2) return fail(ctx, SCAN3D_ERR_STATE, "no point cloud in a one-direction configuration");
+    if (!ctx->have_points) return fail(ctx, SCAN3D_ERR_STATE, "align before the points are computed");
+    rc = align_run(ctx, points_of(ctx), ctx->d_count, (long long)npix(ctx), p, out);
+    if (rc == SCAN3D_OK && p->apply) ctx->have_mesh = false;
+    return rc;
+}
+
+int scan3d_align_to_voxels_dev(scan3d_ctx* ctx, float* xyz_dev, int64_t n, const scan3d_align_params* p,
+                               scan3d_align_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (n < 0) return fail(ctx, SCAN3D_ERR_ARG, "n < 0");
+    if (!xyz_dev && n > 0) return fail(ctx, SCAN3D_ERR_ARG, "null xyz_dev");
+    if ((uintptr_t)xyz_dev & 3) return fail(ctx, SCAN3D_ERR_ARG, "xyz_dev must be 4-byte aligned");
+    const int rc = check_align_args(ctx, p, out);
+    if (rc) return rc;
+    return align_run(ctx, xyz_dev, nullptr, (long long)n, p, out);
 }
 
 // ------------------------------------------------------------------------------------------

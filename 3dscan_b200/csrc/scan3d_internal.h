@@ -47,6 +47,32 @@ struct VoxelTable {
     uint32_t cap, max_voxels;
     double S;                  // (double)voxel_size
 };
+
+// the alignment's cell index of the model (scan3d_align_kernels.cu)
+struct AlignIndex {
+    unsigned long long* keys;  // [cap], s3v::EMPTY_KEY = free; key = s3v::pack_key of the cell
+    uint2* cells;              // [cap] (points in the cell, end of its range in entries)
+    uint32_t* model_slot;      // [max_voxels] cell slot of each voxel, VOXEL_NO_SLOT = not in the model
+    float4* entries;           // [2 max_voxels] per model point: (x, y, z, ordinal bits), (nx, ny, nz, 0)
+    uint32_t* cursor;          // [1]
+    uint32_t cap;
+};
+// the device state of one alignment run
+struct AlignState {
+    double T[12];              // current estimate [R | t], row-major
+    double rms_first, rms_last;
+    long long pairs_first, pairs_last;
+    int iterations, status, done, rounds;   // updates applied, scan3d_align_result.status, run ended, solves run
+    int overflow;              // the voxel accumulator overflowed (read when the index is built)
+    uint32_t n_src;            // the ctx route's point count (read when the index is built)
+};
+struct AlignRun {
+    double T0[12];             // T_init
+    double S;                  // cell edge
+    double r2;                 // max_distance^2
+    double stop_rotation, stop_translation;
+    int max_iterations;
+};
 }  // namespace s3d
 
 struct scan3d_ctx {
@@ -124,6 +150,13 @@ struct scan3d_ctx {
     float* vox_nrm = nullptr;             // [max_voxels][3]
     uint8_t* vox_rgb = nullptr;           // [max_voxels][3]
     uint32_t* vox_cnt = nullptr;          // [max_voxels]
+
+    // scan3d_align_to_voxels (allocated by the first align, grown with max_voxels and the sample count)
+    s3d::AlignIndex aln{};
+    uint32_t aln_alloc_max = 0;           // max_voxels the index buffers hold
+    uint32_t aln_alloc_blocks = 0;        // blocks of match partials the partial buffer holds
+    double* aln_partials = nullptr;       // [ALIGN_NSUM + 1][blocks]
+    s3d::AlignState* aln_state = nullptr;
 
     int cta_limit = 0;             // scan3d_set_cta_limit
 
@@ -256,6 +289,25 @@ uint32_t voxel_table_capacity(uint32_t max_voxels, int sm_count);
 // 1 launch: the merged voxels in first-point order into xyz / nrm [max_voxels][3], rgb [max_voxels][3], cnt
 cudaError_t launch_voxel_finish(const VoxelTable& t, int par, float* xyz, float* nrm, uint8_t* rgb, uint32_t* cnt,
                                 int sm_count, cudaStream_t st);
+
+// ---- scan-to-model alignment (scan3d_align_kernels.cu; common/scan3d_align_math.h has the arithmetic) ----
+// ALIGN_INDEX_LAUNCHES launches: cell keys and counts (which also initialises *state from run, the voxel overflow
+// flag and, when n_dev is set, the source count), cell ranges, scatter of the model points.  The model is the first
+// min(total, max_voxels) voxel outputs of t (total = t.state->total[par]); xyz / nrm [max_voxels][3].  The index holds
+// ALIGN_CELLS_PER_VOXEL * max_voxels slots (at most half of them taken) and must be reset before (keys 0xff, cells and
+// cursor 0).
+constexpr int ALIGN_INDEX_LAUNCHES = 3;
+constexpr uint32_t ALIGN_CELLS_PER_VOXEL = 2;
+cudaError_t launch_align_index(const AlignIndex& ix, const VoxelTable& t, int par, const float* xyz, const float* nrm,
+                               double S, AlignState* state, const AlignRun& run, const uint32_t* n_dev, int sm_count,
+                               cudaStream_t st);
+// One match + one solve launch per iteration.  The source is xyz[i * stride] for i * stride < n, n = min(*n_dev, n_max)
+// when n_dev is set, else n_max; the grid depends on n_max and stride only (align_match_blocks).  partials
+// [ALIGN_NSUM + 1][blocks].
+constexpr int ALIGN_NSUM = 28;
+uint32_t align_match_blocks(long long n_max, int stride);
+cudaError_t launch_align_iteration(const AlignIndex& ix, AlignState* state, const AlignRun& run, const float* xyz,
+                                   const uint32_t* n_dev, long long n_max, int stride, double* partials, cudaStream_t st);
 
 // ---- debug / self-test ----
 cudaError_t launch_debug_atan2(const double* y, const double* x, float* out, int n, int mode,

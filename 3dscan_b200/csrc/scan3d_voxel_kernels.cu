@@ -8,6 +8,7 @@
 // orders them by their first point inside the add.  That takes a grid-wide step after the inserts, so an add is
 // 5 launches: insert, flag, the compaction's k_count + k_scan over the flags, assign.
 #include "scan3d_internal.h"
+#include "scan3d_hash.cuh"
 #include "../common/scan3d_voxel_math.h"
 
 namespace s3d {
@@ -16,40 +17,6 @@ namespace {
 
 constexpr int VT = 256;                 // threads per block of the insert / flag kernels
 constexpr unsigned FULL = 0xffffffffu;
-
-// splitmix64's finaliser: the table position must not follow the raster order of the keys
-__device__ __forceinline__ unsigned long long mix64(unsigned long long x)
-{
-    x ^= x >> 30;
-    x *= 0xbf58476d1ce4e5b9ull;
-    x ^= x >> 27;
-    x *= 0x94d049bb133111ebull;
-    x ^= x >> 31;
-    return x;
-}
-
-// The key's slot, inserting it if absent.  At most cap probes, so a full table cannot hang the add (the capacity
-// rule in scan3d_voxel_begin keeps the table at most half full, so the bound is never reached in practice).
-// *claimed = this call took a new slot.  VOXEL_NO_SLOT if the table is full.
-__device__ __forceinline__ uint32_t find_or_insert(unsigned long long* keys, uint32_t cap, unsigned long long key,
-                                                   bool* claimed)
-{
-    uint32_t s = (uint32_t)(((mix64(key) >> 32) * (unsigned long long)cap) >> 32);
-    *claimed = false;
-    for (uint32_t p = 0; p < cap; p++) {
-        unsigned long long k = __ldcg(keys + s);   // keys never change once set: a stale EMPTY only costs a CAS
-        if (k == s3v::EMPTY_KEY) {
-            k = atomicCAS(keys + s, s3v::EMPTY_KEY, key);
-            if (k == s3v::EMPTY_KEY) {
-                *claimed = true;
-                return s;
-            }
-        }
-        if (k == key) return s;
-        s = s + 1 == cap ? 0 : s + 1;
-    }
-    return VOXEL_NO_SLOT;
-}
 
 }  // namespace
 

@@ -242,8 +242,8 @@ int scan3d_write_pcd(scan3d_ctx *ctx, const char *path);
  * SCAN3D_ERR_STATE without points or with dirs == 1; SCAN3D_ERR_CONFIG for a row-sharded ctx (a shard's last cell row
  * needs the next shard's first row) or W*H >= 2^31.  The face buffer (2(W-1)(H-1) faces) and the normal buffer (W*H)
  * are ctx-owned, allocated by the first build.  Every entry that rewrites or drops the points (a reconstruct,
- * scan3d_compact_points, scan3d_set_points_buffer) makes the mesh stale: the getters below then return
- * SCAN3D_ERR_STATE (the device pointers NULL) until scan3d_build_mesh runs again. */
+ * scan3d_compact_points, scan3d_set_points_buffer, scan3d_align_to_voxels with apply) makes the mesh stale: the getters
+ * below then return SCAN3D_ERR_STATE (the device pointers NULL) until scan3d_build_mesh runs again. */
 int scan3d_build_mesh(scan3d_ctx *ctx, float max_edge);
 int scan3d_mesh_face_count(scan3d_ctx *ctx, int64_t *count_out);             /* syncs */
 /* faces int32[n][3], normals f32[point_count][3]; either may be NULL; max_faces bounds the face copy */
@@ -306,6 +306,71 @@ int scan3d_get_voxels(scan3d_ctx *ctx, float *xyz_host, float *normals_host, uin
 /* the vertex element of scan3d_write_mesh_ply ("x y z nx ny nz red green blue"), no face element; ascii (%.9g) or
  * binary_little_endian */
 int scan3d_write_voxel_ply(scan3d_ctx *ctx, const char *path, int binary);
+
+/* ---- scan-to-model alignment: point-to-plane ICP of a view against the merged voxel cloud (the reference's users ran
+ * MeshLab's ICP on the exported clouds) -------------------------------------------------------------------------------
+ * Refines a rigid estimate T (p_model = T p_source) of a roughly registered view before it is added to the merge, so
+ * that an error of the turntable angle or pivot (register_point_clouds' Pi = 22/7 alone rotates by theta * 1.000402)
+ * does not place one surface in the merge several times.
+ *
+ * Model: the outputs of the last scan3d_voxel_finish whose normal is not (0,0,0).  The align reads the accumulator and
+ * never changes it: the voxel getters return the same bytes before and after.
+ * Source: scan3d_align_to_voxels uses the ctx's current points, wherever they are (scan3d_set_points_buffer and
+ * row-sharded contexts included); scan3d_align_to_voxels_dev uses n points xyz f32[n][3] in device memory of the ctx's
+ * GPU, ordered on the ctx stream.  Sample j is point j * stride.  A point with a non-finite coordinate, or whose
+ * transformed coordinate / max_distance (1 + 2^-20) has a cell outside [-2^20, 2^20) on some axis, is never paired.
+ * Correspondence: for p' = T p (double), the model point q with the smallest ((dx*dx + dy*dy) + dz*dz) in double, a
+ * tie going to the smaller voxel ordinal; the pair is kept when that is <= max_distance^2.  This is the exact nearest
+ * neighbour within the radius: the search covers every model point that can qualify (a cell index of edge
+ * max_distance (1 + 2^-20) and the 27 cells around the query's).
+ * Update: each pair gives J = [p' x n_q, n_q] and r = (p' - q) . n_q; with A = sum J^T J and b = sum J^T r the update
+ * solves (A + mu I) x = -b by an LDL^T factorisation, mu = 1e-6 * trace(A) / 6, which keeps a rank-deficient scene (a
+ * plane alone; the synthetic plane + sphere, free to turn about the plane normal through the sphere centre) finite.
+ * x = (omega, v); dR = Rodrigues(omega) exactly (sin and cos by a fixed polynomial, not the small-angle matrix);
+ * T <- [dR | v] T.  The run ends converged (status 0) after an update with |omega| <= stop_rotation and |v| <=
+ * stop_translation (stop_rotation = stop_translation = 0: never), at the iteration limit (status 1), or with fewer than
+ * 6 pairs or a solve that fails its pivot test (every pivot > mu / 2, mu finite and > 0; status 2, T = the last good
+ * estimate, T_init when no update succeeded).  rms_* = sqrt(sum r^2 / pairs) of an iteration's pairs before its
+ * update (0 without pairs).  The exact arithmetic is in 3dscan_b200/common/scan3d_align_math.h; the sums are reduced
+ * in a fixed order, so results are bit-reproducible and independent of the GPU's SM count.
+ * apply = 1: the source is then transformed in place by the returned T rounded to float, by scan3d_register_points'
+ * kernel with the translation in R's fourth column and a zero pivot (register_point's float operation order).  On the
+ * ctx variant this rewrites the points, so the mesh becomes stale, as after every other rewriting entry.
+ * Synchronisation: the iteration loop, the convergence test and the state live in device memory; the host does not
+ * wait between iterations.  The entry synchronises the ctx stream once, at the end, to copy the result out (the
+ * apply, if any, is queued after that and runs asynchronously).
+ * Launches: always 3 (cell index of the model) + 2 per max_iterations (match, solve; those after the run ended return
+ * at once) + 1 with apply when the source is not empty.  The index buffers (about 60 B per max_voxels) are ctx-owned,
+ * allocated by the first align and grown with max_voxels.
+ * Errors: SCAN3D_ERR_ARG for null pointers (xyz_dev may be NULL when n = 0), a max_distance not finite or <= 0,
+ * max_iterations outside 1..64, stride < 1, a negative or NaN stop threshold, n < 0, xyz_dev not 4-byte aligned, or a
+ * T_init that is not finite, whose last row is not (0, 0, 0, 1) or whose 3x3 block R is not a rotation within 1e-6
+ * (every element of R^T R - I, and det R - 1, within 1e-6).  SCAN3D_ERR_STATE before scan3d_voxel_begin, before the
+ * first scan3d_voxel_finish or after an add since it; for the ctx variant also without points or with dirs == 1.
+ * SCAN3D_ERR_CONFIG when the accumulator overflowed (max_voxels too small), found on the device and reported after the
+ * final synchronisation, without applying. */
+typedef struct {
+    double T_init[16];         /* row-major 4x4 rigid start estimate (identity when the nominal registration is already
+                                  folded into the points) */
+    float max_distance;        /* correspondence radius, finite, > 0 (model units) */
+    int32_t max_iterations;    /* 1..64 */
+    int32_t stride;            /* >= 1: source sample j is point j * stride */
+    double stop_rotation;      /* radians, >= 0 */
+    double stop_translation;   /* model units, >= 0; 0 and 0 = always run max_iterations */
+    int32_t apply;             /* 1: transform the source cloud in place by the returned T */
+} scan3d_align_params;
+
+typedef struct {
+    double T[16];              /* p_model = T p_source; T_init when no update succeeded */
+    int32_t iterations;        /* updates applied */
+    int32_t status;            /* 0 converged, 1 iteration limit, 2 too few pairs / singular system (T = last good) */
+    int64_t pairs_first, pairs_last;   /* correspondences of the first / last iteration */
+    double rms_first, rms_last;        /* point-to-plane RMS of those iterations, before their update */
+} scan3d_align_result;
+
+int scan3d_align_to_voxels(scan3d_ctx *ctx, const scan3d_align_params *p, scan3d_align_result *out);
+int scan3d_align_to_voxels_dev(scan3d_ctx *ctx, float *xyz_dev, int64_t n, const scan3d_align_params *p,
+                               scan3d_align_result *out);
 
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
