@@ -82,6 +82,22 @@ class AlignResult:
                 f"{self.pairs_last}, rms={self.rms_first:.6g}->{self.rms_last:.6g})")
 
 
+class SurfaceParams(C.Structure):
+    _fields_ = [("max_distance", C.c_float), ("max_points", C.c_int64)]
+
+
+class SurfaceResultC(C.Structure):
+    _fields_ = [("vertices", C.c_int64), ("faces", C.c_int64), ("lattice_points", C.c_int64),
+                ("undefined_points", C.c_int64)]
+
+
+# voxel_surface's default max_points per merged voxel: the smallest power of two >= 1.5x the largest lattice points
+# per voxel measured on tools/bench_surface.py's workloads (29.2 on workload A, profiles/r3_bench_surface.json).  64 is
+# also the most a voxel can add (the 4 x 4 x 4 corners of its 27 cells), so the default never overflows; pass
+# max_points from a previous result's lattice_points to hold less memory.
+SURFACE_POINTS_PER_VOXEL = 64
+
+
 class Scan3DError(RuntimeError):
     pass
 
@@ -201,6 +217,9 @@ def cuda_lib():
     L.scan3d_write_voxel_ply.argtypes = [vp, C.c_char_p, i32]
     L.scan3d_align_to_voxels.argtypes = [vp, C.POINTER(AlignParams), C.POINTER(AlignResultC)]
     L.scan3d_align_to_voxels_dev.argtypes = [vp, vp, i64, C.POINTER(AlignParams), C.POINTER(AlignResultC)]
+    L.scan3d_voxel_surface.argtypes = [vp, C.POINTER(SurfaceParams), C.POINTER(SurfaceResultC)]
+    L.scan3d_get_voxel_surface.argtypes = [vp, vp, vp, vp, vp, i64, i64]
+    L.scan3d_write_voxel_surface_ply.argtypes = [vp, C.c_char_p, i32]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -572,6 +591,7 @@ class Scan3D:
     def voxel_begin(self, voxel_size, max_voxels):
         """Reset the ctx's merge accumulator: voxels of edge voxel_size, up to max_voxels of them."""
         self._ck(self.L.scan3d_voxel_begin(self.h, voxel_size, int(max_voxels)))
+        self._voxel_size = float(C.c_float(voxel_size).value)
 
     def voxel_add(self):
         """Add the ctx's current points (with the fresh mesh's normals and the texture's colours); asynchronous."""
@@ -605,6 +625,34 @@ class Scan3D:
 
     def write_voxel_ply(self, path, binary=False):
         self._ck(self.L.scan3d_write_voxel_ply(self.h, path.encode(), 1 if binary else 0))
+
+    # -- triangle surface of the voxel outputs (include/scan3d.h has the exact rules)
+    def voxel_surface(self, max_distance=None, max_points=None):
+        """Extract the surface of the outputs of the last voxel_finish; synchronises once and returns a dict with
+        vertices, faces, lattice_points and undefined_points.  max_distance None = 2 voxel_size; max_points None =
+        SURFACE_POINTS_PER_VOXEL * the voxel count (within [1, 2^31 - 1])."""
+        if max_distance is None:
+            max_distance = 2.0 * self._voxel_size
+        if max_points is None:
+            max_points = min(max(SURFACE_POINTS_PER_VOXEL * self.voxel_count()[0], 1), 2 ** 31 - 1)
+        p = SurfaceParams(max_distance, int(max_points))
+        r = SurfaceResultC()
+        self._ck(self.L.scan3d_voxel_surface(self.h, C.byref(p), C.byref(r)))
+        self._surface_counts = (r.vertices, r.faces)
+        return dict(vertices=r.vertices, faces=r.faces, lattice_points=r.lattice_points,
+                    undefined_points=r.undefined_points)
+
+    def voxel_surface_mesh(self):
+        """(xyz float32 [v][3], normals float32 [v][3], rgb uint8 [v][3], faces int32 [f][3]) of the last
+        voxel_surface."""
+        v, f = getattr(self, "_surface_counts", (0, 0))
+        out = (np.empty((v, 3), np.float32), np.empty((v, 3), np.float32), np.empty((v, 3), np.uint8),
+               np.empty((f, 3), np.int32))
+        self._ck(self.L.scan3d_get_voxel_surface(self.h, *[_ptr(a) for a in out], v, f))
+        return out
+
+    def write_voxel_surface_ply(self, path, binary=False):
+        self._ck(self.L.scan3d_write_voxel_surface_ply(self.h, path.encode(), 1 if binary else 0))
 
     # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
     @staticmethod

@@ -87,6 +87,13 @@ S3A_HD bool closer(double d, uint32_t ord, double best_d, uint32_t best_ord)
     return d < best_d || (d == best_d && ord < best_ord);
 }
 
+// the point-to-plane residual (p' - q) . n_q of a pair
+S3A_HD double residual(const double p[3], float qx, float qy, float qz, float nx, float ny, float nz)
+{
+    const double dx = S3A_SUB(p[0], (double)qx), dy = S3A_SUB(p[1], (double)qy), dz = S3A_SUB(p[2], (double)qz);
+    return S3A_ADD(S3A_ADD(S3A_MUL(dx, (double)nx), S3A_MUL(dy, (double)ny)), S3A_MUL(dz, (double)nz));
+}
+
 // the Jacobian row and the residual of a pair (p', q, n_q)
 S3A_HD void row(const double p[3], float qx, float qy, float qz, float nx, float ny, float nz, double J[6], double* r)
 {
@@ -97,8 +104,7 @@ S3A_HD void row(const double p[3], float qx, float qy, float qz, float nx, float
     J[3] = n0;
     J[4] = n1;
     J[5] = n2;
-    const double dx = S3A_SUB(p[0], (double)qx), dy = S3A_SUB(p[1], (double)qy), dz = S3A_SUB(p[2], (double)qz);
-    *r = S3A_ADD(S3A_ADD(S3A_MUL(dx, n0), S3A_MUL(dy, n1)), S3A_MUL(dz, n2));
+    *r = residual(p, qx, qy, qz, nx, ny, nz);
 }
 
 // s += the products of one pair

@@ -130,32 +130,8 @@ __global__ void __launch_bounds__(MT) k_align_match(AlignIndex ix, const AlignSt
         const size_t i = (size_t)j * (size_t)stride;
         double p[3];
         s3l::transform(T, xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2], p);
-        long long c[3];
-        if (!s3l::cell_of(p, run.S, c)) continue;
-        double best = 0.0;
-        uint32_t best_o = VOXEL_NO_SLOT, best_e = 0;
-        for (int dz = -1; dz <= 1; dz++)
-            for (int dy = -1; dy <= 1; dy++)
-                for (int dx = -1; dx <= 1; dx++) {
-                    const long long a = c[0] + dx, b = c[1] + dy, e = c[2] + dz;
-                    if (a < s3v::I_MIN || a >= s3v::I_MAX || b < s3v::I_MIN || b >= s3v::I_MAX || e < s3v::I_MIN ||
-                        e >= s3v::I_MAX)
-                        continue;
-                    const uint32_t slot = find_slot(ix.keys, ix.cap, s3v::pack_key(a, b, e));
-                    if (slot == VOXEL_NO_SLOT) continue;
-                    const uint2 cell = ix.cells[slot];
-                    for (uint32_t u = cell.y - cell.x; u < cell.y; u++) {
-                        const float4 q = ix.entries[2 * (size_t)u];
-                        const double d = s3l::dist2(p, q.x, q.y, q.z);
-                        const uint32_t o = __float_as_uint(q.w);
-                        if (d <= run.r2 && (best_o == VOXEL_NO_SLOT || s3l::closer(d, o, best, best_o))) {
-                            best = d;
-                            best_o = o;
-                            best_e = u;
-                        }
-                    }
-                }
-        if (best_o == VOXEL_NO_SLOT) continue;
+        uint32_t best_e;
+        if (align_nearest(ix, p, run.S, run.r2, &best_e) == VOXEL_NO_SLOT) continue;
         const float4 q = ix.entries[2 * (size_t)best_e], nq = ix.entries[2 * (size_t)best_e + 1];
         double J[6], r;
         s3l::row(p, q.x, q.y, q.z, nq.x, nq.y, nq.z, J, &r);

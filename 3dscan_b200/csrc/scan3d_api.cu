@@ -14,6 +14,7 @@
 #include "../common/scan3d_pattern_profile.h"
 #include "../common/scan3d_aux_math.h"
 #include "../common/scan3d_align_math.h"
+#include "../common/scan3d_surface_math.h"
 
 using namespace s3d;
 
@@ -212,7 +213,10 @@ void scan3d_destroy(scan3d_ctx* ctx)
                     ctx->vox.keys, ctx->vox.acc, ctx->vox.ordinal, ctx->vox.ord2slot, ctx->vox.state,
                     ctx->vox_point_slot, ctx->vox_flags, ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb, ctx->vox_cnt,
                     ctx->aln.keys, ctx->aln.cells, ctx->aln.model_slot, ctx->aln.entries, ctx->aln.cursor,
-                    ctx->aln_partials, ctx->aln_state};
+                    ctx->aln_partials, ctx->aln_state,
+                    ctx->srf.keys, ctx->srf.owner, ctx->srf.f, ctx->srf.nearest, ctx->srf.vert, ctx->srf.state,
+                    ctx->srf_flags, ctx->srf_flag_counts, ctx->srf_vert_slot, ctx->srf_face_counts, ctx->srf_xyz,
+                    ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
@@ -909,6 +913,26 @@ static void write_ply_with_normals(FILE* f, int binary, int64_t n, const float* 
     }
 }
 
+// The vertex element of write_ply_with_normals and the face element "vertex_indices" (uchar count, int indices) of
+// scan3d_write_mesh_ply and scan3d_write_voxel_surface_ply.
+static void write_ply_with_faces(FILE* f, int binary, int64_t nv, const float* xyz, const float* nrm, const uint8_t* rgb,
+                                 int64_t nf, const int32_t* faces)
+{
+    char face_header[96];
+    snprintf(face_header, sizeof(face_header), "element face %lld\nproperty list uchar int vertex_indices\n", (long long)nf);
+    write_ply_with_normals(f, binary, nv, xyz, nrm, rgb, face_header);
+    if (binary) {
+        std::vector<uint8_t> frec((size_t)nf * 13);
+        for (int64_t i = 0; i < nf; i++) {
+            frec[(size_t)i * 13] = 3;
+            memcpy(&frec[(size_t)i * 13 + 1], &faces[(size_t)i * 3], 12);
+        }
+        fwrite(frec.data(), 1, frec.size(), f);
+    } else {
+        for (int64_t i = 0; i < nf; i++) fprintf(f, "3 %d %d %d\n", faces[3 * i], faces[3 * i + 1], faces[3 * i + 2]);
+    }
+}
+
 // ------------------------------------------------------------------------------------------
 // camera-grid mesh of the compacted points (common/scan3d_mesh_math.h has the exact rules)
 // ------------------------------------------------------------------------------------------
@@ -988,19 +1012,7 @@ int scan3d_write_mesh_ply(scan3d_ctx* ctx, const char* path, int binary)
     if (rc) return rc;
     FILE* f = fopen(path, "wb");
     if (!f) return fail(ctx, SCAN3D_ERR_IO, "cannot open PLY for writing");
-    char face_header[96];
-    snprintf(face_header, sizeof(face_header), "element face %lld\nproperty list uchar int vertex_indices\n", (long long)nf);
-    write_ply_with_normals(f, binary, np, xyz.data(), nrm.data(), rgb.data(), face_header);
-    if (binary) {
-        std::vector<uint8_t> frec((size_t)nf * 13);
-        for (int64_t i = 0; i < nf; i++) {
-            frec[(size_t)i * 13] = 3;
-            memcpy(&frec[(size_t)i * 13 + 1], &faces[(size_t)i * 3], 12);
-        }
-        fwrite(frec.data(), 1, frec.size(), f);
-    } else {
-        for (int64_t i = 0; i < nf; i++) fprintf(f, "3 %d %d %d\n", faces[3 * i], faces[3 * i + 1], faces[3 * i + 2]);
-    }
+    write_ply_with_faces(f, binary, np, xyz.data(), nrm.data(), rgb.data(), nf, faces.data());
     const bool ok = fclose(f) == 0;
     return ok ? SCAN3D_OK : fail(ctx, SCAN3D_ERR_IO, "PLY write failed");
 }
@@ -1021,6 +1033,7 @@ int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
     if (max_voxels < 1 || max_voxels >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_ARG, "max_voxels must be in [1, 2^31)");
     CK(cudaSetDevice(ctx->device));
     ctx->vox_begun = ctx->vox_fresh = false;
+    ctx->srf_ready = false;
     VoxelTable& t = ctx->vox;
     const uint32_t cap = voxel_table_capacity((uint32_t)max_voxels, ctx->sm_count);
     if (cap > ctx->vox_alloc_cap) {
@@ -1086,7 +1099,7 @@ int scan3d_voxel_add_points(scan3d_ctx* ctx)
         return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^32 - 1 points since scan3d_voxel_begin (W*H counted per ctx add)");
     CK(cudaSetDevice(ctx->device));
     ctx->vox_bound += ub;
-    ctx->vox_fresh = false;
+    ctx->vox_fresh = ctx->srf_ready = false;
     return voxel_add(ctx, points_of(ctx), ctx->have_mesh ? ctx->mesh_normals : nullptr,
                      ctx->texture && ctx->rgb ? ctx->rgb : nullptr, ctx->d_count, (uint32_t)ub);
 }
@@ -1104,7 +1117,7 @@ int scan3d_voxel_add_points_dev(scan3d_ctx* ctx, const float* xyz_dev, const flo
         return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^32 - 1 points since scan3d_voxel_begin");
     CK(cudaSetDevice(ctx->device));
     ctx->vox_bound += (uint64_t)n;
-    ctx->vox_fresh = false;
+    ctx->vox_fresh = ctx->srf_ready = false;
     const int64_t chunk = (int64_t)npix(ctx);   // the per-point scratch holds W*H points
     for (int64_t off = 0; off < n; off += chunk) {
         const int64_t k = std::min(chunk, n - off);
@@ -1124,6 +1137,7 @@ int scan3d_voxel_finish(scan3d_ctx* ctx)
                            ctx->sm_count, ctx->stream));
     ctx->launches += 1;
     ctx->vox_fresh = true;
+    ctx->srf_ready = false;
     return SCAN3D_OK;
 }
 
@@ -1212,11 +1226,10 @@ static int check_align_args(scan3d_ctx* ctx, const scan3d_align_params* p, scan3
     return SCAN3D_OK;
 }
 
-// the whole run on the source xyz (n_dev: its count is on the device, <= n_max)
-static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long long n_max, const scan3d_align_params* p,
-                     scan3d_align_result* out)
+// the model's cell index of edge run.S (ALIGN_INDEX_LAUNCHES), in ctx-owned buffers grown with max_voxels; it also
+// initialises ctx->aln_state from run (n_dev: the source count to record, or null)
+static int align_index(scan3d_ctx* ctx, const AlignRun& run, const uint32_t* n_dev)
 {
-    CK(cudaSetDevice(ctx->device));
     const uint32_t maxv = ctx->vox.max_voxels;
     AlignIndex& ix = ctx->aln;
     if (maxv > ctx->aln_alloc_max) {
@@ -1232,6 +1245,21 @@ static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long lo
     }
     if (!ctx->aln_state) CK(dalloc(&ctx->aln_state, 1));
     if (!ix.cursor) CK(dalloc(&ix.cursor, 1));
+    ix.cap = ALIGN_CELLS_PER_VOXEL * maxv;
+    CK(cudaMemsetAsync(ix.keys, 0xff, (size_t)ix.cap * sizeof(*ix.keys), ctx->stream));
+    CK(cudaMemsetAsync(ix.cells, 0, (size_t)ix.cap * sizeof(*ix.cells), ctx->stream));
+    CK(cudaMemsetAsync(ix.cursor, 0, sizeof(*ix.cursor), ctx->stream));
+    CK(launch_align_index(ix, ctx->vox, (int)(ctx->vox_chunks & 1), ctx->vox_xyz, ctx->vox_nrm, run.S, ctx->aln_state,
+                          run, n_dev, ctx->sm_count, ctx->stream));
+    ctx->launches += ALIGN_INDEX_LAUNCHES;
+    return SCAN3D_OK;
+}
+
+// the whole run on the source xyz (n_dev: its count is on the device, <= n_max)
+static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long long n_max, const scan3d_align_params* p,
+                     scan3d_align_result* out)
+{
+    CK(cudaSetDevice(ctx->device));
     const uint32_t blocks = align_match_blocks(n_max, p->stride);
     if (blocks > ctx->aln_alloc_blocks) {
         free_ptr(ctx->aln_partials);
@@ -1240,10 +1268,6 @@ static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long lo
         CK(dalloc(&ctx->aln_partials, (size_t)(ALIGN_NSUM + 1) * blocks));
         ctx->aln_alloc_blocks = blocks;
     }
-    ix.cap = ALIGN_CELLS_PER_VOXEL * maxv;
-    CK(cudaMemsetAsync(ix.keys, 0xff, (size_t)ix.cap * sizeof(*ix.keys), ctx->stream));
-    CK(cudaMemsetAsync(ix.cells, 0, (size_t)ix.cap * sizeof(*ix.cells), ctx->stream));
-    CK(cudaMemsetAsync(ix.cursor, 0, sizeof(*ix.cursor), ctx->stream));
     AlignRun run;
     for (int k = 0; k < 12; k++) run.T0[k] = p->T_init[k];
     run.S = s3l::cell_edge(p->max_distance);
@@ -1251,12 +1275,10 @@ static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long lo
     run.stop_rotation = p->stop_rotation;
     run.stop_translation = p->stop_translation;
     run.max_iterations = p->max_iterations;
-    const int par = (int)(ctx->vox_chunks & 1);
-    CK(launch_align_index(ix, ctx->vox, par, ctx->vox_xyz, ctx->vox_nrm, run.S, ctx->aln_state, run, n_dev,
-                          ctx->sm_count, ctx->stream));
-    ctx->launches += ALIGN_INDEX_LAUNCHES;
+    const int rc = align_index(ctx, run, n_dev);
+    if (rc) return rc;
     for (int it = 0; it < p->max_iterations; it++) {
-        CK(launch_align_iteration(ix, ctx->aln_state, run, xyz, n_dev, n_max, p->stride, ctx->aln_partials, ctx->stream));
+        CK(launch_align_iteration(ctx->aln, ctx->aln_state, run, xyz, n_dev, n_max, p->stride, ctx->aln_partials, ctx->stream));
         ctx->launches += 2;
     }
     AlignState st;
@@ -1305,6 +1327,144 @@ int scan3d_align_to_voxels_dev(scan3d_ctx* ctx, float* xyz_dev, int64_t n, const
     const int rc = check_align_args(ctx, p, out);
     if (rc) return rc;
     return align_run(ctx, xyz_dev, nullptr, (long long)n, p, out);
+}
+
+// ------------------------------------------------------------------------------------------
+// triangle surface of the merged voxels (include/scan3d.h and common/scan3d_surface_math.h have the exact rules)
+// ------------------------------------------------------------------------------------------
+int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d_surface_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!p || !out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (!(p->max_distance > 0.0f && p->max_distance - p->max_distance == 0.0f))
+        return fail(ctx, SCAN3D_ERR_ARG, "max_distance must be finite and > 0");
+    if (p->max_points < 1 || p->max_points >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_ARG, "max_points must be in [1, 2^31)");
+    if (!ctx->vox_begun || !ctx->vox_fresh)
+        return fail(ctx, SCAN3D_ERR_STATE, "no voxel outputs of the current adds to mesh: call scan3d_voxel_finish");
+    CK(cudaSetDevice(ctx->device));
+    ctx->srf_ready = false;
+    AlignRun run{};                                      // the index only; T0 = I for the state it initialises
+    run.T0[0] = run.T0[5] = run.T0[10] = 1.0;
+    run.S = s3l::cell_edge(p->max_distance);
+    int rc = align_index(ctx, run, nullptr);
+    if (rc) return rc;
+    SurfaceTable& s = ctx->srf;
+    const uint32_t maxp = (uint32_t)p->max_points;
+    const uint32_t cap = surface_table_capacity(maxp, ctx->sm_count);
+    if (cap > ctx->srf_alloc_cap) {
+        free_ptr(s.keys); free_ptr(s.owner); free_ptr(s.f); free_ptr(s.nearest); free_ptr(s.vert);
+        s.keys = s.owner = nullptr; s.f = nullptr; s.nearest = s.vert = nullptr;
+        ctx->srf_alloc_cap = 0;
+        CK(dalloc(&s.keys, cap));
+        CK(dalloc(&s.owner, cap));
+        CK(dalloc(&s.f, cap));
+        CK(dalloc(&s.nearest, cap));
+        CK(dalloc(&s.vert, cap));
+        ctx->srf_alloc_cap = cap;
+    }
+    const size_t nvb = (maxp + SURFACE_VB - 1) / SURFACE_VB;
+    if (maxp > ctx->srf_alloc_points) {
+        free_ptr(ctx->srf_vert_slot); free_ptr(ctx->srf_face_counts);
+        ctx->srf_vert_slot = ctx->srf_face_counts = nullptr;
+        ctx->srf_alloc_points = 0;
+        CK(dalloc(&ctx->srf_vert_slot, maxp));
+        CK(dalloc(&ctx->srf_face_counts, nvb + 1));
+        ctx->srf_alloc_points = maxp;
+    }
+    const uint64_t nflags = (uint64_t)s3s::OFFSETS * ctx->vox.max_voxels;
+    if (nflags > ctx->srf_alloc_flags) {
+        free_ptr(ctx->srf_flags); free_ptr(ctx->srf_flag_counts);
+        ctx->srf_flags = nullptr; ctx->srf_flag_counts = nullptr;
+        ctx->srf_alloc_flags = 0;
+        CK(dalloc(&ctx->srf_flags, nflags));
+        CK(dalloc(&ctx->srf_flag_counts, (nflags + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+        ctx->srf_alloc_flags = nflags;
+    }
+    if (!s.state) CK(dalloc(&s.state, 1));
+    s.cap = cap;
+    s.max_points = maxp;
+    s.S = ctx->vox.S;
+    CK(cudaMemsetAsync(s.keys, 0xff, (size_t)cap * sizeof(*s.keys), ctx->stream));
+    CK(cudaMemsetAsync(s.owner, 0xff, (size_t)cap * sizeof(*s.owner), ctx->stream));
+    CK(cudaMemsetAsync(s.vert, 0xff, (size_t)cap * sizeof(*s.vert), ctx->stream));
+    CK(cudaMemsetAsync(s.state, 0, sizeof(*s.state), ctx->stream));
+    CK(cudaMemsetAsync(ctx->srf_face_counts, 0, nvb * sizeof(uint32_t), ctx->stream));
+    CK(launch_surface_counts(s, ctx->aln, ctx->vox, (int)(ctx->vox_chunks & 1), ctx->vox_nrm, p->max_distance,
+                             ctx->srf_flags, ctx->srf_flag_counts, ctx->srf_vert_slot, ctx->srf_face_counts, ctx->stream));
+    ctx->launches += SURFACE_COUNT_LAUNCHES;
+    SurfaceState st;
+    int vox_overflow = 0;
+    CK(cudaMemcpyAsync(&st, s.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&vox_overflow, &ctx->aln_state->overflow, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (vox_overflow)
+        return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct voxels than max_voxels: begin again with a larger max_voxels");
+    if (st.overflow || st.occupied > maxp)
+        return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct lattice points than max_points: extract again with a larger max_points");
+    if ((uint64_t)st.vertices * 6 > 0xffffffffull)   // the face count is a 32-bit sum of <= 6 per vertex
+        return fail(ctx, SCAN3D_ERR_CONFIG, "more than (2^32 - 1) / 6 surface vertices");
+    if (st.vertices > ctx->srf_alloc_v) {
+        free_ptr(ctx->srf_xyz); free_ptr(ctx->srf_nrm); free_ptr(ctx->srf_rgb);
+        ctx->srf_xyz = ctx->srf_nrm = nullptr; ctx->srf_rgb = nullptr;
+        ctx->srf_alloc_v = 0;
+        CK(dalloc(&ctx->srf_xyz, 3 * (size_t)st.vertices));
+        CK(dalloc(&ctx->srf_nrm, 3 * (size_t)st.vertices));
+        CK(dalloc(&ctx->srf_rgb, 3 * (size_t)st.vertices));
+        ctx->srf_alloc_v = st.vertices;
+    }
+    if (st.faces > ctx->srf_alloc_f) {
+        free_ptr(ctx->srf_tri);
+        ctx->srf_tri = nullptr;
+        ctx->srf_alloc_f = 0;
+        CK(dalloc(&ctx->srf_tri, 3 * (size_t)st.faces));
+        ctx->srf_alloc_f = st.faces;
+    }
+    CK(launch_surface_emit(s, ctx->vox_rgb, ctx->srf_vert_slot, ctx->srf_face_counts, st.vertices, ctx->srf_xyz,
+                           ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri, ctx->stream));
+    ctx->launches += 1;
+    ctx->srf_vertices = st.vertices;
+    ctx->srf_faces = st.faces;
+    ctx->srf_ready = true;
+    out->vertices = st.vertices;
+    out->faces = st.faces;
+    out->lattice_points = st.occupied;
+    out->undefined_points = (int64_t)st.undefined;
+    return SCAN3D_OK;
+}
+
+int scan3d_get_voxel_surface(scan3d_ctx* ctx, float* xyz, float* normals, uint8_t* rgb, int32_t* faces,
+                             int64_t max_vertices, int64_t max_faces)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!ctx->srf_ready)
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    CK(cudaSetDevice(ctx->device));
+    const int64_t nv = std::max<int64_t>(0, std::min(ctx->srf_vertices, max_vertices));
+    const int64_t nf = std::max<int64_t>(0, std::min(ctx->srf_faces, max_faces));
+    if (xyz && nv) CK(cudaMemcpyAsync(xyz, ctx->srf_xyz, (size_t)nv * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    if (normals && nv) CK(cudaMemcpyAsync(normals, ctx->srf_nrm, (size_t)nv * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    if (rgb && nv) CK(cudaMemcpyAsync(rgb, ctx->srf_rgb, (size_t)nv * 3, cudaMemcpyDeviceToHost, ctx->stream));
+    if (faces && nf) CK(cudaMemcpyAsync(faces, ctx->srf_tri, (size_t)nf * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return SCAN3D_OK;
+}
+
+int scan3d_write_voxel_surface_ply(scan3d_ctx* ctx, const char* path, int binary)
+{
+    if (!ctx || !path) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (!ctx->srf_ready)
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
+    std::vector<float> xyz((size_t)nv * 3), nrm((size_t)nv * 3);
+    std::vector<uint8_t> rgb((size_t)nv * 3);
+    std::vector<int32_t> faces((size_t)nf * 3);
+    const int rc = scan3d_get_voxel_surface(ctx, xyz.data(), nrm.data(), rgb.data(), faces.data(), nv, nf);
+    if (rc) return rc;
+    FILE* f = fopen(path, "wb");
+    if (!f) return fail(ctx, SCAN3D_ERR_IO, "cannot open PLY for writing");
+    write_ply_with_faces(f, binary, nv, xyz.data(), nrm.data(), rgb.data(), nf, faces.data());
+    const bool ok = fclose(f) == 0;
+    return ok ? SCAN3D_OK : fail(ctx, SCAN3D_ERR_IO, "PLY write failed");
 }
 
 // ------------------------------------------------------------------------------------------

@@ -73,6 +73,24 @@ struct AlignRun {
     double stop_rotation, stop_translation;
     int max_iterations;
 };
+
+// the surface extraction's lattice table (scan3d_surface_kernels.cu), one slot per distinct lattice point
+struct SurfaceState {
+    unsigned long long undefined;  // lattice points without a model point within max_distance
+    uint32_t occupied;             // slots taken = distinct lattice points
+    uint32_t overflow;             // an insert found no free slot, or a vertex ordinal reached max_points
+    uint32_t vertices, faces;
+};
+struct SurfaceTable {
+    unsigned long long* keys;      // [cap] s3v::pack_key of the lattice point, s3v::EMPTY_KEY = free
+    unsigned long long* owner;     // [cap] min(27 o + k) of a candidate cell, ~0 = not a candidate
+    double* f;                     // [cap] corner value
+    uint32_t* nearest;             // [cap] ordinal of the nearest model point, VOXEL_NO_SLOT = f undefined
+    uint32_t* vert;                // [cap] VOXEL_NO_SLOT = not an active cell, else its vertex ordinal
+    SurfaceState* state;
+    uint32_t cap, max_points;
+    double S;                      // (double)voxel_size
+};
 }  // namespace s3d
 
 struct scan3d_ctx {
@@ -157,6 +175,22 @@ struct scan3d_ctx {
     uint32_t aln_alloc_blocks = 0;        // blocks of match partials the partial buffer holds
     double* aln_partials = nullptr;       // [ALIGN_NSUM + 1][blocks]
     s3d::AlignState* aln_state = nullptr;
+
+    // scan3d_voxel_surface (allocated by the first extraction, grown on demand)
+    s3d::SurfaceTable srf{};
+    bool srf_ready = false;               // the surface of the current voxel outputs is held
+    uint32_t srf_alloc_cap = 0, srf_alloc_points = 0;   // what the table and the per-vertex buffers hold
+    uint64_t srf_alloc_flags = 0;         // what the flag plane holds (27 max_voxels)
+    uint8_t* srf_flags = nullptr;         // [27 max_voxels] (o, k) owns an active cell
+    uint32_t* srf_flag_counts = nullptr;  // [cdiv(27 max_voxels, POINT_BLOCK) + 1]
+    uint32_t* srf_vert_slot = nullptr;    // [max_points] lattice slot of each vertex
+    uint32_t* srf_face_counts = nullptr;  // [cdiv(max_points, SURFACE_VB) + 1] faces per block of vertices, then offsets
+    int64_t srf_vertices = 0, srf_faces = 0;
+    int64_t srf_alloc_v = 0, srf_alloc_f = 0;
+    float* srf_xyz = nullptr;             // [vertices][3]
+    float* srf_nrm = nullptr;             // [vertices][3]
+    uint8_t* srf_rgb = nullptr;           // [vertices][3]
+    int32_t* srf_tri = nullptr;           // [faces][3]
 
     int cta_limit = 0;             // scan3d_set_cta_limit
 
@@ -308,6 +342,25 @@ constexpr int ALIGN_NSUM = 28;
 uint32_t align_match_blocks(long long n_max, int stride);
 cudaError_t launch_align_iteration(const AlignIndex& ix, AlignState* state, const AlignRun& run, const float* xyz,
                                    const uint32_t* n_dev, long long n_max, int stride, double* partials, cudaStream_t st);
+
+// ---- surface extraction (scan3d_surface_kernels.cu; common/scan3d_surface_math.h has the arithmetic) ----
+// launch_surface_counts: SURFACE_COUNT_LAUNCHES launches after launch_align_index built the model's index (cell edge
+// s3l::cell_edge(max_distance)): candidate cells (27 per model voxel, with their order key), their other 7 corners,
+// the corner values, the (o, k) flags of active cells, k_count + k_scan over them (the vertex ordinals), vertex
+// assignment with the faces per block of SURFACE_VB vertices, and the scan of those.  The table must be reset before
+// (keys 0xff, owner 0xff, vert 0xff, state 0).  flags [27 max_voxels], flag_counts [cdiv(27 max_voxels, POINT_BLOCK)],
+// vert_slot [max_points], face_counts [cdiv(max_points, SURFACE_VB)].
+// launch_surface_emit: 1 launch, the vertices (xyz, normals, rgb) and faces once the counts are known.
+constexpr int SURFACE_COUNT_LAUNCHES = 8;
+constexpr int SURFACE_VB = 256;
+cudaError_t launch_surface_counts(const SurfaceTable& s, const AlignIndex& ix, const VoxelTable& t, int par,
+                                  const float* vox_nrm, float max_distance, uint8_t* flags, uint32_t* flag_counts,
+                                  uint32_t* vert_slot, uint32_t* face_counts, cudaStream_t st);
+cudaError_t launch_surface_emit(const SurfaceTable& s, const uint8_t* vox_rgb, const uint32_t* vert_slot,
+                                const uint32_t* face_counts, uint32_t vertices, float* xyz, float* nrm, uint8_t* rgb,
+                                int32_t* faces, cudaStream_t st);
+// slots of the lattice table for max_points: at most half of them are ever taken
+uint32_t surface_table_capacity(uint32_t max_points, int sm_count);
 
 // ---- debug / self-test ----
 cudaError_t launch_debug_atan2(const double* y, const double* x, float* out, int n, int mode,

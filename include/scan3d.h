@@ -372,6 +372,75 @@ int scan3d_align_to_voxels(scan3d_ctx *ctx, const scan3d_align_params *p, scan3d
 int scan3d_align_to_voxels_dev(scan3d_ctx *ctx, float *xyz_dev, int64_t n, const scan3d_align_params *p,
                                scan3d_align_result *out);
 
+/* ---- triangle surface of the merged voxels: point-to-plane distance on the voxel lattice (Hoppe et al. 1992), meshed
+ * by naive surface nets (Gibson 1998) --------------------------------------------------------------------------------
+ * One closed, oriented triangle surface of the whole object from the merge, in place of the reconstruction the
+ * reference's users ran in another tool.  A pure function of the merge outputs, their order and max_distance: the
+ * result is bit-reproducible and does not depend on the hash, the scheduling or the GPU's SM count.
+ *
+ * s = the voxel_size of the last scan3d_voxel_begin, S = (double)s.  The model is the outputs of the last
+ * scan3d_voxel_finish whose normal is not (0,0,0), with their ordinals o (the alignment's model).
+ * Lattice point g = (i, j, k), integers in [-2^20, 2^20); x_g = ((double)i*S, (double)j*S, (double)k*S).  Cell g is the
+ * cube with min corner g, corners g + (a, b, c), a, b, c in {0, 1}.  A model voxel sits in the cell of its own merge
+ * index (not recomputed from its rounded output coordinate).
+ * Candidate cell: some model voxel v has max(|g - v|) <= 1 on every axis.  A cell with a corner outside the key range is
+ * never active and is not held.
+ * Corner value f(g): q = the nearest model point to x_g by the alignment's rule (d = ((dx*dx + dy*dy) + dz*dz) in
+ * double, dx = x_g - (double)q_x; q qualifies when d <= R*R, R = (double)max_distance; a tie goes to the smaller
+ * ordinal); f(g) = (dx*n_x + dy*n_y) + dz*n_z with q's normal n (the alignment's residual).  Undefined when no model
+ * point is within R.  g is inside when f < 0, outside when f >= 0.
+ * Active cell: a candidate whose 8 corners are all defined and not all on one side.
+ * Vertex of an active cell: its 12 edges in the order: the four x-edges at (b, c) = (0,0), (1,0), (0,1), (1,1), then the
+ * four y-edges at (a, c) and the four z-edges at (a, b) in the same pattern.  On each edge whose lower end u and upper
+ * end w lie on different sides, t = f_u / (f_u - f_w); the crossing takes ((double)g_u,axis + t)*S on the edge's axis
+ * and x_u's other two coordinates.  Per axis the crossings are summed in edge order from +0, divided by their number
+ * in double and rounded to float.
+ * Vertex normal: the trilinear gradient g_x = ((f100 - f000) + (f110 - f010)) + ((f101 - f001) + (f111 - f011)), g_y,
+ * g_z likewise over the (0,0), (1,0), (0,1), (1,1) pattern of the other two axes, divided by sqrt((g_x^2 + g_y^2) +
+ * g_z^2) in double and rounded to float; (0,0,0) when that length is 0 or not finite.
+ * Vertex colour: per channel (sum of the 8 corners' nearest model points' colours + 4) / 8, integer division.
+ * Faces: for each active cell g and axis a = x, y, z, with (b, d) the next two axes in cyclic order ((y,z), (z,x),
+ * (x,y)): lattice edge g -> g + e_a gives a quad when its ends are on different sides and cells g, g - e_b,
+ * g - e_b - e_d and g - e_d are all active.  v0..v3 = the vertices of g - e_b - e_d, g - e_d, g, g - e_b; when
+ * f(g) < 0 <= f(g + e_a) the triangles are (v0, v1, v2), (v0, v2, v3), else (v0, v2, v1), (v0, v3, v2): every face's
+ * right-hand normal points from inside to outside, the direction of the model normals.
+ * Order: vertices by their cell's key min(27*o + k) over the model voxels v_o that make it a candidate, k = ((dz+1)*3 +
+ * (dy+1))*3 + (dx+1) for the offset g - v_o; faces by their v2, then the axis, then the two triangles.  Vertex indices
+ * are int32.  The exact arithmetic is in 3dscan_b200/common/scan3d_surface_math.h.
+ * Synchronisation: scan3d_voxel_surface synchronises the ctx stream once, after the counts are known; the vertex and
+ * face buffers are then sized, *out is filled and the emission is queued asynchronously.
+ * Launches: always 3 (the alignment's cell index of the model, cell edge max_distance (1 + 2^-20)) + 8 (candidate
+ * cells, their corners, corner values, active-cell flags, their k_count + k_scan, vertex ordinals with face counts,
+ * the scan of those) before the synchronisation, + 1 (the emission) when it succeeds.
+ * Memory (ctx-owned, allocated by the first extraction, grown on demand): about 68 B per max_points, 27 B + the index's
+ * ~60 B per max_voxels, and 27 B per vertex + 12 B per face.
+ * The extraction never changes the accumulator: the voxel getters return the same bytes before and after.  A later
+ * begin, add or finish makes the surface stale (the getters and the writer then return SCAN3D_ERR_STATE); an align,
+ * with or without apply, does not.  A failed extraction leaves no surface behind.
+ * Errors: SCAN3D_ERR_ARG for null pointers, a max_distance not finite or <= 0, max_points outside [1, 2^31), a null
+ * path.  SCAN3D_ERR_STATE before scan3d_voxel_begin, before the first scan3d_voxel_finish or after an add since it.
+ * SCAN3D_ERR_CONFIG when the accumulator overflowed (max_voxels too small), or when more than max_points distinct
+ * lattice points were needed: both are found on the device (inserting stops, so nothing hangs or overruns) and reported
+ * at the synchronisation.  A model without normals gives 0 vertices and 0 faces, with SCAN3D_OK. */
+typedef struct {
+    float max_distance;        /* R: finite, > 0 (model units) */
+    int64_t max_points;        /* capacity in distinct lattice points (candidate cells and their corners), 1 .. 2^31 - 1 */
+} scan3d_surface_params;
+
+typedef struct {
+    int64_t vertices, faces;
+    int64_t lattice_points;    /* distinct lattice points held (to size max_points) */
+    int64_t undefined_points;  /* of them, without a model point within R (to choose R) */
+} scan3d_surface_result;
+
+int scan3d_voxel_surface(scan3d_ctx *ctx, const scan3d_surface_params *p, scan3d_surface_result *out);
+/* xyz f32[v][3], normals f32[v][3], rgb u8[v][3] of the first v = min(vertices, max_vertices) vertices, faces
+ * int32[f][3] of the first f = min(faces, max_faces) faces; any pointer may be NULL; syncs */
+int scan3d_get_voxel_surface(scan3d_ctx *ctx, float *xyz, float *normals, uint8_t *rgb, int32_t *faces,
+                             int64_t max_vertices, int64_t max_faces);
+/* the vertex element of scan3d_write_mesh_ply plus its face element; ascii (%.9g) or binary_little_endian */
+int scan3d_write_voxel_surface_ply(scan3d_ctx *ctx, const char *path, int binary);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,
