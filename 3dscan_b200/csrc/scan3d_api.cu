@@ -164,6 +164,11 @@ int scan3d_create(const scan3d_config* cfg, int device, scan3d_ctx** out)
         double tab[ATAN_TAB_DOUBLES];
         fill_atan_table(tab);
         CK(cudaMemcpyAsync(ctx->atan_tab, tab, sizeof(tab), cudaMemcpyHostToDevice, ctx->stream));
+        const int n_codes = 1 << (cfg->dirs == 2 && cfg->M_h > cfg->M_v ? cfg->M_h : cfg->M_v);
+        std::vector<double> code_term(n_codes);
+        fill_code_term_table(code_term.data(), n_codes);
+        CK(dalloc(&ctx->code_term, (size_t)n_codes));
+        CK(cudaMemcpyAsync(ctx->code_term, code_term.data(), n_codes * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
         CK(dalloc(&ctx->nstep_w, 128));
         double w[128];
         memset(w, 0, sizeof(w));
@@ -204,7 +209,7 @@ void scan3d_destroy(scan3d_ctx* ctx)
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     if (ctx->own_stream) cudaStreamSynchronize(ctx->own_stream);
-    void* ptrs[] = {ctx->cam_lut, ctx->proj_lut, ctx->atan_tab, ctx->nstep_w, ctx->wrapped[0], ctx->wrapped[1],
+    void* ptrs[] = {ctx->cam_lut, ctx->proj_lut, ctx->atan_tab, ctx->code_term, ctx->nstep_w, ctx->wrapped[0], ctx->wrapped[1],
                     ctx->unwrapped[0], ctx->unwrapped[1], ctx->code[0], ctx->code[1], ctx->mask[0],
                     ctx->mask[1], ctx->valid, ctx->cpmap, ctx->xyz, ctx->pts, ctx->pix, ctx->rgb,
                     ctx->texture, ctx->d_count, ctx->block_counts, ctx->tile_state, ctx->tile_flags, ctx->tile_list, ctx->trace, ctx->d_stack, ctx->d_roi, ctx->d_undist, ctx->roi_eff, ctx->roi_eff_h, ctx->roi_strict, ctx->pattern_profiles,
@@ -259,6 +264,11 @@ int scan3d_set_calibration(scan3d_ctx* ctx, const scan3d_calib* cal)
         return K[1] == 0.0 && K[3] == 0.0 && K[6] == 0.0 && K[7] == 0.0 && K[8] == 1.0;
     };
     d.cam_std = std_form(cal->Kc);
+    {
+        double Rc[9];
+        rodrigues_host(cal->rc, Rc);
+        camera_frame_calib(cal->Kc, Rc, cal->tc, d.Ap, &d);
+    }
     d.proj_std = std_form(cal->Kp);
     d.fast_div_ok = ctx->fast_div_ok ? 1 : 0;
     d.cam_distorted = d.proj_distorted = 0;
@@ -564,7 +574,7 @@ int scan3d_reconstruct_dev(scan3d_ctx* ctx, const uint8_t* stack_dev, const uint
     a.pts = points_of(ctx); a.pix = ctx->pix;
     a.rgb = ctx->texture ? ctx->rgb : nullptr; a.texture = ctx->texture;
     a.d_count = ctx->d_count; a.tile_state = ctx->tile_state; a.trace = ctx->trace; a.tile_flags = ctx->tile_flags; a.tile_list = ctx->tile_list + 1; a.n_list = ctx->tile_list;
-    a.cam_lut = ctx->cam_lut; a.proj_lut = ctx->proj_lut; a.atan_tab = ctx->atan_tab;
+    a.cam_lut = ctx->cam_lut; a.proj_lut = ctx->proj_lut; a.atan_tab = ctx->atan_tab; a.code_term = ctx->code_term;
     if (ctx->trace) CK(cudaMemsetAsync(ctx->trace, 0, (size_t)1024 * 64 * 8 * 8, ctx->stream));   // diagnostics only
     a.epoch = ++ctx->epoch;
     if ((ctx->epoch & 0x3fffffffu) == 0) {   // epoch wrapped: clear the look-back words once

@@ -113,7 +113,6 @@ k_fused7(const __grid_constant__ FusedArgs a, const __grid_constant__ DeviceCali
     constexpr int NCONS = 32 * CW;
     constexpr int WPF = T / 4;
     constexpr Geom7 G = geom7(T);
-    constexpr bool fastdiv = true;   // host verified (else this kernel is not used)
 
     extern __shared__ __align__(128) uint8_t smem[];
     // MV / MH != 0: the Gray depths as compile-time constants (the named configurations): plane loops without guards,
@@ -481,23 +480,27 @@ k_fused7(const __grid_constant__ FusedArgs a, const __grid_constant__ DeviceCali
                     const bool m = mv && mh;                                             // merge_valid_maps, 5/compute_correspondance.cpp:60-77
                     const int cv = code_of_pair(gvA_h, gvB_h, u, M_v);
                     const float wv = add_pi(phase_of_pair<N>(Pv, u, tab));               // 4/phase_unwrap.cpp:290
-                    float unwv = (x == 0 || x == W - 1) ? 0.0f : unwrap_abs(wv, cv, fastdiv);  // :285, :291
+                    // two directions: the unwrap term comes from the per-order table (one cached load instead of 4 FP64
+                    // instructions); one direction has too few independent chains per pass to cover the load (1080p
+                    // 3-step measured 4 % slower with it) and divides
+                    float unwv = (x == 0 || x == W - 1) ? 0.0f
+                                 : DIRS == 2 ? unwrap_abs_k(wv, __ldg(a.code_term + cv)) : unwrap_abs(wv, cv, true);  // :285, :291
                     unwv = mv ? unwv : 0.0f;
                     bool v = mv;
                     r_cv[u] = mv ? cv : -1;
                     if (DIRS == 2) {
                         const int ch = code_of_pair(ghA_h, ghB_h, u, M_h);
                         const float wh = add_pi(phase_of_pair<N>(Ph, u, tab));
-                        float unwh = (y == 0 || y == a.H_total - 1) ? 0.0f : unwrap_abs(wh, ch, fastdiv);  // :304, :309
+                        float unwh = (y == 0 || y == a.H_total - 1) ? 0.0f : unwrap_abs_k(wh, __ldg(a.code_term + ch));  // :304, :309
                         unwh = mh ? unwh : 0.0f;
-                        int px, py;                                                       // 5/compute_correspondance.cpp:648-675
-                        const bool okx = correspond32(unwv, a.fw_v_d, &px);
-                        const bool oky = correspond32(unwh, a.fw_h_d, &py);
-                        // FE_INVALID on x rejects before y is computed (:650-655); on y after x is stored
-                        r_cp[u].x = (m && okx) ? px : 0;
-                        r_cp[u].y = (m && okx && oky) ? py : 0;
+                        // 5/compute_correspondance.cpp:648-675.  Both phases are finite here (see
+                        // correspond32_finite), so lrint's FE_INVALID rejection never fires.
+                        const int px = correspond32_finite(unwv, a.fw_v_d);
+                        const int py = correspond32_finite(unwh, a.fw_h_d);
+                        r_cp[u].x = m ? px : 0;
+                        r_cp[u].y = m ? py : 0;
                         // 0 <= p <= P-1 as one unsigned compare (saturated values fall outside as well)
-                        v = m && okx && oky && (unsigned)px <= (unsigned)(a.PW - 1) && (unsigned)py <= (unsigned)(a.PH - 1);
+                        v = m && (unsigned)px <= (unsigned)(a.PW - 1) && (unsigned)py <= (unsigned)(a.PH - 1);
                         r_unwh[u] = unwh;
                         r_ch[u] = mh ? ch : -1;
                     }
@@ -590,7 +593,7 @@ k_fused7(const __grid_constant__ FusedArgs a, const __grid_constant__ DeviceCali
                     up = (double)cpx; vp = (double)cpy;
                 }
                 if (EXACT) triangulate_point(cal.Ac, cal.Ap, uc, vc, up, vp, Xd);
-                else triangulate_point_fast(cal.Ac, cal.Ap, uc, vc, up, vp, Xd);
+                else triangulate_point_camframe(cal, uc, vc, up, vp, Xd);   // cam_std (launch_fused7)
                 float px = __double2float_rn(Xd[0]), py = __double2float_rn(Xd[1]), pz = __double2float_rn(Xd[2]);   // 8/save_point_cloud.cpp:94-96
                 // optional: register_point_clouds' turntable transform on the float point (9/register_point_clouds.cpp:117-137)
                 if (REG) s3a::register_point(a.reg_R, a.reg_t[0], a.reg_t[1], a.reg_t[2], px, py, pz);
@@ -756,7 +759,8 @@ cudaError_t launch_fused7(const scan3d_config& c, const FusedArgs& a_in, const D
     FusedArgs a = a_in;
     const int T = 128 * p.cw;
     a.n_tiles = (int)(((size_t)c.W * c.H + T - 1) / T);
-    const bool exact = !(c.flags & SCAN3D_FLAG_FAST_TRIANGULATION);
+    // the fast solve runs in the camera's frame and needs the standard camera matrix; otherwise the exact one runs
+    const bool exact = !(c.flags & SCAN3D_FLAG_FAST_TRIANGULATION) || !cal.cam_std;
     if (mod7(c)) {
         if (!a.roi2 || !a.roi_list) return cudaErrorInvalidValue;
         return c.dirs == 2 ? launch7_mod<2>(a, cal, sm_count, p, exact, st) : launch7_mod<1>(a, cal, sm_count, p, exact, st);

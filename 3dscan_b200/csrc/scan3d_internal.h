@@ -110,6 +110,7 @@ struct scan3d_ctx {
     double2* cam_lut = nullptr;    // [H][W] (u',v') of the local rows, only if the camera is distorted
     double2* proj_lut = nullptr;   // [PH][PW], only if the projector is distorted
     double* atan_tab = nullptr;    // hi[33] then lo[33]
+    double* code_term = nullptr;   // [2^max(M_v, M_h)] the unwrap term of every fringe order
     float* pts_ext = nullptr;      // scan3d_set_points_buffer: caller-owned (possibly peer) destination of the points
     uint8_t* pattern_profiles = nullptr;   // scan3d_generate_patterns: 1-D profiles of both directions' patterns
     bool have_profiles[2] = {false, false};
@@ -278,6 +279,7 @@ struct FusedArgs {
     unsigned long long* trace;    // optional timeline buffer (SCAN3D_TRACE), else null
     const double2* cam_lut; const double2* proj_lut;
     const double* atan_tab;
+    const double* code_term;      // [2^max(M_v, M_h)] code*2.0*Pi per fringe order (fill_code_term_table)
     uint32_t epoch;
     int W, H, row0, H_total, PW, PH;
     int N, M_v, M_h, fw_v, fw_h;

@@ -113,13 +113,20 @@ __device__ __forceinline__ double fast_div(double num, double den)
 //   atan2 = K + s*atan(mn/mx):  (|y|<=|x|, x>=0): K=0, s=+   (|y|>|x|, x>=0): K=pi/2, s=-
 //                               (|y|<=|x|, x<0):  K=pi, s=-  (|y|>|x|, x<0):  K=pi/2, s=+
 // then the sign of y.
+// mx and mn are selected from the words of x and y; the high word goes through a float select with |.| operands, which
+// clears its sign bit in the same instruction (fabs of a double in a register costs a DADD on the FP64 pipe).  Read as
+// a float, a high word is never NaN or subnormal here (|x|, |y| lie in [2^-1000, 2^1000] or are 0).  The sign of x is
+// its high word's: x is never -0 (every caller passes an integer, or a round-to-nearest sum that starts from one, and
+// such a sum is -0 only when both of its operands are).
 __device__ __forceinline__ float atan2_to_float(double y, double x, float yf, float xf,
                                                 const double* __restrict__ tab)
 {
-    const double ax = fabs(x), ay = fabs(y);
-    const bool swap = ay > ax;
-    const bool xneg = x < 0.0;
-    const double mx = swap ? ay : ax, mn = swap ? ax : ay;
+    const bool swap = fabs(y) > fabs(x);
+    const int xh = __double2hiint(x), xl = __double2loint(x), yh = __double2hiint(y), yl = __double2loint(y);
+    const bool xneg = xh < 0;
+    const float axh = fabsf(__int_as_float(xh)), ayh = fabsf(__int_as_float(yh));
+    const double mx = __hiloint2double(__float_as_int(swap ? ayh : axh), swap ? yl : xl);
+    const double mn = __hiloint2double(__float_as_int(swap ? axh : ayh), swap ? xl : yl);
     (void)yf; (void)xf;
     // Table row i = round(32 * mn / mx) and c = i / 32, both out of ONE double: 2^47 + q has an ulp of exactly 1/32,
     // so adding q = mn * (reciprocal seed of mx) to 2^47 rounds it to a multiple of 1/32, leaves i in the low word of
@@ -288,6 +295,17 @@ __device__ __forceinline__ float unwrap_abs(float wrapped_plus_pi, int code, boo
     const double k = div_const((double)(code * 44), 7.0, K_RCP_7, fast);   // code*44 < 2^21: exact
     return __double2float_rn(dadd((double)wrapped_plus_pi, k));
 }
+// the same with k = code*2.0*Pi looked up (fill_code_term_table)
+__device__ __forceinline__ float unwrap_abs_k(float wrapped_plus_pi, double k)
+{
+    return __double2float_rn(dadd((double)wrapped_plus_pi, k));
+}
+// host side: code*2.0*Pi of every fringe order below n, in the reference's IEEE order.  The single-pass kernel loads
+// it (one cached load per pixel and direction) instead of converting the order and dividing (4 FP64 instructions).
+inline void fill_code_term_table(double* t, int n)
+{
+    for (int code = 0; code < n; code++) t[code] = (((double)code * 2.0) * 22.0) / 7.0;
+}
 // 5/compute_correspondance.cpp:648 : lrint(fw * (Phi / (2.0*Pi))), round-half-even; FE_INVALID
 // (NaN/inf/out of range) rejects the pixel.  Returns false on FE_INVALID.
 __device__ __forceinline__ bool correspond(float phi_abs, int fw, long long* out, bool fast = false)
@@ -305,6 +323,14 @@ __device__ __forceinline__ bool correspond32(float phi_abs, double fw, int* out)
     *out = __double2int_rn(v);
     return fabs(v) < 9223372036854775808.0;
 }
+// correspond32 for a phase that is known to be finite and below 2^18 in magnitude (k_fused7: 0, or
+// RN(RN(w + 22/7) + code*44/7) with w in [-pi, pi] and code < 2^15): with fw < 2^31, |v| < 2^47, so the
+// FE_INVALID test always passes and is left out.  An out-of-range v still saturates, and the caller's unsigned
+// bounds compare rejects both saturated values.
+__device__ __forceinline__ int correspond32_finite(float phi_abs, double fw)
+{
+    return __double2int_rn(dmul(fw, div_const((double)phi_abs, K_TWO_PI_REF, K_RCP_TWO_PI_REF, true)));
+}
 
 // ---------------------------------------------------------------------------------------
 // calibration algebra on the device
@@ -319,7 +345,39 @@ struct DeviceCalib {
     int cam_std;        // Kc == [fx 0 cx; 0 fy cy; 0 0 1]: the K*[x;y;1] product has exact shortcuts
     int proj_std;
     int fast_div_ok;    // host verified: the 3-operation exact quotients below equal IEEE division
+    // the fast solve in the camera's frame (triangulate_point_camframe; filled by camera_frame_calib)
+    double Apc[12];     // Ap * [Rc|tc]^-1: the projector's matrix for camera-frame points
+    double Rct[9];      // Rc^T (row-major): camera frame -> world
+    double oc[3];       // -Rc^T tc: the camera centre in the world
+    double fx2, fy2;    // Kc[0]^2, Kc[4]^2
 };
+
+// Host side: the camera-frame set-up from the camera's rotation Rc (row-major), translation tc and intrinsics Kc and
+// the projector's world matrix Ap.
+inline void camera_frame_calib(const double Kc[9], const double Rc[9], const double tc[3], const double Ap[12],
+                               DeviceCalib* d)
+{
+    for (int i = 0; i < 3; i++)
+        for (int j = 0; j < 3; j++) d->Rct[i * 3 + j] = Rc[j * 3 + i];
+    for (int i = 0; i < 3; i++) {
+        long double s = 0.0L;
+        for (int k = 0; k < 3; k++) s -= (long double)Rc[k * 3 + i] * tc[k];
+        d->oc[i] = (double)s;
+    }
+    // [Rc|tc]^-1 = [Rc^T | -Rc^T tc]
+    for (int i = 0; i < 3; i++) {
+        for (int j = 0; j < 3; j++) {
+            long double s = 0.0L;
+            for (int k = 0; k < 3; k++) s += (long double)Ap[i * 4 + k] * Rc[j * 3 + k];
+            d->Apc[i * 4 + j] = (double)s;
+        }
+        long double s = Ap[i * 4 + 3];
+        for (int k = 0; k < 3; k++) s += (long double)Ap[i * 4 + k] * d->oc[k];
+        d->Apc[i * 4 + 3] = (double)s;
+    }
+    d->fx2 = Kc[0] * Kc[0];
+    d->fy2 = Kc[4] * Kc[4];
+}
 
 // One pixel of cvUndistortPoints (5 fixed iterations, 5-coefficient model) followed by
 // K*[xn;yn;1] and the divide by the third row (7/triangulation.cpp:290-307 / :363-378).
@@ -500,6 +558,55 @@ __device__ __forceinline__ void triangulate_point_fast(const double* __restrict_
     X[0] = fma(c02, b[2], fma(c01, b[1], c00 * b[0])) * r;
     X[1] = fma(c12, b[2], fma(c11, b[1], c01 * b[0])) * r;
     X[2] = fma(c22, b[2], fma(c12, b[1], c02 * b[0])) * r;
+}
+
+// triangulate_point_fast solved in the camera's frame, for a camera matrix in the standard form (cam_std).  The
+// residuals P_i X - F_i are the same functions of the point in any frame reached by a rigid motion, so the
+// least-squares point is the same and so is the conditioning of the normal equations.  With the camera at the
+// origin, its rows become [fx, 0, cx - uc] and [0, fy, cy - vc] with F = 0: 73 FP64 operations instead of 84,
+// including the 9 that take the point back to the world frame.
+__device__ __forceinline__ void triangulate_point_camframe(const DeviceCalib& cal, double uc, double vc, double up,
+                                                           double vp, double* X)
+{
+    const double* __restrict__ A = cal.Apc;
+    const double du = cal.Kc[2] - uc, dv = cal.Kc[5] - vc;
+    double P2[3], P3[3];
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+        P2[j] = fma(-up, A[8 + j], A[0 + j]);
+        P3[j] = fma(-vp, A[8 + j], A[4 + j]);
+    }
+    const double F2 = fma(A[11], up, -A[3]);
+    const double F3 = fma(A[11], vp, -A[7]);
+#define S3D_DOT2(a, b, c0) fma(P3[a], P3[b], fma(P2[a], P2[b], c0))
+    const double S00 = S3D_DOT2(0, 0, cal.fx2), S01 = fma(P3[0], P3[1], P2[0] * P2[1]);
+    const double S02 = S3D_DOT2(0, 2, cal.Kc[0] * du);
+    const double S11 = S3D_DOT2(1, 1, cal.fy2), S12 = S3D_DOT2(1, 2, cal.Kc[4] * dv);
+    const double S22 = S3D_DOT2(2, 2, fma(dv, dv, du * du));
+#undef S3D_DOT2
+    double b[3];
+#pragma unroll
+    for (int j = 0; j < 3; j++) b[j] = fma(P3[j], F3, P2[j] * F2);
+    const double c00 = fma(S11, S22, -S12 * S12);
+    const double c01 = fma(S02, S12, -S01 * S22);
+    const double c02 = fma(S01, S12, -S02 * S11);
+    const double c11 = fma(S00, S22, -S02 * S02);
+    const double c12 = fma(S01, S02, -S00 * S12);
+    const double c22 = fma(S00, S11, -S01 * S01);
+    const double det = fma(S02, c02, fma(S01, c01, S00 * c00));
+    // one Newton step on the 20-bit seed leaves 1/det within ~2^-40 relative, far inside the mode's 1e-6 bound
+    // against the reference order (the world-frame solve above takes two)
+    double r = rcp_seed(det);
+    r = fma(r, fma(-det, r, 1.0), r);
+    const double x0 = fma(c02, b[2], fma(c01, b[1], c00 * b[0])) * r;
+    const double x1 = fma(c12, b[2], fma(c11, b[1], c01 * b[0])) * r;
+    const double x2 = fma(c22, b[2], fma(c12, b[1], c02 * b[0])) * r;
+    if (det == 0.0) {   // cvInvert returns a zero matrix for a singular input: the world origin
+        X[0] = X[1] = X[2] = 0.0;
+        return;
+    }
+#pragma unroll
+    for (int i = 0; i < 3; i++) X[i] = fma(cal.Rct[3 * i + 2], x2, fma(cal.Rct[3 * i + 1], x1, fma(cal.Rct[3 * i], x0, cal.oc[i])));
 }
 
 // ---------------------------------------------------------------------------------------
