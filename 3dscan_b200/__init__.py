@@ -91,6 +91,15 @@ class SurfaceResultC(C.Structure):
                 ("undefined_points", C.c_int64)]
 
 
+class ComponentsParams(C.Structure):
+    _fields_ = [("min_faces", C.c_int64), ("max_components", C.c_int64)]
+
+
+class ComponentsResultC(C.Structure):
+    _fields_ = [("components", C.c_int64), ("kept", C.c_int64), ("vertices", C.c_int64), ("faces", C.c_int64),
+                ("largest_faces", C.c_int64)]
+
+
 # voxel_surface's default max_points per merged voxel: the smallest power of two >= 1.5x the largest lattice points
 # per voxel measured on tools/bench_surface.py's workloads (29.2 on workload A, profiles/r3_bench_surface.json).  64 is
 # also the most a voxel can add (the 4 x 4 x 4 corners of its 27 cells), so the default never overflows; pass
@@ -220,6 +229,9 @@ def cuda_lib():
     L.scan3d_voxel_surface.argtypes = [vp, C.POINTER(SurfaceParams), C.POINTER(SurfaceResultC)]
     L.scan3d_get_voxel_surface.argtypes = [vp, vp, vp, vp, vp, i64, i64]
     L.scan3d_write_voxel_surface_ply.argtypes = [vp, C.c_char_p, i32]
+    L.scan3d_voxel_surface_components.argtypes = [vp, C.POINTER(ComponentsParams), C.POINTER(ComponentsResultC)]
+    L.scan3d_get_surface_components.argtypes = [vp, vp, vp, vp, i64]
+    L.scan3d_mesh_components_dev.argtypes = [vp, vp, i64, i64, vp, C.POINTER(i64)]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -653,6 +665,43 @@ class Scan3D:
 
     def write_voxel_surface_ply(self, path, binary=False):
         self._ck(self.L.scan3d_write_voxel_surface_ply(self.h, path.encode(), 1 if binary else 0))
+
+    # -- connected components (include/scan3d.h has the exact rules)
+    def surface_components(self, min_faces=0, max_components=0):
+        """Label the held voxel surface and keep, in place, its components with at least min_faces faces, at most
+        max_components of them (0 = no limit) by faces descending; synchronises once and returns a dict with
+        components, kept, vertices, faces and largest_faces.  voxel_surface_mesh() then returns the kept surface."""
+        p = ComponentsParams(int(min_faces), int(max_components))
+        r = ComponentsResultC()
+        self._ck(self.L.scan3d_voxel_surface_components(self.h, C.byref(p), C.byref(r)))
+        self._surface_counts = (r.vertices, r.faces)
+        self._components = r.components
+        return dict(components=r.components, kept=r.kept, vertices=r.vertices, faces=r.faces,
+                    largest_faces=r.largest_faces)
+
+    def surface_component_table(self):
+        """(vertices int64 [c], faces int64 [c], kept bool [c]) per component of the last surface_components, in id
+        order."""
+        c = getattr(self, "_components", 0)
+        v, f, k = np.empty(c, np.int64), np.empty(c, np.int64), np.empty(c, np.uint8)
+        self._ck(self.L.scan3d_get_surface_components(self.h, _ptr(v), _ptr(f), _ptr(k), c))
+        return v, f, k.astype(bool)
+
+    def mesh_components_dev(self, faces, n_vertices):
+        """Connected components of a triangle mesh on the ctx's GPU: faces is a CUDA int32 tensor [f][3].  torch's
+        current stream is synchronised first, so faces written there are ready and the new labels tensor is not in
+        use by earlier work.  Returns (labels int32 tensor [n_vertices], component count)."""
+        import torch
+        if not (isinstance(faces, torch.Tensor) and faces.is_cuda and faces.dtype == torch.int32 and faces.dim() == 2
+                and faces.shape[1] == 3):
+            raise Scan3DError("faces must be a CUDA int32 tensor of shape [f][3]")
+        faces = faces.contiguous()
+        labels = torch.empty(int(n_vertices), dtype=torch.int32, device=faces.device)
+        torch.cuda.current_stream(faces.device).synchronize()
+        n = C.c_int64()
+        self._ck(self.L.scan3d_mesh_components_dev(self.h, C.c_void_p(faces.data_ptr()), faces.shape[0],
+                                                   int(n_vertices), C.c_void_p(labels.data_ptr()), C.byref(n)))
+        return labels, n.value
 
     # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
     @staticmethod

@@ -221,7 +221,10 @@ void scan3d_destroy(scan3d_ctx* ctx)
                     ctx->aln_partials, ctx->aln_state,
                     ctx->srf.keys, ctx->srf.owner, ctx->srf.f, ctx->srf.nearest, ctx->srf.vert, ctx->srf.state,
                     ctx->srf_flags, ctx->srf_flag_counts, ctx->srf_vert_slot, ctx->srf_face_counts, ctx->srf_xyz,
-                    ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri};
+                    ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri,
+                    ctx->cc_parent, ctx->cc_flags, ctx->cc_vert_counts, ctx->cc_label, ctx->cc_comp_v, ctx->cc_comp_f,
+                    ctx->cc_kept, ctx->cc_keep_f, ctx->cc_face_counts, ctx->cc_state, ctx->cc_xyz, ctx->cc_nrm,
+                    ctx->cc_rgb, ctx->cc_tri};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
@@ -1043,7 +1046,7 @@ int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
     if (max_voxels < 1 || max_voxels >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_ARG, "max_voxels must be in [1, 2^31)");
     CK(cudaSetDevice(ctx->device));
     ctx->vox_begun = ctx->vox_fresh = false;
-    ctx->srf_ready = false;
+    ctx->srf_ready = ctx->cc_ready = false;
     VoxelTable& t = ctx->vox;
     const uint32_t cap = voxel_table_capacity((uint32_t)max_voxels, ctx->sm_count);
     if (cap > ctx->vox_alloc_cap) {
@@ -1109,7 +1112,7 @@ int scan3d_voxel_add_points(scan3d_ctx* ctx)
         return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^32 - 1 points since scan3d_voxel_begin (W*H counted per ctx add)");
     CK(cudaSetDevice(ctx->device));
     ctx->vox_bound += ub;
-    ctx->vox_fresh = ctx->srf_ready = false;
+    ctx->vox_fresh = ctx->srf_ready = ctx->cc_ready = false;
     return voxel_add(ctx, points_of(ctx), ctx->have_mesh ? ctx->mesh_normals : nullptr,
                      ctx->texture && ctx->rgb ? ctx->rgb : nullptr, ctx->d_count, (uint32_t)ub);
 }
@@ -1127,7 +1130,7 @@ int scan3d_voxel_add_points_dev(scan3d_ctx* ctx, const float* xyz_dev, const flo
         return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^32 - 1 points since scan3d_voxel_begin");
     CK(cudaSetDevice(ctx->device));
     ctx->vox_bound += (uint64_t)n;
-    ctx->vox_fresh = ctx->srf_ready = false;
+    ctx->vox_fresh = ctx->srf_ready = ctx->cc_ready = false;
     const int64_t chunk = (int64_t)npix(ctx);   // the per-point scratch holds W*H points
     for (int64_t off = 0; off < n; off += chunk) {
         const int64_t k = std::min(chunk, n - off);
@@ -1147,7 +1150,7 @@ int scan3d_voxel_finish(scan3d_ctx* ctx)
                            ctx->sm_count, ctx->stream));
     ctx->launches += 1;
     ctx->vox_fresh = true;
-    ctx->srf_ready = false;
+    ctx->srf_ready = ctx->cc_ready = false;
     return SCAN3D_OK;
 }
 
@@ -1352,7 +1355,7 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
     if (!ctx->vox_begun || !ctx->vox_fresh)
         return fail(ctx, SCAN3D_ERR_STATE, "no voxel outputs of the current adds to mesh: call scan3d_voxel_finish");
     CK(cudaSetDevice(ctx->device));
-    ctx->srf_ready = false;
+    ctx->srf_ready = ctx->cc_ready = false;
     AlignRun run{};                                      // the index only; T0 = I for the state it initialises
     run.T0[0] = run.T0[5] = run.T0[10] = 1.0;
     run.S = s3l::cell_edge(p->max_distance);
@@ -1475,6 +1478,151 @@ int scan3d_write_voxel_surface_ply(scan3d_ctx* ctx, const char* path, int binary
     write_ply_with_faces(f, binary, nv, xyz.data(), nrm.data(), rgb.data(), nf, faces.data());
     const bool ok = fclose(f) == 0;
     return ok ? SCAN3D_OK : fail(ctx, SCAN3D_ERR_IO, "PLY write failed");
+}
+
+// ------------------------------------------------------------------------------------------
+// connected components of a triangle mesh (include/scan3d.h has the exact rules)
+// ------------------------------------------------------------------------------------------
+// the labelling scratch for n vertices: parent, root flags, their block offsets, the device state
+static int cc_label_scratch(scan3d_ctx* ctx, int64_t n)
+{
+    n = std::max<int64_t>(n, 1);
+    if (n > ctx->cc_alloc_label) {
+        free_ptr(ctx->cc_parent); free_ptr(ctx->cc_flags); free_ptr(ctx->cc_vert_counts);
+        ctx->cc_parent = ctx->cc_vert_counts = nullptr; ctx->cc_flags = nullptr;
+        ctx->cc_alloc_label = 0;
+        CK(dalloc(&ctx->cc_parent, (size_t)n));
+        CK(dalloc(&ctx->cc_flags, (size_t)n));
+        CK(dalloc(&ctx->cc_vert_counts, (size_t)(n + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+        ctx->cc_alloc_label = n;
+    }
+    if (!ctx->cc_state) CK(dalloc(&ctx->cc_state, 1));
+    CK(cudaMemsetAsync(ctx->cc_state, 0, sizeof(ComponentsState), ctx->stream));
+    return SCAN3D_OK;
+}
+
+int scan3d_voxel_surface_components(scan3d_ctx* ctx, const scan3d_components_params* p, scan3d_components_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!p || !out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (p->min_faces < 0 || p->max_components < 0) return fail(ctx, SCAN3D_ERR_ARG, "min_faces and max_components must be >= 0");
+    if (!ctx->srf_ready)
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    CK(cudaSetDevice(ctx->device));
+    ctx->cc_ready = false;
+    const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
+    int rc = cc_label_scratch(ctx, nv);
+    if (rc) return rc;
+    const int64_t av = std::max<int64_t>(nv, 1), af = std::max<int64_t>(nf, 1);
+    if (av > ctx->cc_alloc_v) {
+        free_ptr(ctx->cc_label); free_ptr(ctx->cc_comp_v); free_ptr(ctx->cc_comp_f); free_ptr(ctx->cc_kept);
+        ctx->cc_label = nullptr; ctx->cc_comp_v = ctx->cc_comp_f = nullptr; ctx->cc_kept = nullptr;
+        ctx->cc_alloc_v = 0;
+        CK(dalloc(&ctx->cc_label, (size_t)av));
+        CK(dalloc(&ctx->cc_comp_v, (size_t)av));
+        CK(dalloc(&ctx->cc_comp_f, (size_t)av));
+        CK(dalloc(&ctx->cc_kept, (size_t)av));
+        ctx->cc_alloc_v = av;
+    }
+    if (af > ctx->cc_alloc_f) {
+        free_ptr(ctx->cc_keep_f); free_ptr(ctx->cc_face_counts);
+        ctx->cc_keep_f = nullptr; ctx->cc_face_counts = nullptr;
+        ctx->cc_alloc_f = 0;
+        CK(dalloc(&ctx->cc_keep_f, (size_t)af));
+        CK(dalloc(&ctx->cc_face_counts, (size_t)(af + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+        ctx->cc_alloc_f = af;
+    }
+    CK(cudaMemsetAsync(ctx->cc_comp_v, 0, (size_t)nv * sizeof(uint32_t), ctx->stream));
+    CK(cudaMemsetAsync(ctx->cc_comp_f, 0, (size_t)nv * sizeof(uint32_t), ctx->stream));
+    CK(launch_cc_labels(ctx->srf_tri, (uint32_t)nf, (uint32_t)nv, ctx->cc_parent, ctx->cc_flags, ctx->cc_vert_counts,
+                        ctx->cc_label, ctx->cc_state, ctx->stream));
+    CK(launch_cc_select(ctx->srf_tri, (uint32_t)nf, (uint32_t)nv, ctx->cc_label, (unsigned long long)p->min_faces,
+                        (unsigned long long)p->max_components, ctx->cc_comp_v, ctx->cc_comp_f, ctx->cc_kept,
+                        ctx->cc_flags, ctx->cc_keep_f, ctx->cc_vert_counts, ctx->cc_face_counts, ctx->cc_state,
+                        ctx->stream));
+    ctx->launches += COMPONENT_LABEL_LAUNCHES + COMPONENT_SELECT_LAUNCHES;
+    ComponentsState st;
+    CK(cudaMemcpyAsync(&st, ctx->cc_state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st.vertices > ctx->cc_out_alloc_v) {
+        free_ptr(ctx->cc_xyz); free_ptr(ctx->cc_nrm); free_ptr(ctx->cc_rgb);
+        ctx->cc_xyz = ctx->cc_nrm = nullptr; ctx->cc_rgb = nullptr;
+        ctx->cc_out_alloc_v = 0;
+        CK(dalloc(&ctx->cc_xyz, 3 * (size_t)st.vertices));
+        CK(dalloc(&ctx->cc_nrm, 3 * (size_t)st.vertices));
+        CK(dalloc(&ctx->cc_rgb, 3 * (size_t)st.vertices));
+        ctx->cc_out_alloc_v = st.vertices;
+    }
+    if (st.faces > ctx->cc_out_alloc_f) {
+        free_ptr(ctx->cc_tri);
+        ctx->cc_tri = nullptr;
+        ctx->cc_out_alloc_f = 0;
+        CK(dalloc(&ctx->cc_tri, 3 * (size_t)st.faces));
+        ctx->cc_out_alloc_f = st.faces;
+    }
+    CK(launch_cc_emit(ctx->cc_flags, ctx->cc_vert_counts, (uint32_t)nv, ctx->srf_xyz, ctx->srf_nrm, ctx->srf_rgb,
+                      ctx->cc_keep_f, ctx->cc_face_counts, (uint32_t)nf, ctx->srf_tri, ctx->cc_label, ctx->cc_xyz,
+                      ctx->cc_nrm, ctx->cc_rgb, ctx->cc_tri, ctx->stream));
+    ctx->launches += COMPONENT_EMIT_LAUNCHES;
+    // the compacted set becomes the held surface; the old one is the next compaction's destination
+    std::swap(ctx->srf_xyz, ctx->cc_xyz);
+    std::swap(ctx->srf_nrm, ctx->cc_nrm);
+    std::swap(ctx->srf_rgb, ctx->cc_rgb);
+    std::swap(ctx->srf_tri, ctx->cc_tri);
+    std::swap(ctx->srf_alloc_v, ctx->cc_out_alloc_v);
+    std::swap(ctx->srf_alloc_f, ctx->cc_out_alloc_f);
+    ctx->srf_vertices = st.vertices;
+    ctx->srf_faces = st.faces;
+    ctx->cc_components = st.components;
+    ctx->cc_ready = true;
+    out->components = st.components;
+    out->kept = st.kept;
+    out->vertices = st.vertices;
+    out->faces = st.faces;
+    out->largest_faces = st.largest;
+    return SCAN3D_OK;
+}
+
+int scan3d_get_surface_components(scan3d_ctx* ctx, int64_t* vertices, int64_t* faces, uint8_t* kept,
+                                  int64_t max_components)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!ctx->cc_ready)
+        return fail(ctx, SCAN3D_ERR_STATE, "no component table of the held surface: call scan3d_voxel_surface_components");
+    CK(cudaSetDevice(ctx->device));
+    const int64_t n = std::max<int64_t>(0, std::min(ctx->cc_components, max_components));
+    std::vector<uint32_t> v(vertices ? n : 0), f(faces ? n : 0);
+    if (vertices && n) CK(cudaMemcpyAsync(v.data(), ctx->cc_comp_v, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (faces && n) CK(cudaMemcpyAsync(f.data(), ctx->cc_comp_f, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (kept && n) CK(cudaMemcpyAsync(kept, ctx->cc_kept, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    for (int64_t c = 0; vertices && c < n; c++) vertices[c] = v[c];
+    for (int64_t c = 0; faces && c < n; c++) faces[c] = f[c];
+    return SCAN3D_OK;
+}
+
+int scan3d_mesh_components_dev(scan3d_ctx* ctx, const int32_t* faces_dev, int64_t n_faces, int64_t n_vertices,
+                               int32_t* label_dev, int64_t* components_out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!components_out) return fail(ctx, SCAN3D_ERR_ARG, "null components_out");
+    if (n_faces < 0 || n_faces >= (1LL << 31) || n_vertices < 0 || n_vertices >= (1LL << 31))
+        return fail(ctx, SCAN3D_ERR_ARG, "n_faces and n_vertices must be in [0, 2^31)");
+    if ((!faces_dev && n_faces > 0) || (!label_dev && n_vertices > 0)) return fail(ctx, SCAN3D_ERR_ARG, "null device pointer");
+    if (((uintptr_t)faces_dev & 3) || ((uintptr_t)label_dev & 3))
+        return fail(ctx, SCAN3D_ERR_ARG, "faces_dev and label_dev must be 4-byte aligned");
+    CK(cudaSetDevice(ctx->device));
+    const int rc = cc_label_scratch(ctx, n_vertices);
+    if (rc) return rc;
+    CK(launch_cc_labels(faces_dev, (uint32_t)n_faces, (uint32_t)n_vertices, ctx->cc_parent, ctx->cc_flags,
+                        ctx->cc_vert_counts, label_dev, ctx->cc_state, ctx->stream));
+    ctx->launches += COMPONENT_LABEL_LAUNCHES;
+    ComponentsState st;
+    CK(cudaMemcpyAsync(&st, ctx->cc_state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st.bad) return fail(ctx, SCAN3D_ERR_ARG, "a face index outside [0, n_vertices)");
+    *components_out = st.components;
+    return SCAN3D_OK;
 }
 
 // ------------------------------------------------------------------------------------------

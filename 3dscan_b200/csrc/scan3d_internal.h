@@ -91,6 +91,16 @@ struct SurfaceTable {
     uint32_t cap, max_points;
     double S;                      // (double)voxel_size
 };
+
+// the connected components of a triangle mesh (scan3d_components_kernels.cu)
+struct ComponentsState {
+    unsigned long long threshold;  // K of the keep rule: component c is kept when eligible and its key is >= K
+    uint32_t components;           // of the mesh
+    uint32_t kept, largest;        // components kept; the most faces of one component
+    uint32_t vertices, faces;      // kept
+    uint32_t bad;                  // a face index outside [0, vertices)
+    uint32_t pad;
+};
 }  // namespace s3d
 
 struct scan3d_ctx {
@@ -193,6 +203,27 @@ struct scan3d_ctx {
     uint8_t* srf_rgb = nullptr;           // [vertices][3]
     int32_t* srf_tri = nullptr;           // [faces][3]
 
+    // scan3d_voxel_surface_components / scan3d_mesh_components_dev (allocated on first use, grown on demand)
+    bool cc_ready = false;                // the component table of the last scan3d_voxel_surface_components is held
+    int64_t cc_components = 0;
+    int64_t cc_alloc_label = 0;           // vertices the labelling scratch holds
+    int64_t cc_alloc_v = 0, cc_alloc_f = 0;   // vertices and faces the table, keep flags and block counts hold
+    uint32_t* cc_parent = nullptr;        // [vertices] union-find forest, then each vertex's root
+    uint8_t* cc_flags = nullptr;          // [vertices] root flags, then the vertices' keep flags
+    uint32_t* cc_vert_counts = nullptr;   // [cdiv(vertices, POINT_BLOCK) + 1] block offsets of the flags
+    int32_t* cc_label = nullptr;          // [vertices] component ids, then the kept vertices' new indices
+    uint32_t* cc_comp_v = nullptr;        // [vertices] per component: vertices, faces, kept flag
+    uint32_t* cc_comp_f = nullptr;
+    uint8_t* cc_kept = nullptr;
+    uint8_t* cc_keep_f = nullptr;         // [faces]
+    uint32_t* cc_face_counts = nullptr;   // [cdiv(faces, POINT_BLOCK) + 1]
+    s3d::ComponentsState* cc_state = nullptr;
+    int64_t cc_out_alloc_v = 0, cc_out_alloc_f = 0;   // the second surface set, swapped with srf_* after a compaction
+    float* cc_xyz = nullptr;
+    float* cc_nrm = nullptr;
+    uint8_t* cc_rgb = nullptr;
+    int32_t* cc_tri = nullptr;
+
     int cta_limit = 0;             // scan3d_set_cta_limit
 
     // scan3d_set_registration
@@ -245,7 +276,7 @@ cudaError_t launch_triangulate(const Shape& s, const DeviceCalib& cal, const dou
 cudaError_t launch_undistort_lut(const double* K9_k5_dev_unused, const DeviceCalib& cal, bool projector,
                                  int W, int H, int row0, double2* lut, cudaStream_t st);
 // Raster-order point offsets of the valid plane, 2 launches (k_count, k_scan): block_counts[b] = number of valid
-// pixels before block b of POINT_BLOCK pixels, *total = all of them.
+// pixels before block b of POINT_BLOCK pixels, *total = all of them.  An empty plane takes one block (total 0).
 constexpr int POINT_BLOCK = 1024;
 cudaError_t launch_point_offsets(const uint8_t* valid, size_t plane, uint32_t* block_counts, uint32_t* total,
                                  cudaStream_t st);
@@ -363,6 +394,30 @@ cudaError_t launch_surface_emit(const SurfaceTable& s, const uint8_t* vox_rgb, c
                                 int32_t* faces, cudaStream_t st);
 // slots of the lattice table for max_points: at most half of them are ever taken
 uint32_t surface_table_capacity(uint32_t max_points, int sm_count);
+
+// ---- connected components of a triangle mesh (scan3d_components_kernels.cu) ----
+// launch_cc_labels: COMPONENT_LABEL_LAUNCHES launches for n vertices and n_faces faces [n_faces][3]: parent = v,
+// union per face, find per vertex with the root flags, k_count + k_scan over them (state->components), the roots' ids,
+// every vertex's id into label [n].  state must be zeroed before; parent and flags [n], block_counts [cdiv(n,
+// POINT_BLOCK) + 1].  Any n below 2^31 and n_faces below 2^32, 0 included.
+// launch_cc_select: COMPONENT_SELECT_LAUNCHES launches after it: vertices and faces per component (comp_v, comp_f [n],
+// zeroed before), the selection (state->threshold, kept, largest), the keep flags (keep_v [n], keep_f [n_faces], kept
+// [components]), k_count + k_scan over each of keep_v (state->vertices) and keep_f (state->faces).
+// launch_cc_emit: COMPONENT_EMIT_LAUNCHES launches: the kept vertices into xyz2 / nrm2 / rgb2 (their new indices into
+// new_index [n]), then the kept faces, remapped, into faces2.
+constexpr int COMPONENT_LABEL_LAUNCHES = 7;
+constexpr int COMPONENT_SELECT_LAUNCHES = 7;
+constexpr int COMPONENT_EMIT_LAUNCHES = 2;
+cudaError_t launch_cc_labels(const int32_t* faces, uint32_t n_faces, uint32_t n, uint32_t* parent, uint8_t* flags,
+                             uint32_t* block_counts, int32_t* label, ComponentsState* state, cudaStream_t st);
+cudaError_t launch_cc_select(const int32_t* faces, uint32_t n_faces, uint32_t n, const int32_t* label,
+                             unsigned long long min_faces, unsigned long long max_components, uint32_t* comp_v,
+                             uint32_t* comp_f, uint8_t* kept, uint8_t* keep_v, uint8_t* keep_f, uint32_t* vert_counts,
+                             uint32_t* face_counts, ComponentsState* state, cudaStream_t st);
+cudaError_t launch_cc_emit(const uint8_t* keep_v, const uint32_t* vert_counts, uint32_t n, const float* xyz,
+                           const float* nrm, const uint8_t* rgb, const uint8_t* keep_f, const uint32_t* face_counts,
+                           uint32_t n_faces, const int32_t* faces, int32_t* new_index, float* xyz2, float* nrm2,
+                           uint8_t* rgb2, int32_t* faces2, cudaStream_t st);
 
 // ---- debug / self-test ----
 cudaError_t launch_debug_atan2(const double* y, const double* x, float* out, int n, int mode,

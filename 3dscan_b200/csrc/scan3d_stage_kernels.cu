@@ -413,7 +413,7 @@ __global__ void k_scatter(const double* __restrict__ xyz, const uint8_t* __restr
 cudaError_t launch_point_offsets(const uint8_t* valid, size_t plane, uint32_t* block_counts, uint32_t* total,
                                  cudaStream_t st)
 {
-    const int nb = (int)cdiv((long)plane, CB);
+    const int nb = plane ? (int)cdiv((long)plane, CB) : 1;
     k_count<<<nb, CB, 0, st>>>(valid, block_counts, plane);
     k_scan<<<1, 1024, 0, st>>>(block_counts, nb, total);
     return cudaGetLastError();

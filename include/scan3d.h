@@ -441,6 +441,66 @@ int scan3d_get_voxel_surface(scan3d_ctx *ctx, float *xyz, float *normals, uint8_
 /* the vertex element of scan3d_write_mesh_ply plus its face element; ascii (%.9g) or binary_little_endian */
 int scan3d_write_voxel_surface_ply(scan3d_ctx *ctx, const char *path, int binary);
 
+/* ---- connected components of a triangle mesh; removal of the small pieces of the surface ----------------
+ * Component: two vertices are connected when some face contains both; a face connects its three vertices (a degenerate
+ * face such as (a, a, b) is allowed).  A vertex that no face uses is a component by itself, with 0 faces.  A face
+ * belongs to the component of its vertices.
+ * Component id: components are ranked by their smallest vertex index (the component of vertex 0 has id 0).  The labels
+ * are a pure function of the faces and the vertex count: they do not depend on scheduling or on the SM count.
+ * Keep rule (min_faces >= 0, max_components >= 0, 0 = no limit): of the components with at least min_faces faces, the
+ * first max_components ranked by faces in descending order, ties going to the smaller id.  (0, 0) keeps everything;
+ * min_faces = 1 drops the vertices that no face uses.
+ * Compaction: kept vertices keep their relative order and their xyz, normal and rgb bytes; kept faces keep their
+ * relative order with their indices remapped to the new vertex positions: new = cumsum(keep_v) - 1,
+ * faces = new[faces[keep_f]].
+ * Method: a lock-free union-find (ECL-CC: atomicCAS links the larger root under the smaller, finds halve the path), so
+ * every root is its component's smallest vertex; the roots ranked by k_count + k_scan give the ids.  Counts per
+ * component are integer atomics and the selection is an integer radix select, so every result is bit-reproducible.
+ * scan3d_voxel_surface_components labels the held voxel surface, then replaces it in place by its kept components:
+ * scan3d_get_voxel_surface and scan3d_write_voxel_surface_ply then return the cleaned surface, and a second call with
+ * the same parameters changes nothing.  It needs a held surface (SCAN3D_ERR_STATE otherwise).  A later
+ * scan3d_voxel_surface, begin, add or finish makes the component table stale (scan3d_get_surface_components then
+ * returns SCAN3D_ERR_STATE); the staleness of the surface itself is unchanged; an align changes neither the surface nor
+ * the table; the accumulator is never touched.
+ * scan3d_mesh_components_dev labels any triangle mesh in device memory of the ctx's GPU (faces int32 [n_faces][3],
+ * labels int32 [n_vertices]), ordered on the ctx stream; it leaves the held surface and the table alone.
+ * Synchronisation: one per entry.  scan3d_voxel_surface_components synchronises once the counts, the selection and
+ * the kept totals are known; *out is then filled and the compaction is queued asynchronously.
+ * Launches: scan3d_mesh_components_dev always 7 (parent = v, one union per face, find per vertex with the root flags,
+ * their k_count + k_scan, the roots' ids, every vertex's id).  scan3d_voxel_surface_components always 16, even for
+ * (0, 0): those 7, then the counts per component, the selection, the keep flags, k_count + k_scan over the vertex
+ * flags and over the face flags before the synchronisation, and 2 after it (kept vertices, kept faces).  With (0, 0)
+ * the surface's bytes are unchanged.
+ * Memory (ctx-owned, allocated on first use, grown on demand): 18 B per vertex and 1 B per face of scratch and
+ * component table, plus a second surface set of 27 B per kept vertex and 12 B per kept face that is swapped with the
+ * held one.
+ * Errors: SCAN3D_ERR_ARG for a null ctx, params, result or components_out; faces_dev NULL with n_faces > 0 or
+ * label_dev NULL with n_vertices > 0; a negative min_faces or max_components; n_faces or n_vertices outside
+ * [0, 2^31); device pointers not 4-byte aligned; and in scan3d_mesh_components_dev a face index outside
+ * [0, n_vertices), which is found on the device and reported at the synchronisation (the labels are then
+ * unspecified).  An argument or state error launches nothing and leaves the surface as it was. */
+typedef struct {
+    int64_t min_faces;       /* >= 0 */
+    int64_t max_components;  /* >= 0, 0 = no limit */
+} scan3d_components_params;
+
+typedef struct {
+    int64_t components;      /* of the surface as it was when the call began */
+    int64_t kept;            /* components kept */
+    int64_t vertices, faces; /* of the surface after the call */
+    int64_t largest_faces;   /* faces of the component with the most, 0 for an empty surface */
+} scan3d_components_result;
+
+/* labels the held voxel surface, then replaces it in place by its kept components */
+int scan3d_voxel_surface_components(scan3d_ctx *ctx, const scan3d_components_params *p, scan3d_components_result *out);
+/* per component of the last call, in id order: vertex count, face count, kept flag of the first
+ * min(components, max_components); any pointer may be NULL; syncs */
+int scan3d_get_surface_components(scan3d_ctx *ctx, int64_t *vertices, int64_t *faces, uint8_t *kept,
+                                  int64_t max_components);
+/* labels of any triangle mesh in device memory of the ctx's GPU, ordered on the ctx stream; syncs once */
+int scan3d_mesh_components_dev(scan3d_ctx *ctx, const int32_t *faces_dev, int64_t n_faces, int64_t n_vertices,
+                               int32_t *label_dev, int64_t *components_out);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,

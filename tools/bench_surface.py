@@ -115,30 +115,51 @@ def run(name, ctx, views, voxel):
     return out
 
 
-c = scaled_calib(load_calib_c1(), W / 1600.0, PW / 1280.0)
-cal = s3.make_calib(*[c[k] for k in ("Kc", "dc", "Kp", "dp", "rc", "tc", "rp", "tp")])
-cfg = s3.make_config(W, H, PW, PH, 8, 10, 10, 4, 4, 2, flags=s3.FLAG_FAST_TRIANGULATION)
-params = s3.default_synth_params(seed=0x3D5CA9)
-stack, roi, truth = s3.synth_stack(cfg, cal, params, want_truth=True)
-stream = torch.cuda.Stream()
-ctx = s3.Scan3D(cfg, 0, cal, stream=stream.cuda_stream)
-ctx.set_texture(np.random.default_rng(0x3D5CA9).integers(0, 256, (H, W, 3), dtype=np.uint8))
+def setup():
+    """the ctx on its own stream and the c3 scan (stack, roi, truth, synth params) both workloads are captured from"""
+    global stream
+    c = scaled_calib(load_calib_c1(), W / 1600.0, PW / 1280.0)
+    cal = s3.make_calib(*[c[k] for k in ("Kc", "dc", "Kp", "dp", "rc", "tc", "rp", "tp")])
+    cfg = s3.make_config(W, H, PW, PH, 8, 10, 10, 4, 4, 2, flags=s3.FLAG_FAST_TRIANGULATION)
+    params = s3.default_synth_params(seed=0x3D5CA9)
+    stack, roi, truth = s3.synth_stack(cfg, cal, params, want_truth=True)
+    stream = torch.cuda.Stream()
+    ctx = s3.Scan3D(cfg, 0, cal, stream=stream.cuda_stream)
+    ctx.set_texture(np.random.default_rng(0x3D5CA9).integers(0, 256, (H, W, 3), dtype=np.uint8))
+    return ctx, stack, roi, truth, params
 
-name, plim = gpu_info()
-result = dict(kernel="scan3d_voxel_surface (R = 2 voxels) + stream synchronise",
-              scan="4096x3000 c3 synthetic scan, 8-step, 10+10 bits, fast triangulation, seed 0x3D5CA9, texture, mesh",
-              gpu=name, power_limit=plim)
-views = capture_views(ctx, stack, roi, [45.0 * k for k in range(8)])
-ctx.set_registration(True, 0.0, *CENTRE)
-ctx.reconstruct(stack, roi)
-voxel = 2.0 * median_spacing(ctx, views[0][0])
-result["A"] = run("A: 8 whole views at 45 deg", ctx, views, voxel)
-del views
-torch.cuda.synchronize()
-on_sphere = np.abs(np.linalg.norm(truth.astype(np.float64) - np.array(CENTRE), axis=2) - params.sphere_r) < 1e-3
-roi_b = (roi * on_sphere).astype(np.uint8)
-views = capture_views(ctx, stack, roi_b, [10.0 * k for k in range(36)])
-del stack, truth
-result["B"] = run("B: 36 sphere-only views at 10 deg", ctx, views, voxel)
-print(json.dumps(result, indent=1), flush=True)
-ctx.close()
+
+def workload_a(ctx, stack, roi):
+    """(views, voxel size) of workload A"""
+    views = capture_views(ctx, stack, roi, [45.0 * k for k in range(8)])
+    ctx.set_registration(True, 0.0, *CENTRE)
+    ctx.reconstruct(stack, roi)
+    return views, 2.0 * median_spacing(ctx, views[0][0])
+
+
+def workload_b(ctx, stack, roi, truth, params):
+    """views of workload B (the voxel size is A's)"""
+    on_sphere = np.abs(np.linalg.norm(truth.astype(np.float64) - np.array(CENTRE), axis=2) - params.sphere_r) < 1e-3
+    roi_b = (roi * on_sphere).astype(np.uint8)
+    return capture_views(ctx, stack, roi_b, [10.0 * k for k in range(36)])
+
+
+def main():
+    ctx, stack, roi, truth, params = setup()
+    name, plim = gpu_info()
+    result = dict(kernel="scan3d_voxel_surface (R = 2 voxels) + stream synchronise",
+                  scan="4096x3000 c3 synthetic scan, 8-step, 10+10 bits, fast triangulation, seed 0x3D5CA9, texture, mesh",
+                  gpu=name, power_limit=plim)
+    views, voxel = workload_a(ctx, stack, roi)
+    result["A"] = run("A: 8 whole views at 45 deg", ctx, views, voxel)
+    del views
+    torch.cuda.synchronize()
+    views = workload_b(ctx, stack, roi, truth, params)
+    del stack, truth
+    result["B"] = run("B: 36 sphere-only views at 10 deg", ctx, views, voxel)
+    print(json.dumps(result, indent=1), flush=True)
+    ctx.close()
+
+
+if __name__ == "__main__":
+    main()
