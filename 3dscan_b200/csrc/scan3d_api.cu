@@ -20,28 +20,7 @@ using namespace s3d;
 
 static thread_local std::string g_create_error;
 
-#define CK(call)                                                                          \
-    do {                                                                                  \
-        cudaError_t e_ = (call);                                                          \
-        if (e_ != cudaSuccess) {                                                          \
-            ctx->err = std::string(#call) + ": " + cudaGetErrorString(e_);                \
-            return SCAN3D_ERR_CUDA;                                                       \
-        }                                                                                 \
-    } while (0)
-
-static int fail(scan3d_ctx* ctx, int code, const char* msg)
-{
-    if (ctx) ctx->err = msg;
-    return code;
-}
-
 static size_t npix(const scan3d_ctx* c) { return (size_t)c->cfg.W * c->cfg.H; }
-
-template <class T>
-static cudaError_t dalloc(T** p, size_t n)
-{
-    return cudaMalloc((void**)p, n * sizeof(T));
-}
 
 // ---- host-side calibration algebra (once per calibration; 7/triangulation.cpp:1061-1126) ----
 static void rodrigues_host(const double r[3], double R[9])
@@ -139,37 +118,37 @@ int scan3d_create(const scan3d_config* cfg, int device, scan3d_ctx** out)
         const size_t n = npix(ctx);
         const int D = cfg->dirs;
         for (int d = 0; d < D; d++) {
-            CK(dalloc(&ctx->unwrapped[d], n));
-            CK(dalloc(&ctx->code[d], n));
+            CK(ctx->unwrapped[d].ensure(n));
+            CK(ctx->code[d].ensure(n));
         }
-        CK(dalloc(&ctx->mask[0], n));
-        CK(dalloc(&ctx->valid, n));
+        CK(ctx->mask[0].ensure(n));
+        CK(ctx->valid.ensure(n));
         if (D == 2) {
-            CK(dalloc(&ctx->cpmap, n));
-            CK(dalloc(&ctx->pts, 3 * n));
-            if (cfg->flags & SCAN3D_FLAG_POINT_PIXELS) CK(dalloc(&ctx->pix, n));
+            CK(ctx->cpmap.ensure(n));
+            CK(ctx->pts.ensure(3 * n));
+            if (cfg->flags & SCAN3D_FLAG_POINT_PIXELS) CK(ctx->pix.ensure(n));
         }
-        CK(dalloc(&ctx->d_count, 4));
+        CK(ctx->d_count.ensure(4));
         CK(cudaMemsetAsync(ctx->d_count, 0, 16, ctx->stream));
         const int ntiles = fused_num_tiles(ctx->cfg);
-        CK(dalloc(&ctx->tile_state, (size_t)ntiles + 1));
+        CK(ctx->tile_state.ensure((size_t)ntiles + 1));
         CK(cudaMemsetAsync(ctx->tile_state, 0, ((size_t)ntiles + 1) * 8, ctx->stream));
         if (getenv("SCAN3D_TRACE")) {
-            CK(dalloc(&ctx->trace, (size_t)1024 * 64 * 8));
+            CK(ctx->trace.ensure((size_t)1024 * 64 * 8));
             CK(cudaMemsetAsync(ctx->trace, 0, (size_t)1024 * 64 * 8 * 8, ctx->stream));
         }
-        CK(dalloc(&ctx->tile_flags, (size_t)ntiles + 16));
-        CK(dalloc(&ctx->tile_list, (size_t)ntiles + 16));
-        CK(dalloc(&ctx->atan_tab, (size_t)ATAN_TAB_DOUBLES));
+        CK(ctx->tile_flags.ensure((size_t)ntiles + 16));
+        CK(ctx->tile_list.ensure((size_t)ntiles + 16));
+        CK(ctx->atan_tab.ensure((size_t)ATAN_TAB_DOUBLES));
         double tab[ATAN_TAB_DOUBLES];
         fill_atan_table(tab);
         CK(cudaMemcpyAsync(ctx->atan_tab, tab, sizeof(tab), cudaMemcpyHostToDevice, ctx->stream));
         const int n_codes = 1 << (cfg->dirs == 2 && cfg->M_h > cfg->M_v ? cfg->M_h : cfg->M_v);
         std::vector<double> code_term(n_codes);
         fill_code_term_table(code_term.data(), n_codes);
-        CK(dalloc(&ctx->code_term, (size_t)n_codes));
+        CK(ctx->code_term.ensure((size_t)n_codes));
         CK(cudaMemcpyAsync(ctx->code_term, code_term.data(), n_codes * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        CK(dalloc(&ctx->nstep_w, 128));
+        CK(ctx->nstep_w.ensure(128));
         double w[128];
         memset(w, 0, sizeof(w));
         for (int k = 0; k < cfg->N && k < 64; k++) {
@@ -208,27 +187,10 @@ void scan3d_destroy(scan3d_ctx* ctx)
 {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    if (ctx->own_stream) cudaStreamSynchronize(ctx->own_stream);
-    void* ptrs[] = {ctx->cam_lut, ctx->proj_lut, ctx->atan_tab, ctx->code_term, ctx->nstep_w, ctx->wrapped[0], ctx->wrapped[1],
-                    ctx->unwrapped[0], ctx->unwrapped[1], ctx->code[0], ctx->code[1], ctx->mask[0],
-                    ctx->mask[1], ctx->valid, ctx->cpmap, ctx->xyz, ctx->pts, ctx->pix, ctx->rgb,
-                    ctx->texture, ctx->d_count, ctx->block_counts, ctx->tile_state, ctx->tile_flags, ctx->tile_list, ctx->trace, ctx->d_stack, ctx->d_roi, ctx->d_undist, ctx->roi_eff, ctx->roi_eff_h, ctx->roi_strict, ctx->pattern_profiles,
-                    ctx->undist_xy[0], ctx->undist_xy[1], ctx->undist_frac[0], ctx->undist_frac[1],
-                    ctx->mesh_idx, ctx->mesh_counts, ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals,
-                    ctx->vox.keys, ctx->vox.acc, ctx->vox.ordinal, ctx->vox.ord2slot, ctx->vox.state,
-                    ctx->vox_point_slot, ctx->vox_flags, ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb, ctx->vox_cnt,
-                    ctx->aln.keys, ctx->aln.cells, ctx->aln.model_slot, ctx->aln.entries, ctx->aln.cursor,
-                    ctx->aln_partials, ctx->aln_state,
-                    ctx->srf.keys, ctx->srf.owner, ctx->srf.f, ctx->srf.nearest, ctx->srf.vert, ctx->srf.state,
-                    ctx->srf_flags, ctx->srf_flag_counts, ctx->srf_vert_slot, ctx->srf_face_counts, ctx->srf_xyz,
-                    ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri,
-                    ctx->cc_parent, ctx->cc_flags, ctx->cc_vert_counts, ctx->cc_label, ctx->cc_comp_v, ctx->cc_comp_f,
-                    ctx->cc_kept, ctx->cc_keep_f, ctx->cc_face_counts, ctx->cc_state, ctx->cc_xyz, ctx->cc_nrm,
-                    ctx->cc_rgb, ctx->cc_tri};
-    for (void* p : ptrs)
-        if (p) cudaFree(p);
-    if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
-    delete ctx;
+    const cudaStream_t own = ctx->own_stream;
+    if (own) cudaStreamSynchronize(own);
+    delete ctx;                                   // frees every buffer, before their stream goes
+    if (own) cudaStreamDestroy(own);
 }
 
 int scan3d_set_stream(scan3d_ctx* ctx, void* cuda_stream)
@@ -279,22 +241,22 @@ int scan3d_set_calibration(scan3d_ctx* ctx, const scan3d_calib* cal)
         if (cal->dc[i] != 0.0) d.cam_distorted = 1;
         if (cal->dp[i] != 0.0) d.proj_distorted = 1;
     }
-    if (ctx->cam_lut) { cudaFree(ctx->cam_lut); ctx->cam_lut = nullptr; }
-    if (ctx->proj_lut) { cudaFree(ctx->proj_lut); ctx->proj_lut = nullptr; }
+    ctx->cam_lut.release();
+    ctx->proj_lut.release();
     for (int k = 0; k < 2; k++) {   // cv::undistort maps belong to the previous calibration
-        if (ctx->undist_xy[k]) { cudaFree(ctx->undist_xy[k]); ctx->undist_xy[k] = nullptr; }
-        if (ctx->undist_frac[k]) { cudaFree(ctx->undist_frac[k]); ctx->undist_frac[k] = nullptr; }
+        ctx->undist_xy[k].release();
+        ctx->undist_frac[k].release();
     }
     if (ctx->cfg.dirs == 2) {
         // a table also for an intrinsic matrix that is not [fx 0 cx; 0 fy cy; 0 0 1] (skew, ...): the kernels' table-free
         // route then only ever sees the standard form (4 operations per coordinate, no division)
         if (d.cam_distorted || !d.cam_std) {
-            CK(dalloc(&ctx->cam_lut, npix(ctx)));
+            CK(ctx->cam_lut.ensure(npix(ctx)));
             CK(launch_undistort_lut(nullptr, d, false, ctx->cfg.W, ctx->cfg.H, ctx->cfg.row0, ctx->cam_lut, ctx->stream));
             ctx->launches++;
         }
         if (d.proj_distorted || !d.proj_std) {
-            CK(dalloc(&ctx->proj_lut, (size_t)ctx->cfg.PW * ctx->cfg.PH));
+            CK(ctx->proj_lut.ensure((size_t)ctx->cfg.PW * ctx->cfg.PH));
             CK(launch_undistort_lut(nullptr, d, true, ctx->cfg.PW, ctx->cfg.PH, 0, ctx->proj_lut, ctx->stream));
             ctx->launches++;
         }
@@ -317,11 +279,11 @@ int scan3d_set_texture(scan3d_ctx* ctx, const uint8_t* bgr_host)
     if (!ctx) return SCAN3D_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     if (!bgr_host) {
-        if (ctx->texture) { cudaFree(ctx->texture); ctx->texture = nullptr; }
+        ctx->texture.release();
         return SCAN3D_OK;
     }
-    if (!ctx->texture) CK(dalloc(&ctx->texture, 3 * npix(ctx)));
-    if (!ctx->rgb) CK(dalloc(&ctx->rgb, 3 * npix(ctx)));
+    CK(ctx->texture.ensure(3 * npix(ctx)));
+    CK(ctx->rgb.ensure(3 * npix(ctx)));
     CK(cudaMemcpyAsync(ctx->texture, bgr_host, 3 * npix(ctx), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return SCAN3D_OK;
@@ -333,8 +295,8 @@ int scan3d_set_texture(scan3d_ctx* ctx, const uint8_t* bgr_host)
 static int ensure_stage_planes(scan3d_ctx* ctx, int dir)
 {
     const size_t n = npix(ctx);
-    if (!ctx->wrapped[dir]) CK(dalloc(&ctx->wrapped[dir], n));
-    if (!ctx->mask[dir]) CK(dalloc(&ctx->mask[dir], n));
+    CK(ctx->wrapped[dir].ensure(n));
+    CK(ctx->mask[dir].ensure(n));
     return SCAN3D_OK;
 }
 
@@ -345,7 +307,7 @@ static int strict_roi(scan3d_ctx* ctx, const uint8_t** roi_dev)
 {
     if (!(ctx->cfg.flags & SCAN3D_FLAG_STRICT_REFERENCE)) return SCAN3D_OK;
     const size_t n = (size_t)ctx->cfg.W * ctx->cfg.H_total;
-    if (!ctx->roi_strict) CK(dalloc(&ctx->roi_strict, n));
+    CK(ctx->roi_strict.ensure(n));
     CK(launch_strict_roi(*roi_dev, ctx->roi_strict, n, ctx->cfg.N, ctx->stream));
     ctx->launches++;
     *roi_dev = ctx->roi_strict;
@@ -371,7 +333,7 @@ int scan3d_compute_wrapped_phase_dev(scan3d_ctx* ctx, int dir, const uint8_t* fr
         if (rc) return rc;
     }
     if (ctx->cfg.flags & SCAN3D_FLAG_MODULATION_MASK) {
-        if (!ctx->roi_eff) CK(dalloc(&ctx->roi_eff, npix(ctx)));
+        CK(ctx->roi_eff.ensure(npix(ctx)));
         CK(launch_modulation_roi(s, fringe_dev, roi_dev, ctx->roi_eff, ctx->stream));
         ctx->launches++;
         roi_dev = ctx->roi_eff;
@@ -392,8 +354,8 @@ static int ensure_staging(scan3d_ctx* ctx)
     const size_t sb = (size_t)scan3d_stack_bytes(&ctx->cfg);
     size_t rb;
     roi_bytes(ctx, &rb);
-    if (!ctx->d_stack) CK(cudaMalloc((void**)&ctx->d_stack, sb));
-    if (!ctx->d_roi) CK(cudaMalloc((void**)&ctx->d_roi, rb));
+    CK(ctx->d_stack.ensure(sb));
+    CK(ctx->d_roi.ensure(rb));
     return SCAN3D_OK;
 }
 
@@ -467,7 +429,7 @@ int scan3d_triangulate(scan3d_ctx* ctx)
     if (!ctx->has_calib) return fail(ctx, SCAN3D_ERR_STATE, "triangulate before set_calibration");
     if (!ctx->have_cpmap) return fail(ctx, SCAN3D_ERR_STATE, "triangulate before compute_c_p_map");
     CK(cudaSetDevice(ctx->device));
-    if (!ctx->xyz) CK(dalloc(&ctx->xyz, 3 * npix(ctx)));
+    CK(ctx->xyz.ensure(3 * npix(ctx)));
     const Shape s = shape_of(ctx->cfg);
     CK(launch_triangulate(s, ctx->dcal, ctx->cam_lut, ctx->proj_lut, ctx->cpmap, ctx->valid, ctx->xyz, ctx->stream));
     ctx->launches++;
@@ -482,13 +444,13 @@ int scan3d_compact_points(scan3d_ctx* ctx, int64_t* count_out)
     if (!ctx->have_xyz) return fail(ctx, SCAN3D_ERR_STATE, "compact_points before triangulate");
     CK(cudaSetDevice(ctx->device));
     const size_t n = npix(ctx);
-    if (!ctx->block_counts) CK(dalloc(&ctx->block_counts, (n + 1023) / 1024 + 1));
-    if (!ctx->pix) CK(dalloc(&ctx->pix, n));
-    if (ctx->texture && !ctx->rgb) CK(dalloc(&ctx->rgb, 3 * n));
+    CK(ctx->block_counts.ensure((n + 1023) / 1024 + 1));
+    CK(ctx->pix.ensure(n));
+    if (ctx->texture) CK(ctx->rgb.ensure(3 * n));
     const Shape s = shape_of(ctx->cfg);
     int nl = 0;
     CK(launch_compact(s, ctx->xyz, ctx->valid, ctx->texture, ctx->block_counts, points_of(ctx), ctx->pix,
-                      ctx->texture ? ctx->rgb : nullptr, ctx->d_count, ctx->stream, &nl));
+                      ctx->texture ? ctx->rgb.get() : nullptr, ctx->d_count, ctx->stream, &nl));
     ctx->launches += nl;
     ctx->have_points = true;
     ctx->have_mesh = false;
@@ -558,14 +520,14 @@ int scan3d_reconstruct_dev(scan3d_ctx* ctx, const uint8_t* stack_dev, const uint
         // direction from that direction's three fringe images (a pre-pass: the mask recurrence needs it two rows up)
         const Shape s = shape_of(c);
         const size_t n = npix(ctx);
-        if (!ctx->roi_eff) CK(dalloc(&ctx->roi_eff, n));
+        CK(ctx->roi_eff.ensure(n));
         CK(launch_modulation_roi(s, stack_dev, roi_dev, ctx->roi_eff, ctx->stream));
         ctx->launches++;
         a.roi = ctx->roi_eff;
         a.roi2 = ctx->roi_eff;
         a.roi_list = roi_dev;
         if (c.dirs == 2) {
-            if (!ctx->roi_eff_h) CK(dalloc(&ctx->roi_eff_h, n));
+            CK(ctx->roi_eff_h.ensure(n));
             CK(launch_modulation_roi(s, stack_dev + (size_t)(c.N + 2 * c.M_v) * n, roi_dev, ctx->roi_eff_h, ctx->stream));
             ctx->launches++;
             a.roi2 = ctx->roi_eff_h;
@@ -575,7 +537,7 @@ int scan3d_reconstruct_dev(scan3d_ctx* ctx, const uint8_t* stack_dev, const uint
     a.code_v = ctx->code[0]; a.code_h = ctx->code[1];
     a.valid = ctx->valid; a.cpmap = ctx->cpmap;
     a.pts = points_of(ctx); a.pix = ctx->pix;
-    a.rgb = ctx->texture ? ctx->rgb : nullptr; a.texture = ctx->texture;
+    a.rgb = ctx->texture ? ctx->rgb.get() : nullptr; a.texture = ctx->texture;
     a.d_count = ctx->d_count; a.tile_state = ctx->tile_state; a.trace = ctx->trace; a.tile_flags = ctx->tile_flags; a.tile_list = ctx->tile_list + 1; a.n_list = ctx->tile_list;
     a.cam_lut = ctx->cam_lut; a.proj_lut = ctx->proj_lut; a.atan_tab = ctx->atan_tab; a.code_term = ctx->code_term;
     if (ctx->trace) CK(cudaMemsetAsync(ctx->trace, 0, (size_t)1024 * 64 * 8 * 8, ctx->stream));   // diagnostics only
@@ -655,7 +617,7 @@ int scan3d_reconstruct_raw_dev(scan3d_ctx* ctx, const uint8_t* raw_stack_dev, co
     if (!ctx || !raw_stack_dev || !roi_dev) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
     CK(cudaSetDevice(ctx->device));
     const size_t sb = (size_t)scan3d_stack_bytes(&ctx->cfg);
-    if (!ctx->d_undist) CK(cudaMalloc((void**)&ctx->d_undist, sb));
+    CK(ctx->d_undist.ensure(sb));
     const int frames = (int)(sb / npix(ctx));
     int rc = scan3d_undistort_frames_dev(ctx, 0, raw_stack_dev, frames, ctx->d_undist);      // 2/project_pattern.cpp:220,234
     if (rc) return rc;
@@ -865,8 +827,8 @@ int scan3d_set_points_buffer(scan3d_ctx* ctx, void* points_dev, int64_t capacity
     ctx->have_points = ctx->have_mesh = false;
     return SCAN3D_OK;
 }
-void* scan3d_device_point_pixels(scan3d_ctx* ctx) { return ctx ? ctx->pix : nullptr; }
-void* scan3d_device_point_count(scan3d_ctx* ctx) { return ctx ? ctx->d_count : nullptr; }
+void* scan3d_device_point_pixels(scan3d_ctx* ctx) { return ctx ? ctx->pix.get() : nullptr; }
+void* scan3d_device_point_count(scan3d_ctx* ctx) { return ctx ? ctx->d_count.get() : nullptr; }
 
 // pcl::io::savePLYFile-style vertex list (8/save_point_cloud.cpp:216-217)
 int scan3d_write_ply(scan3d_ctx* ctx, const char* path, int binary)
@@ -963,12 +925,12 @@ int scan3d_build_mesh(scan3d_ctx* ctx, float max_edge)
     const size_t n = npix(ctx);
     const size_t nb = (n + POINT_BLOCK - 1) / POINT_BLOCK;
     const size_t max_faces = 2 * (size_t)(c.W - 1) * (size_t)(c.H - 1);
-    if (!ctx->block_counts) CK(dalloc(&ctx->block_counts, nb + 1));
-    if (!ctx->mesh_idx) CK(dalloc(&ctx->mesh_idx, n));
-    if (!ctx->mesh_counts) CK(dalloc(&ctx->mesh_counts, nb));
-    if (!ctx->mesh_totals) CK(dalloc(&ctx->mesh_totals, 2));
-    if (!ctx->mesh_faces) CK(dalloc(&ctx->mesh_faces, 3 * std::max(max_faces, (size_t)1)));
-    if (!ctx->mesh_normals) CK(dalloc(&ctx->mesh_normals, 3 * n));
+    CK(ctx->block_counts.ensure(nb + 1));
+    CK(ctx->mesh_idx.ensure(n));
+    CK(ctx->mesh_counts.ensure(nb));
+    CK(ctx->mesh_totals.ensure(2));
+    CK(ctx->mesh_faces.ensure(3 * std::max(max_faces, (size_t)1)));
+    CK(ctx->mesh_normals.ensure(3 * n));
     CK(launch_mesh(ctx->valid, points_of(ctx), c.W, c.H, max_edge, ctx->mesh_idx, ctx->block_counts, ctx->mesh_counts,
                    ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals, ctx->stream));
     ctx->launches += MESH_LAUNCHES;
@@ -1005,8 +967,8 @@ int scan3d_get_mesh(scan3d_ctx* ctx, int32_t* faces_host, float* normals_host, i
     return SCAN3D_OK;
 }
 
-void* scan3d_device_mesh_faces(scan3d_ctx* ctx) { return ctx && ctx->have_mesh ? ctx->mesh_faces : nullptr; }
-void* scan3d_device_point_normals(scan3d_ctx* ctx) { return ctx && ctx->have_mesh ? ctx->mesh_normals : nullptr; }
+void* scan3d_device_mesh_faces(scan3d_ctx* ctx) { return ctx && ctx->have_mesh ? ctx->mesh_faces.get() : nullptr; }
+void* scan3d_device_point_normals(scan3d_ctx* ctx) { return ctx && ctx->have_mesh ? ctx->mesh_normals.get() : nullptr; }
 
 int scan3d_write_mesh_ply(scan3d_ctx* ctx, const char* path, int binary)
 {
@@ -1033,11 +995,6 @@ int scan3d_write_mesh_ply(scan3d_ctx* ctx, const char* path, int binary)
 // ------------------------------------------------------------------------------------------
 // voxel-grid merge of registered views (include/scan3d.h and common/scan3d_voxel_math.h have the exact rules)
 // ------------------------------------------------------------------------------------------
-static void free_ptr(void* p)
-{
-    if (p) cudaFree(p);
-}
-
 int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
@@ -1049,32 +1006,17 @@ int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
     ctx->srf_ready = ctx->cc_ready = false;
     VoxelTable& t = ctx->vox;
     const uint32_t cap = voxel_table_capacity((uint32_t)max_voxels, ctx->sm_count);
-    if (cap > ctx->vox_alloc_cap) {
-        free_ptr(t.keys); free_ptr(t.acc); free_ptr(t.ordinal);
-        t.keys = nullptr; t.acc = nullptr; t.ordinal = nullptr;
-        ctx->vox_alloc_cap = 0;
-        CK(dalloc(&t.keys, cap));
-        CK(dalloc(&t.acc, cap));
-        CK(dalloc(&t.ordinal, cap));
-        ctx->vox_alloc_cap = cap;
-    }
-    if ((uint32_t)max_voxels > ctx->vox_alloc_max) {
-        free_ptr(t.ord2slot); free_ptr(ctx->vox_xyz); free_ptr(ctx->vox_nrm); free_ptr(ctx->vox_rgb); free_ptr(ctx->vox_cnt);
-        t.ord2slot = nullptr; ctx->vox_xyz = ctx->vox_nrm = nullptr; ctx->vox_rgb = nullptr; ctx->vox_cnt = nullptr;
-        ctx->vox_alloc_max = 0;
-        const size_t m = (size_t)max_voxels;
-        CK(dalloc(&t.ord2slot, m));
-        CK(dalloc(&ctx->vox_xyz, 3 * m));
-        CK(dalloc(&ctx->vox_nrm, 3 * m));
-        CK(dalloc(&ctx->vox_rgb, 3 * m));
-        CK(dalloc(&ctx->vox_cnt, m));
-        ctx->vox_alloc_max = (uint32_t)max_voxels;
-    }
+    CK(grow_group(Grow(ctx->vox_keys, cap), Grow(ctx->vox_acc, cap), Grow(ctx->vox_ordinal, cap)));
+    const size_t m = (size_t)max_voxels;
+    CK(grow_group(Grow(ctx->vox_ord2slot, m), Grow(ctx->vox_xyz, 3 * m), Grow(ctx->vox_nrm, 3 * m),
+                  Grow(ctx->vox_rgb, 3 * m), Grow(ctx->vox_cnt, m)));
     const size_t n = npix(ctx);
-    if (!t.state) CK(dalloc(&t.state, 1));
-    if (!ctx->vox_point_slot) CK(dalloc(&ctx->vox_point_slot, n));
-    if (!ctx->vox_flags) CK(dalloc(&ctx->vox_flags, n));
-    if (!ctx->block_counts) CK(dalloc(&ctx->block_counts, (n + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+    CK(ctx->vox_state.ensure(1));
+    CK(ctx->vox_point_slot.ensure(n));
+    CK(ctx->vox_flags.ensure(n));
+    CK(ctx->block_counts.ensure((n + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+    t.keys = ctx->vox_keys; t.acc = ctx->vox_acc; t.ordinal = ctx->vox_ordinal;
+    t.ord2slot = ctx->vox_ord2slot; t.state = ctx->vox_state;
     CK(cudaMemsetAsync(t.keys, 0xff, (size_t)cap * sizeof(*t.keys), ctx->stream));
     CK(cudaMemsetAsync(t.acc, 0, (size_t)cap * sizeof(*t.acc), ctx->stream));
     CK(cudaMemsetAsync(t.ordinal, 0xff, (size_t)cap * sizeof(*t.ordinal), ctx->stream));
@@ -1113,8 +1055,8 @@ int scan3d_voxel_add_points(scan3d_ctx* ctx)
     CK(cudaSetDevice(ctx->device));
     ctx->vox_bound += ub;
     ctx->vox_fresh = ctx->srf_ready = ctx->cc_ready = false;
-    return voxel_add(ctx, points_of(ctx), ctx->have_mesh ? ctx->mesh_normals : nullptr,
-                     ctx->texture && ctx->rgb ? ctx->rgb : nullptr, ctx->d_count, (uint32_t)ub);
+    return voxel_add(ctx, points_of(ctx), ctx->have_mesh ? ctx->mesh_normals.get() : nullptr,
+                     ctx->texture && ctx->rgb ? ctx->rgb.get() : nullptr, ctx->d_count, (uint32_t)ub);
 }
 
 int scan3d_voxel_add_points_dev(scan3d_ctx* ctx, const float* xyz_dev, const float* normals_dev, const uint8_t* rgb_dev,
@@ -1245,19 +1187,13 @@ static int align_index(scan3d_ctx* ctx, const AlignRun& run, const uint32_t* n_d
 {
     const uint32_t maxv = ctx->vox.max_voxels;
     AlignIndex& ix = ctx->aln;
-    if (maxv > ctx->aln_alloc_max) {
-        free_ptr(ix.keys); free_ptr(ix.cells); free_ptr(ix.model_slot); free_ptr(ix.entries);
-        ix.keys = nullptr; ix.cells = nullptr; ix.model_slot = nullptr; ix.entries = nullptr;
-        ctx->aln_alloc_max = 0;
-        const size_t cap = (size_t)ALIGN_CELLS_PER_VOXEL * maxv;
-        CK(dalloc(&ix.keys, cap));
-        CK(dalloc(&ix.cells, cap));
-        CK(dalloc(&ix.model_slot, (size_t)maxv));
-        CK(dalloc(&ix.entries, 2 * (size_t)maxv));
-        ctx->aln_alloc_max = maxv;
-    }
-    if (!ctx->aln_state) CK(dalloc(&ctx->aln_state, 1));
-    if (!ix.cursor) CK(dalloc(&ix.cursor, 1));
+    const size_t cap = (size_t)ALIGN_CELLS_PER_VOXEL * maxv;
+    CK(grow_group(Grow(ctx->aln_keys, cap), Grow(ctx->aln_cells, cap), Grow(ctx->aln_model_slot, (size_t)maxv),
+                  Grow(ctx->aln_entries, 2 * (size_t)maxv)));
+    CK(ctx->aln_state.ensure(1));
+    CK(ctx->aln_cursor.ensure(1));
+    ix.keys = ctx->aln_keys; ix.cells = ctx->aln_cells; ix.model_slot = ctx->aln_model_slot;
+    ix.entries = ctx->aln_entries; ix.cursor = ctx->aln_cursor;
     ix.cap = ALIGN_CELLS_PER_VOXEL * maxv;
     CK(cudaMemsetAsync(ix.keys, 0xff, (size_t)ix.cap * sizeof(*ix.keys), ctx->stream));
     CK(cudaMemsetAsync(ix.cells, 0, (size_t)ix.cap * sizeof(*ix.cells), ctx->stream));
@@ -1274,13 +1210,7 @@ static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long lo
 {
     CK(cudaSetDevice(ctx->device));
     const uint32_t blocks = align_match_blocks(n_max, p->stride);
-    if (blocks > ctx->aln_alloc_blocks) {
-        free_ptr(ctx->aln_partials);
-        ctx->aln_partials = nullptr;
-        ctx->aln_alloc_blocks = 0;
-        CK(dalloc(&ctx->aln_partials, (size_t)(ALIGN_NSUM + 1) * blocks));
-        ctx->aln_alloc_blocks = blocks;
-    }
+    CK(ctx->aln_partials.ensure((size_t)(ALIGN_NSUM + 1) * blocks));
     AlignRun run;
     for (int k = 0; k < 12; k++) run.T0[k] = p->T_init[k];
     run.S = s3l::cell_edge(p->max_distance);
@@ -1364,36 +1294,15 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
     SurfaceTable& s = ctx->srf;
     const uint32_t maxp = (uint32_t)p->max_points;
     const uint32_t cap = surface_table_capacity(maxp, ctx->sm_count);
-    if (cap > ctx->srf_alloc_cap) {
-        free_ptr(s.keys); free_ptr(s.owner); free_ptr(s.f); free_ptr(s.nearest); free_ptr(s.vert);
-        s.keys = s.owner = nullptr; s.f = nullptr; s.nearest = s.vert = nullptr;
-        ctx->srf_alloc_cap = 0;
-        CK(dalloc(&s.keys, cap));
-        CK(dalloc(&s.owner, cap));
-        CK(dalloc(&s.f, cap));
-        CK(dalloc(&s.nearest, cap));
-        CK(dalloc(&s.vert, cap));
-        ctx->srf_alloc_cap = cap;
-    }
+    CK(grow_group(Grow(ctx->srf_keys, cap), Grow(ctx->srf_owner, cap), Grow(ctx->srf_f, cap),
+                  Grow(ctx->srf_nearest, cap), Grow(ctx->srf_vert, cap)));
     const size_t nvb = (maxp + SURFACE_VB - 1) / SURFACE_VB;
-    if (maxp > ctx->srf_alloc_points) {
-        free_ptr(ctx->srf_vert_slot); free_ptr(ctx->srf_face_counts);
-        ctx->srf_vert_slot = ctx->srf_face_counts = nullptr;
-        ctx->srf_alloc_points = 0;
-        CK(dalloc(&ctx->srf_vert_slot, maxp));
-        CK(dalloc(&ctx->srf_face_counts, nvb + 1));
-        ctx->srf_alloc_points = maxp;
-    }
+    CK(grow_group(Grow(ctx->srf_vert_slot, maxp), Grow(ctx->srf_face_counts, nvb + 1)));
     const uint64_t nflags = (uint64_t)s3s::OFFSETS * ctx->vox.max_voxels;
-    if (nflags > ctx->srf_alloc_flags) {
-        free_ptr(ctx->srf_flags); free_ptr(ctx->srf_flag_counts);
-        ctx->srf_flags = nullptr; ctx->srf_flag_counts = nullptr;
-        ctx->srf_alloc_flags = 0;
-        CK(dalloc(&ctx->srf_flags, nflags));
-        CK(dalloc(&ctx->srf_flag_counts, (nflags + POINT_BLOCK - 1) / POINT_BLOCK + 1));
-        ctx->srf_alloc_flags = nflags;
-    }
-    if (!s.state) CK(dalloc(&s.state, 1));
+    CK(grow_group(Grow(ctx->srf_flags, nflags), Grow(ctx->srf_flag_counts, (nflags + POINT_BLOCK - 1) / POINT_BLOCK + 1)));
+    CK(ctx->srf_state.ensure(1));
+    s.keys = ctx->srf_keys; s.owner = ctx->srf_owner; s.f = ctx->srf_f; s.nearest = ctx->srf_nearest;
+    s.vert = ctx->srf_vert; s.state = ctx->srf_state;
     s.cap = cap;
     s.max_points = maxp;
     s.S = ctx->vox.S;
@@ -1408,7 +1317,7 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
     SurfaceState st;
     int vox_overflow = 0;
     CK(cudaMemcpyAsync(&st, s.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(&vox_overflow, &ctx->aln_state->overflow, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&vox_overflow, &ctx->aln_state.get()->overflow, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     if (vox_overflow)
         return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct voxels than max_voxels: begin again with a larger max_voxels");
@@ -1416,22 +1325,9 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
         return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct lattice points than max_points: extract again with a larger max_points");
     if ((uint64_t)st.vertices * 6 > 0xffffffffull)   // the face count is a 32-bit sum of <= 6 per vertex
         return fail(ctx, SCAN3D_ERR_CONFIG, "more than (2^32 - 1) / 6 surface vertices");
-    if (st.vertices > ctx->srf_alloc_v) {
-        free_ptr(ctx->srf_xyz); free_ptr(ctx->srf_nrm); free_ptr(ctx->srf_rgb);
-        ctx->srf_xyz = ctx->srf_nrm = nullptr; ctx->srf_rgb = nullptr;
-        ctx->srf_alloc_v = 0;
-        CK(dalloc(&ctx->srf_xyz, 3 * (size_t)st.vertices));
-        CK(dalloc(&ctx->srf_nrm, 3 * (size_t)st.vertices));
-        CK(dalloc(&ctx->srf_rgb, 3 * (size_t)st.vertices));
-        ctx->srf_alloc_v = st.vertices;
-    }
-    if (st.faces > ctx->srf_alloc_f) {
-        free_ptr(ctx->srf_tri);
-        ctx->srf_tri = nullptr;
-        ctx->srf_alloc_f = 0;
-        CK(dalloc(&ctx->srf_tri, 3 * (size_t)st.faces));
-        ctx->srf_alloc_f = st.faces;
-    }
+    const size_t nv3 = 3 * (size_t)st.vertices;
+    CK(grow_group(Grow(ctx->srf_xyz, nv3), Grow(ctx->srf_nrm, nv3), Grow(ctx->srf_rgb, nv3)));
+    CK(ctx->srf_tri.ensure(3 * (size_t)st.faces));
     CK(launch_surface_emit(s, ctx->vox_rgb, ctx->srf_vert_slot, ctx->srf_face_counts, st.vertices, ctx->srf_xyz,
                            ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri, ctx->stream));
     ctx->launches += 1;
@@ -1487,16 +1383,9 @@ int scan3d_write_voxel_surface_ply(scan3d_ctx* ctx, const char* path, int binary
 static int cc_label_scratch(scan3d_ctx* ctx, int64_t n)
 {
     n = std::max<int64_t>(n, 1);
-    if (n > ctx->cc_alloc_label) {
-        free_ptr(ctx->cc_parent); free_ptr(ctx->cc_flags); free_ptr(ctx->cc_vert_counts);
-        ctx->cc_parent = ctx->cc_vert_counts = nullptr; ctx->cc_flags = nullptr;
-        ctx->cc_alloc_label = 0;
-        CK(dalloc(&ctx->cc_parent, (size_t)n));
-        CK(dalloc(&ctx->cc_flags, (size_t)n));
-        CK(dalloc(&ctx->cc_vert_counts, (size_t)(n + POINT_BLOCK - 1) / POINT_BLOCK + 1));
-        ctx->cc_alloc_label = n;
-    }
-    if (!ctx->cc_state) CK(dalloc(&ctx->cc_state, 1));
+    CK(grow_group(Grow(ctx->cc_parent, (size_t)n), Grow(ctx->cc_flags, (size_t)n),
+                  Grow(ctx->cc_vert_counts, (size_t)(n + POINT_BLOCK - 1) / POINT_BLOCK + 1)));
+    CK(ctx->cc_state.ensure(1));
     CK(cudaMemsetAsync(ctx->cc_state, 0, sizeof(ComponentsState), ctx->stream));
     return SCAN3D_OK;
 }
@@ -1513,25 +1402,9 @@ int scan3d_voxel_surface_components(scan3d_ctx* ctx, const scan3d_components_par
     const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
     int rc = cc_label_scratch(ctx, nv);
     if (rc) return rc;
-    const int64_t av = std::max<int64_t>(nv, 1), af = std::max<int64_t>(nf, 1);
-    if (av > ctx->cc_alloc_v) {
-        free_ptr(ctx->cc_label); free_ptr(ctx->cc_comp_v); free_ptr(ctx->cc_comp_f); free_ptr(ctx->cc_kept);
-        ctx->cc_label = nullptr; ctx->cc_comp_v = ctx->cc_comp_f = nullptr; ctx->cc_kept = nullptr;
-        ctx->cc_alloc_v = 0;
-        CK(dalloc(&ctx->cc_label, (size_t)av));
-        CK(dalloc(&ctx->cc_comp_v, (size_t)av));
-        CK(dalloc(&ctx->cc_comp_f, (size_t)av));
-        CK(dalloc(&ctx->cc_kept, (size_t)av));
-        ctx->cc_alloc_v = av;
-    }
-    if (af > ctx->cc_alloc_f) {
-        free_ptr(ctx->cc_keep_f); free_ptr(ctx->cc_face_counts);
-        ctx->cc_keep_f = nullptr; ctx->cc_face_counts = nullptr;
-        ctx->cc_alloc_f = 0;
-        CK(dalloc(&ctx->cc_keep_f, (size_t)af));
-        CK(dalloc(&ctx->cc_face_counts, (size_t)(af + POINT_BLOCK - 1) / POINT_BLOCK + 1));
-        ctx->cc_alloc_f = af;
-    }
+    const size_t av = (size_t)std::max<int64_t>(nv, 1), af = (size_t)std::max<int64_t>(nf, 1);
+    CK(grow_group(Grow(ctx->cc_label, av), Grow(ctx->cc_comp_v, av), Grow(ctx->cc_comp_f, av), Grow(ctx->cc_kept, av)));
+    CK(grow_group(Grow(ctx->cc_keep_f, af), Grow(ctx->cc_face_counts, (af + POINT_BLOCK - 1) / POINT_BLOCK + 1)));
     CK(cudaMemsetAsync(ctx->cc_comp_v, 0, (size_t)nv * sizeof(uint32_t), ctx->stream));
     CK(cudaMemsetAsync(ctx->cc_comp_f, 0, (size_t)nv * sizeof(uint32_t), ctx->stream));
     CK(launch_cc_labels(ctx->srf_tri, (uint32_t)nf, (uint32_t)nv, ctx->cc_parent, ctx->cc_flags, ctx->cc_vert_counts,
@@ -1544,22 +1417,9 @@ int scan3d_voxel_surface_components(scan3d_ctx* ctx, const scan3d_components_par
     ComponentsState st;
     CK(cudaMemcpyAsync(&st, ctx->cc_state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (st.vertices > ctx->cc_out_alloc_v) {
-        free_ptr(ctx->cc_xyz); free_ptr(ctx->cc_nrm); free_ptr(ctx->cc_rgb);
-        ctx->cc_xyz = ctx->cc_nrm = nullptr; ctx->cc_rgb = nullptr;
-        ctx->cc_out_alloc_v = 0;
-        CK(dalloc(&ctx->cc_xyz, 3 * (size_t)st.vertices));
-        CK(dalloc(&ctx->cc_nrm, 3 * (size_t)st.vertices));
-        CK(dalloc(&ctx->cc_rgb, 3 * (size_t)st.vertices));
-        ctx->cc_out_alloc_v = st.vertices;
-    }
-    if (st.faces > ctx->cc_out_alloc_f) {
-        free_ptr(ctx->cc_tri);
-        ctx->cc_tri = nullptr;
-        ctx->cc_out_alloc_f = 0;
-        CK(dalloc(&ctx->cc_tri, 3 * (size_t)st.faces));
-        ctx->cc_out_alloc_f = st.faces;
-    }
+    const size_t kv3 = 3 * (size_t)st.vertices;
+    CK(grow_group(Grow(ctx->cc_xyz, kv3), Grow(ctx->cc_nrm, kv3), Grow(ctx->cc_rgb, kv3)));
+    CK(ctx->cc_tri.ensure(3 * (size_t)st.faces));
     CK(launch_cc_emit(ctx->cc_flags, ctx->cc_vert_counts, (uint32_t)nv, ctx->srf_xyz, ctx->srf_nrm, ctx->srf_rgb,
                       ctx->cc_keep_f, ctx->cc_face_counts, (uint32_t)nf, ctx->srf_tri, ctx->cc_label, ctx->cc_xyz,
                       ctx->cc_nrm, ctx->cc_rgb, ctx->cc_tri, ctx->stream));
@@ -1569,8 +1429,6 @@ int scan3d_voxel_surface_components(scan3d_ctx* ctx, const scan3d_components_par
     std::swap(ctx->srf_nrm, ctx->cc_nrm);
     std::swap(ctx->srf_rgb, ctx->cc_rgb);
     std::swap(ctx->srf_tri, ctx->cc_tri);
-    std::swap(ctx->srf_alloc_v, ctx->cc_out_alloc_v);
-    std::swap(ctx->srf_alloc_f, ctx->cc_out_alloc_f);
     ctx->srf_vertices = st.vertices;
     ctx->srf_faces = st.faces;
     ctx->cc_components = st.components;
@@ -1644,7 +1502,7 @@ int scan3d_generate_patterns_dev(scan3d_ctx* ctx, int dir, uint8_t* patterns_dev
     const int M = dir == 0 ? c.M_v : c.M_h, fw = dir == 0 ? c.fw_v : c.fw_h;
     const int len = dir == 0 ? c.PW : c.PH, lenp = (len + 15) & ~15, np = c.N + 2 * M;
     const size_t max_prof = (size_t)(16 + 2 * 15) * (((size_t)std::max(c.PW, c.PH) + 15) & ~(size_t)15);
-    if (!ctx->pattern_profiles) CK(dalloc(&ctx->pattern_profiles, 2 * max_prof));
+    CK(ctx->pattern_profiles.ensure(2 * max_prof));
     uint8_t* d_prof = ctx->pattern_profiles + (size_t)dir * max_prof;
     if (!ctx->have_profiles[dir]) {      // the profiles depend on the configuration only: once per context
         std::vector<uint8_t> prof((size_t)np * lenp, 0);
@@ -1668,15 +1526,12 @@ int scan3d_generate_patterns(scan3d_ctx* ctx, int dir, uint8_t* patterns_host)
     const int64_t bytes = scan3d_pattern_bytes(&ctx->cfg, dir);
     if (bytes <= 0) return fail(ctx, SCAN3D_ERR_ARG, "bad direction or projector size");
     CK(cudaSetDevice(ctx->device));
-    uint8_t* d = nullptr;
-    CK(cudaMalloc((void**)&d, (size_t)bytes));
-    int rc = scan3d_generate_patterns_dev(ctx, dir, d);
-    cudaError_t e = cudaSuccess;
-    if (rc == SCAN3D_OK) e = cudaMemcpyAsync(patterns_host, d, (size_t)bytes, cudaMemcpyDeviceToHost, ctx->stream);
-    const cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d);
+    DeviceBuffer<uint8_t> d;
+    CK(d.ensure((size_t)bytes));
+    const int rc = scan3d_generate_patterns_dev(ctx, dir, d);
     if (rc) return rc;
-    if (e != cudaSuccess || e2 != cudaSuccess) return fail(ctx, SCAN3D_ERR_CUDA, cudaGetErrorString(e != cudaSuccess ? e : e2));
+    CK(cudaMemcpyAsync(patterns_host, d, (size_t)bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     return SCAN3D_OK;
 }
 
@@ -1710,21 +1565,17 @@ int scan3d_debug_atan2(scan3d_ctx* ctx, const double* y_host, const double* x_ho
 {
     if (!ctx || !y_host || !x_host || !out_host || n <= 0) return fail(ctx, SCAN3D_ERR_ARG, "bad argument");
     CK(cudaSetDevice(ctx->device));
-    double *dy = nullptr, *dx = nullptr;
-    float* dout = nullptr;
-    cudaError_t e = cudaMalloc((void**)&dy, (size_t)n * 8);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&dx, (size_t)n * 8);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&dout, (size_t)n * 4);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dy, y_host, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dx, x_host, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = launch_debug_atan2(dy, dx, dout, n, mode, ctx->atan_tab, ctx->stream);
-    if (e == cudaSuccess) {
-        ctx->launches++;
-        e = cudaMemcpyAsync(out_host, dout, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream);
-    }
-    const cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-    cudaFree(dy); cudaFree(dx); cudaFree(dout);
-    if (e != cudaSuccess || e2 != cudaSuccess) return fail(ctx, SCAN3D_ERR_CUDA, cudaGetErrorString(e != cudaSuccess ? e : e2));
+    DeviceBuffer<double> dy, dx;
+    DeviceBuffer<float> dout;
+    CK(dy.ensure((size_t)n));
+    CK(dx.ensure((size_t)n));
+    CK(dout.ensure((size_t)n));
+    CK(cudaMemcpyAsync(dy, y_host, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(dx, x_host, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(launch_debug_atan2(dy, dx, dout, n, mode, ctx->atan_tab, ctx->stream));
+    ctx->launches++;
+    CK(cudaMemcpyAsync(out_host, dout, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     return SCAN3D_OK;
 }
 
@@ -1748,15 +1599,14 @@ int scan3d_debug_divcheck(scan3d_ctx* ctx, uint64_t* mismatches)
 {
     if (!ctx || !mismatches) return fail(ctx, SCAN3D_ERR_ARG, "bad argument");
     CK(cudaSetDevice(ctx->device));
-    unsigned long long* d = nullptr;
-    CK(cudaMalloc((void**)&d, 8));
+    DeviceBuffer<unsigned long long> d;
+    CK(d.ensure(1));
     unsigned long long h = 0;
-    cudaError_t e = cudaMemsetAsync(d, 0, 8, ctx->stream);
-    if (e == cudaSuccess) e = launch_debug_divcheck(d, ctx->stream);
-    if (e == cudaSuccess) { ctx->launches++; e = cudaMemcpyAsync(&h, d, 8, cudaMemcpyDeviceToHost, ctx->stream); }
-    const cudaError_t e2 = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d);
-    if (e != cudaSuccess || e2 != cudaSuccess) return fail(ctx, SCAN3D_ERR_CUDA, cudaGetErrorString(e != cudaSuccess ? e : e2));
+    CK(cudaMemsetAsync(d, 0, 8, ctx->stream));
+    CK(launch_debug_divcheck(d, ctx->stream));
+    ctx->launches++;
+    CK(cudaMemcpyAsync(&h, d, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     *mismatches = h;
     return SCAN3D_OK;
 }

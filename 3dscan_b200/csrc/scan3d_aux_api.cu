@@ -5,26 +5,12 @@
 #include <string.h>
 
 #include <string>
+#include <utility>
 
 #include "scan3d_internal.h"
 #include "../common/scan3d_aux_math.h"
 
 using namespace s3d;
-
-#define CK(call)                                                                          \
-    do {                                                                                  \
-        cudaError_t e_ = (call);                                                          \
-        if (e_ != cudaSuccess) {                                                          \
-            ctx->err = std::string(#call) + ": " + cudaGetErrorString(e_);                \
-            return SCAN3D_ERR_CUDA;                                                       \
-        }                                                                                 \
-    } while (0)
-
-static int fail(scan3d_ctx* ctx, int code, const char* msg)
-{
-    if (ctx) ctx->err = msg;
-    return code;
-}
 
 // frame shape of the device whose images are undistorted: 0 = camera, 1 = projector
 static int kind_shape(scan3d_ctx* ctx, int kind, int* W, int* H)
@@ -46,22 +32,20 @@ static int ensure_map(scan3d_ctx* ctx, int kind, int W, int H)
 {
     if (ctx->undist_xy[kind]) return SCAN3D_OK;
     const size_t n = (size_t)W * H;
-    short2* xy = nullptr;
-    uint16_t* frac = nullptr;
+    DeviceBuffer<short2> xy;
+    DeviceBuffer<uint16_t> frac;
     const double* K = kind == 0 ? ctx->hcal.Kc : ctx->hcal.Kp;
     const double* d = kind == 0 ? ctx->hcal.dc : ctx->hcal.dp;
-    cudaError_t e = cudaMalloc((void**)&xy, n * sizeof(short2));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&frac, n * sizeof(uint16_t));
+    cudaError_t e = xy.ensure(n);
+    if (e == cudaSuccess) e = frac.ensure(n);
     if (e == cudaSuccess) e = launch_undistort_map(K, d, W, H, xy, frac, ctx->stream);
     if (e != cudaSuccess) {      // both maps or none: a half-built pair must never look usable
-        cudaFree(xy);
-        cudaFree(frac);
         cudaGetLastError();
         ctx->err = std::string("undistortion map: ") + cudaGetErrorString(e);
         return SCAN3D_ERR_CUDA;
     }
-    ctx->undist_xy[kind] = xy;
-    ctx->undist_frac[kind] = frac;
+    ctx->undist_xy[kind] = std::move(xy);
+    ctx->undist_frac[kind] = std::move(frac);
     ctx->launches++;
     return SCAN3D_OK;
 }
@@ -96,18 +80,14 @@ int scan3d_undistort_frames(scan3d_ctx* ctx, int device_kind, const uint8_t* src
     if (n_frames == 0) return SCAN3D_OK;
     CK(cudaSetDevice(ctx->device));
     const size_t bytes = (size_t)W * H * n_frames;
-    uint8_t* buf = nullptr;
-    CK(cudaMalloc((void**)&buf, 2 * bytes));
-    rc = [&]() -> int {
-        CK(cudaMemcpyAsync(buf, src_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
-        int r = scan3d_undistort_frames_dev(ctx, device_kind, buf, n_frames, buf + bytes);
-        if (r) return r;
-        CK(cudaMemcpyAsync(dst_host, buf + bytes, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        return SCAN3D_OK;
-    }();
-    cudaFree(buf);
-    return rc;
+    DeviceBuffer<uint8_t> buf;
+    CK(buf.ensure(2 * bytes));
+    CK(cudaMemcpyAsync(buf, src_host, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    rc = scan3d_undistort_frames_dev(ctx, device_kind, buf, n_frames, buf + bytes);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(dst_host, buf + bytes, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return SCAN3D_OK;
 }
 
 int scan3d_get_undistort_map(scan3d_ctx* ctx, int device_kind, int16_t* xy_host, uint16_t* frac_host)
@@ -142,19 +122,15 @@ int scan3d_roi_fill(scan3d_ctx* ctx, const uint8_t* outline_host, uint8_t* roi_h
     if (!ctx || !outline_host || !roi_host) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
     CK(cudaSetDevice(ctx->device));
     const size_t n = (size_t)ctx->cfg.W * ctx->cfg.H_total;
-    uint8_t* buf = nullptr;
-    CK(cudaMalloc((void**)&buf, 2 * n));
-    int rc = [&]() -> int {
-        CK(cudaMemcpyAsync(buf, outline_host, n, cudaMemcpyHostToDevice, ctx->stream));
-        int r = scan3d_roi_fill_dev(ctx, buf, buf + n, filled_host ? buf : nullptr);   // outline filled in place, like the reference
-        if (r) return r;
-        CK(cudaMemcpyAsync(roi_host, buf + n, n, cudaMemcpyDeviceToHost, ctx->stream));
-        if (filled_host) CK(cudaMemcpyAsync(filled_host, buf, n, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        return SCAN3D_OK;
-    }();
-    cudaFree(buf);
-    return rc;
+    DeviceBuffer<uint8_t> buf;
+    CK(buf.ensure(2 * n));
+    CK(cudaMemcpyAsync(buf, outline_host, n, cudaMemcpyHostToDevice, ctx->stream));
+    const int rc = scan3d_roi_fill_dev(ctx, buf, buf + n, filled_host ? buf.get() : nullptr);   // outline filled in place, like the reference
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(roi_host, buf + n, n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (filled_host) CK(cudaMemcpyAsync(filled_host, buf, n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return SCAN3D_OK;
 }
 
 int scan3d_register_rotation(float theta_deg, float R[16])
@@ -185,18 +161,14 @@ int scan3d_register_points(scan3d_ctx* ctx, const float* src_host, float* dst_ho
     if (n < 0) return fail(ctx, SCAN3D_ERR_ARG, "negative point count");
     if (n == 0) return SCAN3D_OK;
     CK(cudaSetDevice(ctx->device));
-    float* buf = nullptr;
-    CK(cudaMalloc((void**)&buf, (size_t)n * 12));
-    int rc = [&]() -> int {
-        CK(cudaMemcpyAsync(buf, src_host, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
-        int r = scan3d_register_points_dev(ctx, buf, buf, n, theta_deg, tx, ty, tz);   // element-wise: in place is fine
-        if (r) return r;
-        CK(cudaMemcpyAsync(dst_host, buf, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        return SCAN3D_OK;
-    }();
-    cudaFree(buf);
-    return rc;
+    DeviceBuffer<float> buf;
+    CK(buf.ensure(3 * (size_t)n));
+    CK(cudaMemcpyAsync(buf, src_host, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
+    const int rc = scan3d_register_points_dev(ctx, buf, buf, n, theta_deg, tx, ty, tz);   // element-wise: in place is fine
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(dst_host, buf, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return SCAN3D_OK;
 }
 
 }  // extern "C"

@@ -7,6 +7,7 @@
 #include <string>
 
 #include "../../include/scan3d.h"
+#include "scan3d_device_buffer.h"
 #include "scan3d_math.cuh"
 
 #define S3D_PLANE_MASK_H 10   // internal: valid_map_horizontal when the stage API is used
@@ -103,7 +104,11 @@ struct ComponentsState {
 };
 }  // namespace s3d
 
+// Every device buffer the context owns is a DeviceBuffer: scan3d_destroy frees them all by deleting the context.
 struct scan3d_ctx {
+    template <class T>
+    using Buf = s3d::DeviceBuffer<T>;
+
     scan3d_config cfg{};
     int device = 0;
     int sm_count = 148;
@@ -117,112 +122,122 @@ struct scan3d_ctx {
     bool fast_div_ok = false;      // see scan3d_math.cuh div_const
     scan3d_calib hcal{};
     s3d::DeviceCalib dcal{};
-    double2* cam_lut = nullptr;    // [H][W] (u',v') of the local rows, only if the camera is distorted
-    double2* proj_lut = nullptr;   // [PH][PW], only if the projector is distorted
-    double* atan_tab = nullptr;    // hi[33] then lo[33]
-    double* code_term = nullptr;   // [2^max(M_v, M_h)] the unwrap term of every fringe order
+    Buf<double2> cam_lut;          // [H][W] (u',v') of the local rows, only if the camera is distorted
+    Buf<double2> proj_lut;         // [PH][PW], only if the projector is distorted
+    Buf<double> atan_tab;          // hi[33] then lo[33]
+    Buf<double> code_term;         // [2^max(M_v, M_h)] the unwrap term of every fringe order
     float* pts_ext = nullptr;      // scan3d_set_points_buffer: caller-owned (possibly peer) destination of the points
-    uint8_t* pattern_profiles = nullptr;   // scan3d_generate_patterns: 1-D profiles of both directions' patterns
+    Buf<uint8_t> pattern_profiles; // scan3d_generate_patterns: 1-D profiles of both directions' patterns
     bool have_profiles[2] = {false, false};
-    uint8_t* roi_eff = nullptr;    // SCAN3D_FLAG_MODULATION_MASK: ROI && modulation criterion of the current direction
-    uint8_t* roi_eff_h = nullptr;  // ... single-pass entry: the horizontal direction's plane (roi_eff = the vertical one's)
-    uint8_t* roi_strict = nullptr; // SCAN3D_FLAG_STRICT_REFERENCE: (ROI == 1) && N in {3, 4}, whole frame
-    double* nstep_w = nullptr;     // sin[64] then cos[64] (generic-N extension)
-    short2* undist_xy[2] = {nullptr, nullptr};     // cv::undistort's fixed-point map of the camera [0] / projector [1]
-    uint16_t* undist_frac[2] = {nullptr, nullptr}; // (scan3d_undistort_frames; built on first use per calibration)
+    Buf<uint8_t> roi_eff;          // SCAN3D_FLAG_MODULATION_MASK: ROI && modulation criterion of the current direction
+    Buf<uint8_t> roi_eff_h;        // ... single-pass entry: the horizontal direction's plane (roi_eff = the vertical one's)
+    Buf<uint8_t> roi_strict;       // SCAN3D_FLAG_STRICT_REFERENCE: (ROI == 1) && N in {3, 4}, whole frame
+    Buf<double> nstep_w;           // sin[64] then cos[64] (generic-N extension)
+    Buf<short2> undist_xy[2];      // cv::undistort's fixed-point map of the camera [0] / projector [1]
+    Buf<uint16_t> undist_frac[2];  // (scan3d_undistort_frames; built on first use per calibration)
 
     // planes (row-major [H][W])
-    float* wrapped[2] = {nullptr, nullptr};
-    float* unwrapped[2] = {nullptr, nullptr};
-    int16_t* code[2] = {nullptr, nullptr};
-    uint8_t* mask[2] = {nullptr, nullptr};
-    uint8_t* valid = nullptr;
-    int2* cpmap = nullptr;
-    double* xyz = nullptr;         // lazily allocated by scan3d_triangulate
+    Buf<float> wrapped[2];
+    Buf<float> unwrapped[2];
+    Buf<int16_t> code[2];
+    Buf<uint8_t> mask[2];
+    Buf<uint8_t> valid;
+    Buf<int2> cpmap;
+    Buf<double> xyz;               // lazily allocated by scan3d_triangulate
 
     // compacted points
-    float* pts = nullptr;          // [H*W][3]
-    uint32_t* pix = nullptr;       // [H*W]   (only with SCAN3D_FLAG_POINT_PIXELS / stage API)
-    uint8_t* rgb = nullptr;        // [H*W][3] (only when a texture is set)
-    uint8_t* texture = nullptr;    // [H][W][3] BGR
-    uint32_t* d_count = nullptr;   // [1]
-    uint32_t* block_counts = nullptr;  // stage-API compaction scratch
-    unsigned long long* tile_state = nullptr;  // fused kernel decoupled look-back
-    uint8_t* tile_flags = nullptr;             // fused kernel work list (see k_tile_flags)
-    int* tile_list = nullptr;
-    unsigned long long* trace = nullptr;       // SCAN3D_TRACE=1: per-CTA pipeline timeline
+    Buf<float> pts;                // [H*W][3]
+    Buf<uint32_t> pix;             // [H*W]   (only with SCAN3D_FLAG_POINT_PIXELS / stage API)
+    Buf<uint8_t> rgb;              // [H*W][3] (only when a texture is set)
+    Buf<uint8_t> texture;          // [H][W][3] BGR
+    Buf<uint32_t> d_count;         // [1]
+    Buf<uint32_t> block_counts;    // stage-API compaction scratch
+    Buf<unsigned long long> tile_state;  // fused kernel decoupled look-back
+    Buf<uint8_t> tile_flags;             // fused kernel work list (see k_tile_flags)
+    Buf<int> tile_list;
+    Buf<unsigned long long> trace;       // SCAN3D_TRACE=1: per-CTA pipeline timeline
     uint32_t epoch = 0;
     s3d::TensorMapCache tmaps;
 
     // staging for the host-buffer entries
-    uint8_t* d_stack = nullptr;
-    uint8_t* d_roi = nullptr;
-    uint8_t* d_undist = nullptr;   // scan3d_reconstruct_raw: the undistorted stack
+    Buf<uint8_t> d_stack;
+    Buf<uint8_t> d_roi;
+    Buf<uint8_t> d_undist;         // scan3d_reconstruct_raw: the undistorted stack
 
     // scan3d_build_mesh (allocated on the first build)
-    int32_t* mesh_idx = nullptr;          // [H*W] point index of each pixel, -1 = invalid
-    uint32_t* mesh_counts = nullptr;      // face counts / offsets per block of POINT_BLOCK pixels
-    uint32_t* mesh_totals = nullptr;      // [2] points, faces
-    int32_t* mesh_faces = nullptr;        // [2(W-1)(H-1)][3]
-    float* mesh_normals = nullptr;        // [H*W][3]
+    Buf<int32_t> mesh_idx;         // [H*W] point index of each pixel, -1 = invalid
+    Buf<uint32_t> mesh_counts;     // face counts / offsets per block of POINT_BLOCK pixels
+    Buf<uint32_t> mesh_totals;     // [2] points, faces
+    Buf<int32_t> mesh_faces;       // [2(W-1)(H-1)][3]
+    Buf<float> mesh_normals;       // [H*W][3]
 
-    // scan3d_voxel_begin: the merge accumulator (independent of the points; reallocated when a begin asks for more)
+    // scan3d_voxel_begin: the merge accumulator (independent of the points; reallocated when a begin asks for more).
+    // vox is the kernels' view of the vox_* buffers below.
     s3d::VoxelTable vox{};
     bool vox_begun = false;        // a begin has run
     bool vox_fresh = false;        // the outputs are those of the adds since begin (a finish ran after the last add)
     uint64_t vox_bound = 0;        // upper bound of the points added since begin (W*H per ctx add, n per dev add)
     uint32_t vox_chunks = 0;       // adds (chunks of <= W*H points) since begin
-    uint32_t vox_alloc_cap = 0, vox_alloc_max = 0;   // what the buffers hold
-    uint32_t* vox_point_slot = nullptr;   // [H*W] per-point scratch of an add
-    uint8_t* vox_flags = nullptr;         // [H*W]
-    float* vox_xyz = nullptr;             // [max_voxels][3] outputs of scan3d_voxel_finish
-    float* vox_nrm = nullptr;             // [max_voxels][3]
-    uint8_t* vox_rgb = nullptr;           // [max_voxels][3]
-    uint32_t* vox_cnt = nullptr;          // [max_voxels]
+    Buf<unsigned long long> vox_keys;     // [cap] the table
+    Buf<s3d::VoxelSlot> vox_acc;          // [cap]
+    Buf<uint32_t> vox_ordinal;            // [cap]
+    Buf<uint32_t> vox_ord2slot;           // [max_voxels]
+    Buf<s3d::VoxelState> vox_state;
+    Buf<uint32_t> vox_point_slot;         // [H*W] per-point scratch of an add
+    Buf<uint8_t> vox_flags;               // [H*W]
+    Buf<float> vox_xyz;                   // [max_voxels][3] outputs of scan3d_voxel_finish
+    Buf<float> vox_nrm;                   // [max_voxels][3]
+    Buf<uint8_t> vox_rgb;                 // [max_voxels][3]
+    Buf<uint32_t> vox_cnt;                // [max_voxels]
 
-    // scan3d_align_to_voxels (allocated by the first align, grown with max_voxels and the sample count)
+    // scan3d_align_to_voxels (allocated by the first align, grown with max_voxels and the sample count); aln is the
+    // kernels' view of the aln_* index buffers
     s3d::AlignIndex aln{};
-    uint32_t aln_alloc_max = 0;           // max_voxels the index buffers hold
-    uint32_t aln_alloc_blocks = 0;        // blocks of match partials the partial buffer holds
-    double* aln_partials = nullptr;       // [ALIGN_NSUM + 1][blocks]
-    s3d::AlignState* aln_state = nullptr;
+    Buf<unsigned long long> aln_keys;     // [2 max_voxels]
+    Buf<uint2> aln_cells;                 // [2 max_voxels]
+    Buf<uint32_t> aln_model_slot;         // [max_voxels]
+    Buf<float4> aln_entries;              // [2 max_voxels]
+    Buf<uint32_t> aln_cursor;             // [1]
+    Buf<double> aln_partials;             // [ALIGN_NSUM + 1][blocks]
+    Buf<s3d::AlignState> aln_state;
 
-    // scan3d_voxel_surface (allocated by the first extraction, grown on demand)
+    // scan3d_voxel_surface (allocated by the first extraction, grown on demand); srf is the kernels' view of the
+    // lattice table srf_keys ... srf_state
     s3d::SurfaceTable srf{};
     bool srf_ready = false;               // the surface of the current voxel outputs is held
-    uint32_t srf_alloc_cap = 0, srf_alloc_points = 0;   // what the table and the per-vertex buffers hold
-    uint64_t srf_alloc_flags = 0;         // what the flag plane holds (27 max_voxels)
-    uint8_t* srf_flags = nullptr;         // [27 max_voxels] (o, k) owns an active cell
-    uint32_t* srf_flag_counts = nullptr;  // [cdiv(27 max_voxels, POINT_BLOCK) + 1]
-    uint32_t* srf_vert_slot = nullptr;    // [max_points] lattice slot of each vertex
-    uint32_t* srf_face_counts = nullptr;  // [cdiv(max_points, SURFACE_VB) + 1] faces per block of vertices, then offsets
+    Buf<unsigned long long> srf_keys;     // [cap]
+    Buf<unsigned long long> srf_owner;    // [cap]
+    Buf<double> srf_f;                    // [cap]
+    Buf<uint32_t> srf_nearest;            // [cap]
+    Buf<uint32_t> srf_vert;               // [cap]
+    Buf<s3d::SurfaceState> srf_state;
+    Buf<uint8_t> srf_flags;               // [27 max_voxels] (o, k) owns an active cell
+    Buf<uint32_t> srf_flag_counts;        // [cdiv(27 max_voxels, POINT_BLOCK) + 1]
+    Buf<uint32_t> srf_vert_slot;          // [max_points] lattice slot of each vertex
+    Buf<uint32_t> srf_face_counts;        // [cdiv(max_points, SURFACE_VB) + 1] faces per block of vertices, then offsets
     int64_t srf_vertices = 0, srf_faces = 0;
-    int64_t srf_alloc_v = 0, srf_alloc_f = 0;
-    float* srf_xyz = nullptr;             // [vertices][3]
-    float* srf_nrm = nullptr;             // [vertices][3]
-    uint8_t* srf_rgb = nullptr;           // [vertices][3]
-    int32_t* srf_tri = nullptr;           // [faces][3]
+    Buf<float> srf_xyz;                   // [vertices][3]
+    Buf<float> srf_nrm;                   // [vertices][3]
+    Buf<uint8_t> srf_rgb;                 // [vertices][3]
+    Buf<int32_t> srf_tri;                 // [faces][3]
 
     // scan3d_voxel_surface_components / scan3d_mesh_components_dev (allocated on first use, grown on demand)
     bool cc_ready = false;                // the component table of the last scan3d_voxel_surface_components is held
     int64_t cc_components = 0;
-    int64_t cc_alloc_label = 0;           // vertices the labelling scratch holds
-    int64_t cc_alloc_v = 0, cc_alloc_f = 0;   // vertices and faces the table, keep flags and block counts hold
-    uint32_t* cc_parent = nullptr;        // [vertices] union-find forest, then each vertex's root
-    uint8_t* cc_flags = nullptr;          // [vertices] root flags, then the vertices' keep flags
-    uint32_t* cc_vert_counts = nullptr;   // [cdiv(vertices, POINT_BLOCK) + 1] block offsets of the flags
-    int32_t* cc_label = nullptr;          // [vertices] component ids, then the kept vertices' new indices
-    uint32_t* cc_comp_v = nullptr;        // [vertices] per component: vertices, faces, kept flag
-    uint32_t* cc_comp_f = nullptr;
-    uint8_t* cc_kept = nullptr;
-    uint8_t* cc_keep_f = nullptr;         // [faces]
-    uint32_t* cc_face_counts = nullptr;   // [cdiv(faces, POINT_BLOCK) + 1]
-    s3d::ComponentsState* cc_state = nullptr;
-    int64_t cc_out_alloc_v = 0, cc_out_alloc_f = 0;   // the second surface set, swapped with srf_* after a compaction
-    float* cc_xyz = nullptr;
-    float* cc_nrm = nullptr;
-    uint8_t* cc_rgb = nullptr;
-    int32_t* cc_tri = nullptr;
+    Buf<uint32_t> cc_parent;              // [vertices] union-find forest, then each vertex's root
+    Buf<uint8_t> cc_flags;                // [vertices] root flags, then the vertices' keep flags
+    Buf<uint32_t> cc_vert_counts;         // [cdiv(vertices, POINT_BLOCK) + 1] block offsets of the flags
+    Buf<int32_t> cc_label;                // [vertices] component ids, then the kept vertices' new indices
+    Buf<uint32_t> cc_comp_v;              // [vertices] per component: vertices, faces, kept flag
+    Buf<uint32_t> cc_comp_f;
+    Buf<uint8_t> cc_kept;
+    Buf<uint8_t> cc_keep_f;               // [faces]
+    Buf<uint32_t> cc_face_counts;         // [cdiv(faces, POINT_BLOCK) + 1]
+    Buf<s3d::ComponentsState> cc_state;
+    Buf<float> cc_xyz;                    // the second surface set, swapped with srf_* after a compaction
+    Buf<float> cc_nrm;
+    Buf<uint8_t> cc_rgb;
+    Buf<int32_t> cc_tri;
 
     int cta_limit = 0;             // scan3d_set_cta_limit
 
@@ -238,7 +253,23 @@ struct scan3d_ctx {
     bool in_reconstruct = false;   // stage entries called from scan3d_reconstruct_dev's stage chain
 };
 
+// the C entries' error returns: a failed CUDA call names itself in ctx->err
+#define CK(call)                                                                          \
+    do {                                                                                  \
+        cudaError_t e_ = (call);                                                          \
+        if (e_ != cudaSuccess) {                                                          \
+            ctx->err = std::string(#call) + ": " + cudaGetErrorString(e_);                \
+            return SCAN3D_ERR_CUDA;                                                       \
+        }                                                                                 \
+    } while (0)
+
 namespace s3d {
+
+inline int fail(scan3d_ctx* ctx, int code, const char* msg)
+{
+    if (ctx) ctx->err = msg;
+    return code;
+}
 
 struct Shape {
     int W, H;         // local frame
