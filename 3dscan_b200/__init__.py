@@ -100,6 +100,11 @@ class ComponentsResultC(C.Structure):
                 ("largest_faces", C.c_int64)]
 
 
+class DecimateResultC(C.Structure):
+    _fields_ = [("vertices", C.c_int64), ("faces", C.c_int64), ("collapsed_faces", C.c_int64),
+                ("duplicate_faces", C.c_int64), ("mean_fallbacks", C.c_int64)]
+
+
 # voxel_surface's default max_points per merged voxel: the smallest power of two >= 1.5x the largest lattice points
 # per voxel measured on tools/bench_surface.py's workloads (29.2 on workload A, profiles/r3_bench_surface.json).  64 is
 # also the most a voxel can add (the 4 x 4 x 4 corners of its 27 cells), so the default never overflows; pass
@@ -232,6 +237,7 @@ def cuda_lib():
     L.scan3d_voxel_surface_components.argtypes = [vp, C.POINTER(ComponentsParams), C.POINTER(ComponentsResultC)]
     L.scan3d_get_surface_components.argtypes = [vp, vp, vp, vp, i64]
     L.scan3d_mesh_components_dev.argtypes = [vp, vp, i64, i64, vp, C.POINTER(i64)]
+    L.scan3d_voxel_surface_decimate.argtypes = [vp, C.c_float, C.POINTER(DecimateResultC)]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -702,6 +708,19 @@ class Scan3D:
         self._ck(self.L.scan3d_mesh_components_dev(self.h, C.c_void_p(faces.data_ptr()), faces.shape[0],
                                                    int(n_vertices), C.c_void_p(labels.data_ptr()), C.byref(n)))
         return labels, n.value
+
+    # -- simplification of the voxel surface (include/scan3d.h has the exact rules)
+    def surface_decimate(self, cell_size):
+        """Replace the held voxel surface, in place, by its vertex clustering on a grid of edge cell_size (voxel_size
+        to 256 voxel_size) with quadric placement; synchronises once and returns a dict with vertices, faces,
+        collapsed_faces, duplicate_faces and mean_fallbacks.  voxel_surface_mesh() then returns the simplified
+        surface; the component table goes stale."""
+        r = DecimateResultC()
+        self._ck(self.L.scan3d_voxel_surface_decimate(self.h, float(cell_size), C.byref(r)))
+        self._surface_counts = (r.vertices, r.faces)
+        self._components = 0
+        return dict(vertices=r.vertices, faces=r.faces, collapsed_faces=r.collapsed_faces,
+                    duplicate_faces=r.duplicate_faces, mean_fallbacks=r.mean_fallbacks)
 
     # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
     @staticmethod

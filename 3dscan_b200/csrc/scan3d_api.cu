@@ -15,6 +15,7 @@
 #include "../common/scan3d_aux_math.h"
 #include "../common/scan3d_align_math.h"
 #include "../common/scan3d_surface_math.h"
+#include "../common/scan3d_decimate_math.h"
 
 using namespace s3d;
 
@@ -1334,6 +1335,7 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
     ctx->srf_vertices = st.vertices;
     ctx->srf_faces = st.faces;
     ctx->srf_ready = true;
+    ctx->srf_decimated = false;
     out->vertices = st.vertices;
     out->faces = st.faces;
     out->lattice_points = st.occupied;
@@ -1480,6 +1482,82 @@ int scan3d_mesh_components_dev(scan3d_ctx* ctx, const int32_t* faces_dev, int64_
     CK(cudaStreamSynchronize(ctx->stream));
     if (st.bad) return fail(ctx, SCAN3D_ERR_ARG, "a face index outside [0, n_vertices)");
     *components_out = st.components;
+    return SCAN3D_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// simplification of the voxel surface (include/scan3d.h and common/scan3d_decimate_math.h have the exact rules)
+// ------------------------------------------------------------------------------------------
+int scan3d_voxel_surface_decimate(scan3d_ctx* ctx, float cell_size, scan3d_decimate_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (!(cell_size - cell_size == 0.0f)) return fail(ctx, SCAN3D_ERR_ARG, "cell_size must be finite");
+    if (!ctx->srf_ready)
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    const double H = (double)cell_size, s = ctx->vox.S;
+    if (!(H >= s && H <= s3q::RATIO_MAX * s))
+        return fail(ctx, SCAN3D_ERR_ARG, "cell_size must be in [voxel_size, 256 voxel_size]");
+    if (ctx->srf_decimated)
+        return fail(ctx, SCAN3D_ERR_STATE, "the held surface is already simplified: extract it again first");
+    const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
+    if (nf >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^31 - 1 surface faces");
+    CK(cudaSetDevice(ctx->device));
+    ctx->cc_ready = false;
+    // the cluster table, sized as scan3d_voxel_begin sizes the merge's for max_voxels = the vertex count
+    const uint32_t maxv = (uint32_t)std::max<int64_t>(nv, 1);
+    const size_t av = maxv, af = (size_t)std::max<int64_t>(nf, 1);
+    VoxelTable& t = ctx->dec;
+    const uint32_t cap = voxel_table_capacity(maxv, ctx->sm_count);
+    CK(grow_group(Grow(ctx->dec_keys, cap), Grow(ctx->dec_acc, cap), Grow(ctx->dec_ordinal, cap)));
+    CK(grow_group(Grow(ctx->dec_ord2slot, av), Grow(ctx->dec_point_slot, av), Grow(ctx->dec_vert_flags, av),
+                  Grow(ctx->dec_vert_counts, (av + POINT_BLOCK - 1) / POINT_BLOCK + 1),
+                  Grow(ctx->dec_quad, s3q::NQ * av)));
+    CK(grow_group(Grow(ctx->dec_ctri, 3 * af), Grow(ctx->dec_table, 2 * af), Grow(ctx->dec_slot_of, af),
+                  Grow(ctx->dec_keep, af), Grow(ctx->dec_face_counts, (af + POINT_BLOCK - 1) / POINT_BLOCK + 1)));
+    CK(ctx->dec_vstate.ensure(1));
+    CK(ctx->dec_state.ensure(1));
+    // the emission runs before the synchronisation, so the second set holds the whole input
+    CK(grow_group(Grow(ctx->cc_xyz, 3 * av), Grow(ctx->cc_nrm, 3 * av), Grow(ctx->cc_rgb, 3 * av)));
+    CK(ctx->cc_tri.ensure(3 * af));
+    t.keys = ctx->dec_keys; t.acc = ctx->dec_acc; t.ordinal = ctx->dec_ordinal;
+    t.ord2slot = ctx->dec_ord2slot; t.state = ctx->dec_vstate;
+    t.cap = cap;
+    t.max_voxels = maxv;
+    t.S = H;
+    DecimateBuffers b;
+    b.point_slot = ctx->dec_point_slot; b.vert_flags = ctx->dec_vert_flags; b.vert_counts = ctx->dec_vert_counts;
+    b.quad = ctx->dec_quad; b.ctri = ctx->dec_ctri; b.table = ctx->dec_table; b.table_cap = (uint32_t)(2 * af);
+    b.slot_of = ctx->dec_slot_of; b.keep = ctx->dec_keep; b.face_counts = ctx->dec_face_counts;
+    b.state = ctx->dec_state;
+    CK(cudaMemsetAsync(t.keys, 0xff, (size_t)cap * sizeof(*t.keys), ctx->stream));
+    CK(cudaMemsetAsync(t.acc, 0, (size_t)cap * sizeof(*t.acc), ctx->stream));
+    CK(cudaMemsetAsync(t.ordinal, 0xff, (size_t)cap * sizeof(*t.ordinal), ctx->stream));
+    CK(cudaMemsetAsync(t.state, 0, sizeof(*t.state), ctx->stream));
+    CK(cudaMemsetAsync(b.quad, 0, s3q::NQ * av * sizeof(*b.quad), ctx->stream));
+    CK(cudaMemsetAsync(b.table, 0xff, (size_t)b.table_cap * sizeof(*b.table), ctx->stream));
+    CK(cudaMemsetAsync(b.state, 0, sizeof(*b.state), ctx->stream));
+    CK(launch_decimate(t, b, ctx->srf_xyz, ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri, (uint32_t)nv, (uint32_t)nf, H,
+                       ctx->cc_xyz, ctx->cc_nrm, ctx->cc_rgb, ctx->cc_tri, ctx->sm_count, ctx->stream));
+    ctx->launches += DECIMATE_LAUNCHES;
+    DecimateState st;
+    VoxelState vst;
+    CK(cudaMemcpyAsync(&st, b.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&vst, t.state, sizeof(vst), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    // the simplified set becomes the held surface; the old one is the next compaction's destination
+    std::swap(ctx->srf_xyz, ctx->cc_xyz);
+    std::swap(ctx->srf_nrm, ctx->cc_nrm);
+    std::swap(ctx->srf_rgb, ctx->cc_rgb);
+    std::swap(ctx->srf_tri, ctx->cc_tri);
+    ctx->srf_vertices = vst.total[1];
+    ctx->srf_faces = st.faces;
+    ctx->srf_decimated = true;
+    out->vertices = vst.total[1];
+    out->faces = st.faces;
+    out->collapsed_faces = st.collapsed;
+    out->duplicate_faces = nf - st.collapsed - st.faces;
+    out->mean_fallbacks = st.fallbacks;
     return SCAN3D_OK;
 }
 

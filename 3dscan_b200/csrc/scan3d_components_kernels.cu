@@ -78,19 +78,6 @@ __device__ __forceinline__ bool keep_component(const uint32_t* comp_f, const Com
     return f >= min_faces && key_of(f, c) >= st->threshold;
 }
 
-// rank of this thread's flag among the flags of its POINT_BLOCK block (every thread of the block calls it)
-__device__ __forceinline__ uint32_t block_rank(bool flag)
-{
-    __shared__ uint32_t wsum[POINT_BLOCK / 32];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const unsigned b = __ballot_sync(FULL, flag);
-    if (lane == 0) wsum[w] = __popc(b);
-    __syncthreads();
-    uint32_t before = 0;
-    for (int k = 0; k < w; k++) before += wsum[k];
-    return before + __popc(b & ((1u << lane) - 1));
-}
-
 }  // namespace
 
 __global__ void __launch_bounds__(CT) k_cc_init(uint32_t* __restrict__ parent, uint32_t n)

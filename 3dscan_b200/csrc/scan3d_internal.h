@@ -102,6 +102,27 @@ struct ComponentsState {
     uint32_t bad;                  // a face index outside [0, vertices)
     uint32_t pad;
 };
+
+// the surface simplification (scan3d_decimate_kernels.cu); the clusters are a second VoxelTable
+struct DecimateState {
+    uint32_t collapsed;            // faces with two corners in one cluster
+    uint32_t fallbacks;            // clusters placed at their mean after a failed solve
+    uint32_t faces;                // kept faces
+    uint32_t zero;                 // stays 0: the vertex count of an empty surface's voxel add
+};
+struct DecimateBuffers {
+    uint32_t* point_slot;          // [vertices] cluster slot of each vertex
+    uint8_t* vert_flags;           // [vertices]
+    uint32_t* vert_counts;         // [cdiv(vertices, POINT_BLOCK) + 1]
+    unsigned long long* quad;      // [vertices][10] quadric sums per cluster ordinal (int64 two's complement), zeroed
+    int32_t* ctri;                 // [faces][3] cluster ordinals of the corners
+    uint32_t* table;               // [table_cap] face indices, VOXEL_NO_SLOT = free
+    uint32_t table_cap;
+    uint32_t* slot_of;             // [faces] table slot of each face, VOXEL_NO_SLOT = collapsed
+    uint8_t* keep;                 // [faces]
+    uint32_t* face_counts;         // [cdiv(faces, POINT_BLOCK) + 1]
+    DecimateState* state;          // zeroed
+};
 }  // namespace s3d
 
 // Every device buffer the context owns is a DeviceBuffer: scan3d_destroy frees them all by deleting the context.
@@ -239,6 +260,26 @@ struct scan3d_ctx {
     Buf<uint8_t> cc_rgb;
     Buf<int32_t> cc_tri;
 
+    // scan3d_voxel_surface_decimate (allocated on first use, grown on demand); dec is the kernels' view of the cluster
+    // table dec_keys ... dec_state, never the merge's ctx->vox.  The emission writes the components' second set.
+    bool srf_decimated = false;           // the held surface is a simplification (it is not simplified again)
+    s3d::VoxelTable dec{};
+    Buf<unsigned long long> dec_keys;     // [cap] the cluster table
+    Buf<s3d::VoxelSlot> dec_acc;          // [cap]
+    Buf<uint32_t> dec_ordinal;            // [cap]
+    Buf<uint32_t> dec_ord2slot;           // [vertices]
+    Buf<s3d::VoxelState> dec_vstate;
+    Buf<uint32_t> dec_point_slot;         // [vertices]
+    Buf<uint8_t> dec_vert_flags;          // [vertices]
+    Buf<uint32_t> dec_vert_counts;        // [cdiv(vertices, POINT_BLOCK) + 1]
+    Buf<unsigned long long> dec_quad;     // [vertices][10]
+    Buf<int32_t> dec_ctri;                // [faces][3]
+    Buf<uint32_t> dec_table;              // [2 faces]
+    Buf<uint32_t> dec_slot_of;            // [faces]
+    Buf<uint8_t> dec_keep;                // [faces]
+    Buf<uint32_t> dec_face_counts;        // [cdiv(faces, POINT_BLOCK) + 1]
+    Buf<s3d::DecimateState> dec_state;
+
     int cta_limit = 0;             // scan3d_set_cta_limit
 
     // scan3d_set_registration
@@ -313,6 +354,20 @@ cudaError_t launch_point_offsets(const uint8_t* valid, size_t plane, uint32_t* b
                                  cudaStream_t st);
 // exclusive scan of counts[n] in place by one CTA (k_scan), *total = the sum; 1 launch
 cudaError_t launch_block_scan(uint32_t* counts, int n, uint32_t* total, cudaStream_t st);
+
+// rank of this thread's flag among the flags of its POINT_BLOCK block (every thread of the block calls it); with the
+// block offsets of launch_point_offsets this places a flagged item at its compacted position
+__device__ __forceinline__ uint32_t block_rank(bool flag)
+{
+    __shared__ uint32_t wsum[POINT_BLOCK / 32];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const unsigned b = __ballot_sync(0xffffffffu, flag);
+    if (lane == 0) wsum[w] = __popc(b);
+    __syncthreads();
+    uint32_t before = 0;
+    for (int k = 0; k < w; k++) before += wsum[k];
+    return before + __popc(b & ((1u << lane) - 1));
+}
 // 3 launches: count, scan, scatter.  pix / rgb / texture may be null.
 cudaError_t launch_compact(const Shape& s, const double* xyz, const uint8_t* valid,
                            const uint8_t* texture, uint32_t* block_counts, float* pts, uint32_t* pix,
@@ -449,6 +504,17 @@ cudaError_t launch_cc_emit(const uint8_t* keep_v, const uint32_t* vert_counts, u
                            const float* nrm, const uint8_t* rgb, const uint8_t* keep_f, const uint32_t* face_counts,
                            uint32_t n_faces, const int32_t* faces, int32_t* new_index, float* xyz2, float* nrm2,
                            uint8_t* rgb2, int32_t* faces2, cudaStream_t st);
+
+// ---- surface simplification (scan3d_decimate_kernels.cu; common/scan3d_decimate_math.h has the arithmetic) ----
+// DECIMATE_LAUNCHES launches for a surface of n_vertices (xyz, nrm, rgb) and n_faces (tri): launch_voxel_add over the
+// vertices into t (the clusters, edge t.S = H; t must be reset as scan3d_voxel_begin resets the merge's table, with
+// max_voxels >= max(n_vertices, 1)), the face quadrics with the cluster triples, the duplicate-face table, the keep
+// flags, k_count + k_scan over them (b.state->faces), then the vertices of the clusters into xyz2 / nrm2 / rgb2 [n_vertices]
+// and the kept faces into faces2 [n_faces].  b.quad, b.state zeroed and b.table set to 0xff before.
+constexpr int DECIMATE_LAUNCHES = VOXEL_ADD_LAUNCHES + 7;
+cudaError_t launch_decimate(const VoxelTable& t, const DecimateBuffers& b, const float* xyz, const float* nrm,
+                            const uint8_t* rgb, const int32_t* tri, uint32_t n_vertices, uint32_t n_faces, double H,
+                            float* xyz2, float* nrm2, uint8_t* rgb2, int32_t* faces2, int sm_count, cudaStream_t st);
 
 // ---- debug / self-test ----
 cudaError_t launch_debug_atan2(const double* y, const double* x, float* out, int n, int mode,

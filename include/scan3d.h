@@ -501,6 +501,62 @@ int scan3d_get_surface_components(scan3d_ctx *ctx, int64_t *vertices, int64_t *f
 int scan3d_mesh_components_dev(scan3d_ctx *ctx, const int32_t *faces_dev, int64_t n_faces, int64_t n_vertices,
                                int32_t *label_dev, int64_t *components_out);
 
+/* ---- simplification of the voxel surface: vertex clustering on a coarser grid with quadric placement (Rossignac &
+ * Borrel 1993; Lindstrom 2000) ---------------------------------------------------------------------------------------
+ * scan3d_voxel_surface_decimate replaces the held voxel surface in place by its simplification: scan3d_get_voxel_surface,
+ * scan3d_write_voxel_surface_ply and scan3d_voxel_surface_components then work on the simplified surface.  The result
+ * is a pure function of the held surface and cell_size: bit-reproducible, independent of scheduling and SM count.
+ *
+ * s = the voxel_size of the last scan3d_voxel_begin, H = (double)cell_size, r = H / s in [1, 256].
+ * Cluster: a vertex's voxel of edge H in the merge's sense (per axis t = (double)x / H, i = floor(t), fraction
+ * f = t - i in [0, 1]; the merge's key range).  Clusters are numbered in order of their first vertex (the merge's order
+ * rule).  Each cluster becomes one output vertex, at the cluster's ordinal: its normal and colour are the merge's rules
+ * over the cluster's vertices (the vertex normals as the points' normals, the vertex colours as their colours); its
+ * position is the placement below.  Every cluster is output, including clusters that no kept face uses: a later
+ * scan3d_voxel_surface_components with min_faces = 1 removes those.
+ * Face quadric: for a face (a, b, c), d1 = p_b - p_a, d2 = p_c - p_a per axis in double; n = (d1y d2z - d1z d2y,
+ * d1z d2x - d1x d2z, d1x d2y - d1y d2x); l2 = (nx nx + ny ny) + nz nz.  l2 == 0: the face adds no quadric (it still
+ * counts for the faces below).  Else u = n / sqrt(l2) and w = (sqrt(l2) * 0.5) / (H * H), the face's area in cell units.
+ * Each corner k, with its fractions f_k in its own cluster, has e = (u_x f_x + u_y f_y) + u_z f_z and adds the 10
+ * coefficients (w * c_j) for c = (u_x u_x, u_x u_y, u_x u_z, u_y u_y, u_y u_z, u_z u_z, u_x e, u_y e, u_z e, e e), each
+ * rounded to the int64 rint((w * c_j) * 2^40), half to even, to its cluster's sums (int64, two's complement; the bound
+ * that keeps them below 2^63 for r in [1, 256] is derived in 3dscan_b200/common/scan3d_decimate_math.h).
+ * Placement: A = the symmetric 3x3 matrix of the first 6 sums * 2^-40 (A00, A01, A02, A11, A12, A22), b = the next 3
+ * * 2^-40; ybar = the cluster's mean in cell units from the merge's sums, sum q_a / (2^24 n).  tr = (A00 + A11) + A22;
+ * tr == 0: y = ybar.  Else mu = 1e-3 * (tr / 3) and (A + mu I) y = b + mu ybar is solved by the alignment's LDL^T
+ * (pivot test: mu finite and > 0, every pivot > mu / 2).  When the pivot test fails, or some y_a is not finite or not
+ * in [0, 1], y = ybar and the cluster counts in mean_fallbacks.  The output coordinate is (float)(((double)i_a + y_a)
+ * * H).  The exact operation order is in 3dscan_b200/common/scan3d_decimate_math.h.
+ * Faces: face (a, b, c) maps to (C(a), C(b), C(c)), the cluster ordinals.  A face with two of them equal is dropped
+ * (collapsed_faces).  The canonical triple is the cyclic rotation that puts the smallest ordinal first, which keeps
+ * the winding; of the faces with the same canonical triple the first by face index is kept, the others are dropped
+ * (duplicate_faces).  Opposite windings are different triples, so both are kept.  Kept faces keep their relative
+ * order and their rotation.  The output can be non-manifold where a cluster joins two sheets of the surface.
+ * State: needs a held surface (SCAN3D_ERR_STATE otherwise).  A surface is simplified once: a second call returns
+ * SCAN3D_ERR_STATE until a new scan3d_voxel_surface (the overflow bound rests on surface-nets faces).  Components
+ * before and after are allowed; the call makes the component table stale.  A later begin, add or finish makes the
+ * surface stale as before; an align touches neither; the accumulator is never changed.
+ * Synchronisation: one, after every launch, when the counts are known; *out is then filled and the simplified set
+ * swapped in.
+ * Launches: always 12, an empty surface included: 5 (the merge's add over the vertices), the face quadrics, the
+ * duplicate-face table, the keep flags, k_count + k_scan over them, the vertices (placement), the faces.
+ * Memory (ctx-owned, allocated on first use, grown on demand): about 275 B per vertex (the cluster table at ~184 B, the
+ * quadric sums indexed by cluster ordinal at 80 B, 9 B of scratch) and 25 B per face (cluster triples, duplicate
+ * table, slots and flags), plus the components' second surface set, grown to 27 B per vertex and 12 B per face of the
+ * input, which is swapped with the held one.
+ * Errors: SCAN3D_ERR_ARG for a null ctx or out, a cell_size that is not finite, and (with a held surface) cell_size <
+ * voxel_size or > 256 voxel_size; SCAN3D_ERR_CONFIG for a surface of 2^31 faces or more.  An argument, state or
+ * size error launches nothing and leaves the surface as it was.  An empty surface gives 0 vertices and 0 faces,
+ * with SCAN3D_OK. */
+typedef struct {
+    int64_t vertices, faces;     /* of the surface after the call */
+    int64_t collapsed_faces;     /* dropped: two corners in one cluster */
+    int64_t duplicate_faces;     /* dropped: same oriented cluster triple as an earlier face */
+    int64_t mean_fallbacks;      /* clusters placed at their mean instead of the quadric minimum */
+} scan3d_decimate_result;
+
+int scan3d_voxel_surface_decimate(scan3d_ctx *ctx, float cell_size, scan3d_decimate_result *out);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,
