@@ -105,6 +105,15 @@ class DecimateResultC(C.Structure):
                 ("duplicate_faces", C.c_int64), ("mean_fallbacks", C.c_int64)]
 
 
+class SmoothParams(C.Structure):
+    _fields_ = [("iterations", C.c_int32), ("lam", C.c_float), ("mu", C.c_float)]
+
+
+class SmoothResultC(C.Structure):
+    _fields_ = [("vertices", C.c_int64), ("faces", C.c_int64), ("held_vertices", C.c_int64),
+                ("isolated_vertices", C.c_int64), ("passes", C.c_int64), ("max_displacement", C.c_double)]
+
+
 # voxel_surface's default max_points per merged voxel: the smallest power of two >= 1.5x the largest lattice points
 # per voxel measured on tools/bench_surface.py's workloads (29.2 on workload A, profiles/r3_bench_surface.json).  64 is
 # also the most a voxel can add (the 4 x 4 x 4 corners of its 27 cells), so the default never overflows; pass
@@ -238,6 +247,8 @@ def cuda_lib():
     L.scan3d_get_surface_components.argtypes = [vp, vp, vp, vp, i64]
     L.scan3d_mesh_components_dev.argtypes = [vp, vp, i64, i64, vp, C.POINTER(i64)]
     L.scan3d_voxel_surface_decimate.argtypes = [vp, C.c_float, C.POINTER(DecimateResultC)]
+    L.scan3d_voxel_surface_smooth.argtypes = [vp, C.POINTER(SmoothParams), C.POINTER(SmoothResultC)]
+    L.scan3d_mesh_smooth_dev.argtypes = [vp, vp, vp, i64, vp, i64, C.POINTER(SmoothParams), C.POINTER(SmoothResultC)]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -721,6 +732,46 @@ class Scan3D:
         self._components = 0
         return dict(vertices=r.vertices, faces=r.faces, collapsed_faces=r.collapsed_faces,
                     duplicate_faces=r.duplicate_faces, mean_fallbacks=r.mean_fallbacks)
+
+    # -- smoothing of the voxel surface and of device meshes (include/scan3d.h has the exact rules)
+    @staticmethod
+    def _smooth_result(r):
+        return dict(vertices=r.vertices, faces=r.faces, held_vertices=r.held_vertices,
+                    isolated_vertices=r.isolated_vertices, passes=r.passes, max_displacement=r.max_displacement)
+
+    def surface_smooth(self, iterations=10, lam=0.5, mu=-0.53):
+        """Taubin lambda|mu smoothing of the held voxel surface, in place (MeshLab's defaults); boundary and
+        non-manifold vertices are held.  Synchronises once and returns a dict with vertices, faces, held_vertices,
+        isolated_vertices, passes and max_displacement.  voxel_surface_mesh() then returns the smoothed surface; the
+        component table stays valid."""
+        r = SmoothResultC()
+        self._ck(self.L.scan3d_voxel_surface_smooth(self.h, C.byref(SmoothParams(int(iterations), lam, mu)),
+                                                    C.byref(r)))
+        self._surface_counts = (r.vertices, r.faces)
+        return self._smooth_result(r)
+
+    def mesh_smooth_dev(self, xyz, faces, normals=None, iterations=10, lam=0.5, mu=-0.53):
+        """surface_smooth() for a triangle mesh on the ctx's GPU, in place: xyz a CUDA float32 tensor [v][3], faces a
+        CUDA int32 tensor [f][3], normals None or a CUDA float32 tensor [v][3] (then recomputed).  torch's current
+        stream is synchronised first, so data written there is ready.  Returns the dict of surface_smooth()."""
+        import torch
+
+        def ok(t, dtype, rows):
+            return (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dtype and t.dim() == 2 and
+                    t.shape[1] == 3 and t.is_contiguous() and (rows is None or t.shape[0] == rows))
+        if not ok(xyz, torch.float32, None):
+            raise Scan3DError("xyz must be a contiguous CUDA float32 tensor of shape [v][3]")
+        if not ok(faces, torch.int32, None):
+            raise Scan3DError("faces must be a contiguous CUDA int32 tensor of shape [f][3]")
+        if normals is not None and not ok(normals, torch.float32, xyz.shape[0]):
+            raise Scan3DError("normals must be None or a contiguous CUDA float32 tensor of the shape of xyz")
+        torch.cuda.current_stream(xyz.device).synchronize()
+        r = SmoothResultC()
+        self._ck(self.L.scan3d_mesh_smooth_dev(self.h, C.c_void_p(xyz.data_ptr()),
+                                               None if normals is None else C.c_void_p(normals.data_ptr()),
+                                               xyz.shape[0], C.c_void_p(faces.data_ptr()), faces.shape[0],
+                                               C.byref(SmoothParams(int(iterations), lam, mu)), C.byref(r)))
+        return self._smooth_result(r)
 
     # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
     @staticmethod

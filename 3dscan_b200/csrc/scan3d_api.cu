@@ -1336,6 +1336,7 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
     ctx->srf_faces = st.faces;
     ctx->srf_ready = true;
     ctx->srf_decimated = false;
+    ctx->srf_smoothed = false;
     out->vertices = st.vertices;
     out->faces = st.faces;
     out->lattice_points = st.occupied;
@@ -1500,6 +1501,8 @@ int scan3d_voxel_surface_decimate(scan3d_ctx* ctx, float cell_size, scan3d_decim
         return fail(ctx, SCAN3D_ERR_ARG, "cell_size must be in [voxel_size, 256 voxel_size]");
     if (ctx->srf_decimated)
         return fail(ctx, SCAN3D_ERR_STATE, "the held surface is already simplified: extract it again first");
+    if (ctx->srf_smoothed)
+        return fail(ctx, SCAN3D_ERR_STATE, "the held surface is smoothed: extract it again to simplify it");
     const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
     if (nf >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^31 - 1 surface faces");
     CK(cudaSetDevice(ctx->device));
@@ -1559,6 +1562,102 @@ int scan3d_voxel_surface_decimate(scan3d_ctx* ctx, float cell_size, scan3d_decim
     out->duplicate_faces = nf - st.collapsed - st.faces;
     out->mean_fallbacks = st.fallbacks;
     return SCAN3D_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// smoothing of the voxel surface and of device meshes (include/scan3d.h and common/scan3d_smooth_math.h have the exact
+// rules)
+// ------------------------------------------------------------------------------------------
+static int check_smooth_args(scan3d_ctx* ctx, const scan3d_smooth_params* p, scan3d_smooth_result* out)
+{
+    if (!p || !out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (p->iterations < 0 || p->iterations > SCAN3D_SMOOTH_MAX_ITERATIONS)
+        return fail(ctx, SCAN3D_ERR_ARG, "iterations must be in [0, 4096]");
+    if (!(p->lambda > 0.0f && p->lambda <= 1.0f)) return fail(ctx, SCAN3D_ERR_ARG, "lambda must be in (0, 1]");
+    if (!(p->mu >= -1.0f && p->mu <= 0.0f)) return fail(ctx, SCAN3D_ERR_ARG, "mu must be in [-1, 0]");
+    return SCAN3D_OK;
+}
+
+// smooths the mesh (xyz, nrm, faces) into xyz_out / nrm_out (the same buffers or others; nrm and nrm_out may be null);
+// one synchronisation; on an error found on the device nothing is written
+static int smooth_run(scan3d_ctx* ctx, const float* xyz, const float* nrm, const int32_t* faces, int64_t nv, int64_t nf,
+                      const scan3d_smooth_params* p, float* xyz_out, float* nrm_out, scan3d_smooth_result* out)
+{
+    if (6 * nf >= (1LL << 32)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than (2^32 - 1) / 6 faces");
+    const int passes = p->iterations * (p->mu == 0.0f ? 1 : 2);
+    const size_t av = (size_t)std::max<int64_t>(nv, 1);
+    const uint32_t cap = (uint32_t)std::max<int64_t>(6 * nf, 64);   // two slots per side: at most half are taken
+    CK(grow_group(Grow(ctx->sm_keys, cap), Grow(ctx->sm_sides, cap), Grow(ctx->sm_rows, cap)));
+    CK(grow_group(Grow(ctx->sm_degree, av), Grow(ctx->sm_held, av),
+                  Grow(ctx->sm_block_counts, (av + POINT_BLOCK - 1) / POINT_BLOCK + 1), Grow(ctx->sm_cursor, av),
+                  Grow(ctx->sm_q[0], 3 * av), Grow(ctx->sm_q[1], 3 * av)));
+    CK(ctx->sm_nsum.ensure(3 * av));
+    CK(ctx->sm_state.ensure(1));
+    SmoothBuffers b;
+    b.keys = ctx->sm_keys; b.sides = ctx->sm_sides; b.cap = cap; b.rows = ctx->sm_rows;
+    b.degree = ctx->sm_degree; b.held = ctx->sm_held; b.block_counts = ctx->sm_block_counts; b.cursor = ctx->sm_cursor;
+    b.q[0] = ctx->sm_q[0]; b.q[1] = ctx->sm_q[1]; b.nsum = ctx->sm_nsum; b.state = ctx->sm_state;
+    CK(cudaMemsetAsync(b.keys, 0xff, (size_t)cap * sizeof(*b.keys), ctx->stream));
+    CK(cudaMemsetAsync(b.sides, 0, (size_t)cap * sizeof(*b.sides), ctx->stream));
+    CK(cudaMemsetAsync(b.degree, 0, av * sizeof(*b.degree), ctx->stream));
+    CK(cudaMemsetAsync(b.held, 0, av * sizeof(*b.held), ctx->stream));
+    CK(cudaMemsetAsync(b.nsum, 0, 3 * av * sizeof(*b.nsum), ctx->stream));
+    CK(cudaMemsetAsync(b.state, 0, sizeof(*b.state), ctx->stream));
+    CK(launch_smooth(b, xyz, nrm, faces, (uint32_t)nv, (uint32_t)nf, passes, (double)p->lambda, (double)p->mu, xyz_out,
+                     nrm_out, ctx->stream));
+    ctx->launches += SMOOTH_BUILD_LAUNCHES + passes + SMOOTH_END_LAUNCHES;
+    SmoothState st;
+    CK(cudaMemcpyAsync(&st, b.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st.bad) return fail(ctx, SCAN3D_ERR_ARG, "a coordinate that is not finite or a face index outside [0, n_vertices)");
+    if (st.overflow)
+        return fail(ctx, SCAN3D_ERR_CONFIG,
+                    "a free vertex with more than 2^20 neighbours, or moved beyond the fixed-point limit");
+    out->vertices = nv;
+    out->faces = nf;
+    out->held_vertices = st.held;
+    out->isolated_vertices = st.isolated;
+    out->passes = passes;
+    double move;
+    memcpy(&move, &st.max_move, sizeof(move));
+    out->max_displacement = move;
+    return SCAN3D_OK;
+}
+
+int scan3d_voxel_surface_smooth(scan3d_ctx* ctx, const scan3d_smooth_params* p, scan3d_smooth_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    int rc = check_smooth_args(ctx, p, out);
+    if (rc) return rc;
+    if (!ctx->srf_ready)
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    CK(cudaSetDevice(ctx->device));
+    const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
+    const size_t av3 = 3 * (size_t)std::max<int64_t>(nv, 1);
+    CK(grow_group(Grow(ctx->cc_xyz, av3), Grow(ctx->cc_nrm, av3)));
+    rc = smooth_run(ctx, ctx->srf_xyz, ctx->srf_nrm, ctx->srf_tri, nv, nf, p, ctx->cc_xyz, ctx->cc_nrm, out);
+    if (rc) return rc;
+    // the smoothed positions and normals become the held surface; faces, colours and the vertex order are unchanged
+    std::swap(ctx->srf_xyz, ctx->cc_xyz);
+    std::swap(ctx->srf_nrm, ctx->cc_nrm);
+    ctx->srf_smoothed = true;
+    return SCAN3D_OK;
+}
+
+int scan3d_mesh_smooth_dev(scan3d_ctx* ctx, float* xyz_dev, float* normals_dev, int64_t n_vertices,
+                           const int32_t* faces_dev, int64_t n_faces, const scan3d_smooth_params* p,
+                           scan3d_smooth_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    const int rc = check_smooth_args(ctx, p, out);
+    if (rc) return rc;
+    if (n_faces < 0 || n_faces >= (1LL << 31) || n_vertices < 0 || n_vertices >= (1LL << 31))
+        return fail(ctx, SCAN3D_ERR_ARG, "n_faces and n_vertices must be in [0, 2^31)");
+    if ((!xyz_dev && n_vertices > 0) || (!faces_dev && n_faces > 0)) return fail(ctx, SCAN3D_ERR_ARG, "null device pointer");
+    if (((uintptr_t)xyz_dev & 3) || ((uintptr_t)normals_dev & 3) || ((uintptr_t)faces_dev & 3))
+        return fail(ctx, SCAN3D_ERR_ARG, "xyz_dev, normals_dev and faces_dev must be 4-byte aligned");
+    CK(cudaSetDevice(ctx->device));
+    return smooth_run(ctx, xyz_dev, normals_dev, faces_dev, n_vertices, n_faces, p, xyz_dev, normals_dev, out);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -123,6 +123,29 @@ struct DecimateBuffers {
     uint32_t* face_counts;         // [cdiv(faces, POINT_BLOCK) + 1]
     DecimateState* state;          // zeroed
 };
+
+// the surface smoothing (scan3d_smooth_kernels.cu); the undirected edges are a hash of (min << 32 | max) keys
+struct SmoothState {
+    unsigned long long max_move;   // bits of the largest displacement (a non-negative double, so the bits order it)
+    uint32_t exp_field;            // the largest biased float exponent field of the coordinates
+    uint32_t bad;                  // a coordinate not finite or a face index outside [0, vertices): SCAN3D_ERR_ARG
+    uint32_t overflow;             // a free vertex over a limit of common/scan3d_smooth_math.h: SCAN3D_ERR_CONFIG
+    uint32_t held, isolated;       // vertices on an edge whose count is not 2; vertices without a neighbour
+    uint32_t entries;              // neighbour row entries (the sum of the degrees)
+};
+struct SmoothBuffers {
+    unsigned long long* keys;      // [cap] edge keys, s3v::EMPTY_KEY = free
+    uint32_t* sides;               // [cap] sides on each edge, zeroed
+    uint32_t cap;
+    uint32_t* degree;              // [vertices] distinct neighbours, zeroed
+    uint8_t* held;                 // [vertices] zeroed
+    uint32_t* block_counts;        // [cdiv(vertices, POINT_BLOCK) + 1]
+    uint32_t* cursor;              // [vertices] row start, then (after the scatter) row end
+    uint32_t* rows;                // [cap] neighbour indices (2 per edge, at most 2 * 3 nf)
+    long long* q[2];               // [vertices][3] fixed-point positions, ping-pong
+    unsigned long long* nsum;      // [vertices][3] fixed-point normal sums (int64 two's complement), zeroed
+    SmoothState* state;            // zeroed
+};
 }  // namespace s3d
 
 // Every device buffer the context owns is a DeviceBuffer: scan3d_destroy frees them all by deleting the context.
@@ -279,6 +302,20 @@ struct scan3d_ctx {
     Buf<uint8_t> dec_keep;                // [faces]
     Buf<uint32_t> dec_face_counts;        // [cdiv(faces, POINT_BLOCK) + 1]
     Buf<s3d::DecimateState> dec_state;
+
+    // scan3d_voxel_surface_smooth / scan3d_mesh_smooth_dev (allocated on first use, grown on demand).  The surface
+    // route writes the components' second set's xyz and normals.
+    bool srf_smoothed = false;            // the held surface is smoothed (scan3d_voxel_surface_decimate refuses it)
+    Buf<unsigned long long> sm_keys;      // [6 faces] the edge table
+    Buf<uint32_t> sm_sides;               // [6 faces]
+    Buf<uint32_t> sm_rows;                // [6 faces]
+    Buf<uint32_t> sm_degree;              // [vertices]
+    Buf<uint8_t> sm_held;                 // [vertices]
+    Buf<uint32_t> sm_block_counts;        // [cdiv(vertices, POINT_BLOCK) + 1]
+    Buf<uint32_t> sm_cursor;              // [vertices]
+    Buf<long long> sm_q[2];               // [vertices][3]
+    Buf<unsigned long long> sm_nsum;      // [vertices][3]
+    Buf<s3d::SmoothState> sm_state;
 
     int cta_limit = 0;             // scan3d_set_cta_limit
 
@@ -515,6 +552,20 @@ constexpr int DECIMATE_LAUNCHES = VOXEL_ADD_LAUNCHES + 7;
 cudaError_t launch_decimate(const VoxelTable& t, const DecimateBuffers& b, const float* xyz, const float* nrm,
                             const uint8_t* rgb, const int32_t* tri, uint32_t n_vertices, uint32_t n_faces, double H,
                             float* xyz2, float* nrm2, uint8_t* rgb2, int32_t* faces2, int sm_count, cudaStream_t st);
+
+// ---- surface smoothing (scan3d_smooth_kernels.cu; common/scan3d_smooth_math.h has the arithmetic) ----
+// SMOOTH_BUILD_LAUNCHES + passes + SMOOTH_END_LAUNCHES launches for n vertices (xyz, nrm may be null) and nf faces
+// [nf][3]: the exponent max and the finiteness check over the vertices, the sides into the edge table, the degrees and
+// held flags per edge, the degree sums per POINT_BLOCK vertices, their k_scan, the row starts with the fixed-point
+// positions, the neighbour rows; then one gather per pass (k = lambda, or lambda and mu alternating when mu != 0);
+// then the face normals and the write of xyz_out / nrm_out (nrm_out may be null), which writes nothing when the state
+// holds an error.  xyz_out may be xyz and nrm_out nrm.  b.keys 0xff; b.sides, b.degree, b.held, b.nsum, b.state zeroed
+// before; b.cap >= 2 * 3 nf.
+constexpr int SMOOTH_BUILD_LAUNCHES = 7;
+constexpr int SMOOTH_END_LAUNCHES = 2;
+cudaError_t launch_smooth(const SmoothBuffers& b, const float* xyz, const float* nrm, const int32_t* faces, uint32_t n,
+                          uint32_t nf, int passes, double lambda, double mu, float* xyz_out, float* nrm_out,
+                          cudaStream_t st);
 
 // ---- debug / self-test ----
 cudaError_t launch_debug_atan2(const double* y, const double* x, float* out, int n, int mode,

@@ -557,6 +557,78 @@ typedef struct {
 
 int scan3d_voxel_surface_decimate(scan3d_ctx *ctx, float cell_size, scan3d_decimate_result *out);
 
+/* ---- smoothing of the voxel surface and of device meshes: Taubin lambda|mu fairing with the uniform umbrella
+ * operator (Taubin 1995), boundaries held ------------------------------------------------------------------------------
+ * The result is a pure function of the mesh and the parameters: bit-reproducible, independent of scheduling, of the
+ * hash and of the SM count.  The exact operation order is in 3dscan_b200/common/scan3d_smooth_math.h.
+ *
+ * Neighbours: each face (a, b, c) contributes its sides (a, b), (b, c), (c, a); a side with equal ends is skipped.
+ * Two vertices are neighbours when some side joins them; the count of an undirected edge is the number of sides on it.
+ * A vertex on an edge whose count is not 2 is held: open boundaries (count 1) and non-manifold edges (3 or more).
+ * Held vertices and vertices without a neighbour (isolated) keep their xyz bytes exactly; the others are free.
+ * Fixed point: 2^E is the smallest power of two above every |coordinate| of the mesh (E = the largest biased float
+ * exponent field - 126, an exact max on the device); every vertex's position is the int64 Q = rint((double)x *
+ * 2^(40 - E)), half to even, so coordinates down to 2^(E - 17) are held exactly.
+ * Pass: every free vertex with d distinct neighbours, per axis, S = sum of the neighbours' Q (exact integers, so the
+ * order of the neighbours does not matter), m = (double)S / (double)d, Q' = Q + rint(k * (m - (double)Q)), with
+ * separately rounded IEEE operations (no FMA) and k = (double)lambda or (double)mu.  An iteration is a lambda pass then
+ * a mu pass; mu = 0 gives plain Laplacian smoothing with one pass per iteration.  At the end a free vertex takes
+ * (float)((double)Q * 2^(E - 40)).  iterations = 0 only quantises the free vertices and recomputes the normals.
+ * Normals, recomputed from the final float positions: for each face with three distinct indices, the unit normal of
+ * (p_b - p_a) x (p_c - p_a) in double, as a float, in the merge's fixed point (clamped to [-1, 1], rint(v * 2^24)), is
+ * added to each of its three vertices (a face with a zero or non-finite cross product adds nothing); a vertex's normal
+ * is then the merge's normalisation of its integer sums, and a vertex whose sums are all zero keeps its normal bytes.
+ * Equal-weight face normals keep the sums of any hub below 2^55.
+ * Limits (derived in the math header; each fails the whole call with SCAN3D_ERR_CONFIG and nothing is written): a free
+ * vertex with more than 2^20 neighbours; a free vertex with some |Q| > 2^42 after a pass (a mu pass moves vertices away
+ * from their neighbours' mean); a free vertex whose output coordinate rounds to +-inf; 6 * n_faces >= 2^32.
+ *
+ * scan3d_voxel_surface_smooth smooths the held voxel surface in place: scan3d_get_voxel_surface and
+ * scan3d_write_voxel_surface_ply then return it.  Faces, colours and the vertex order do not change, so a component
+ * table of scan3d_voxel_surface_components stays valid.  It needs a held surface (SCAN3D_ERR_STATE otherwise).
+ * Smoothing after components or decimation is allowed, and so is smoothing again.  scan3d_voxel_surface_decimate
+ * refuses a smoothed surface with SCAN3D_ERR_STATE until a new scan3d_voxel_surface (its overflow bound rests on
+ * surface-nets geometry, which smoothing does not keep).  A later begin, add or finish makes the surface stale as
+ * before; the accumulator is never touched.  The result is computed into the components' second surface set and
+ * swapped with the held one after the synchronisation, so on any error the surface is untouched.
+ * scan3d_mesh_smooth_dev smooths any triangle mesh in device memory of the ctx's GPU in place: xyz_dev float
+ * [n_vertices][3], normals_dev float [n_vertices][3] or NULL (no normals), faces_dev int32 [n_faces][3]; ordered on the
+ * ctx stream.  It leaves the held surface and the component table alone, and on any error leaves the buffers as they
+ * were.  The ctx's own camera-grid mesh is a valid target: scan3d_device_points, scan3d_device_point_normals and
+ * scan3d_device_mesh_faces with the counts of scan3d_point_count and scan3d_mesh_face_count; the mesh stays valid, and
+ * scan3d_write_mesh_ply then writes the smoothed single view.  The next reconstruct overwrites the points.
+ * Synchronisation: one per call, after every launch.
+ * Launches: 7 + passes + 2, with passes = iterations * 2 (mu != 0) or iterations (mu = 0), an empty mesh included:
+ * the exponent max, the sides into the edge table, the degrees and held flags, the degree sums per block, their scan,
+ * the row starts with the fixed-point positions, the neighbour rows; one gather per pass; the face normals; the write.
+ * Memory (ctx-owned, allocated on first use, grown on demand): 81 B per vertex (two fixed-point position sets at 24 B,
+ * the normal sums at 24 B, degree, row start and held flag) and 96 B per face (the edge table of 6 slots of 12 B, and
+ * 6 row entries of 4 B); the surface route also grows the components' second set's xyz and normals to 24 B per vertex.
+ * Errors: SCAN3D_ERR_ARG for a null ctx, params or result; iterations outside [0, 4096]; lambda not in (0, 1] or mu not
+ * in [-1, 0] (NaN and infinities included); and in scan3d_mesh_smooth_dev n_vertices or n_faces outside [0, 2^31), a
+ * NULL xyz_dev or faces_dev with a non-zero count, a buffer not 4-byte aligned, and, found on the device, a coordinate
+ * that is not finite or a face index outside [0, n_vertices).  An argument or state error launches nothing; an error
+ * found on the device is reported at the synchronisation and nothing is written. */
+#define SCAN3D_SMOOTH_MAX_ITERATIONS 4096
+typedef struct {
+    int32_t iterations;          /* [0, 4096]; MeshLab's default is 10 */
+    float lambda;                /* (0, 1]; MeshLab's default is 0.5 */
+    float mu;                    /* [-1, 0]; MeshLab's default is -0.53; 0 = Laplacian smoothing */
+} scan3d_smooth_params;
+
+typedef struct {
+    int64_t vertices, faces;     /* of the mesh */
+    int64_t held_vertices;       /* on an edge whose count is not 2 */
+    int64_t isolated_vertices;   /* without a neighbour */
+    int64_t passes;              /* gathers run */
+    double max_displacement;     /* the largest Euclidean move of a vertex, model units */
+} scan3d_smooth_result;
+
+int scan3d_voxel_surface_smooth(scan3d_ctx *ctx, const scan3d_smooth_params *p, scan3d_smooth_result *out);
+int scan3d_mesh_smooth_dev(scan3d_ctx *ctx, float *xyz_dev, float *normals_dev, int64_t n_vertices,
+                           const int32_t *faces_dev, int64_t n_faces, const scan3d_smooth_params *p,
+                           scan3d_smooth_result *out);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,
