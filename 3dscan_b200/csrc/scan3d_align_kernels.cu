@@ -29,9 +29,9 @@ constexpr int IT = 256;                  // threads per block of the index kerne
 constexpr int MT = 256;                  // threads per match block
 constexpr int SPT = 8;                   // samples per match thread
 constexpr long long SPB = (long long)MT * SPT;
-constexpr int NV = ALIGN_NSUM + 1;       // the sums and the pair count
+constexpr int NV = s3l::NSUM + 1;        // the sums and the pair count
 constexpr unsigned FULL = 0xffffffffu;
-static_assert(ALIGN_NSUM == s3l::NSUM, "sum count");
+constexpr uint32_t CELLS_PER_VOXEL = 2;  // index slots per model voxel: at most half of them are taken
 
 __device__ __forceinline__ uint32_t model_count(const VoxelTable& t, int par)
 {
@@ -211,31 +211,49 @@ static unsigned index_grid(unsigned long long n, int sm_count)
     return (unsigned)(b < 1 ? 1 : b);
 }
 
-cudaError_t launch_align_index(const AlignIndex& ix, const VoxelTable& t, int par, const float* xyz, const float* nrm,
-                               double S, AlignState* state, const AlignRun& run, const uint32_t* n_dev, int sm_count,
-                               cudaStream_t st)
-{
-    const unsigned gm = index_grid(t.max_voxels, sm_count);
-    k_align_cells<<<gm, IT, 0, st>>>(ix, t, par, xyz, nrm, S, state, run, n_dev);
-    k_align_ranges<<<index_grid(ix.cap, sm_count), IT, 0, st>>>(ix);
-    k_align_scatter<<<gm, IT, 0, st>>>(ix, t, par, xyz, nrm);
-    return cudaGetLastError();
-}
-
-uint32_t align_match_blocks(long long n_max, int stride)
+static uint32_t match_blocks(long long n_max, int stride)
 {
     const long long samples = (n_max + stride - 1) / stride;
     const long long b = (samples + SPB - 1) / SPB;
     return (uint32_t)(b < 1 ? 1 : b);
 }
 
-cudaError_t launch_align_iteration(const AlignIndex& ix, AlignState* state, const AlignRun& run, const float* xyz,
-                                   const uint32_t* n_dev, long long n_max, int stride, double* partials, cudaStream_t st)
+cudaError_t AlignWorkspace::index(const VoxelTable& t, int par, const float* xyz, const float* nrm, const AlignRun& run,
+                                  const uint32_t* n_dev, int sm_count, cudaStream_t st, int64_t* launches)
 {
-    const uint32_t blocks = align_match_blocks(n_max, stride);
-    k_align_match<<<blocks, MT, 0, st>>>(ix, state, run, xyz, n_dev, n_max, stride, partials);
-    k_align_solve<<<1, MT, 0, st>>>(state, run, partials, blocks);
+    const uint32_t maxv = t.max_voxels, cap = CELLS_PER_VOXEL * maxv;
+    cudaError_t e =
+        grow_group(Grow(keys, cap), Grow(cells, cap), Grow(model_slot, maxv), Grow(entries, 2 * (size_t)maxv));
+    if (e == cudaSuccess) e = state.ensure(1);
+    if (e == cudaSuccess) e = cursor.ensure(1);
+    if (e != cudaSuccess) return e;
+    view = AlignIndex{keys, cells, model_slot, entries, cursor, cap};
+    e = cudaMemsetAsync(keys, 0xff, (size_t)cap * sizeof(*view.keys), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(cells, 0, (size_t)cap * sizeof(*view.cells), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(cursor, 0, sizeof(*view.cursor), st);
+    if (e != cudaSuccess) return e;
+    const unsigned gm = index_grid(maxv, sm_count);
+    k_align_cells<<<gm, IT, 0, st>>>(view, t, par, xyz, nrm, run.S, state, run, n_dev);
+    k_align_ranges<<<index_grid(cap, sm_count), IT, 0, st>>>(view);
+    k_align_scatter<<<gm, IT, 0, st>>>(view, t, par, xyz, nrm);
+    *launches += 3;
     return cudaGetLastError();
+}
+
+cudaError_t AlignWorkspace::align(const VoxelTable& t, int par, const float* xyz, const float* nrm, const AlignRun& run,
+                                  const float* src, const uint32_t* n_dev, long long n_max, int stride, int sm_count,
+                                  cudaStream_t st, int64_t* launches)
+{
+    const uint32_t blocks = match_blocks(n_max, stride);
+    cudaError_t e = partials.ensure((size_t)NV * blocks);
+    if (e == cudaSuccess) e = index(t, par, xyz, nrm, run, n_dev, sm_count, st, launches);
+    for (int it = 0; it < run.max_iterations && e == cudaSuccess; it++) {
+        k_align_match<<<blocks, MT, 0, st>>>(view, state, run, src, n_dev, n_max, stride, partials);
+        k_align_solve<<<1, MT, 0, st>>>(state, run, partials, blocks);
+        *launches += 2;
+        e = cudaGetLastError();
+    }
+    return e;
 }
 
 }  // namespace s3d

@@ -933,8 +933,7 @@ int scan3d_build_mesh(scan3d_ctx* ctx, float max_edge)
     CK(ctx->mesh_faces.ensure(3 * std::max(max_faces, (size_t)1)));
     CK(ctx->mesh_normals.ensure(3 * n));
     CK(launch_mesh(ctx->valid, points_of(ctx), c.W, c.H, max_edge, ctx->mesh_idx, ctx->block_counts, ctx->mesh_counts,
-                   ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals, ctx->stream));
-    ctx->launches += MESH_LAUNCHES;
+                   ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals, ctx->stream, &ctx->launches));
     ctx->have_mesh = true;
     return SCAN3D_OK;
 }
@@ -1005,26 +1004,13 @@ int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
     CK(cudaSetDevice(ctx->device));
     ctx->vox_begun = ctx->vox_fresh = false;
     ctx->srf_ready = ctx->cc_ready = false;
-    VoxelTable& t = ctx->vox;
-    const uint32_t cap = voxel_table_capacity((uint32_t)max_voxels, ctx->sm_count);
-    CK(grow_group(Grow(ctx->vox_keys, cap), Grow(ctx->vox_acc, cap), Grow(ctx->vox_ordinal, cap)));
-    const size_t m = (size_t)max_voxels;
-    CK(grow_group(Grow(ctx->vox_ord2slot, m), Grow(ctx->vox_xyz, 3 * m), Grow(ctx->vox_nrm, 3 * m),
-                  Grow(ctx->vox_rgb, 3 * m), Grow(ctx->vox_cnt, m)));
-    const size_t n = npix(ctx);
-    CK(ctx->vox_state.ensure(1));
+    CK(ctx->vox.reset((uint32_t)max_voxels, (double)voxel_size, ctx->sm_count, ctx->stream));
+    const size_t m = (size_t)max_voxels, n = npix(ctx);
+    CK(grow_group(Grow(ctx->vox_xyz, 3 * m), Grow(ctx->vox_nrm, 3 * m), Grow(ctx->vox_rgb, 3 * m),
+                  Grow(ctx->vox_cnt, m)));
     CK(ctx->vox_point_slot.ensure(n));
     CK(ctx->vox_flags.ensure(n));
     CK(ctx->block_counts.ensure((n + POINT_BLOCK - 1) / POINT_BLOCK + 1));
-    t.keys = ctx->vox_keys; t.acc = ctx->vox_acc; t.ordinal = ctx->vox_ordinal;
-    t.ord2slot = ctx->vox_ord2slot; t.state = ctx->vox_state;
-    CK(cudaMemsetAsync(t.keys, 0xff, (size_t)cap * sizeof(*t.keys), ctx->stream));
-    CK(cudaMemsetAsync(t.acc, 0, (size_t)cap * sizeof(*t.acc), ctx->stream));
-    CK(cudaMemsetAsync(t.ordinal, 0xff, (size_t)cap * sizeof(*t.ordinal), ctx->stream));
-    CK(cudaMemsetAsync(t.state, 0, sizeof(*t.state), ctx->stream));
-    t.cap = cap;
-    t.max_voxels = (uint32_t)max_voxels;
-    t.S = (double)voxel_size;
     ctx->vox_bound = 0;
     ctx->vox_chunks = 0;
     ctx->vox_begun = true;
@@ -1035,10 +1021,9 @@ int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
 static int voxel_add(scan3d_ctx* ctx, const float* xyz, const float* nrm, const uint8_t* rgb, const uint32_t* n_dev,
                      uint32_t plane)
 {
-    CK(launch_voxel_add(ctx->vox, xyz, nrm, rgb, n_dev, plane, ctx->vox_point_slot, ctx->vox_flags, ctx->block_counts,
-                        (int)(ctx->vox_chunks & 1), ctx->stream));
+    CK(launch_voxel_add(ctx->vox.view, xyz, nrm, rgb, n_dev, plane, ctx->vox_point_slot, ctx->vox_flags,
+                        ctx->block_counts, (int)(ctx->vox_chunks & 1), ctx->stream, &ctx->launches));
     ctx->vox_chunks++;
-    ctx->launches += VOXEL_ADD_LAUNCHES;
     return SCAN3D_OK;
 }
 
@@ -1089,8 +1074,8 @@ int scan3d_voxel_finish(scan3d_ctx* ctx)
     if (!ctx) return SCAN3D_ERR_ARG;
     if (!ctx->vox_begun) return fail(ctx, SCAN3D_ERR_STATE, "voxel finish before scan3d_voxel_begin");
     CK(cudaSetDevice(ctx->device));
-    CK(launch_voxel_finish(ctx->vox, (int)(ctx->vox_chunks & 1), ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb, ctx->vox_cnt,
-                           ctx->sm_count, ctx->stream));
+    CK(launch_voxel_finish(ctx->vox.view, (int)(ctx->vox_chunks & 1), ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb,
+                           ctx->vox_cnt, ctx->sm_count, ctx->stream));
     ctx->launches += 1;
     ctx->vox_fresh = true;
     ctx->srf_ready = ctx->cc_ready = false;
@@ -1106,7 +1091,7 @@ int scan3d_voxel_count(scan3d_ctx* ctx, int64_t* voxels_out, int64_t* dropped_ou
     VoxelState st;
     CK(cudaMemcpyAsync(&st, ctx->vox.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (st.overflow || st.occupied > ctx->vox.max_voxels)
+    if (st.overflow || st.occupied > ctx->vox.view.max_voxels)
         return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct voxels than max_voxels: begin again with a larger max_voxels");
     if (voxels_out) *voxels_out = st.total[ctx->vox_chunks & 1];
     if (dropped_out) *dropped_out = (int64_t)st.dropped;
@@ -1182,36 +1167,11 @@ static int check_align_args(scan3d_ctx* ctx, const scan3d_align_params* p, scan3
     return SCAN3D_OK;
 }
 
-// the model's cell index of edge run.S (ALIGN_INDEX_LAUNCHES), in ctx-owned buffers grown with max_voxels; it also
-// initialises ctx->aln_state from run (n_dev: the source count to record, or null)
-static int align_index(scan3d_ctx* ctx, const AlignRun& run, const uint32_t* n_dev)
-{
-    const uint32_t maxv = ctx->vox.max_voxels;
-    AlignIndex& ix = ctx->aln;
-    const size_t cap = (size_t)ALIGN_CELLS_PER_VOXEL * maxv;
-    CK(grow_group(Grow(ctx->aln_keys, cap), Grow(ctx->aln_cells, cap), Grow(ctx->aln_model_slot, (size_t)maxv),
-                  Grow(ctx->aln_entries, 2 * (size_t)maxv)));
-    CK(ctx->aln_state.ensure(1));
-    CK(ctx->aln_cursor.ensure(1));
-    ix.keys = ctx->aln_keys; ix.cells = ctx->aln_cells; ix.model_slot = ctx->aln_model_slot;
-    ix.entries = ctx->aln_entries; ix.cursor = ctx->aln_cursor;
-    ix.cap = ALIGN_CELLS_PER_VOXEL * maxv;
-    CK(cudaMemsetAsync(ix.keys, 0xff, (size_t)ix.cap * sizeof(*ix.keys), ctx->stream));
-    CK(cudaMemsetAsync(ix.cells, 0, (size_t)ix.cap * sizeof(*ix.cells), ctx->stream));
-    CK(cudaMemsetAsync(ix.cursor, 0, sizeof(*ix.cursor), ctx->stream));
-    CK(launch_align_index(ix, ctx->vox, (int)(ctx->vox_chunks & 1), ctx->vox_xyz, ctx->vox_nrm, run.S, ctx->aln_state,
-                          run, n_dev, ctx->sm_count, ctx->stream));
-    ctx->launches += ALIGN_INDEX_LAUNCHES;
-    return SCAN3D_OK;
-}
-
 // the whole run on the source xyz (n_dev: its count is on the device, <= n_max)
 static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long long n_max, const scan3d_align_params* p,
                      scan3d_align_result* out)
 {
     CK(cudaSetDevice(ctx->device));
-    const uint32_t blocks = align_match_blocks(n_max, p->stride);
-    CK(ctx->aln_partials.ensure((size_t)(ALIGN_NSUM + 1) * blocks));
     AlignRun run;
     for (int k = 0; k < 12; k++) run.T0[k] = p->T_init[k];
     run.S = s3l::cell_edge(p->max_distance);
@@ -1219,14 +1179,10 @@ static int align_run(scan3d_ctx* ctx, float* xyz, const uint32_t* n_dev, long lo
     run.stop_rotation = p->stop_rotation;
     run.stop_translation = p->stop_translation;
     run.max_iterations = p->max_iterations;
-    const int rc = align_index(ctx, run, n_dev);
-    if (rc) return rc;
-    for (int it = 0; it < p->max_iterations; it++) {
-        CK(launch_align_iteration(ctx->aln, ctx->aln_state, run, xyz, n_dev, n_max, p->stride, ctx->aln_partials, ctx->stream));
-        ctx->launches += 2;
-    }
+    CK(ctx->aln.align(ctx->vox.view, (int)(ctx->vox_chunks & 1), ctx->vox_xyz, ctx->vox_nrm, run, xyz, n_dev, n_max,
+                      p->stride, ctx->sm_count, ctx->stream, &ctx->launches));
     AlignState st;
-    CK(cudaMemcpyAsync(&st, ctx->aln_state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&st, ctx->aln.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     if (st.overflow)
         return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct voxels than max_voxels: begin again with a larger max_voxels");
@@ -1290,35 +1246,17 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
     AlignRun run{};                                      // the index only; T0 = I for the state it initialises
     run.T0[0] = run.T0[5] = run.T0[10] = 1.0;
     run.S = s3l::cell_edge(p->max_distance);
-    int rc = align_index(ctx, run, nullptr);
-    if (rc) return rc;
-    SurfaceTable& s = ctx->srf;
+    const int par = (int)(ctx->vox_chunks & 1);
     const uint32_t maxp = (uint32_t)p->max_points;
-    const uint32_t cap = surface_table_capacity(maxp, ctx->sm_count);
-    CK(grow_group(Grow(ctx->srf_keys, cap), Grow(ctx->srf_owner, cap), Grow(ctx->srf_f, cap),
-                  Grow(ctx->srf_nearest, cap), Grow(ctx->srf_vert, cap)));
-    const size_t nvb = (maxp + SURFACE_VB - 1) / SURFACE_VB;
-    CK(grow_group(Grow(ctx->srf_vert_slot, maxp), Grow(ctx->srf_face_counts, nvb + 1)));
-    const uint64_t nflags = (uint64_t)s3s::OFFSETS * ctx->vox.max_voxels;
-    CK(grow_group(Grow(ctx->srf_flags, nflags), Grow(ctx->srf_flag_counts, (nflags + POINT_BLOCK - 1) / POINT_BLOCK + 1)));
-    CK(ctx->srf_state.ensure(1));
-    s.keys = ctx->srf_keys; s.owner = ctx->srf_owner; s.f = ctx->srf_f; s.nearest = ctx->srf_nearest;
-    s.vert = ctx->srf_vert; s.state = ctx->srf_state;
-    s.cap = cap;
-    s.max_points = maxp;
-    s.S = ctx->vox.S;
-    CK(cudaMemsetAsync(s.keys, 0xff, (size_t)cap * sizeof(*s.keys), ctx->stream));
-    CK(cudaMemsetAsync(s.owner, 0xff, (size_t)cap * sizeof(*s.owner), ctx->stream));
-    CK(cudaMemsetAsync(s.vert, 0xff, (size_t)cap * sizeof(*s.vert), ctx->stream));
-    CK(cudaMemsetAsync(s.state, 0, sizeof(*s.state), ctx->stream));
-    CK(cudaMemsetAsync(ctx->srf_face_counts, 0, nvb * sizeof(uint32_t), ctx->stream));
-    CK(launch_surface_counts(s, ctx->aln, ctx->vox, (int)(ctx->vox_chunks & 1), ctx->vox_nrm, p->max_distance,
-                             ctx->srf_flags, ctx->srf_flag_counts, ctx->srf_vert_slot, ctx->srf_face_counts, ctx->stream));
-    ctx->launches += SURFACE_COUNT_LAUNCHES;
+    CK(ctx->aln.index(ctx->vox.view, par, ctx->vox_xyz, ctx->vox_nrm, run, nullptr, ctx->sm_count, ctx->stream,
+                      &ctx->launches));
+    CK(ctx->lattice.count(ctx->aln.view, ctx->vox.view, par, ctx->vox_nrm, p->max_distance, maxp, ctx->sm_count,
+                          ctx->stream, &ctx->launches));
     SurfaceState st;
     int vox_overflow = 0;
-    CK(cudaMemcpyAsync(&st, s.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(&vox_overflow, &ctx->aln_state.get()->overflow, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&st, ctx->lattice.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&vox_overflow, &ctx->aln.state.get()->overflow, sizeof(int), cudaMemcpyDeviceToHost,
+                       ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     if (vox_overflow)
         return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct voxels than max_voxels: begin again with a larger max_voxels");
@@ -1326,14 +1264,10 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
         return fail(ctx, SCAN3D_ERR_CONFIG, "more distinct lattice points than max_points: extract again with a larger max_points");
     if ((uint64_t)st.vertices * 6 > 0xffffffffull)   // the face count is a 32-bit sum of <= 6 per vertex
         return fail(ctx, SCAN3D_ERR_CONFIG, "more than (2^32 - 1) / 6 surface vertices");
-    const size_t nv3 = 3 * (size_t)st.vertices;
-    CK(grow_group(Grow(ctx->srf_xyz, nv3), Grow(ctx->srf_nrm, nv3), Grow(ctx->srf_rgb, nv3)));
-    CK(ctx->srf_tri.ensure(3 * (size_t)st.faces));
-    CK(launch_surface_emit(s, ctx->vox_rgb, ctx->srf_vert_slot, ctx->srf_face_counts, st.vertices, ctx->srf_xyz,
-                           ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri, ctx->stream));
-    ctx->launches += 1;
-    ctx->srf_vertices = st.vertices;
-    ctx->srf_faces = st.faces;
+    CK(ctx->surface.grow(st.vertices, st.faces));
+    CK(ctx->lattice.emit(ctx->vox_rgb, st.vertices, ctx->surface, ctx->stream, &ctx->launches));
+    ctx->surface.vertices = st.vertices;
+    ctx->surface.faces = st.faces;
     ctx->srf_ready = true;
     ctx->srf_decimated = false;
     ctx->srf_smoothed = false;
@@ -1351,12 +1285,13 @@ int scan3d_get_voxel_surface(scan3d_ctx* ctx, float* xyz, float* normals, uint8_
     if (!ctx->srf_ready)
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
     CK(cudaSetDevice(ctx->device));
-    const int64_t nv = std::max<int64_t>(0, std::min(ctx->srf_vertices, max_vertices));
-    const int64_t nf = std::max<int64_t>(0, std::min(ctx->srf_faces, max_faces));
-    if (xyz && nv) CK(cudaMemcpyAsync(xyz, ctx->srf_xyz, (size_t)nv * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    if (normals && nv) CK(cudaMemcpyAsync(normals, ctx->srf_nrm, (size_t)nv * 12, cudaMemcpyDeviceToHost, ctx->stream));
-    if (rgb && nv) CK(cudaMemcpyAsync(rgb, ctx->srf_rgb, (size_t)nv * 3, cudaMemcpyDeviceToHost, ctx->stream));
-    if (faces && nf) CK(cudaMemcpyAsync(faces, ctx->srf_tri, (size_t)nf * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    const SurfaceMesh& s = ctx->surface;
+    const int64_t nv = std::max<int64_t>(0, std::min(s.vertices, max_vertices));
+    const int64_t nf = std::max<int64_t>(0, std::min(s.faces, max_faces));
+    if (xyz && nv) CK(cudaMemcpyAsync(xyz, s.xyz, (size_t)nv * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    if (normals && nv) CK(cudaMemcpyAsync(normals, s.nrm, (size_t)nv * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    if (rgb && nv) CK(cudaMemcpyAsync(rgb, s.rgb, (size_t)nv * 3, cudaMemcpyDeviceToHost, ctx->stream));
+    if (faces && nf) CK(cudaMemcpyAsync(faces, s.tri, (size_t)nf * 12, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return SCAN3D_OK;
 }
@@ -1366,7 +1301,7 @@ int scan3d_write_voxel_surface_ply(scan3d_ctx* ctx, const char* path, int binary
     if (!ctx || !path) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
     if (!ctx->srf_ready)
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
-    const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
+    const int64_t nv = ctx->surface.vertices, nf = ctx->surface.faces;
     std::vector<float> xyz((size_t)nv * 3), nrm((size_t)nv * 3);
     std::vector<uint8_t> rgb((size_t)nv * 3);
     std::vector<int32_t> faces((size_t)nf * 3);
@@ -1382,17 +1317,6 @@ int scan3d_write_voxel_surface_ply(scan3d_ctx* ctx, const char* path, int binary
 // ------------------------------------------------------------------------------------------
 // connected components of a triangle mesh (include/scan3d.h has the exact rules)
 // ------------------------------------------------------------------------------------------
-// the labelling scratch for n vertices: parent, root flags, their block offsets, the device state
-static int cc_label_scratch(scan3d_ctx* ctx, int64_t n)
-{
-    n = std::max<int64_t>(n, 1);
-    CK(grow_group(Grow(ctx->cc_parent, (size_t)n), Grow(ctx->cc_flags, (size_t)n),
-                  Grow(ctx->cc_vert_counts, (size_t)(n + POINT_BLOCK - 1) / POINT_BLOCK + 1)));
-    CK(ctx->cc_state.ensure(1));
-    CK(cudaMemsetAsync(ctx->cc_state, 0, sizeof(ComponentsState), ctx->stream));
-    return SCAN3D_OK;
-}
-
 int scan3d_voxel_surface_components(scan3d_ctx* ctx, const scan3d_components_params* p, scan3d_components_result* out)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
@@ -1402,38 +1326,17 @@ int scan3d_voxel_surface_components(scan3d_ctx* ctx, const scan3d_components_par
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
     CK(cudaSetDevice(ctx->device));
     ctx->cc_ready = false;
-    const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
-    int rc = cc_label_scratch(ctx, nv);
-    if (rc) return rc;
-    const size_t av = (size_t)std::max<int64_t>(nv, 1), af = (size_t)std::max<int64_t>(nf, 1);
-    CK(grow_group(Grow(ctx->cc_label, av), Grow(ctx->cc_comp_v, av), Grow(ctx->cc_comp_f, av), Grow(ctx->cc_kept, av)));
-    CK(grow_group(Grow(ctx->cc_keep_f, af), Grow(ctx->cc_face_counts, (af + POINT_BLOCK - 1) / POINT_BLOCK + 1)));
-    CK(cudaMemsetAsync(ctx->cc_comp_v, 0, (size_t)nv * sizeof(uint32_t), ctx->stream));
-    CK(cudaMemsetAsync(ctx->cc_comp_f, 0, (size_t)nv * sizeof(uint32_t), ctx->stream));
-    CK(launch_cc_labels(ctx->srf_tri, (uint32_t)nf, (uint32_t)nv, ctx->cc_parent, ctx->cc_flags, ctx->cc_vert_counts,
-                        ctx->cc_label, ctx->cc_state, ctx->stream));
-    CK(launch_cc_select(ctx->srf_tri, (uint32_t)nf, (uint32_t)nv, ctx->cc_label, (unsigned long long)p->min_faces,
-                        (unsigned long long)p->max_components, ctx->cc_comp_v, ctx->cc_comp_f, ctx->cc_kept,
-                        ctx->cc_flags, ctx->cc_keep_f, ctx->cc_vert_counts, ctx->cc_face_counts, ctx->cc_state,
-                        ctx->stream));
-    ctx->launches += COMPONENT_LABEL_LAUNCHES + COMPONENT_SELECT_LAUNCHES;
+    CK(ctx->cc.select(ctx->surface, (unsigned long long)p->min_faces, (unsigned long long)p->max_components,
+                      ctx->stream, &ctx->launches));
     ComponentsState st;
-    CK(cudaMemcpyAsync(&st, ctx->cc_state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&st, ctx->cc.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    const size_t kv3 = 3 * (size_t)st.vertices;
-    CK(grow_group(Grow(ctx->cc_xyz, kv3), Grow(ctx->cc_nrm, kv3), Grow(ctx->cc_rgb, kv3)));
-    CK(ctx->cc_tri.ensure(3 * (size_t)st.faces));
-    CK(launch_cc_emit(ctx->cc_flags, ctx->cc_vert_counts, (uint32_t)nv, ctx->srf_xyz, ctx->srf_nrm, ctx->srf_rgb,
-                      ctx->cc_keep_f, ctx->cc_face_counts, (uint32_t)nf, ctx->srf_tri, ctx->cc_label, ctx->cc_xyz,
-                      ctx->cc_nrm, ctx->cc_rgb, ctx->cc_tri, ctx->stream));
-    ctx->launches += COMPONENT_EMIT_LAUNCHES;
+    CK(ctx->spare.grow(st.vertices, st.faces));
+    CK(ctx->cc.emit(ctx->surface, ctx->spare, ctx->stream, &ctx->launches));
     // the compacted set becomes the held surface; the old one is the next compaction's destination
-    std::swap(ctx->srf_xyz, ctx->cc_xyz);
-    std::swap(ctx->srf_nrm, ctx->cc_nrm);
-    std::swap(ctx->srf_rgb, ctx->cc_rgb);
-    std::swap(ctx->srf_tri, ctx->cc_tri);
-    ctx->srf_vertices = st.vertices;
-    ctx->srf_faces = st.faces;
+    std::swap(ctx->surface, ctx->spare);
+    ctx->surface.vertices = st.vertices;
+    ctx->surface.faces = st.faces;
     ctx->cc_components = st.components;
     ctx->cc_ready = true;
     out->components = st.components;
@@ -1453,9 +1356,9 @@ int scan3d_get_surface_components(scan3d_ctx* ctx, int64_t* vertices, int64_t* f
     CK(cudaSetDevice(ctx->device));
     const int64_t n = std::max<int64_t>(0, std::min(ctx->cc_components, max_components));
     std::vector<uint32_t> v(vertices ? n : 0), f(faces ? n : 0);
-    if (vertices && n) CK(cudaMemcpyAsync(v.data(), ctx->cc_comp_v, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    if (faces && n) CK(cudaMemcpyAsync(f.data(), ctx->cc_comp_f, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    if (kept && n) CK(cudaMemcpyAsync(kept, ctx->cc_kept, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (vertices && n) CK(cudaMemcpyAsync(v.data(), ctx->cc.comp_v, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (faces && n) CK(cudaMemcpyAsync(f.data(), ctx->cc.comp_f, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    if (kept && n) CK(cudaMemcpyAsync(kept, ctx->cc.kept, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     for (int64_t c = 0; vertices && c < n; c++) vertices[c] = v[c];
     for (int64_t c = 0; faces && c < n; c++) faces[c] = f[c];
@@ -1473,13 +1376,9 @@ int scan3d_mesh_components_dev(scan3d_ctx* ctx, const int32_t* faces_dev, int64_
     if (((uintptr_t)faces_dev & 3) || ((uintptr_t)label_dev & 3))
         return fail(ctx, SCAN3D_ERR_ARG, "faces_dev and label_dev must be 4-byte aligned");
     CK(cudaSetDevice(ctx->device));
-    const int rc = cc_label_scratch(ctx, n_vertices);
-    if (rc) return rc;
-    CK(launch_cc_labels(faces_dev, (uint32_t)n_faces, (uint32_t)n_vertices, ctx->cc_parent, ctx->cc_flags,
-                        ctx->cc_vert_counts, label_dev, ctx->cc_state, ctx->stream));
-    ctx->launches += COMPONENT_LABEL_LAUNCHES;
+    CK(ctx->cc.labels(faces_dev, (uint32_t)n_faces, (uint32_t)n_vertices, label_dev, ctx->stream, &ctx->launches));
     ComponentsState st;
-    CK(cudaMemcpyAsync(&st, ctx->cc_state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&st, ctx->cc.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     if (st.bad) return fail(ctx, SCAN3D_ERR_ARG, "a face index outside [0, n_vertices)");
     *components_out = st.components;
@@ -1496,65 +1395,29 @@ int scan3d_voxel_surface_decimate(scan3d_ctx* ctx, float cell_size, scan3d_decim
     if (!(cell_size - cell_size == 0.0f)) return fail(ctx, SCAN3D_ERR_ARG, "cell_size must be finite");
     if (!ctx->srf_ready)
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
-    const double H = (double)cell_size, s = ctx->vox.S;
+    const double H = (double)cell_size, s = ctx->vox.view.S;
     if (!(H >= s && H <= s3q::RATIO_MAX * s))
         return fail(ctx, SCAN3D_ERR_ARG, "cell_size must be in [voxel_size, 256 voxel_size]");
     if (ctx->srf_decimated)
         return fail(ctx, SCAN3D_ERR_STATE, "the held surface is already simplified: extract it again first");
     if (ctx->srf_smoothed)
         return fail(ctx, SCAN3D_ERR_STATE, "the held surface is smoothed: extract it again to simplify it");
-    const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
+    const int64_t nv = ctx->surface.vertices, nf = ctx->surface.faces;
     if (nf >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^31 - 1 surface faces");
     CK(cudaSetDevice(ctx->device));
     ctx->cc_ready = false;
-    // the cluster table, sized as scan3d_voxel_begin sizes the merge's for max_voxels = the vertex count
-    const uint32_t maxv = (uint32_t)std::max<int64_t>(nv, 1);
-    const size_t av = maxv, af = (size_t)std::max<int64_t>(nf, 1);
-    VoxelTable& t = ctx->dec;
-    const uint32_t cap = voxel_table_capacity(maxv, ctx->sm_count);
-    CK(grow_group(Grow(ctx->dec_keys, cap), Grow(ctx->dec_acc, cap), Grow(ctx->dec_ordinal, cap)));
-    CK(grow_group(Grow(ctx->dec_ord2slot, av), Grow(ctx->dec_point_slot, av), Grow(ctx->dec_vert_flags, av),
-                  Grow(ctx->dec_vert_counts, (av + POINT_BLOCK - 1) / POINT_BLOCK + 1),
-                  Grow(ctx->dec_quad, s3q::NQ * av)));
-    CK(grow_group(Grow(ctx->dec_ctri, 3 * af), Grow(ctx->dec_table, 2 * af), Grow(ctx->dec_slot_of, af),
-                  Grow(ctx->dec_keep, af), Grow(ctx->dec_face_counts, (af + POINT_BLOCK - 1) / POINT_BLOCK + 1)));
-    CK(ctx->dec_vstate.ensure(1));
-    CK(ctx->dec_state.ensure(1));
-    // the emission runs before the synchronisation, so the second set holds the whole input
-    CK(grow_group(Grow(ctx->cc_xyz, 3 * av), Grow(ctx->cc_nrm, 3 * av), Grow(ctx->cc_rgb, 3 * av)));
-    CK(ctx->cc_tri.ensure(3 * af));
-    t.keys = ctx->dec_keys; t.acc = ctx->dec_acc; t.ordinal = ctx->dec_ordinal;
-    t.ord2slot = ctx->dec_ord2slot; t.state = ctx->dec_vstate;
-    t.cap = cap;
-    t.max_voxels = maxv;
-    t.S = H;
-    DecimateBuffers b;
-    b.point_slot = ctx->dec_point_slot; b.vert_flags = ctx->dec_vert_flags; b.vert_counts = ctx->dec_vert_counts;
-    b.quad = ctx->dec_quad; b.ctri = ctx->dec_ctri; b.table = ctx->dec_table; b.table_cap = (uint32_t)(2 * af);
-    b.slot_of = ctx->dec_slot_of; b.keep = ctx->dec_keep; b.face_counts = ctx->dec_face_counts;
-    b.state = ctx->dec_state;
-    CK(cudaMemsetAsync(t.keys, 0xff, (size_t)cap * sizeof(*t.keys), ctx->stream));
-    CK(cudaMemsetAsync(t.acc, 0, (size_t)cap * sizeof(*t.acc), ctx->stream));
-    CK(cudaMemsetAsync(t.ordinal, 0xff, (size_t)cap * sizeof(*t.ordinal), ctx->stream));
-    CK(cudaMemsetAsync(t.state, 0, sizeof(*t.state), ctx->stream));
-    CK(cudaMemsetAsync(b.quad, 0, s3q::NQ * av * sizeof(*b.quad), ctx->stream));
-    CK(cudaMemsetAsync(b.table, 0xff, (size_t)b.table_cap * sizeof(*b.table), ctx->stream));
-    CK(cudaMemsetAsync(b.state, 0, sizeof(*b.state), ctx->stream));
-    CK(launch_decimate(t, b, ctx->srf_xyz, ctx->srf_nrm, ctx->srf_rgb, ctx->srf_tri, (uint32_t)nv, (uint32_t)nf, H,
-                       ctx->cc_xyz, ctx->cc_nrm, ctx->cc_rgb, ctx->cc_tri, ctx->sm_count, ctx->stream));
-    ctx->launches += DECIMATE_LAUNCHES;
+    // the emission runs before the synchronisation, so the spare set holds the whole input
+    CK(ctx->spare.grow(std::max<int64_t>(nv, 1), std::max<int64_t>(nf, 1)));
+    CK(ctx->dec.run(ctx->surface, H, ctx->spare, ctx->sm_count, ctx->stream, &ctx->launches));
     DecimateState st;
     VoxelState vst;
-    CK(cudaMemcpyAsync(&st, b.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(&vst, t.state, sizeof(vst), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&st, ctx->dec.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&vst, ctx->dec.clusters.state, sizeof(vst), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     // the simplified set becomes the held surface; the old one is the next compaction's destination
-    std::swap(ctx->srf_xyz, ctx->cc_xyz);
-    std::swap(ctx->srf_nrm, ctx->cc_nrm);
-    std::swap(ctx->srf_rgb, ctx->cc_rgb);
-    std::swap(ctx->srf_tri, ctx->cc_tri);
-    ctx->srf_vertices = vst.total[1];
-    ctx->srf_faces = st.faces;
+    std::swap(ctx->surface, ctx->spare);
+    ctx->surface.vertices = vst.total[1];
+    ctx->surface.faces = st.faces;
     ctx->srf_decimated = true;
     out->vertices = vst.total[1];
     out->faces = st.faces;
@@ -1585,29 +1448,10 @@ static int smooth_run(scan3d_ctx* ctx, const float* xyz, const float* nrm, const
 {
     if (6 * nf >= (1LL << 32)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than (2^32 - 1) / 6 faces");
     const int passes = p->iterations * (p->mu == 0.0f ? 1 : 2);
-    const size_t av = (size_t)std::max<int64_t>(nv, 1);
-    const uint32_t cap = (uint32_t)std::max<int64_t>(6 * nf, 64);   // two slots per side: at most half are taken
-    CK(grow_group(Grow(ctx->sm_keys, cap), Grow(ctx->sm_sides, cap), Grow(ctx->sm_rows, cap)));
-    CK(grow_group(Grow(ctx->sm_degree, av), Grow(ctx->sm_held, av),
-                  Grow(ctx->sm_block_counts, (av + POINT_BLOCK - 1) / POINT_BLOCK + 1), Grow(ctx->sm_cursor, av),
-                  Grow(ctx->sm_q[0], 3 * av), Grow(ctx->sm_q[1], 3 * av)));
-    CK(ctx->sm_nsum.ensure(3 * av));
-    CK(ctx->sm_state.ensure(1));
-    SmoothBuffers b;
-    b.keys = ctx->sm_keys; b.sides = ctx->sm_sides; b.cap = cap; b.rows = ctx->sm_rows;
-    b.degree = ctx->sm_degree; b.held = ctx->sm_held; b.block_counts = ctx->sm_block_counts; b.cursor = ctx->sm_cursor;
-    b.q[0] = ctx->sm_q[0]; b.q[1] = ctx->sm_q[1]; b.nsum = ctx->sm_nsum; b.state = ctx->sm_state;
-    CK(cudaMemsetAsync(b.keys, 0xff, (size_t)cap * sizeof(*b.keys), ctx->stream));
-    CK(cudaMemsetAsync(b.sides, 0, (size_t)cap * sizeof(*b.sides), ctx->stream));
-    CK(cudaMemsetAsync(b.degree, 0, av * sizeof(*b.degree), ctx->stream));
-    CK(cudaMemsetAsync(b.held, 0, av * sizeof(*b.held), ctx->stream));
-    CK(cudaMemsetAsync(b.nsum, 0, 3 * av * sizeof(*b.nsum), ctx->stream));
-    CK(cudaMemsetAsync(b.state, 0, sizeof(*b.state), ctx->stream));
-    CK(launch_smooth(b, xyz, nrm, faces, (uint32_t)nv, (uint32_t)nf, passes, (double)p->lambda, (double)p->mu, xyz_out,
-                     nrm_out, ctx->stream));
-    ctx->launches += SMOOTH_BUILD_LAUNCHES + passes + SMOOTH_END_LAUNCHES;
+    CK(ctx->smooth.run(xyz, nrm, faces, (uint32_t)nv, (uint32_t)nf, passes, (double)p->lambda, (double)p->mu, xyz_out,
+                       nrm_out, ctx->stream, &ctx->launches));
     SmoothState st;
-    CK(cudaMemcpyAsync(&st, b.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&st, ctx->smooth.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     if (st.bad) return fail(ctx, SCAN3D_ERR_ARG, "a coordinate that is not finite or a face index outside [0, n_vertices)");
     if (st.overflow)
@@ -1632,14 +1476,13 @@ int scan3d_voxel_surface_smooth(scan3d_ctx* ctx, const scan3d_smooth_params* p, 
     if (!ctx->srf_ready)
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
     CK(cudaSetDevice(ctx->device));
-    const int64_t nv = ctx->srf_vertices, nf = ctx->srf_faces;
-    const size_t av3 = 3 * (size_t)std::max<int64_t>(nv, 1);
-    CK(grow_group(Grow(ctx->cc_xyz, av3), Grow(ctx->cc_nrm, av3)));
-    rc = smooth_run(ctx, ctx->srf_xyz, ctx->srf_nrm, ctx->srf_tri, nv, nf, p, ctx->cc_xyz, ctx->cc_nrm, out);
+    SurfaceMesh &s = ctx->surface, &spare = ctx->spare;
+    CK(spare.grow_positions(std::max<int64_t>(s.vertices, 1)));
+    rc = smooth_run(ctx, s.xyz, s.nrm, s.tri, s.vertices, s.faces, p, spare.xyz, spare.nrm, out);
     if (rc) return rc;
     // the smoothed positions and normals become the held surface; faces, colours and the vertex order are unchanged
-    std::swap(ctx->srf_xyz, ctx->cc_xyz);
-    std::swap(ctx->srf_nrm, ctx->cc_nrm);
+    std::swap(s.xyz, spare.xyz);
+    std::swap(s.nrm, spare.nrm);
     ctx->srf_smoothed = true;
     return SCAN3D_OK;
 }

@@ -287,44 +287,70 @@ __global__ void __launch_bounds__(POINT_BLOCK) k_cc_emit_faces(const uint8_t* __
 namespace {
 // at least one block, so that every launch runs for an empty mesh too
 unsigned grid(uint32_t n, int threads) { return n ? (unsigned)((n + (uint64_t)threads - 1) / threads) : 1u; }
-}  // namespace
 
-cudaError_t launch_cc_labels(const int32_t* faces, uint32_t n_faces, uint32_t n, uint32_t* parent, uint8_t* flags,
-                             uint32_t* block_counts, int32_t* label, ComponentsState* state, cudaStream_t st)
+// the labelling scratch for n vertices, and the state zeroed
+cudaError_t reset_labels(ComponentsWorkspace& w, uint32_t n, cudaStream_t st)
 {
-    k_cc_init<<<grid(n, CT), CT, 0, st>>>(parent, n);
-    k_cc_hook<<<grid(n_faces, CT), CT, 0, st>>>(faces, n_faces, n, parent, state);
-    k_cc_compress<<<grid(n, CT), CT, 0, st>>>(parent, flags, n);
-    cudaError_t e = launch_point_offsets(flags, n, block_counts, &state->components, st);
+    const size_t a = n ? n : 1;
+    cudaError_t e =
+        grow_group(Grow(w.parent, a), Grow(w.flags, a), Grow(w.vert_counts, (a + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+    if (e == cudaSuccess) e = w.state.ensure(1);
+    if (e == cudaSuccess) e = cudaMemsetAsync(w.state, 0, sizeof(ComponentsState), st);
+    return e;
+}
+
+cudaError_t launch_labels(ComponentsWorkspace& w, const int32_t* faces, uint32_t n_faces, uint32_t n, int32_t* label,
+                          cudaStream_t st, int64_t* launches)
+{
+    k_cc_init<<<grid(n, CT), CT, 0, st>>>(w.parent, n);
+    k_cc_hook<<<grid(n_faces, CT), CT, 0, st>>>(faces, n_faces, n, w.parent, w.state);
+    k_cc_compress<<<grid(n, CT), CT, 0, st>>>(w.parent, w.flags, n);
+    cudaError_t e = launch_point_offsets(w.flags, n, w.vert_counts, &w.state.get()->components, st);
     if (e != cudaSuccess) return e;
-    k_cc_root_ids<<<grid(n, POINT_BLOCK), POINT_BLOCK, 0, st>>>(flags, block_counts, n, label);
-    k_cc_labels<<<grid(n, CT), CT, 0, st>>>(parent, n, label);
+    k_cc_root_ids<<<grid(n, POINT_BLOCK), POINT_BLOCK, 0, st>>>(w.flags, w.vert_counts, n, label);
+    k_cc_labels<<<grid(n, CT), CT, 0, st>>>(w.parent, n, label);
+    *launches += 7;
     return cudaGetLastError();
 }
+}  // namespace
 
-cudaError_t launch_cc_select(const int32_t* faces, uint32_t n_faces, uint32_t n, const int32_t* label,
-                             unsigned long long min_faces, unsigned long long max_components, uint32_t* comp_v,
-                             uint32_t* comp_f, uint8_t* kept, uint8_t* keep_v, uint8_t* keep_f, uint32_t* vert_counts,
-                             uint32_t* face_counts, ComponentsState* state, cudaStream_t st)
+cudaError_t ComponentsWorkspace::labels(const int32_t* faces, uint32_t n_faces, uint32_t n, int32_t* out,
+                                        cudaStream_t st, int64_t* launches)
 {
-    const uint32_t m = n > n_faces ? n : n_faces;
-    k_cc_count<<<grid(m, CT), CT, 0, st>>>(label, faces, n, n_faces, comp_v, comp_f);
-    k_cc_select<<<1, SELECT_THREADS, 0, st>>>(comp_f, state, min_faces, max_components);
-    k_cc_keep<<<grid(m, CT), CT, 0, st>>>(label, faces, comp_f, state, min_faces, n, n_faces, keep_v, keep_f, kept);
-    cudaError_t e = launch_point_offsets(keep_v, n, vert_counts, &state->vertices, st);
-    if (e != cudaSuccess) return e;
-    return launch_point_offsets(keep_f, n_faces, face_counts, &state->faces, st);
+    const cudaError_t e = reset_labels(*this, n, st);
+    return e != cudaSuccess ? e : launch_labels(*this, faces, n_faces, n, out, st, launches);
 }
 
-cudaError_t launch_cc_emit(const uint8_t* keep_v, const uint32_t* vert_counts, uint32_t n, const float* xyz,
-                           const float* nrm, const uint8_t* rgb, const uint8_t* keep_f, const uint32_t* face_counts,
-                           uint32_t n_faces, const int32_t* faces, int32_t* new_index, float* xyz2, float* nrm2,
-                           uint8_t* rgb2, int32_t* faces2, cudaStream_t st)
+cudaError_t ComponentsWorkspace::select(const SurfaceMesh& in, unsigned long long min_faces,
+                                        unsigned long long max_components, cudaStream_t st, int64_t* launches)
 {
-    k_cc_emit_vertices<<<grid(n, POINT_BLOCK), POINT_BLOCK, 0, st>>>(keep_v, vert_counts, n, xyz, nrm, rgb, xyz2, nrm2,
-                                                                     rgb2, new_index);
-    k_cc_emit_faces<<<grid(n_faces, POINT_BLOCK), POINT_BLOCK, 0, st>>>(keep_f, face_counts, n_faces, faces, new_index,
-                                                                        faces2);
+    const uint32_t n = (uint32_t)in.vertices, n_faces = (uint32_t)in.faces;
+    const size_t av = n ? n : 1, af = n_faces ? n_faces : 1;
+    cudaError_t e = reset_labels(*this, n, st);
+    if (e == cudaSuccess) e = grow_group(Grow(label, av), Grow(comp_v, av), Grow(comp_f, av), Grow(kept, av));
+    if (e == cudaSuccess) e = grow_group(Grow(keep_f, af), Grow(face_counts, (af + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+    if (e == cudaSuccess) e = cudaMemsetAsync(comp_v, 0, (size_t)n * sizeof(uint32_t), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(comp_f, 0, (size_t)n * sizeof(uint32_t), st);
+    if (e == cudaSuccess) e = launch_labels(*this, in.tri, n_faces, n, label, st, launches);
+    if (e != cudaSuccess) return e;
+    const uint32_t m = n > n_faces ? n : n_faces;
+    k_cc_count<<<grid(m, CT), CT, 0, st>>>(label, in.tri, n, n_faces, comp_v, comp_f);
+    k_cc_select<<<1, SELECT_THREADS, 0, st>>>(comp_f, state, min_faces, max_components);
+    k_cc_keep<<<grid(m, CT), CT, 0, st>>>(label, in.tri, comp_f, state, min_faces, n, n_faces, flags, keep_f, kept);
+    e = launch_point_offsets(flags, n, vert_counts, &state.get()->vertices, st);
+    if (e != cudaSuccess) return e;
+    *launches += 7;
+    return launch_point_offsets(keep_f, n_faces, face_counts, &state.get()->faces, st);
+}
+
+cudaError_t ComponentsWorkspace::emit(const SurfaceMesh& in, SurfaceMesh& out, cudaStream_t st, int64_t* launches)
+{
+    const uint32_t n = (uint32_t)in.vertices, n_faces = (uint32_t)in.faces;
+    k_cc_emit_vertices<<<grid(n, POINT_BLOCK), POINT_BLOCK, 0, st>>>(flags, vert_counts, n, in.xyz, in.nrm, in.rgb,
+                                                                     out.xyz, out.nrm, out.rgb, label);
+    k_cc_emit_faces<<<grid(n_faces, POINT_BLOCK), POINT_BLOCK, 0, st>>>(keep_f, face_counts, n_faces, in.tri, label,
+                                                                        out.tri);
+    *launches += 2;
     return cudaGetLastError();
 }
 

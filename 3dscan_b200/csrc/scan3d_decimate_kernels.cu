@@ -181,22 +181,40 @@ __global__ void __launch_bounds__(POINT_BLOCK) k_dec_faces(const uint8_t* __rest
     for (int j = 0; j < 3; j++) faces2[3 * (size_t)r + j] = ctri[3 * (size_t)f + j];
 }
 
-cudaError_t launch_decimate(const VoxelTable& t, const DecimateBuffers& b, const float* xyz, const float* nrm,
-                            const uint8_t* rgb, const int32_t* tri, uint32_t n_vertices, uint32_t n_faces, double H,
-                            float* xyz2, float* nrm2, uint8_t* rgb2, int32_t* faces2, int sm_count, cudaStream_t st)
+cudaError_t DecimateWorkspace::run(const SurfaceMesh& in, double H, SurfaceMesh& out, int sm_count, cudaStream_t st,
+                                   int64_t* launches)
 {
+    const uint32_t n_vertices = (uint32_t)in.vertices, n_faces = (uint32_t)in.faces;
+    // the cluster table is sized as the merge's for max_voxels = the vertex count
+    const size_t av = n_vertices ? n_vertices : 1, af = n_faces ? n_faces : 1;
+    const uint32_t table_cap = (uint32_t)(2 * af);
+    cudaError_t e = clusters.reset((uint32_t)av, H, sm_count, st);
+    if (e == cudaSuccess)
+        e = grow_group(Grow(point_slot, av), Grow(vert_flags, av),
+                       Grow(vert_counts, (av + POINT_BLOCK - 1) / POINT_BLOCK + 1), Grow(quad, s3q::NQ * av));
+    if (e == cudaSuccess)
+        e = grow_group(Grow(ctri, 3 * af), Grow(table, table_cap), Grow(slot_of, af), Grow(keep, af),
+                       Grow(face_counts, (af + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+    if (e == cudaSuccess) e = state.ensure(1);
+    if (e == cudaSuccess) e = cudaMemsetAsync(quad, 0, s3q::NQ * av * sizeof(unsigned long long), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(table, 0xff, (size_t)table_cap * sizeof(uint32_t), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(state, 0, sizeof(DecimateState), st);
+    if (e != cudaSuccess) return e;
+    const VoxelTable& t = clusters.view;
+    DecimateState* ds = state;
     // an empty surface still runs every launch: one block that reads a vertex count of 0
     const uint32_t plane = n_vertices ? n_vertices : 1;
-    cudaError_t e = launch_voxel_add(t, xyz, nrm, rgb, n_vertices ? nullptr : &b.state->zero, plane, b.point_slot,
-                                     b.vert_flags, b.vert_counts, 0, st);
+    e = launch_voxel_add(t, in.xyz, in.nrm, in.rgb, n_vertices ? nullptr : &ds->zero, plane, point_slot, vert_flags,
+                         vert_counts, 0, st, launches);
     if (e != cudaSuccess) return e;
-    k_dec_quadrics<<<grid(n_faces, DT), DT, 0, st>>>(t, xyz, tri, n_faces, H, b.point_slot, b.ctri, b.quad);
-    k_dec_insert<<<grid(n_faces, DT), DT, 0, st>>>(b.ctri, n_faces, b.table, b.table_cap, b.slot_of, b.state);
-    k_dec_flags<<<grid(n_faces, DT), DT, 0, st>>>(b.table, b.slot_of, n_faces, b.keep);
-    e = launch_point_offsets(b.keep, n_faces, b.face_counts, &b.state->faces, st);
+    k_dec_quadrics<<<grid(n_faces, DT), DT, 0, st>>>(t, in.xyz, in.tri, n_faces, H, point_slot, ctri, quad);
+    k_dec_insert<<<grid(n_faces, DT), DT, 0, st>>>(ctri, n_faces, table, table_cap, slot_of, ds);
+    k_dec_flags<<<grid(n_faces, DT), DT, 0, st>>>(table, slot_of, n_faces, keep);
+    e = launch_point_offsets(keep, n_faces, face_counts, &ds->faces, st);
     if (e != cudaSuccess) return e;
-    k_dec_vertices<<<4 * sm_count, 256, 0, st>>>(t, b.quad, H, xyz2, nrm2, rgb2, b.state);
-    k_dec_faces<<<grid(n_faces, POINT_BLOCK), POINT_BLOCK, 0, st>>>(b.keep, b.face_counts, n_faces, b.ctri, faces2);
+    k_dec_vertices<<<4 * sm_count, 256, 0, st>>>(t, quad, H, out.xyz, out.nrm, out.rgb, ds);
+    k_dec_faces<<<grid(n_faces, POINT_BLOCK), POINT_BLOCK, 0, st>>>(keep, face_counts, n_faces, ctri, out.tri);
+    *launches += 7;
     return cudaGetLastError();
 }
 

@@ -61,7 +61,7 @@ __device__ __forceinline__ uint32_t find_slot(const unsigned long long* __restri
     return VOXEL_NO_SLOT;
 }
 
-// The exact nearest model point to p within r2 in the alignment's cell index (launch_align_index, cell edge S): the
+// The exact nearest model point to p within r2 in the alignment's cell index (AlignWorkspace::index, cell edge S): the
 // smallest s3l::dist2, a tie going to the smaller ordinal.  Returns its ordinal and sets *entry to its entry, or
 // VOXEL_NO_SLOT when no model point qualifies.
 __device__ __forceinline__ uint32_t align_nearest(const AlignIndex& ix, const double p[3], double S, double r2,

@@ -22,6 +22,10 @@ struct TensorMapCache {
     int next = 0;
 };
 
+// Each stage on the merged model owns its device scratch in a workspace below.  The workspace's functions, defined next
+// to the stage's kernels, grow the scratch, clear what the kernels need cleared and launch.  A function or launcher
+// with an int64_t* launches argument adds the kernels it launches to *launches.
+
 // the voxel-grid merge's hash table (scan3d_voxel_kernels.cu)
 constexpr uint32_t VOXEL_NO_SLOT = 0xffffffffu;   // no slot / no ordinal yet
 // the integer sums of one voxel (zero-initialised); first_inv = ~(index of the first point within the current add)
@@ -47,6 +51,17 @@ struct VoxelTable {
     VoxelState* state;
     uint32_t cap, max_voxels;
     double S;                  // (double)voxel_size
+};
+// One voxel hash table and its kernels' view: the merge's accumulator and the simplification's clusters.
+struct VoxelStore {
+    DeviceBuffer<unsigned long long> keys;
+    DeviceBuffer<VoxelSlot> acc;
+    DeviceBuffer<uint32_t> ordinal;
+    DeviceBuffer<uint32_t> ord2slot;
+    DeviceBuffer<VoxelState> state;
+    VoxelTable view{};
+    // an empty table for max_voxels voxels of edge S: grown, the view set, keys and ordinals 0xff, sums and state 0
+    cudaError_t reset(uint32_t max_voxels, double S, int sm_count, cudaStream_t st);
 };
 
 // the alignment's cell index of the model (scan3d_align_kernels.cu)
@@ -74,6 +89,27 @@ struct AlignRun {
     double stop_rotation, stop_translation;
     int max_iterations;
 };
+// The alignment's cell index of the merged model, the state of one run and the match partials.  The model is the first
+// min(total, max_voxels) voxel outputs (xyz, nrm [max_voxels][3]) of t, total = t.state->total[par].
+struct AlignWorkspace {
+    DeviceBuffer<unsigned long long> keys;   // [2 max_voxels]
+    DeviceBuffer<uint2> cells;               // [2 max_voxels]
+    DeviceBuffer<uint32_t> model_slot;       // [max_voxels]
+    DeviceBuffer<float4> entries;            // [2 max_voxels]
+    DeviceBuffer<uint32_t> cursor;           // [1]
+    DeviceBuffer<double> partials;           // [sums + 1][blocks]
+    DeviceBuffer<AlignState> state;
+    AlignIndex view{};
+    // the index of cell edge run.S, 3 launches: cell keys and counts (which also initialises state from run, the voxel
+    // overflow flag and, when n_dev is set, the source count), cell ranges, scatter of the model points
+    cudaError_t index(const VoxelTable& t, int par, const float* xyz, const float* nrm, const AlignRun& run,
+                      const uint32_t* n_dev, int sm_count, cudaStream_t st, int64_t* launches);
+    // the index, then one match + one solve launch per iteration.  The source is src[i * stride] for i * stride < n,
+    // n = min(*n_dev, n_max) when n_dev is set, else n_max; the grid depends on n_max and stride only.
+    cudaError_t align(const VoxelTable& t, int par, const float* xyz, const float* nrm, const AlignRun& run,
+                      const float* src, const uint32_t* n_dev, long long n_max, int stride, int sm_count,
+                      cudaStream_t st, int64_t* launches);
+};
 
 // the surface extraction's lattice table (scan3d_surface_kernels.cu), one slot per distinct lattice point
 struct SurfaceState {
@@ -92,6 +128,41 @@ struct SurfaceTable {
     uint32_t cap, max_points;
     double S;                      // (double)voxel_size
 };
+// A triangle surface.  The context holds two: the held surface and the spare set, which the stage that replaces the
+// held surface writes before the two are swapped.
+struct SurfaceMesh {
+    DeviceBuffer<float> xyz, nrm;  // [vertices][3]
+    DeviceBuffer<uint8_t> rgb;     // [vertices][3]
+    DeviceBuffer<int32_t> tri;     // [faces][3]
+    int64_t vertices = 0, faces = 0;
+    cudaError_t grow(size_t nv, size_t nf)
+    {
+        const cudaError_t e = grow_group(Grow(xyz, 3 * nv), Grow(nrm, 3 * nv), Grow(rgb, 3 * nv));
+        return e != cudaSuccess ? e : tri.ensure(3 * nf);
+    }
+    // positions and normals only: the smoothing writes nothing else
+    cudaError_t grow_positions(size_t nv) { return grow_group(Grow(xyz, 3 * nv), Grow(nrm, 3 * nv)); }
+};
+// The lattice table and the vertex scratch of the surface extraction.
+struct SurfaceWorkspace {
+    DeviceBuffer<unsigned long long> keys, owner;  // [cap]
+    DeviceBuffer<double> f;                        // [cap]
+    DeviceBuffer<uint32_t> nearest, vert;          // [cap]
+    DeviceBuffer<SurfaceState> state;
+    DeviceBuffer<uint8_t> flags;                   // [27 max_voxels] (o, k) owns an active cell
+    DeviceBuffer<uint32_t> flag_counts;            // [cdiv(27 max_voxels, POINT_BLOCK) + 1]
+    DeviceBuffer<uint32_t> vert_slot;              // [max_points] lattice slot of each vertex
+    DeviceBuffer<uint32_t> face_counts;            // [cdiv(max_points, vertex block) + 1] faces per block, then offsets
+    SurfaceTable view{};
+    // 8 launches after ix was built from t's model with cell edge s3l::cell_edge(max_distance): candidate cells (27 per
+    // model voxel, with their order key), their other 7 corners, the corner values, the (o, k) flags of active cells,
+    // k_count + k_scan over them (the vertex ordinals), vertex assignment with the faces per block of vertices, and the
+    // scan of those; state->vertices and state->faces are then known
+    cudaError_t count(const AlignIndex& ix, const VoxelTable& t, int par, const float* vox_nrm, float max_distance,
+                      uint32_t max_points, int sm_count, cudaStream_t st, int64_t* launches);
+    // 1 launch: the vertices (xyz, normals, rgb) and faces into out
+    cudaError_t emit(const uint8_t* vox_rgb, uint32_t vertices, SurfaceMesh& out, cudaStream_t st, int64_t* launches);
+};
 
 // the connected components of a triangle mesh (scan3d_components_kernels.cu)
 struct ComponentsState {
@@ -102,26 +173,58 @@ struct ComponentsState {
     uint32_t bad;                  // a face index outside [0, vertices)
     uint32_t pad;
 };
+// The union-find scratch and the component table.
+struct ComponentsWorkspace {
+    DeviceBuffer<uint32_t> parent;       // [vertices] union-find forest, then each vertex's root
+    DeviceBuffer<uint8_t> flags;         // [vertices] root flags, then the vertices' keep flags
+    DeviceBuffer<uint32_t> vert_counts;  // [cdiv(vertices, POINT_BLOCK) + 1] block offsets of the flags
+    DeviceBuffer<int32_t> label;         // [vertices] component ids, then the kept vertices' new indices
+    DeviceBuffer<uint32_t> comp_v;       // [vertices] per component: vertices, faces, kept flag
+    DeviceBuffer<uint32_t> comp_f;
+    DeviceBuffer<uint8_t> kept;
+    DeviceBuffer<uint8_t> keep_f;        // [faces]
+    DeviceBuffer<uint32_t> face_counts;  // [cdiv(faces, POINT_BLOCK) + 1]
+    DeviceBuffer<ComponentsState> state;
+    // 7 launches for n vertices and n_faces faces [n_faces][3]: parent = v, union per face, find per vertex with the
+    // root flags, k_count + k_scan over them (state->components), the roots' ids, every vertex's id into out [n].  Any
+    // n below 2^31 and n_faces below 2^32, 0 included.
+    cudaError_t labels(const int32_t* faces, uint32_t n_faces, uint32_t n, int32_t* out, cudaStream_t st,
+                       int64_t* launches);
+    // 14 launches on the mesh of in: its labels, then vertices and faces per component, the selection
+    // (state->threshold, kept, largest), the keep flags, k_count + k_scan over each of the vertex flags
+    // (state->vertices) and the face flags (state->faces)
+    cudaError_t select(const SurfaceMesh& in, unsigned long long min_faces, unsigned long long max_components,
+                       cudaStream_t st, int64_t* launches);
+    // 2 launches after select: the kept vertices of in into out (their new indices into label), then the kept faces,
+    // remapped
+    cudaError_t emit(const SurfaceMesh& in, SurfaceMesh& out, cudaStream_t st, int64_t* launches);
+};
 
-// the surface simplification (scan3d_decimate_kernels.cu); the clusters are a second VoxelTable
+// the surface simplification (scan3d_decimate_kernels.cu); the clusters are a second VoxelStore
 struct DecimateState {
     uint32_t collapsed;            // faces with two corners in one cluster
     uint32_t fallbacks;            // clusters placed at their mean after a failed solve
     uint32_t faces;                // kept faces
     uint32_t zero;                 // stays 0: the vertex count of an empty surface's voxel add
 };
-struct DecimateBuffers {
-    uint32_t* point_slot;          // [vertices] cluster slot of each vertex
-    uint8_t* vert_flags;           // [vertices]
-    uint32_t* vert_counts;         // [cdiv(vertices, POINT_BLOCK) + 1]
-    unsigned long long* quad;      // [vertices][10] quadric sums per cluster ordinal (int64 two's complement), zeroed
-    int32_t* ctri;                 // [faces][3] cluster ordinals of the corners
-    uint32_t* table;               // [table_cap] face indices, VOXEL_NO_SLOT = free
-    uint32_t table_cap;
-    uint32_t* slot_of;             // [faces] table slot of each face, VOXEL_NO_SLOT = collapsed
-    uint8_t* keep;                 // [faces]
-    uint32_t* face_counts;         // [cdiv(faces, POINT_BLOCK) + 1]
-    DecimateState* state;          // zeroed
+struct DecimateWorkspace {
+    VoxelStore clusters;                    // edge H, max_voxels = the vertex count
+    DeviceBuffer<uint32_t> point_slot;      // [vertices] cluster slot of each vertex
+    DeviceBuffer<uint8_t> vert_flags;       // [vertices]
+    DeviceBuffer<uint32_t> vert_counts;     // [cdiv(vertices, POINT_BLOCK) + 1]
+    DeviceBuffer<unsigned long long> quad;  // [vertices][10] quadric sums per cluster ordinal (int64 two's complement)
+    DeviceBuffer<int32_t> ctri;             // [faces][3] cluster ordinals of the corners
+    DeviceBuffer<uint32_t> table;           // [2 faces] face indices, VOXEL_NO_SLOT = free
+    DeviceBuffer<uint32_t> slot_of;         // [faces] table slot of each face, VOXEL_NO_SLOT = collapsed
+    DeviceBuffer<uint8_t> keep;             // [faces]
+    DeviceBuffer<uint32_t> face_counts;     // [cdiv(faces, POINT_BLOCK) + 1]
+    DeviceBuffer<DecimateState> state;
+    // 12 launches for the surface in: the merge's voxel add over its vertices into the clusters, the face quadrics
+    // with the cluster triples, the duplicate-face table, the keep flags, k_count + k_scan over them (state->faces),
+    // then the vertices of the clusters (clusters.state->total[1] of them) and the kept faces into out, which holds
+    // in's counts
+    cudaError_t run(const SurfaceMesh& in, double H, SurfaceMesh& out, int sm_count, cudaStream_t st,
+                    int64_t* launches);
 };
 
 // the surface smoothing (scan3d_smooth_kernels.cu); the undirected edges are a hash of (min << 32 | max) keys
@@ -133,18 +236,25 @@ struct SmoothState {
     uint32_t held, isolated;       // vertices on an edge whose count is not 2; vertices without a neighbour
     uint32_t entries;              // neighbour row entries (the sum of the degrees)
 };
-struct SmoothBuffers {
-    unsigned long long* keys;      // [cap] edge keys, s3v::EMPTY_KEY = free
-    uint32_t* sides;               // [cap] sides on each edge, zeroed
-    uint32_t cap;
-    uint32_t* degree;              // [vertices] distinct neighbours, zeroed
-    uint8_t* held;                 // [vertices] zeroed
-    uint32_t* block_counts;        // [cdiv(vertices, POINT_BLOCK) + 1]
-    uint32_t* cursor;              // [vertices] row start, then (after the scatter) row end
-    uint32_t* rows;                // [cap] neighbour indices (2 per edge, at most 2 * 3 nf)
-    long long* q[2];               // [vertices][3] fixed-point positions, ping-pong
-    unsigned long long* nsum;      // [vertices][3] fixed-point normal sums (int64 two's complement), zeroed
-    SmoothState* state;            // zeroed
+struct SmoothWorkspace {
+    DeviceBuffer<unsigned long long> keys;  // [6 faces] the edge table
+    DeviceBuffer<uint32_t> sides;           // [6 faces]
+    DeviceBuffer<uint32_t> rows;            // [6 faces]
+    DeviceBuffer<uint32_t> degree;          // [vertices]
+    DeviceBuffer<uint8_t> held;             // [vertices]
+    DeviceBuffer<uint32_t> block_counts;    // [cdiv(vertices, POINT_BLOCK) + 1]
+    DeviceBuffer<uint32_t> cursor;          // [vertices]
+    DeviceBuffer<long long> q[2];           // [vertices][3]
+    DeviceBuffer<unsigned long long> nsum;  // [vertices][3]
+    DeviceBuffer<SmoothState> state;
+    // 7 + passes + 2 launches for n vertices (xyz, nrm may be null) and nf faces [nf][3], nf < 2^32 / 6: the exponent
+    // max and the finiteness check over the vertices, the sides into the edge table, the degrees and held flags per
+    // edge, the degree sums per POINT_BLOCK vertices, their k_scan, the row starts with the fixed-point positions, the
+    // neighbour rows; then one gather per pass (k = lambda, or lambda and mu alternating when mu != 0); then the face
+    // normals and the write of xyz_out / nrm_out (nrm_out may be null), which writes nothing when the state holds an
+    // error.  xyz_out may be xyz and nrm_out nrm.
+    cudaError_t run(const float* xyz, const float* nrm, const int32_t* faces, uint32_t n, uint32_t nf, int passes,
+                    double lambda, double mu, float* xyz_out, float* nrm_out, cudaStream_t st, int64_t* launches);
 };
 }  // namespace s3d
 
@@ -215,18 +325,12 @@ struct scan3d_ctx {
     Buf<int32_t> mesh_faces;       // [2(W-1)(H-1)][3]
     Buf<float> mesh_normals;       // [H*W][3]
 
-    // scan3d_voxel_begin: the merge accumulator (independent of the points; reallocated when a begin asks for more).
-    // vox is the kernels' view of the vox_* buffers below.
-    s3d::VoxelTable vox{};
+    // scan3d_voxel_begin: the merge accumulator (independent of the points; reallocated when a begin asks for more)
+    s3d::VoxelStore vox;
     bool vox_begun = false;        // a begin has run
     bool vox_fresh = false;        // the outputs are those of the adds since begin (a finish ran after the last add)
     uint64_t vox_bound = 0;        // upper bound of the points added since begin (W*H per ctx add, n per dev add)
     uint32_t vox_chunks = 0;       // adds (chunks of <= W*H points) since begin
-    Buf<unsigned long long> vox_keys;     // [cap] the table
-    Buf<s3d::VoxelSlot> vox_acc;          // [cap]
-    Buf<uint32_t> vox_ordinal;            // [cap]
-    Buf<uint32_t> vox_ord2slot;           // [max_voxels]
-    Buf<s3d::VoxelState> vox_state;
     Buf<uint32_t> vox_point_slot;         // [H*W] per-point scratch of an add
     Buf<uint8_t> vox_flags;               // [H*W]
     Buf<float> vox_xyz;                   // [max_voxels][3] outputs of scan3d_voxel_finish
@@ -234,88 +338,21 @@ struct scan3d_ctx {
     Buf<uint8_t> vox_rgb;                 // [max_voxels][3]
     Buf<uint32_t> vox_cnt;                // [max_voxels]
 
-    // scan3d_align_to_voxels (allocated by the first align, grown with max_voxels and the sample count); aln is the
-    // kernels' view of the aln_* index buffers
-    s3d::AlignIndex aln{};
-    Buf<unsigned long long> aln_keys;     // [2 max_voxels]
-    Buf<uint2> aln_cells;                 // [2 max_voxels]
-    Buf<uint32_t> aln_model_slot;         // [max_voxels]
-    Buf<float4> aln_entries;              // [2 max_voxels]
-    Buf<uint32_t> aln_cursor;             // [1]
-    Buf<double> aln_partials;             // [ALIGN_NSUM + 1][blocks]
-    Buf<s3d::AlignState> aln_state;
+    // The stages on the merged model.  Each owns its device scratch, allocates it on first use, grows it on demand
+    // and clears what its kernels need cleared.
+    s3d::AlignWorkspace aln;              // scan3d_align_to_voxels*, and the model index of scan3d_voxel_surface
+    s3d::SurfaceWorkspace lattice;        // scan3d_voxel_surface
+    s3d::ComponentsWorkspace cc;          // scan3d_voxel_surface_components, scan3d_mesh_components_dev
+    s3d::DecimateWorkspace dec;           // scan3d_voxel_surface_decimate
+    s3d::SmoothWorkspace smooth;          // scan3d_voxel_surface_smooth, scan3d_mesh_smooth_dev
 
-    // scan3d_voxel_surface (allocated by the first extraction, grown on demand); srf is the kernels' view of the
-    // lattice table srf_keys ... srf_state
-    s3d::SurfaceTable srf{};
+    // the held voxel surface, and the spare set that components, decimate and smooth write before they swap it in
+    s3d::SurfaceMesh surface, spare;
     bool srf_ready = false;               // the surface of the current voxel outputs is held
-    Buf<unsigned long long> srf_keys;     // [cap]
-    Buf<unsigned long long> srf_owner;    // [cap]
-    Buf<double> srf_f;                    // [cap]
-    Buf<uint32_t> srf_nearest;            // [cap]
-    Buf<uint32_t> srf_vert;               // [cap]
-    Buf<s3d::SurfaceState> srf_state;
-    Buf<uint8_t> srf_flags;               // [27 max_voxels] (o, k) owns an active cell
-    Buf<uint32_t> srf_flag_counts;        // [cdiv(27 max_voxels, POINT_BLOCK) + 1]
-    Buf<uint32_t> srf_vert_slot;          // [max_points] lattice slot of each vertex
-    Buf<uint32_t> srf_face_counts;        // [cdiv(max_points, SURFACE_VB) + 1] faces per block of vertices, then offsets
-    int64_t srf_vertices = 0, srf_faces = 0;
-    Buf<float> srf_xyz;                   // [vertices][3]
-    Buf<float> srf_nrm;                   // [vertices][3]
-    Buf<uint8_t> srf_rgb;                 // [vertices][3]
-    Buf<int32_t> srf_tri;                 // [faces][3]
-
-    // scan3d_voxel_surface_components / scan3d_mesh_components_dev (allocated on first use, grown on demand)
     bool cc_ready = false;                // the component table of the last scan3d_voxel_surface_components is held
     int64_t cc_components = 0;
-    Buf<uint32_t> cc_parent;              // [vertices] union-find forest, then each vertex's root
-    Buf<uint8_t> cc_flags;                // [vertices] root flags, then the vertices' keep flags
-    Buf<uint32_t> cc_vert_counts;         // [cdiv(vertices, POINT_BLOCK) + 1] block offsets of the flags
-    Buf<int32_t> cc_label;                // [vertices] component ids, then the kept vertices' new indices
-    Buf<uint32_t> cc_comp_v;              // [vertices] per component: vertices, faces, kept flag
-    Buf<uint32_t> cc_comp_f;
-    Buf<uint8_t> cc_kept;
-    Buf<uint8_t> cc_keep_f;               // [faces]
-    Buf<uint32_t> cc_face_counts;         // [cdiv(faces, POINT_BLOCK) + 1]
-    Buf<s3d::ComponentsState> cc_state;
-    Buf<float> cc_xyz;                    // the second surface set, swapped with srf_* after a compaction
-    Buf<float> cc_nrm;
-    Buf<uint8_t> cc_rgb;
-    Buf<int32_t> cc_tri;
-
-    // scan3d_voxel_surface_decimate (allocated on first use, grown on demand); dec is the kernels' view of the cluster
-    // table dec_keys ... dec_state, never the merge's ctx->vox.  The emission writes the components' second set.
     bool srf_decimated = false;           // the held surface is a simplification (it is not simplified again)
-    s3d::VoxelTable dec{};
-    Buf<unsigned long long> dec_keys;     // [cap] the cluster table
-    Buf<s3d::VoxelSlot> dec_acc;          // [cap]
-    Buf<uint32_t> dec_ordinal;            // [cap]
-    Buf<uint32_t> dec_ord2slot;           // [vertices]
-    Buf<s3d::VoxelState> dec_vstate;
-    Buf<uint32_t> dec_point_slot;         // [vertices]
-    Buf<uint8_t> dec_vert_flags;          // [vertices]
-    Buf<uint32_t> dec_vert_counts;        // [cdiv(vertices, POINT_BLOCK) + 1]
-    Buf<unsigned long long> dec_quad;     // [vertices][10]
-    Buf<int32_t> dec_ctri;                // [faces][3]
-    Buf<uint32_t> dec_table;              // [2 faces]
-    Buf<uint32_t> dec_slot_of;            // [faces]
-    Buf<uint8_t> dec_keep;                // [faces]
-    Buf<uint32_t> dec_face_counts;        // [cdiv(faces, POINT_BLOCK) + 1]
-    Buf<s3d::DecimateState> dec_state;
-
-    // scan3d_voxel_surface_smooth / scan3d_mesh_smooth_dev (allocated on first use, grown on demand).  The surface
-    // route writes the components' second set's xyz and normals.
     bool srf_smoothed = false;            // the held surface is smoothed (scan3d_voxel_surface_decimate refuses it)
-    Buf<unsigned long long> sm_keys;      // [6 faces] the edge table
-    Buf<uint32_t> sm_sides;               // [6 faces]
-    Buf<uint32_t> sm_rows;                // [6 faces]
-    Buf<uint32_t> sm_degree;              // [vertices]
-    Buf<uint8_t> sm_held;                 // [vertices]
-    Buf<uint32_t> sm_block_counts;        // [cdiv(vertices, POINT_BLOCK) + 1]
-    Buf<uint32_t> sm_cursor;              // [vertices]
-    Buf<long long> sm_q[2];               // [vertices][3]
-    Buf<unsigned long long> sm_nsum;      // [vertices][3]
-    Buf<s3d::SmoothState> sm_state;
 
     int cta_limit = 0;             // scan3d_set_cta_limit
 
@@ -458,114 +495,23 @@ cudaError_t launch_register_points(const float* src, float* dst, long long n, co
                                    float tz, int sm_count, cudaStream_t st);
 
 // ---- camera-grid mesh (scan3d_mesh_kernels.cu) ----
-// MESH_LAUNCHES launches: point offsets (k_count, k_scan), pixel -> point index plane, face counts per block, their
-// scan, faces + normals.  idx [W*H], block_counts [cdiv(W*H, POINT_BLOCK)], face_counts [same], totals [2]
-// (points, faces); faces [2(W-1)(H-1)][3], normals [W*H][3].
-constexpr int MESH_LAUNCHES = 6;
+// 6 launches: point offsets (k_count, k_scan), pixel -> point index plane, face counts per block, their scan, faces +
+// normals.  idx [W*H], block_counts [cdiv(W*H, POINT_BLOCK)], face_counts [same], totals [2] (points, faces); faces
+// [2(W-1)(H-1)][3], normals [W*H][3].
 cudaError_t launch_mesh(const uint8_t* valid, const float* pts, int W, int H, float max_edge, int32_t* idx,
                         uint32_t* block_counts, uint32_t* face_counts, uint32_t* totals, int32_t* faces, float* normals,
-                        cudaStream_t st);
+                        cudaStream_t st, int64_t* launches);
 
 // ---- voxel-grid merge (scan3d_voxel_kernels.cu; common/scan3d_voxel_math.h has the arithmetic) ----
-// VOXEL_ADD_LAUNCHES launches for `plane` points (the ctx add reads the point count from n_dev, <= plane): insert,
-// flag, k_count + k_scan over the flags, assign.  point_slot and flags [plane], block_counts [cdiv(plane,
-// POINT_BLOCK)]; par = number of adds (chunks) since begin, mod 2.  nrm / rgb may be null (zeros).
-constexpr int VOXEL_ADD_LAUNCHES = 5;
+// 5 launches for `plane` points (the ctx add reads the point count from n_dev, <= plane): insert, flag, k_count +
+// k_scan over the flags, assign.  point_slot and flags [plane], block_counts [cdiv(plane, POINT_BLOCK)]; par = number
+// of adds (chunks) since begin, mod 2.  nrm / rgb may be null (zeros).
 cudaError_t launch_voxel_add(const VoxelTable& t, const float* xyz, const float* nrm, const uint8_t* rgb,
                              const uint32_t* n_dev, uint32_t plane, uint32_t* point_slot, uint8_t* flags,
-                             uint32_t* block_counts, int par, cudaStream_t st);
-// slots of the table for max_voxels: at most half of them are ever taken (scan3d_voxel_kernels.cu)
-uint32_t voxel_table_capacity(uint32_t max_voxels, int sm_count);
+                             uint32_t* block_counts, int par, cudaStream_t st, int64_t* launches);
 // 1 launch: the merged voxels in first-point order into xyz / nrm [max_voxels][3], rgb [max_voxels][3], cnt
 cudaError_t launch_voxel_finish(const VoxelTable& t, int par, float* xyz, float* nrm, uint8_t* rgb, uint32_t* cnt,
                                 int sm_count, cudaStream_t st);
-
-// ---- scan-to-model alignment (scan3d_align_kernels.cu; common/scan3d_align_math.h has the arithmetic) ----
-// ALIGN_INDEX_LAUNCHES launches: cell keys and counts (which also initialises *state from run, the voxel overflow
-// flag and, when n_dev is set, the source count), cell ranges, scatter of the model points.  The model is the first
-// min(total, max_voxels) voxel outputs of t (total = t.state->total[par]); xyz / nrm [max_voxels][3].  The index holds
-// ALIGN_CELLS_PER_VOXEL * max_voxels slots (at most half of them taken) and must be reset before (keys 0xff, cells and
-// cursor 0).
-constexpr int ALIGN_INDEX_LAUNCHES = 3;
-constexpr uint32_t ALIGN_CELLS_PER_VOXEL = 2;
-cudaError_t launch_align_index(const AlignIndex& ix, const VoxelTable& t, int par, const float* xyz, const float* nrm,
-                               double S, AlignState* state, const AlignRun& run, const uint32_t* n_dev, int sm_count,
-                               cudaStream_t st);
-// One match + one solve launch per iteration.  The source is xyz[i * stride] for i * stride < n, n = min(*n_dev, n_max)
-// when n_dev is set, else n_max; the grid depends on n_max and stride only (align_match_blocks).  partials
-// [ALIGN_NSUM + 1][blocks].
-constexpr int ALIGN_NSUM = 28;
-uint32_t align_match_blocks(long long n_max, int stride);
-cudaError_t launch_align_iteration(const AlignIndex& ix, AlignState* state, const AlignRun& run, const float* xyz,
-                                   const uint32_t* n_dev, long long n_max, int stride, double* partials, cudaStream_t st);
-
-// ---- surface extraction (scan3d_surface_kernels.cu; common/scan3d_surface_math.h has the arithmetic) ----
-// launch_surface_counts: SURFACE_COUNT_LAUNCHES launches after launch_align_index built the model's index (cell edge
-// s3l::cell_edge(max_distance)): candidate cells (27 per model voxel, with their order key), their other 7 corners,
-// the corner values, the (o, k) flags of active cells, k_count + k_scan over them (the vertex ordinals), vertex
-// assignment with the faces per block of SURFACE_VB vertices, and the scan of those.  The table must be reset before
-// (keys 0xff, owner 0xff, vert 0xff, state 0).  flags [27 max_voxels], flag_counts [cdiv(27 max_voxels, POINT_BLOCK)],
-// vert_slot [max_points], face_counts [cdiv(max_points, SURFACE_VB)].
-// launch_surface_emit: 1 launch, the vertices (xyz, normals, rgb) and faces once the counts are known.
-constexpr int SURFACE_COUNT_LAUNCHES = 8;
-constexpr int SURFACE_VB = 256;
-cudaError_t launch_surface_counts(const SurfaceTable& s, const AlignIndex& ix, const VoxelTable& t, int par,
-                                  const float* vox_nrm, float max_distance, uint8_t* flags, uint32_t* flag_counts,
-                                  uint32_t* vert_slot, uint32_t* face_counts, cudaStream_t st);
-cudaError_t launch_surface_emit(const SurfaceTable& s, const uint8_t* vox_rgb, const uint32_t* vert_slot,
-                                const uint32_t* face_counts, uint32_t vertices, float* xyz, float* nrm, uint8_t* rgb,
-                                int32_t* faces, cudaStream_t st);
-// slots of the lattice table for max_points: at most half of them are ever taken
-uint32_t surface_table_capacity(uint32_t max_points, int sm_count);
-
-// ---- connected components of a triangle mesh (scan3d_components_kernels.cu) ----
-// launch_cc_labels: COMPONENT_LABEL_LAUNCHES launches for n vertices and n_faces faces [n_faces][3]: parent = v,
-// union per face, find per vertex with the root flags, k_count + k_scan over them (state->components), the roots' ids,
-// every vertex's id into label [n].  state must be zeroed before; parent and flags [n], block_counts [cdiv(n,
-// POINT_BLOCK) + 1].  Any n below 2^31 and n_faces below 2^32, 0 included.
-// launch_cc_select: COMPONENT_SELECT_LAUNCHES launches after it: vertices and faces per component (comp_v, comp_f [n],
-// zeroed before), the selection (state->threshold, kept, largest), the keep flags (keep_v [n], keep_f [n_faces], kept
-// [components]), k_count + k_scan over each of keep_v (state->vertices) and keep_f (state->faces).
-// launch_cc_emit: COMPONENT_EMIT_LAUNCHES launches: the kept vertices into xyz2 / nrm2 / rgb2 (their new indices into
-// new_index [n]), then the kept faces, remapped, into faces2.
-constexpr int COMPONENT_LABEL_LAUNCHES = 7;
-constexpr int COMPONENT_SELECT_LAUNCHES = 7;
-constexpr int COMPONENT_EMIT_LAUNCHES = 2;
-cudaError_t launch_cc_labels(const int32_t* faces, uint32_t n_faces, uint32_t n, uint32_t* parent, uint8_t* flags,
-                             uint32_t* block_counts, int32_t* label, ComponentsState* state, cudaStream_t st);
-cudaError_t launch_cc_select(const int32_t* faces, uint32_t n_faces, uint32_t n, const int32_t* label,
-                             unsigned long long min_faces, unsigned long long max_components, uint32_t* comp_v,
-                             uint32_t* comp_f, uint8_t* kept, uint8_t* keep_v, uint8_t* keep_f, uint32_t* vert_counts,
-                             uint32_t* face_counts, ComponentsState* state, cudaStream_t st);
-cudaError_t launch_cc_emit(const uint8_t* keep_v, const uint32_t* vert_counts, uint32_t n, const float* xyz,
-                           const float* nrm, const uint8_t* rgb, const uint8_t* keep_f, const uint32_t* face_counts,
-                           uint32_t n_faces, const int32_t* faces, int32_t* new_index, float* xyz2, float* nrm2,
-                           uint8_t* rgb2, int32_t* faces2, cudaStream_t st);
-
-// ---- surface simplification (scan3d_decimate_kernels.cu; common/scan3d_decimate_math.h has the arithmetic) ----
-// DECIMATE_LAUNCHES launches for a surface of n_vertices (xyz, nrm, rgb) and n_faces (tri): launch_voxel_add over the
-// vertices into t (the clusters, edge t.S = H; t must be reset as scan3d_voxel_begin resets the merge's table, with
-// max_voxels >= max(n_vertices, 1)), the face quadrics with the cluster triples, the duplicate-face table, the keep
-// flags, k_count + k_scan over them (b.state->faces), then the vertices of the clusters into xyz2 / nrm2 / rgb2 [n_vertices]
-// and the kept faces into faces2 [n_faces].  b.quad, b.state zeroed and b.table set to 0xff before.
-constexpr int DECIMATE_LAUNCHES = VOXEL_ADD_LAUNCHES + 7;
-cudaError_t launch_decimate(const VoxelTable& t, const DecimateBuffers& b, const float* xyz, const float* nrm,
-                            const uint8_t* rgb, const int32_t* tri, uint32_t n_vertices, uint32_t n_faces, double H,
-                            float* xyz2, float* nrm2, uint8_t* rgb2, int32_t* faces2, int sm_count, cudaStream_t st);
-
-// ---- surface smoothing (scan3d_smooth_kernels.cu; common/scan3d_smooth_math.h has the arithmetic) ----
-// SMOOTH_BUILD_LAUNCHES + passes + SMOOTH_END_LAUNCHES launches for n vertices (xyz, nrm may be null) and nf faces
-// [nf][3]: the exponent max and the finiteness check over the vertices, the sides into the edge table, the degrees and
-// held flags per edge, the degree sums per POINT_BLOCK vertices, their k_scan, the row starts with the fixed-point
-// positions, the neighbour rows; then one gather per pass (k = lambda, or lambda and mu alternating when mu != 0);
-// then the face normals and the write of xyz_out / nrm_out (nrm_out may be null), which writes nothing when the state
-// holds an error.  xyz_out may be xyz and nrm_out nrm.  b.keys 0xff; b.sides, b.degree, b.held, b.nsum, b.state zeroed
-// before; b.cap >= 2 * 3 nf.
-constexpr int SMOOTH_BUILD_LAUNCHES = 7;
-constexpr int SMOOTH_END_LAUNCHES = 2;
-cudaError_t launch_smooth(const SmoothBuffers& b, const float* xyz, const float* nrm, const int32_t* faces, uint32_t n,
-                          uint32_t nf, int passes, double lambda, double mu, float* xyz_out, float* nrm_out,
-                          cudaStream_t st);
 
 // ---- debug / self-test ----
 cudaError_t launch_debug_atan2(const double* y, const double* x, float* out, int n, int mode,

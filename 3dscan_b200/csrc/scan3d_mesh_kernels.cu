@@ -198,7 +198,7 @@ __global__ void __launch_bounds__(MT) k_mesh_emit(const int32_t* __restrict__ id
 
 cudaError_t launch_mesh(const uint8_t* valid, const float* pts, int W, int H, float max_edge, int32_t* idx,
                         uint32_t* block_counts, uint32_t* face_counts, uint32_t* totals, int32_t* faces, float* normals,
-                        cudaStream_t st)
+                        cudaStream_t st, int64_t* launches)
 {
     const size_t plane = (size_t)W * H;
     const int nb = (int)((plane + POINT_BLOCK - 1) / POINT_BLOCK);
@@ -210,6 +210,7 @@ cudaError_t launch_mesh(const uint8_t* valid, const float* pts, int W, int H, fl
     e = launch_block_scan(face_counts, nb, totals + 1, st);
     if (e != cudaSuccess) return e;
     k_mesh_emit<<<nb, MT, 0, st>>>(idx, pts, W, H, t2, block_counts, face_counts, faces, normals);
+    *launches += 6;
     return cudaGetLastError();
 }
 

@@ -17,6 +17,21 @@
 
 namespace s3d {
 
+// the kernels' view of a SmoothWorkspace
+struct SmoothBuffers {
+    unsigned long long* keys;      // [cap] edge keys, s3v::EMPTY_KEY = free
+    uint32_t* sides;               // [cap] sides on each edge, zeroed
+    uint32_t cap;
+    uint32_t* degree;              // [vertices] distinct neighbours, zeroed
+    uint8_t* held;                 // [vertices] zeroed
+    uint32_t* block_counts;        // [cdiv(vertices, POINT_BLOCK) + 1]
+    uint32_t* cursor;              // [vertices] row start, then (after the scatter) row end
+    uint32_t* rows;                // [cap] neighbour indices (2 per edge, at most 2 * 3 nf)
+    long long* q[2];               // [vertices][3] fixed-point positions, ping-pong
+    unsigned long long* nsum;      // [vertices][3] fixed-point normal sums (int64 two's complement), zeroed
+    SmoothState* state;            // zeroed
+};
+
 namespace {
 
 constexpr int ST = 256;                                 // threads per block of the per-item kernels
@@ -328,16 +343,33 @@ __global__ void __launch_bounds__(ST) k_sm_write(const float* xyz, const float* 
     if ((threadIdx.x & 31) == 0 && bits) atomicMax(&b.state->max_move, bits);
 }
 
-cudaError_t launch_smooth(const SmoothBuffers& b, const float* xyz, const float* nrm, const int32_t* faces, uint32_t n,
-                          uint32_t nf, int passes, double lambda, double mu, float* xyz_out, float* nrm_out,
-                          cudaStream_t st)
+cudaError_t SmoothWorkspace::run(const float* xyz, const float* nrm, const int32_t* faces, uint32_t n, uint32_t nf,
+                                 int passes, double lambda, double mu, float* xyz_out, float* nrm_out, cudaStream_t st,
+                                 int64_t* launches)
 {
+    const size_t av = n ? n : 1;
+    const uint32_t cap = 6ull * nf > 64 ? (uint32_t)(6ull * nf) : 64u;   // two slots per side: at most half are taken
+    cudaError_t e = grow_group(Grow(keys, cap), Grow(sides, cap), Grow(rows, cap));
+    if (e == cudaSuccess)
+        e = grow_group(Grow(degree, av), Grow(held, av), Grow(block_counts, (av + POINT_BLOCK - 1) / POINT_BLOCK + 1),
+                       Grow(cursor, av), Grow(q[0], 3 * av), Grow(q[1], 3 * av));
+    if (e == cudaSuccess) e = nsum.ensure(3 * av);
+    if (e == cudaSuccess) e = state.ensure(1);
+    if (e != cudaSuccess) return e;
+    const SmoothBuffers b{keys, sides, cap, degree, held, block_counts, cursor, rows, {q[0], q[1]}, nsum, state};
+    e = cudaMemsetAsync(b.keys, 0xff, (size_t)cap * sizeof(*b.keys), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(b.sides, 0, (size_t)cap * sizeof(*b.sides), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(b.degree, 0, av * sizeof(*b.degree), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(b.held, 0, av * sizeof(*b.held), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(b.nsum, 0, 3 * av * sizeof(*b.nsum), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(b.state, 0, sizeof(*b.state), st);
+    if (e != cudaSuccess) return e;
     const int nb = (int)grid(n, POINT_BLOCK);
     k_sm_exponent<<<grid(n, ST), ST, 0, st>>>(xyz, n, b.state);
     k_sm_sides<<<grid(nf, ST), ST, 0, st>>>(faces, nf, n, b);
     k_sm_edges<<<grid(b.cap, ST), ST, 0, st>>>(b);
     k_sm_block_sums<<<nb, POINT_BLOCK, 0, st>>>(b.degree, n, b.block_counts);
-    cudaError_t e = launch_block_scan(b.block_counts, nb, &b.state->entries, st);
+    e = launch_block_scan(b.block_counts, nb, &b.state->entries, st);
     if (e != cudaSuccess) return e;
     k_sm_offsets<<<nb, POINT_BLOCK, 0, st>>>(xyz, b, n);
     k_sm_scatter<<<grid(b.cap, ST), ST, 0, st>>>(b);
@@ -346,9 +378,10 @@ cudaError_t launch_smooth(const SmoothBuffers& b, const float* xyz, const float*
         k_sm_pass<<<grid(n, ST), ST, 0, st>>>(b.q[p & 1], b.q[(p + 1) & 1], b.degree, b.held, b.cursor, b.rows, n, k,
                                               b.state);
     }
-    const long long* q = b.q[passes & 1];
-    k_sm_face_normals<<<grid(nf, ST), ST, 0, st>>>(faces, nf, n, xyz, q, b);
-    k_sm_write<<<grid(n, ST), ST, 0, st>>>(xyz, nrm, n, q, b, xyz_out, nrm_out);
+    const long long* qf = b.q[passes & 1];
+    k_sm_face_normals<<<grid(nf, ST), ST, 0, st>>>(faces, nf, n, xyz, qf, b);
+    k_sm_write<<<grid(n, ST), ST, 0, st>>>(xyz, nrm, n, qf, b, xyz_out, nrm_out);
+    *launches += 7 + passes + 2;
     return cudaGetLastError();
 }
 

@@ -6,7 +6,7 @@
 // The lattice points are held in an open-addressing table (scan3d_hash.cuh) with one slot per distinct point.  Every
 // pair (o, k) of a model voxel o and one of its 27 offsets k inserts its cell and takes the cell's order key
 // 27 o + k with atomicMin; the candidate cells then insert their other 7 corners, and each lattice point is evaluated
-// once against the alignment's cell index of the model (launch_align_index).  The flag of (o, k) is set when (o, k)
+// once against the alignment's cell index of the model (AlignWorkspace::index).  The flag of (o, k) is set when (o, k)
 // owns (has the smallest key of) an active cell, so the compaction's k_count + k_scan over the 27 max_voxels flags rank
 // the vertices by their key whatever the hash or the scheduling did.  Faces are counted per block of SURFACE_VB
 // vertices and scanned; the emission (one thread per vertex) writes each vertex's faces at its block's offset plus
@@ -21,6 +21,7 @@ namespace s3d {
 namespace {
 
 constexpr int ST = 256;                                 // threads per block of the table kernels
+constexpr int SURFACE_VB = 256;                         // vertices per block of the face counts and the emission
 constexpr unsigned FULL = 0xffffffffu;
 constexpr unsigned long long NO_OWNER = ~0ull;
 static_assert(SURFACE_VB % 32 == 0 && SURFACE_VB <= 1024, "vertex block");
@@ -299,7 +300,8 @@ __global__ void __launch_bounds__(SURFACE_VB) k_surface_emit(SurfaceTable s, con
     }
 }
 
-uint32_t surface_table_capacity(uint32_t max_points, int sm_count)
+// slots of the lattice table for max_points: at most half of them are ever taken
+static uint32_t surface_table_capacity(uint32_t max_points, int sm_count)
 {
     // Inserting stops once more than max_points slots are taken.  Blocks that passed that check before claim at most
     // one slot per thread (cells) or seven (corners): the crossing block and every resident one (2048 threads per SM).
@@ -308,32 +310,50 @@ uint32_t surface_table_capacity(uint32_t max_points, int sm_count)
     return (uint32_t)(c < 0xffffffffull ? c : 0xffffffffull);
 }
 
-cudaError_t launch_surface_counts(const SurfaceTable& s, const AlignIndex& ix, const VoxelTable& t, int par,
-                                  const float* vox_nrm, float max_distance, uint8_t* flags, uint32_t* flag_counts,
-                                  uint32_t* vert_slot, uint32_t* face_counts, cudaStream_t st)
+cudaError_t SurfaceWorkspace::count(const AlignIndex& ix, const VoxelTable& t, int par, const float* vox_nrm,
+                                    float max_distance, uint32_t max_points, int sm_count, cudaStream_t st,
+                                    int64_t* launches)
 {
+    const uint32_t cap = surface_table_capacity(max_points, sm_count);
+    const size_t nvb = (max_points + SURFACE_VB - 1) / SURFACE_VB;
     const unsigned long long n = (unsigned long long)s3s::OFFSETS * t.max_voxels;
+    cudaError_t e = grow_group(Grow(keys, cap), Grow(owner, cap), Grow(f, cap), Grow(nearest, cap), Grow(vert, cap));
+    if (e == cudaSuccess) e = grow_group(Grow(vert_slot, max_points), Grow(face_counts, nvb + 1));
+    if (e == cudaSuccess) e = grow_group(Grow(flags, n), Grow(flag_counts, (n + POINT_BLOCK - 1) / POINT_BLOCK + 1));
+    if (e == cudaSuccess) e = state.ensure(1);
+    if (e != cudaSuccess) return e;
+    view = SurfaceTable{keys, owner, f, nearest, vert, state, cap, max_points, t.S};
+    e = cudaMemsetAsync(keys, 0xff, (size_t)cap * sizeof(*view.keys), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(owner, 0xff, (size_t)cap * sizeof(*view.owner), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(vert, 0xff, (size_t)cap * sizeof(*view.vert), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(state, 0, sizeof(*view.state), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(face_counts, 0, nvb * sizeof(uint32_t), st);
+    if (e != cudaSuccess) return e;
+    const SurfaceTable& s = view;
     const unsigned gp = (unsigned)((n + ST - 1) / ST), gs = (unsigned)((s.cap + (unsigned long long)ST - 1) / ST);
     const double R = (double)max_distance;
     k_surface_cells<<<gp, ST, 0, st>>>(s, t, par, vox_nrm, n);
     k_surface_corners<<<gs, ST, 0, st>>>(s);
     k_surface_eval<<<gs, ST, 0, st>>>(s, ix, s3l::cell_edge(max_distance), R * R);
     k_surface_flag<<<gp, ST, 0, st>>>(s, t, par, vox_nrm, n, flags);
-    cudaError_t e = launch_point_offsets(flags, (size_t)n, flag_counts, &s.state->vertices, st);
+    e = launch_point_offsets(flags, (size_t)n, flag_counts, &s.state->vertices, st);
     if (e != cudaSuccess) return e;
     k_surface_assign<<<(unsigned)((n + POINT_BLOCK - 1) / POINT_BLOCK), POINT_BLOCK, 0, st>>>(
         s, t, par, vox_nrm, n, flags, flag_counts, vert_slot, face_counts);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    return launch_block_scan(face_counts, (int)((s.max_points + SURFACE_VB - 1) / SURFACE_VB), &s.state->faces, st);
+    e = launch_block_scan(face_counts, (int)nvb, &s.state->faces, st);
+    *launches += 8;
+    return e;
 }
 
-cudaError_t launch_surface_emit(const SurfaceTable& s, const uint8_t* vox_rgb, const uint32_t* vert_slot,
-                                const uint32_t* face_counts, uint32_t vertices, float* xyz, float* nrm, uint8_t* rgb,
-                                int32_t* faces, cudaStream_t st)
+cudaError_t SurfaceWorkspace::emit(const uint8_t* vox_rgb, uint32_t vertices, SurfaceMesh& out, cudaStream_t st,
+                                   int64_t* launches)
 {
     const unsigned blocks = vertices ? (vertices + SURFACE_VB - 1) / SURFACE_VB : 1;
-    k_surface_emit<<<blocks, SURFACE_VB, 0, st>>>(s, vox_rgb, vert_slot, face_counts, vertices, xyz, nrm, rgb, faces);
+    k_surface_emit<<<blocks, SURFACE_VB, 0, st>>>(view, vox_rgb, vert_slot, face_counts, vertices, out.xyz, out.nrm,
+                                                  out.rgb, out.tri);
+    *launches += 1;
     return cudaGetLastError();
 }
 

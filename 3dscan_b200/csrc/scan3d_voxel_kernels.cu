@@ -149,7 +149,8 @@ __global__ void k_voxel_finish(VoxelTable t, int par, float* __restrict__ out_xy
     }
 }
 
-uint32_t voxel_table_capacity(uint32_t max_voxels, int sm_count)
+// slots of the table for max_voxels: at most half of them are ever taken
+static uint32_t voxel_table_capacity(uint32_t max_voxels, int sm_count)
 {
     // k_voxel_insert stops claiming slots once more than max_voxels are taken.  Blocks that passed that check before
     // claim at most one slot per thread: the crossing block and every resident one (2048 threads per SM).  Twice
@@ -158,9 +159,24 @@ uint32_t voxel_table_capacity(uint32_t max_voxels, int sm_count)
     return (uint32_t)(c < 0xffffffffull ? c : 0xffffffffull);
 }
 
+cudaError_t VoxelStore::reset(uint32_t max_voxels, double S, int sm_count, cudaStream_t st)
+{
+    const uint32_t cap = voxel_table_capacity(max_voxels, sm_count);
+    cudaError_t e = grow_group(Grow(keys, cap), Grow(acc, cap), Grow(ordinal, cap));
+    if (e == cudaSuccess) e = ord2slot.ensure(max_voxels);
+    if (e == cudaSuccess) e = state.ensure(1);
+    if (e != cudaSuccess) return e;
+    view = VoxelTable{keys, acc, ordinal, ord2slot, state, cap, max_voxels, S};
+    e = cudaMemsetAsync(keys, 0xff, (size_t)cap * sizeof(*view.keys), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(acc, 0, (size_t)cap * sizeof(*view.acc), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(ordinal, 0xff, (size_t)cap * sizeof(*view.ordinal), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(state, 0, sizeof(*view.state), st);
+    return e;
+}
+
 cudaError_t launch_voxel_add(const VoxelTable& t, const float* xyz, const float* nrm, const uint8_t* rgb,
                              const uint32_t* n_dev, uint32_t plane, uint32_t* point_slot, uint8_t* flags,
-                             uint32_t* block_counts, int par, cudaStream_t st)
+                             uint32_t* block_counts, int par, cudaStream_t st, int64_t* launches)
 {
     const unsigned grid = (unsigned)((plane + VT - 1) / VT);
     k_voxel_insert<<<grid, VT, 0, st>>>(t, xyz, nrm, rgb, n_dev, plane, point_slot);
@@ -169,6 +185,7 @@ cudaError_t launch_voxel_add(const VoxelTable& t, const float* xyz, const float*
     if (e != cudaSuccess) return e;
     k_voxel_assign<<<(unsigned)((plane + POINT_BLOCK - 1) / POINT_BLOCK), POINT_BLOCK, 0, st>>>(t, flags, plane,
                                                                                                block_counts, point_slot, par);
+    *launches += 5;
     return cudaGetLastError();
 }
 

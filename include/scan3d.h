@@ -472,7 +472,7 @@ int scan3d_write_voxel_surface_ply(scan3d_ctx *ctx, const char *path, int binary
  * flags and over the face flags before the synchronisation, and 2 after it (kept vertices, kept faces).  With (0, 0)
  * the surface's bytes are unchanged.
  * Memory (ctx-owned, allocated on first use, grown on demand): 18 B per vertex and 1 B per face of scratch and
- * component table, plus a second surface set of 27 B per kept vertex and 12 B per kept face that is swapped with the
+ * component table, plus the spare surface set of 27 B per kept vertex and 12 B per kept face that is swapped with the
  * held one.
  * Errors: SCAN3D_ERR_ARG for a null ctx, params, result or components_out; faces_dev NULL with n_faces > 0 or
  * label_dev NULL with n_vertices > 0; a negative min_faces or max_components; n_faces or n_vertices outside
@@ -542,7 +542,7 @@ int scan3d_mesh_components_dev(scan3d_ctx *ctx, const int32_t *faces_dev, int64_
  * duplicate-face table, the keep flags, k_count + k_scan over them, the vertices (placement), the faces.
  * Memory (ctx-owned, allocated on first use, grown on demand): about 275 B per vertex (the cluster table at ~184 B, the
  * quadric sums indexed by cluster ordinal at 80 B, 9 B of scratch) and 25 B per face (cluster triples, duplicate
- * table, slots and flags), plus the components' second surface set, grown to 27 B per vertex and 12 B per face of the
+ * table, slots and flags), plus the spare surface set, grown to 27 B per vertex and 12 B per face of the
  * input, which is swapped with the held one.
  * Errors: SCAN3D_ERR_ARG for a null ctx or out, a cell_size that is not finite, and (with a held surface) cell_size <
  * voxel_size or > 256 voxel_size; SCAN3D_ERR_CONFIG for a surface of 2^31 faces or more.  An argument, state or
@@ -589,7 +589,7 @@ int scan3d_voxel_surface_decimate(scan3d_ctx *ctx, float cell_size, scan3d_decim
  * Smoothing after components or decimation is allowed, and so is smoothing again.  scan3d_voxel_surface_decimate
  * refuses a smoothed surface with SCAN3D_ERR_STATE until a new scan3d_voxel_surface (its overflow bound rests on
  * surface-nets geometry, which smoothing does not keep).  A later begin, add or finish makes the surface stale as
- * before; the accumulator is never touched.  The result is computed into the components' second surface set and
+ * before; the accumulator is never touched.  The result is computed into the spare surface set and
  * swapped with the held one after the synchronisation, so on any error the surface is untouched.
  * scan3d_mesh_smooth_dev smooths any triangle mesh in device memory of the ctx's GPU in place: xyz_dev float
  * [n_vertices][3], normals_dev float [n_vertices][3] or NULL (no normals), faces_dev int32 [n_faces][3]; ordered on the
@@ -603,7 +603,7 @@ int scan3d_voxel_surface_decimate(scan3d_ctx *ctx, float cell_size, scan3d_decim
  * the row starts with the fixed-point positions, the neighbour rows; one gather per pass; the face normals; the write.
  * Memory (ctx-owned, allocated on first use, grown on demand): 81 B per vertex (two fixed-point position sets at 24 B,
  * the normal sums at 24 B, degree, row start and held flag) and 96 B per face (the edge table of 6 slots of 12 B, and
- * 6 row entries of 4 B); the surface route also grows the components' second set's xyz and normals to 24 B per vertex.
+ * 6 row entries of 4 B); the surface route also grows the spare surface set's xyz and normals to 24 B per vertex.
  * Errors: SCAN3D_ERR_ARG for a null ctx, params or result; iterations outside [0, 4096]; lambda not in (0, 1] or mu not
  * in [-1, 0] (NaN and infinities included); and in scan3d_mesh_smooth_dev n_vertices or n_faces outside [0, 2^31), a
  * NULL xyz_dev or faces_dev with a non-zero count, a buffer not 4-byte aligned, and, found on the device, a coordinate

@@ -13,7 +13,7 @@ iterations 1, 10 and 50 with MeshLab's lambda = 0.5, mu = -0.53.  ms per pass is
 iterations (80 passes).  The context's smoothing buffers are grow-only and shared by the three workloads (run in the
 order C3, A, B), so device_bytes_growth is only what a workload's first call added (the drop of the device's free
 memory); device_bytes_owned is what the context holds for the workload by include/scan3d.h's sizes (81 B per vertex,
-96 B per face, and for a surface 24 B per vertex of the components' second set).  A separate torch.profiler pass
+96 B per face, and for a surface 24 B per vertex of the spare surface set).  A separate torch.profiler pass
 over one call at 10 iterations gives the per-kernel split, and the gather's bytes per pass (neighbour rows at 4 B and neighbour positions at 24 B per row entry,
 then degree, row end, held flag, own position and the write at 57 B per vertex) over its mean kernel time give its rate.
 Those are the bytes the algorithm reads, not DRAM traffic: neighbours are mostly close in index order, so many of the
