@@ -281,6 +281,7 @@ int scan3d_set_texture(scan3d_ctx* ctx, const uint8_t* bgr_host)
     CK(cudaSetDevice(ctx->device));
     if (!bgr_host) {
         ctx->texture.release();
+        ctx->results.drop(POINT_COLOURS);
         return SCAN3D_OK;
     }
     CK(ctx->texture.ensure(3 * npix(ctx)));
@@ -321,18 +322,12 @@ static int roi_bytes(const scan3d_ctx* ctx, size_t* out)
     return 0;
 }
 
-int scan3d_compute_wrapped_phase_dev(scan3d_ctx* ctx, int dir, const uint8_t* fringe_dev, const uint8_t* roi_dev)
+// compute_wrapped_phase on the effective ROI (strict_roi applied), after the caller dropped the direction's results
+static int wrapped_phase(scan3d_ctx* ctx, int dir, const uint8_t* fringe_dev, const uint8_t* roi_dev)
 {
-    if (!ctx || !fringe_dev || !roi_dev) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
-    if (dir < 0 || dir >= ctx->cfg.dirs) return fail(ctx, SCAN3D_ERR_ARG, "bad pattern_type");
-    CK(cudaSetDevice(ctx->device));
-    int rc = ensure_stage_planes(ctx, dir);
+    const int rc = ensure_stage_planes(ctx, dir);
     if (rc) return rc;
     const Shape s = shape_of(ctx->cfg);
-    if (!ctx->in_reconstruct) {       // (scan3d_reconstruct_dev has already done it)
-        rc = strict_roi(ctx, &roi_dev);
-        if (rc) return rc;
-    }
     if (ctx->cfg.flags & SCAN3D_FLAG_MODULATION_MASK) {
         CK(ctx->roi_eff.ensure(npix(ctx)));
         CK(launch_modulation_roi(s, fringe_dev, roi_dev, ctx->roi_eff, ctx->stream));
@@ -342,10 +337,19 @@ int scan3d_compute_wrapped_phase_dev(scan3d_ctx* ctx, int dir, const uint8_t* fr
     CK(launch_wrapped(s, ctx->cfg.N, fringe_dev, roi_dev, ctx->wrapped[dir], ctx->atan_tab, ctx->nstep_w, false, ctx->stream));
     CK(launch_mask(s, roi_dev, ctx->mask[dir], ctx->stream));
     ctx->launches += 2;
-    ctx->have_wrapped[dir] = true;
-    ctx->have_unwrapped[dir] = false;
-    ctx->have_cpmap = ctx->have_valid = ctx->have_xyz = ctx->have_points = ctx->have_mesh = false;
+    ctx->results.produce(dir == 0 ? WRAPPED_V : WRAPPED_H);
     return SCAN3D_OK;
+}
+
+int scan3d_compute_wrapped_phase_dev(scan3d_ctx* ctx, int dir, const uint8_t* fringe_dev, const uint8_t* roi_dev)
+{
+    if (!ctx || !fringe_dev || !roi_dev) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (dir < 0 || dir >= ctx->cfg.dirs) return fail(ctx, SCAN3D_ERR_ARG, "bad pattern_type");
+    CK(cudaSetDevice(ctx->device));
+    ctx->results.drop(dir == 0 ? WRAPPED_V : WRAPPED_H);
+    const int rc = strict_roi(ctx, &roi_dev);
+    if (rc) return rc;
+    return wrapped_phase(ctx, dir, fringe_dev, roi_dev);
 }
 
 // The host-pointer entries stage their inputs in the context's own buffers (allocated on first use, sized for a whole
@@ -380,15 +384,17 @@ int scan3d_unwrap_phase_dev(scan3d_ctx* ctx, int dir, const uint8_t* gray_dev, c
 {
     if (!ctx || !gray_dev || !inv_dev) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
     if (dir < 0 || dir >= ctx->cfg.dirs) return fail(ctx, SCAN3D_ERR_ARG, "bad pattern_type");
-    if (!ctx->have_wrapped[dir]) return fail(ctx, SCAN3D_ERR_STATE, "unwrap_phase before compute_wrapped_phase");
+    if (!ctx->results.has(dir == 0 ? WRAPPED_V : WRAPPED_H))
+        return fail(ctx, SCAN3D_ERR_STATE, "unwrap_phase before compute_wrapped_phase");
     CK(cudaSetDevice(ctx->device));
+    const Result unwrapped = dir == 0 ? UNWRAPPED_V : UNWRAPPED_H;
+    ctx->results.drop(unwrapped);
     const Shape s = shape_of(ctx->cfg);
     const int M = dir == 0 ? ctx->cfg.M_v : ctx->cfg.M_h;
     CK(launch_unwrap(s, dir, M, gray_dev, inv_dev, ctx->wrapped[dir], ctx->mask[dir], ctx->code[dir],
                      ctx->unwrapped[dir], ctx->stream));
     ctx->launches++;
-    ctx->have_unwrapped[dir] = true;
-    ctx->have_cpmap = ctx->have_valid = ctx->have_xyz = ctx->have_points = ctx->have_mesh = false;
+    ctx->results.produce(unwrapped);
     return SCAN3D_OK;
 }
 
@@ -413,14 +419,17 @@ int scan3d_compute_c_p_map(scan3d_ctx* ctx)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
     if (ctx->cfg.dirs != 2) return fail(ctx, SCAN3D_ERR_STATE, "compute_c_p_map needs both directions");
-    if (!ctx->have_unwrapped[0] || !ctx->have_unwrapped[1]) return fail(ctx, SCAN3D_ERR_STATE, "compute_c_p_map before unwrap_phase(0) and (1)");
+    if (!ctx->results.has(UNWRAPPED_V) || !ctx->results.has(UNWRAPPED_H))
+        return fail(ctx, SCAN3D_ERR_STATE, "compute_c_p_map before unwrap_phase(0) and (1)");
     CK(cudaSetDevice(ctx->device));
+    ctx->results.drop(CPMAP);
+    ctx->results.drop(VALID);
     const Shape s = shape_of(ctx->cfg);
     CK(launch_cpmap(s, ctx->cfg.fw_v, ctx->cfg.fw_h, ctx->unwrapped[0], ctx->unwrapped[1], ctx->mask[0],
                     ctx->mask[1], ctx->cpmap, ctx->valid, ctx->stream));
     ctx->launches++;
-    ctx->have_cpmap = ctx->have_valid = true;
-    ctx->have_xyz = ctx->have_points = ctx->have_mesh = false;
+    ctx->results.produce(CPMAP);
+    ctx->results.produce(VALID);
     return SCAN3D_OK;
 }
 
@@ -428,22 +437,30 @@ int scan3d_triangulate(scan3d_ctx* ctx)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
     if (!ctx->has_calib) return fail(ctx, SCAN3D_ERR_STATE, "triangulate before set_calibration");
-    if (!ctx->have_cpmap) return fail(ctx, SCAN3D_ERR_STATE, "triangulate before compute_c_p_map");
+    if (!ctx->results.has(CPMAP)) return fail(ctx, SCAN3D_ERR_STATE, "triangulate before compute_c_p_map");
     CK(cudaSetDevice(ctx->device));
+    ctx->results.drop(XYZ);
     CK(ctx->xyz.ensure(3 * npix(ctx)));
     const Shape s = shape_of(ctx->cfg);
     CK(launch_triangulate(s, ctx->dcal, ctx->cam_lut, ctx->proj_lut, ctx->cpmap, ctx->valid, ctx->xyz, ctx->stream));
     ctx->launches++;
-    ctx->have_xyz = true;
-    ctx->have_points = ctx->have_mesh = false;
+    ctx->results.produce(XYZ);
     return SCAN3D_OK;
+}
+
+// the compacted points, and their colours when a texture is set
+static void produce_points(scan3d_ctx* ctx)
+{
+    ctx->results.produce(POINTS);
+    if (ctx->texture) ctx->results.produce(POINT_COLOURS);
 }
 
 int scan3d_compact_points(scan3d_ctx* ctx, int64_t* count_out)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
-    if (!ctx->have_xyz) return fail(ctx, SCAN3D_ERR_STATE, "compact_points before triangulate");
+    if (!ctx->results.has(XYZ)) return fail(ctx, SCAN3D_ERR_STATE, "compact_points before triangulate");
     CK(cudaSetDevice(ctx->device));
+    ctx->results.drop(POINTS);
     const size_t n = npix(ctx);
     CK(ctx->block_counts.ensure((n + 1023) / 1024 + 1));
     CK(ctx->pix.ensure(n));
@@ -453,8 +470,7 @@ int scan3d_compact_points(scan3d_ctx* ctx, int64_t* count_out)
     CK(launch_compact(s, ctx->xyz, ctx->valid, ctx->texture, ctx->block_counts, points_of(ctx), ctx->pix,
                       ctx->texture ? ctx->rgb.get() : nullptr, ctx->d_count, ctx->stream, &nl));
     ctx->launches += nl;
-    ctx->have_points = true;
-    ctx->have_mesh = false;
+    produce_points(ctx);
     if (count_out) return scan3d_point_count(ctx, count_out);
     return SCAN3D_OK;
 }
@@ -471,7 +487,7 @@ static int reconstruct_stagewise(scan3d_ctx* ctx, const uint8_t* stack, const ui
     const uint8_t* p = stack;
     for (int d = 0; d < c.dirs; d++) {
         const int M = d == 0 ? c.M_v : c.M_h;
-        int rc = scan3d_compute_wrapped_phase_dev(ctx, d, p, roi);
+        int rc = wrapped_phase(ctx, d, p, roi);
         if (rc) return rc;
         p += (size_t)c.N * n;
         rc = scan3d_unwrap_phase_dev(ctx, d, p, p + (size_t)M * n);
@@ -480,7 +496,7 @@ static int reconstruct_stagewise(scan3d_ctx* ctx, const uint8_t* stack, const ui
     }
     if (c.dirs == 1) {
         CK(cudaMemcpyAsync(ctx->valid, ctx->mask[0], n, cudaMemcpyDeviceToDevice, ctx->stream));
-        ctx->have_valid = true;
+        ctx->results.produce(VALID);
         return SCAN3D_OK;
     }
     int rc = scan3d_compute_c_p_map(ctx);
@@ -502,17 +518,13 @@ int scan3d_reconstruct_dev(scan3d_ctx* ctx, const uint8_t* stack_dev, const uint
     if (!ctx || !stack_dev || !roi_dev) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
     if (ctx->cfg.dirs == 2 && !ctx->has_calib) return fail(ctx, SCAN3D_ERR_STATE, "reconstruct before set_calibration");
     CK(cudaSetDevice(ctx->device));
-    ctx->have_mesh = false;
+    ctx->results.drop(WRAPPED_V);     // every pixel result is computed from the wrapped phases
+    ctx->results.drop(WRAPPED_H);
     {
         const int rc = strict_roi(ctx, &roi_dev);
         if (rc) return rc;
     }
-    if (!ctx->fast_div_ok || !fused7_supported(ctx->cfg)) {
-        ctx->in_reconstruct = true;
-        const int rc = reconstruct_stagewise(ctx, stack_dev, roi_dev);
-        ctx->in_reconstruct = false;
-        return rc;
-    }
+    if (!ctx->fast_div_ok || !fused7_supported(ctx->cfg)) return reconstruct_stagewise(ctx, stack_dev, roi_dev);
     const scan3d_config& c = ctx->cfg;
     FusedArgs a{};
     a.stack = stack_dev; a.roi = roi_dev;
@@ -564,14 +576,14 @@ int scan3d_reconstruct_dev(scan3d_ctx* ctx, const uint8_t* stack_dev, const uint
                                   ctx->reg_t[2], ctx->sm_count, ctx->stream));
         ctx->launches++;
     }
-    ctx->have_wrapped[0] = ctx->have_wrapped[1] = false;
-    ctx->have_unwrapped[0] = true;
-    ctx->have_unwrapped[1] = c.dirs == 2;
-    ctx->have_cpmap = c.dirs == 2;
-    ctx->have_valid = true;
-    ctx->have_xyz = false;
-    ctx->have_points = c.dirs == 2;
-    ctx->have_mesh = false;
+    // inputs before what is computed from them: producing a result drops what was computed from its old value
+    ctx->results.produce(UNWRAPPED_V);
+    if (c.dirs == 2) ctx->results.produce(UNWRAPPED_H);
+    ctx->results.produce(VALID);
+    if (c.dirs == 2) {
+        ctx->results.produce(CPMAP);
+        produce_points(ctx);
+    }
     return SCAN3D_OK;
 }
 
@@ -647,64 +659,53 @@ int scan3d_reconstruct_raw(scan3d_ctx* ctx, const uint8_t* raw_stack_host, const
 // ------------------------------------------------------------------------------------------
 // results
 // ------------------------------------------------------------------------------------------
-static void* plane_ptr(scan3d_ctx* ctx, int plane, size_t* elt)
-{
-    switch (plane) {
-        case SCAN3D_PLANE_WRAPPED_V: *elt = 4; return ctx->wrapped[0];
-        case SCAN3D_PLANE_WRAPPED_H: *elt = 4; return ctx->wrapped[1];
-        case SCAN3D_PLANE_UNWRAPPED_V: *elt = 4; return ctx->unwrapped[0];
-        case SCAN3D_PLANE_UNWRAPPED_H: *elt = 4; return ctx->unwrapped[1];
-        case SCAN3D_PLANE_CODE_V: *elt = 2; return ctx->code[0];
-        case SCAN3D_PLANE_CODE_H: *elt = 2; return ctx->code[1];
-        case SCAN3D_PLANE_MASK: *elt = 1; return ctx->mask[0];
-        case S3D_PLANE_MASK_H: *elt = 1; return ctx->mask[1];
-        case SCAN3D_PLANE_VALID: *elt = 1; return ctx->valid;
-        case SCAN3D_PLANE_CPMAP: *elt = 8; return ctx->cpmap;
-        case SCAN3D_PLANE_XYZ: *elt = 24; return ctx->xyz;
-        default: *elt = 0; return nullptr;
-    }
-}
+// a plane id's buffer, its element size and the result that holds it
+struct Plane {
+    void* buf;
+    size_t elt;
+    Result result;
+};
 
-// has the plane been produced by a compute entry since the context was created / the inputs last changed?
-static bool plane_ready(const scan3d_ctx* ctx, int plane)
+static Plane plane_of(const scan3d_ctx* ctx, int plane)
 {
     switch (plane) {
-        case SCAN3D_PLANE_WRAPPED_V: case SCAN3D_PLANE_MASK: return ctx->have_wrapped[0];
-        case SCAN3D_PLANE_WRAPPED_H: case S3D_PLANE_MASK_H: return ctx->have_wrapped[1];
-        case SCAN3D_PLANE_UNWRAPPED_V: case SCAN3D_PLANE_CODE_V: return ctx->have_unwrapped[0];
-        case SCAN3D_PLANE_UNWRAPPED_H: case SCAN3D_PLANE_CODE_H: return ctx->have_unwrapped[1];
-        case SCAN3D_PLANE_VALID: return ctx->have_valid;
-        case SCAN3D_PLANE_CPMAP: return ctx->have_cpmap;
-        case SCAN3D_PLANE_XYZ: return ctx->have_xyz;
-        default: return false;
+        case SCAN3D_PLANE_WRAPPED_V: return {ctx->wrapped[0], 4, WRAPPED_V};
+        case SCAN3D_PLANE_WRAPPED_H: return {ctx->wrapped[1], 4, WRAPPED_H};
+        case SCAN3D_PLANE_UNWRAPPED_V: return {ctx->unwrapped[0], 4, UNWRAPPED_V};
+        case SCAN3D_PLANE_UNWRAPPED_H: return {ctx->unwrapped[1], 4, UNWRAPPED_H};
+        case SCAN3D_PLANE_CODE_V: return {ctx->code[0], 2, UNWRAPPED_V};
+        case SCAN3D_PLANE_CODE_H: return {ctx->code[1], 2, UNWRAPPED_H};
+        case SCAN3D_PLANE_MASK: return {ctx->mask[0], 1, WRAPPED_V};
+        case S3D_PLANE_MASK_H: return {ctx->mask[1], 1, WRAPPED_H};
+        case SCAN3D_PLANE_VALID: return {ctx->valid, 1, VALID};
+        case SCAN3D_PLANE_CPMAP: return {ctx->cpmap, 8, CPMAP};
+        case SCAN3D_PLANE_XYZ: return {ctx->xyz, 24, XYZ};
+        default: return {nullptr, 0, RESULT_COUNT};
     }
 }
 
 int64_t scan3d_plane_bytes(const scan3d_ctx* ctx, int plane)
 {
     if (!ctx) return 0;
-    size_t elt = 0;
-    plane_ptr(const_cast<scan3d_ctx*>(ctx), plane, &elt);
-    return (int64_t)(elt * npix(ctx));
+    return (int64_t)(plane_of(ctx, plane).elt * npix(ctx));
 }
 
 void* scan3d_device_plane(scan3d_ctx* ctx, int plane)
 {
-    if (!ctx || !plane_ready(ctx, plane)) return nullptr;     // (a plane nothing has written is not handed out)
-    size_t elt;
-    return plane_ptr(ctx, plane, &elt);
+    if (!ctx) return nullptr;
+    const Plane p = plane_of(ctx, plane);
+    return ctx->results.has(p.result) ? p.buf : nullptr;     // (a plane nothing has written is not handed out)
 }
 
 int scan3d_get_plane(scan3d_ctx* ctx, int plane, void* dst_host)
 {
     if (!ctx || !dst_host) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
-    size_t elt;
-    void* src = plane_ptr(ctx, plane, &elt);
-    if (!src || !plane_ready(ctx, plane))
+    const Plane p = plane_of(ctx, plane);
+    if (!p.buf || !ctx->results.has(p.result))
         return fail(ctx, SCAN3D_ERR_STATE, "plane not available: no compute entry has produced it (the single-pass entry "
                                            "keeps wrapped phases and per-direction masks in registers)");
     CK(cudaSetDevice(ctx->device));
-    CK(cudaMemcpyAsync(dst_host, src, elt * npix(ctx), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(dst_host, p.buf, p.elt * npix(ctx), cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return SCAN3D_OK;
 }
@@ -732,7 +733,7 @@ int scan3d_get_cpmap_i64(scan3d_ctx* ctx, int64_t* dst_host)
 int scan3d_point_count(scan3d_ctx* ctx, int64_t* count_out)
 {
     if (!ctx || !count_out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
-    if (!ctx->have_points) return fail(ctx, SCAN3D_ERR_STATE, "no compacted points yet");
+    if (!ctx->results.has(POINTS)) return fail(ctx, SCAN3D_ERR_STATE, "no compacted points yet");
     CK(cudaSetDevice(ctx->device));
     uint32_t c = 0;
     CK(cudaMemcpyAsync(&c, ctx->d_count, 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -754,7 +755,7 @@ int scan3d_get_points(scan3d_ctx* ctx, float* xyz_host, uint32_t* pix_host, uint
         CK(cudaMemcpyAsync(pix_host, ctx->pix, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
     }
     if (rgb_host) {
-        if (ctx->rgb && ctx->texture) CK(cudaMemcpyAsync(rgb_host, ctx->rgb, (size_t)n * 3, cudaMemcpyDeviceToHost, ctx->stream));
+        if (ctx->results.has(POINT_COLOURS)) CK(cudaMemcpyAsync(rgb_host, ctx->rgb, (size_t)n * 3, cudaMemcpyDeviceToHost, ctx->stream));
         else memset(rgb_host, 0, (size_t)n * 3);
     }
     CK(cudaStreamSynchronize(ctx->stream));
@@ -824,8 +825,8 @@ int scan3d_set_points_buffer(scan3d_ctx* ctx, void* points_dev, int64_t capacity
             else if (e != cudaSuccess) return fail(ctx, SCAN3D_ERR_CUDA, cudaGetErrorString(e));
         }
     }
+    ctx->results.drop(POINTS);
     ctx->pts_ext = (float*)points_dev;
-    ctx->have_points = ctx->have_mesh = false;
     return SCAN3D_OK;
 }
 void* scan3d_device_point_pixels(scan3d_ctx* ctx) { return ctx ? ctx->pix.get() : nullptr; }
@@ -921,8 +922,9 @@ int scan3d_build_mesh(scan3d_ctx* ctx, float max_edge)
         return fail(ctx, SCAN3D_ERR_CONFIG, "the mesh needs the whole frame (a shard's last cell row needs the next shard's first row)");
     if ((int64_t)c.W * c.H >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "W*H must be below 2^31 (int32 point indices)");
     if (!(max_edge > 0.0f)) return fail(ctx, SCAN3D_ERR_ARG, "max_edge must be > 0 (+inf: no length limit)");
-    if (!ctx->have_points) return fail(ctx, SCAN3D_ERR_STATE, "build_mesh before the points are computed");
+    if (!ctx->results.has(POINTS)) return fail(ctx, SCAN3D_ERR_STATE, "build_mesh before the points are computed");
     CK(cudaSetDevice(ctx->device));
+    ctx->results.drop(MESH);
     const size_t n = npix(ctx);
     const size_t nb = (n + POINT_BLOCK - 1) / POINT_BLOCK;
     const size_t max_faces = 2 * (size_t)(c.W - 1) * (size_t)(c.H - 1);
@@ -934,14 +936,14 @@ int scan3d_build_mesh(scan3d_ctx* ctx, float max_edge)
     CK(ctx->mesh_normals.ensure(3 * n));
     CK(launch_mesh(ctx->valid, points_of(ctx), c.W, c.H, max_edge, ctx->mesh_idx, ctx->block_counts, ctx->mesh_counts,
                    ctx->mesh_totals, ctx->mesh_faces, ctx->mesh_normals, ctx->stream, &ctx->launches));
-    ctx->have_mesh = true;
+    ctx->results.produce(MESH);
     return SCAN3D_OK;
 }
 
 int scan3d_mesh_face_count(scan3d_ctx* ctx, int64_t* count_out)
 {
     if (!ctx || !count_out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
-    if (!ctx->have_mesh) return fail(ctx, SCAN3D_ERR_STATE, "no mesh of the current points: call scan3d_build_mesh");
+    if (!ctx->results.has(MESH)) return fail(ctx, SCAN3D_ERR_STATE, "no mesh of the current points: call scan3d_build_mesh");
     CK(cudaSetDevice(ctx->device));
     uint32_t nf = 0;
     CK(cudaMemcpyAsync(&nf, ctx->mesh_totals + 1, 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -967,8 +969,11 @@ int scan3d_get_mesh(scan3d_ctx* ctx, int32_t* faces_host, float* normals_host, i
     return SCAN3D_OK;
 }
 
-void* scan3d_device_mesh_faces(scan3d_ctx* ctx) { return ctx && ctx->have_mesh ? ctx->mesh_faces.get() : nullptr; }
-void* scan3d_device_point_normals(scan3d_ctx* ctx) { return ctx && ctx->have_mesh ? ctx->mesh_normals.get() : nullptr; }
+void* scan3d_device_mesh_faces(scan3d_ctx* ctx) { return ctx && ctx->results.has(MESH) ? ctx->mesh_faces.get() : nullptr; }
+void* scan3d_device_point_normals(scan3d_ctx* ctx)
+{
+    return ctx && ctx->results.has(MESH) ? ctx->mesh_normals.get() : nullptr;
+}
 
 int scan3d_write_mesh_ply(scan3d_ctx* ctx, const char* path, int binary)
 {
@@ -1002,8 +1007,7 @@ int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
         return fail(ctx, SCAN3D_ERR_ARG, "voxel_size must be finite and > 0");
     if (max_voxels < 1 || max_voxels >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_ARG, "max_voxels must be in [1, 2^31)");
     CK(cudaSetDevice(ctx->device));
-    ctx->vox_begun = ctx->vox_fresh = false;
-    ctx->srf_ready = ctx->cc_ready = false;
+    ctx->results.drop(ACCUMULATOR);
     CK(ctx->vox.reset((uint32_t)max_voxels, (double)voxel_size, ctx->sm_count, ctx->stream));
     const size_t m = (size_t)max_voxels, n = npix(ctx);
     CK(grow_group(Grow(ctx->vox_xyz, 3 * m), Grow(ctx->vox_nrm, 3 * m), Grow(ctx->vox_rgb, 3 * m),
@@ -1013,7 +1017,7 @@ int scan3d_voxel_begin(scan3d_ctx* ctx, float voxel_size, int64_t max_voxels)
     CK(ctx->block_counts.ensure((n + POINT_BLOCK - 1) / POINT_BLOCK + 1));
     ctx->vox_bound = 0;
     ctx->vox_chunks = 0;
-    ctx->vox_begun = true;
+    ctx->results.produce(ACCUMULATOR);
     return SCAN3D_OK;
 }
 
@@ -1032,17 +1036,17 @@ static const uint64_t VOXEL_MAX_POINTS = 0xffffffffull;   // point indices since
 int scan3d_voxel_add_points(scan3d_ctx* ctx)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
-    if (!ctx->vox_begun) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before scan3d_voxel_begin");
+    if (!ctx->results.has(ACCUMULATOR)) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before scan3d_voxel_begin");
     if (ctx->cfg.dirs != 2) return fail(ctx, SCAN3D_ERR_STATE, "no point cloud in a one-direction configuration");
-    if (!ctx->have_points) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before the points are computed");
+    if (!ctx->results.has(POINTS)) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before the points are computed");
     const uint64_t ub = npix(ctx);
     if (ctx->vox_bound + ub > VOXEL_MAX_POINTS)
         return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^32 - 1 points since scan3d_voxel_begin (W*H counted per ctx add)");
     CK(cudaSetDevice(ctx->device));
     ctx->vox_bound += ub;
-    ctx->vox_fresh = ctx->srf_ready = ctx->cc_ready = false;
-    return voxel_add(ctx, points_of(ctx), ctx->have_mesh ? ctx->mesh_normals.get() : nullptr,
-                     ctx->texture && ctx->rgb ? ctx->rgb.get() : nullptr, ctx->d_count, (uint32_t)ub);
+    ctx->results.drop(VOXELS);
+    return voxel_add(ctx, points_of(ctx), ctx->results.has(MESH) ? ctx->mesh_normals.get() : nullptr,
+                     ctx->results.has(POINT_COLOURS) ? ctx->rgb.get() : nullptr, ctx->d_count, (uint32_t)ub);
 }
 
 int scan3d_voxel_add_points_dev(scan3d_ctx* ctx, const float* xyz_dev, const float* normals_dev, const uint8_t* rgb_dev,
@@ -1053,12 +1057,12 @@ int scan3d_voxel_add_points_dev(scan3d_ctx* ctx, const float* xyz_dev, const flo
     if (!xyz_dev && n > 0) return fail(ctx, SCAN3D_ERR_ARG, "null xyz_dev");
     if (((uintptr_t)xyz_dev & 3) || ((uintptr_t)normals_dev & 3))
         return fail(ctx, SCAN3D_ERR_ARG, "xyz_dev and normals_dev must be 4-byte aligned");
-    if (!ctx->vox_begun) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before scan3d_voxel_begin");
+    if (!ctx->results.has(ACCUMULATOR)) return fail(ctx, SCAN3D_ERR_STATE, "voxel add before scan3d_voxel_begin");
     if (ctx->vox_bound + (uint64_t)n > VOXEL_MAX_POINTS)
         return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^32 - 1 points since scan3d_voxel_begin");
     CK(cudaSetDevice(ctx->device));
     ctx->vox_bound += (uint64_t)n;
-    ctx->vox_fresh = ctx->srf_ready = ctx->cc_ready = false;
+    ctx->results.drop(VOXELS);
     const int64_t chunk = (int64_t)npix(ctx);   // the per-point scratch holds W*H points
     for (int64_t off = 0; off < n; off += chunk) {
         const int64_t k = std::min(chunk, n - off);
@@ -1072,20 +1076,20 @@ int scan3d_voxel_add_points_dev(scan3d_ctx* ctx, const float* xyz_dev, const flo
 int scan3d_voxel_finish(scan3d_ctx* ctx)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
-    if (!ctx->vox_begun) return fail(ctx, SCAN3D_ERR_STATE, "voxel finish before scan3d_voxel_begin");
+    if (!ctx->results.has(ACCUMULATOR)) return fail(ctx, SCAN3D_ERR_STATE, "voxel finish before scan3d_voxel_begin");
     CK(cudaSetDevice(ctx->device));
+    ctx->results.drop(VOXELS);
     CK(launch_voxel_finish(ctx->vox.view, (int)(ctx->vox_chunks & 1), ctx->vox_xyz, ctx->vox_nrm, ctx->vox_rgb,
                            ctx->vox_cnt, ctx->sm_count, ctx->stream));
     ctx->launches += 1;
-    ctx->vox_fresh = true;
-    ctx->srf_ready = ctx->cc_ready = false;
+    ctx->results.produce(VOXELS);
     return SCAN3D_OK;
 }
 
 int scan3d_voxel_count(scan3d_ctx* ctx, int64_t* voxels_out, int64_t* dropped_out)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
-    if (!ctx->vox_begun || !ctx->vox_fresh)
+    if (!ctx->results.has(VOXELS))
         return fail(ctx, SCAN3D_ERR_STATE, "no voxel outputs of the current adds: call scan3d_voxel_finish");
     CK(cudaSetDevice(ctx->device));
     VoxelState st;
@@ -1162,7 +1166,7 @@ static int check_align_args(scan3d_ctx* ctx, const scan3d_align_params* p, scan3
     if (!(p->stop_rotation >= 0.0) || !(p->stop_translation >= 0.0))
         return fail(ctx, SCAN3D_ERR_ARG, "stop thresholds must be >= 0");
     if (!rigid_4x4(p->T_init)) return fail(ctx, SCAN3D_ERR_ARG, "T_init must be a finite rigid transform (rotation within 1e-6)");
-    if (!ctx->vox_begun || !ctx->vox_fresh)
+    if (!ctx->results.has(VOXELS))
         return fail(ctx, SCAN3D_ERR_STATE, "no voxel outputs of the current adds to align to: call scan3d_voxel_finish");
     return SCAN3D_OK;
 }
@@ -1211,10 +1215,9 @@ int scan3d_align_to_voxels(scan3d_ctx* ctx, const scan3d_align_params* p, scan3d
     int rc = check_align_args(ctx, p, out);
     if (rc) return rc;
     if (ctx->cfg.dirs != 2) return fail(ctx, SCAN3D_ERR_STATE, "no point cloud in a one-direction configuration");
-    if (!ctx->have_points) return fail(ctx, SCAN3D_ERR_STATE, "align before the points are computed");
-    rc = align_run(ctx, points_of(ctx), ctx->d_count, (long long)npix(ctx), p, out);
-    if (rc == SCAN3D_OK && p->apply) ctx->have_mesh = false;
-    return rc;
+    if (!ctx->results.has(POINTS)) return fail(ctx, SCAN3D_ERR_STATE, "align before the points are computed");
+    if (p->apply) ctx->results.drop(MESH);   // the points move; their colours stay theirs
+    return align_run(ctx, points_of(ctx), ctx->d_count, (long long)npix(ctx), p, out);
 }
 
 int scan3d_align_to_voxels_dev(scan3d_ctx* ctx, float* xyz_dev, int64_t n, const scan3d_align_params* p,
@@ -1239,10 +1242,10 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
     if (!(p->max_distance > 0.0f && p->max_distance - p->max_distance == 0.0f))
         return fail(ctx, SCAN3D_ERR_ARG, "max_distance must be finite and > 0");
     if (p->max_points < 1 || p->max_points >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_ARG, "max_points must be in [1, 2^31)");
-    if (!ctx->vox_begun || !ctx->vox_fresh)
+    if (!ctx->results.has(VOXELS))
         return fail(ctx, SCAN3D_ERR_STATE, "no voxel outputs of the current adds to mesh: call scan3d_voxel_finish");
     CK(cudaSetDevice(ctx->device));
-    ctx->srf_ready = ctx->cc_ready = false;
+    ctx->results.drop(SURFACE);
     AlignRun run{};                                      // the index only; T0 = I for the state it initialises
     run.T0[0] = run.T0[5] = run.T0[10] = 1.0;
     run.S = s3l::cell_edge(p->max_distance);
@@ -1268,9 +1271,7 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
     CK(ctx->lattice.emit(ctx->vox_rgb, st.vertices, ctx->surface, ctx->stream, &ctx->launches));
     ctx->surface.vertices = st.vertices;
     ctx->surface.faces = st.faces;
-    ctx->srf_ready = true;
-    ctx->srf_decimated = false;
-    ctx->srf_smoothed = false;
+    ctx->results.produce(SURFACE);
     out->vertices = st.vertices;
     out->faces = st.faces;
     out->lattice_points = st.occupied;
@@ -1282,7 +1283,7 @@ int scan3d_get_voxel_surface(scan3d_ctx* ctx, float* xyz, float* normals, uint8_
                              int64_t max_vertices, int64_t max_faces)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
-    if (!ctx->srf_ready)
+    if (!ctx->results.has(SURFACE))
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
     CK(cudaSetDevice(ctx->device));
     const SurfaceMesh& s = ctx->surface;
@@ -1299,7 +1300,7 @@ int scan3d_get_voxel_surface(scan3d_ctx* ctx, float* xyz, float* normals, uint8_
 int scan3d_write_voxel_surface_ply(scan3d_ctx* ctx, const char* path, int binary)
 {
     if (!ctx || !path) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
-    if (!ctx->srf_ready)
+    if (!ctx->results.has(SURFACE))
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
     const int64_t nv = ctx->surface.vertices, nf = ctx->surface.faces;
     std::vector<float> xyz((size_t)nv * 3), nrm((size_t)nv * 3);
@@ -1322,10 +1323,10 @@ int scan3d_voxel_surface_components(scan3d_ctx* ctx, const scan3d_components_par
     if (!ctx) return SCAN3D_ERR_ARG;
     if (!p || !out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
     if (p->min_faces < 0 || p->max_components < 0) return fail(ctx, SCAN3D_ERR_ARG, "min_faces and max_components must be >= 0");
-    if (!ctx->srf_ready)
+    if (!ctx->results.has(SURFACE))
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
     CK(cudaSetDevice(ctx->device));
-    ctx->cc_ready = false;
+    ctx->results.drop(COMPONENTS);
     CK(ctx->cc.select(ctx->surface, (unsigned long long)p->min_faces, (unsigned long long)p->max_components,
                       ctx->stream, &ctx->launches));
     ComponentsState st;
@@ -1338,7 +1339,7 @@ int scan3d_voxel_surface_components(scan3d_ctx* ctx, const scan3d_components_par
     ctx->surface.vertices = st.vertices;
     ctx->surface.faces = st.faces;
     ctx->cc_components = st.components;
-    ctx->cc_ready = true;
+    ctx->results.produce(COMPONENTS);
     out->components = st.components;
     out->kept = st.kept;
     out->vertices = st.vertices;
@@ -1351,7 +1352,7 @@ int scan3d_get_surface_components(scan3d_ctx* ctx, int64_t* vertices, int64_t* f
                                   int64_t max_components)
 {
     if (!ctx) return SCAN3D_ERR_ARG;
-    if (!ctx->cc_ready)
+    if (!ctx->results.has(COMPONENTS))
         return fail(ctx, SCAN3D_ERR_STATE, "no component table of the held surface: call scan3d_voxel_surface_components");
     CK(cudaSetDevice(ctx->device));
     const int64_t n = std::max<int64_t>(0, std::min(ctx->cc_components, max_components));
@@ -1393,19 +1394,19 @@ int scan3d_voxel_surface_decimate(scan3d_ctx* ctx, float cell_size, scan3d_decim
     if (!ctx) return SCAN3D_ERR_ARG;
     if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
     if (!(cell_size - cell_size == 0.0f)) return fail(ctx, SCAN3D_ERR_ARG, "cell_size must be finite");
-    if (!ctx->srf_ready)
+    if (!ctx->results.has(SURFACE))
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
     const double H = (double)cell_size, s = ctx->vox.view.S;
     if (!(H >= s && H <= s3q::RATIO_MAX * s))
         return fail(ctx, SCAN3D_ERR_ARG, "cell_size must be in [voxel_size, 256 voxel_size]");
-    if (ctx->srf_decimated)
+    if (ctx->results.has(SIMPLIFIED))
         return fail(ctx, SCAN3D_ERR_STATE, "the held surface is already simplified: extract it again first");
-    if (ctx->srf_smoothed)
+    if (ctx->results.has(SMOOTHED))
         return fail(ctx, SCAN3D_ERR_STATE, "the held surface is smoothed: extract it again to simplify it");
     const int64_t nv = ctx->surface.vertices, nf = ctx->surface.faces;
     if (nf >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^31 - 1 surface faces");
     CK(cudaSetDevice(ctx->device));
-    ctx->cc_ready = false;
+    ctx->results.drop(COMPONENTS);
     // the emission runs before the synchronisation, so the spare set holds the whole input
     CK(ctx->spare.grow(std::max<int64_t>(nv, 1), std::max<int64_t>(nf, 1)));
     CK(ctx->dec.run(ctx->surface, H, ctx->spare, ctx->sm_count, ctx->stream, &ctx->launches));
@@ -1418,7 +1419,7 @@ int scan3d_voxel_surface_decimate(scan3d_ctx* ctx, float cell_size, scan3d_decim
     std::swap(ctx->surface, ctx->spare);
     ctx->surface.vertices = vst.total[1];
     ctx->surface.faces = st.faces;
-    ctx->srf_decimated = true;
+    ctx->results.produce(SIMPLIFIED);
     out->vertices = vst.total[1];
     out->faces = st.faces;
     out->collapsed_faces = st.collapsed;
@@ -1473,7 +1474,7 @@ int scan3d_voxel_surface_smooth(scan3d_ctx* ctx, const scan3d_smooth_params* p, 
     if (!ctx) return SCAN3D_ERR_ARG;
     int rc = check_smooth_args(ctx, p, out);
     if (rc) return rc;
-    if (!ctx->srf_ready)
+    if (!ctx->results.has(SURFACE))
         return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
     CK(cudaSetDevice(ctx->device));
     SurfaceMesh &s = ctx->surface, &spare = ctx->spare;
@@ -1483,7 +1484,7 @@ int scan3d_voxel_surface_smooth(scan3d_ctx* ctx, const scan3d_smooth_params* p, 
     // the smoothed positions and normals become the held surface; faces, colours and the vertex order are unchanged
     std::swap(s.xyz, spare.xyz);
     std::swap(s.nrm, spare.nrm);
-    ctx->srf_smoothed = true;
+    ctx->results.produce(SMOOTHED);
     return SCAN3D_OK;
 }
 

@@ -9,6 +9,7 @@
 #include "../../include/scan3d.h"
 #include "scan3d_device_buffer.h"
 #include "scan3d_math.cuh"
+#include "scan3d_results.h"
 
 #define S3D_PLANE_MASK_H 10   // internal: valid_map_horizontal when the stage API is used
 
@@ -327,8 +328,6 @@ struct scan3d_ctx {
 
     // scan3d_voxel_begin: the merge accumulator (independent of the points; reallocated when a begin asks for more)
     s3d::VoxelStore vox;
-    bool vox_begun = false;        // a begin has run
-    bool vox_fresh = false;        // the outputs are those of the adds since begin (a finish ran after the last add)
     uint64_t vox_bound = 0;        // upper bound of the points added since begin (W*H per ctx add, n per dev add)
     uint32_t vox_chunks = 0;       // adds (chunks of <= W*H points) since begin
     Buf<uint32_t> vox_point_slot;         // [H*W] per-point scratch of an add
@@ -348,11 +347,7 @@ struct scan3d_ctx {
 
     // the held voxel surface, and the spare set that components, decimate and smooth write before they swap it in
     s3d::SurfaceMesh surface, spare;
-    bool srf_ready = false;               // the surface of the current voxel outputs is held
-    bool cc_ready = false;                // the component table of the last scan3d_voxel_surface_components is held
     int64_t cc_components = 0;
-    bool srf_decimated = false;           // the held surface is a simplification (it is not simplified again)
-    bool srf_smoothed = false;            // the held surface is smoothed (scan3d_voxel_surface_decimate refuses it)
 
     int cta_limit = 0;             // scan3d_set_cta_limit
 
@@ -360,12 +355,8 @@ struct scan3d_ctx {
     bool reg_on = false;
     float reg_R[16] = {}, reg_t[3] = {};
 
-    // stage bookkeeping
-    bool have_wrapped[2] = {false, false};
-    bool have_unwrapped[2] = {false, false};
-    bool have_cpmap = false, have_valid = false, have_xyz = false, have_points = false;
-    bool have_mesh = false;        // built from the current points; every entry that rewrites or drops them clears it
-    bool in_reconstruct = false;   // stage entries called from scan3d_reconstruct_dev's stage chain
+    // which of the results above are current (scan3d_results.h)
+    s3d::Results results;
 };
 
 // the C entries' error returns: a failed CUDA call names itself in ctx->err

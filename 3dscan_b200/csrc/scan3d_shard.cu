@@ -275,7 +275,7 @@ int scan3d_shard_gather(scan3d_shard* sh, int slot, scan3d_ctx* ctx, int64_t* to
 {
     if (!sh || !ctx || slot < 0 || slot >= sh->slots || sh->host_mode) return sfail(sh, SCAN3D_ERR_ARG, "scan3d_shard_gather: bad argument");
     if (cudaSetDevice(sh->device) != cudaSuccess) return sfail(sh, SCAN3D_ERR_CUDA, "cudaSetDevice failed");
-    if (!ctx->have_points) return sfail(sh, SCAN3D_ERR_STATE, "scan3d_shard_gather before the ctx's reconstruction");
+    if (!ctx->results.has(s3d::POINTS)) return sfail(sh, SCAN3D_ERR_STATE, "scan3d_shard_gather before the ctx's reconstruction");
     // this rank's count (waits for its reconstruction)
     cudaError_t e = cudaMemcpyAsync(sh->h_count, ctx->d_count, 4, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);

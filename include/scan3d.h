@@ -142,7 +142,8 @@ int scan3d_set_calibration(scan3d_ctx *ctx, const scan3d_calib *cal);
 int scan3d_get_projection_matrices(scan3d_ctx *ctx, double A_cam[12], double A_proj[12]);
 
 /* Optional texture ("Point_cloud/texture.bmp", 8/save_point_cloud.cpp:59-66): BGR u8 [H][W][3].
- * NULL clears it (points then carry rgb = 0). */
+ * NULL clears it.  Points carry colours only if a texture was set when they were computed (a reconstruct or
+ * scan3d_compact_points) and scan3d_set_texture(NULL) has not run since; otherwise their colours are zeros. */
 int scan3d_set_texture(scan3d_ctx *ctx, const uint8_t *bgr_host);
 
 /* ---- stage entries (mirror the reference's call sequence) ------------------------------ */
@@ -276,7 +277,8 @@ int scan3d_write_mesh_ply(scan3d_ctx *ctx, const char *path, int binary);
  * accumulator is independent of the ctx's points: a later reconstruct does not touch it.  No kernel launch.
  * scan3d_voxel_add_points: the ctx's current points, wherever they are (scan3d_set_points_buffer included, row-sharded
  * contexts included); each brings its normal from the mesh when the mesh of the current points is fresh
- * (scan3d_build_mesh), else (0,0,0), and its colour when a texture is set, else (0,0,0), as scan3d_write_ply does.
+ * (scan3d_build_mesh), else (0,0,0), and its colour as scan3d_write_ply writes it: the texture's when a texture was
+ * set when the points were computed and scan3d_set_texture(NULL) has not run since, else (0,0,0).
  * Always 5 kernel launches.
  * scan3d_voxel_add_points_dev: n points from caller device memory on the ctx's GPU (xyz f32[n][3], normals f32[n][3]
  * or NULL, rgb u8[n][3] or NULL; NULL means zeros), ordered on the ctx stream.  Runs in chunks of W*H points, 5 kernel

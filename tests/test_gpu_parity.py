@@ -660,3 +660,33 @@ def test_ply_writer(tmp_path):
     packed = (rgb[:, 0].astype(np.uint32) << 16) | (rgb[:, 1].astype(np.uint32) << 8) | rgb[:, 2]
     assert np.allclose(rows[:, 3], packed.view(np.float32).astype(np.float64), rtol=5e-8, atol=0)
     ctx.close()
+
+
+def test_points_carry_the_colours_of_the_texture_they_were_computed_with():
+    """A texture set after the points were computed does not colour them: with texture A, a reconstruct, no texture, a
+    reconstruct, then texture B, the points and the voxels merged from them read zeros, not A's colours."""
+    W, H, PW, PH = 256, 64, 512, 512
+    cal, _, _ = calibs(W / 1600.0, PW / 1280.0)
+    cfg = s3.make_config(W, H, PW, PH, 3, 6, 6, 8, 8, 2)
+    stack, roi = s3.synth_stack(cfg, cal)
+    ctx = _ctx(cfg, cal)
+    rng = np.random.default_rng(3)
+    tex_a, tex_b = (rng.integers(1, 256, (H, W, 3), dtype=np.uint8) for _ in range(2))
+    ctx.set_texture(tex_a)
+    ctx.reconstruct(stack, roi)
+    _, rgb = ctx.points(want_rgb=True)
+    valid = ctx.plane(s3.PLANE_VALID).astype(bool)
+    assert np.array_equal(rgb, tex_a[valid][:, ::-1]) and rgb.all()
+    ctx.set_texture(None)
+    n = ctx.reconstruct(stack, roi)
+    ctx.set_texture(tex_b)
+    xyz, rgb = ctx.points(want_rgb=True)
+    assert n > 1000 and not rgb.any()
+    ctx.voxel_begin(float(np.ptp(xyz, axis=0).max()) / 64, n)
+    ctx.voxel_add()
+    ctx.voxel_finish()
+    assert not ctx.voxels()[2].any()
+    # the next reconstruct is computed with B
+    ctx.reconstruct(stack, roi)
+    assert np.array_equal(ctx.points(want_rgb=True)[1], tex_b[valid][:, ::-1])
+    ctx.close()
