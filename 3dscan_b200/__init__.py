@@ -114,6 +114,17 @@ class SmoothResultC(C.Structure):
                 ("isolated_vertices", C.c_int64), ("passes", C.c_int64), ("max_displacement", C.c_double)]
 
 
+class FillResultC(C.Structure):
+    _fields_ = [("vertices", C.c_int64), ("faces", C.c_int64), ("boundary_edges", C.c_int64), ("holes", C.c_int64),
+                ("filled", C.c_int64), ("faces_added", C.c_int64), ("open_edges", C.c_int64)]
+
+
+# the largest hole scan3d_voxel_surface_fill_holes accepts on a surface that is neither simplified nor smoothed (which
+# stays decimatable after the fill), and on any other mesh (include/scan3d.h)
+FILL_NETS_MAX_EDGES = 22
+FILL_MAX_EDGES = 1024
+
+
 # voxel_surface's default max_points per merged voxel: the smallest power of two >= 1.5x the largest lattice points
 # per voxel measured on tools/bench_surface.py's workloads (29.2 on workload A, profiles/r3_bench_surface.json).  64 is
 # also the most a voxel can add (the 4 x 4 x 4 corners of its 27 cells), so the default never overflows; pass
@@ -249,6 +260,8 @@ def cuda_lib():
     L.scan3d_voxel_surface_decimate.argtypes = [vp, C.c_float, C.POINTER(DecimateResultC)]
     L.scan3d_voxel_surface_smooth.argtypes = [vp, C.POINTER(SmoothParams), C.POINTER(SmoothResultC)]
     L.scan3d_mesh_smooth_dev.argtypes = [vp, vp, vp, i64, vp, i64, C.POINTER(SmoothParams), C.POINTER(SmoothResultC)]
+    L.scan3d_voxel_surface_fill_holes.argtypes = [vp, i32, C.POINTER(FillResultC)]
+    L.scan3d_mesh_fill_holes_dev.argtypes = [vp, vp, i64, vp, i64, i32, vp, i64, C.POINTER(FillResultC)]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -668,6 +681,7 @@ class Scan3D:
         r = SurfaceResultC()
         self._ck(self.L.scan3d_voxel_surface(self.h, C.byref(p), C.byref(r)))
         self._surface_counts = (r.vertices, r.faces)
+        self._surface_refined = False
         return dict(vertices=r.vertices, faces=r.faces, lattice_points=r.lattice_points,
                     undefined_points=r.undefined_points)
 
@@ -730,6 +744,7 @@ class Scan3D:
         self._ck(self.L.scan3d_voxel_surface_decimate(self.h, float(cell_size), C.byref(r)))
         self._surface_counts = (r.vertices, r.faces)
         self._components = 0
+        self._surface_refined = True
         return dict(vertices=r.vertices, faces=r.faces, collapsed_faces=r.collapsed_faces,
                     duplicate_faces=r.duplicate_faces, mean_fallbacks=r.mean_fallbacks)
 
@@ -748,6 +763,7 @@ class Scan3D:
         self._ck(self.L.scan3d_voxel_surface_smooth(self.h, C.byref(SmoothParams(int(iterations), lam, mu)),
                                                     C.byref(r)))
         self._surface_counts = (r.vertices, r.faces)
+        self._surface_refined = True
         return self._smooth_result(r)
 
     def mesh_smooth_dev(self, xyz, faces, normals=None, iterations=10, lam=0.5, mu=-0.53):
@@ -772,6 +788,54 @@ class Scan3D:
                                                xyz.shape[0], C.c_void_p(faces.data_ptr()), faces.shape[0],
                                                C.byref(SmoothParams(int(iterations), lam, mu)), C.byref(r)))
         return self._smooth_result(r)
+
+    # -- hole filling of the voxel surface and of device meshes (include/scan3d.h has the exact rules)
+    @staticmethod
+    def _fill_result(r):
+        return dict(vertices=r.vertices, faces=r.faces, boundary_edges=r.boundary_edges, holes=r.holes,
+                    filled=r.filled, faces_added=r.faces_added, open_edges=r.open_edges)
+
+    def surface_fill_holes(self, max_edges=None):
+        """Close, in place, the holes of the held voxel surface whose boundary loops have at most max_edges edges by
+        minimum-weight triangulation (Liepa's weight).  max_edges None = the largest allowed: FILL_NETS_MAX_EDGES on a
+        surface that is neither simplified nor smoothed (it stays decimatable), else FILL_MAX_EDGES.  Synchronises
+        twice and returns a dict with vertices, faces, boundary_edges, holes, filled, faces_added and open_edges.
+        voxel_surface_mesh() then returns the filled surface; the component table goes stale."""
+        if max_edges is None:
+            max_edges = FILL_MAX_EDGES if getattr(self, "_surface_refined", False) else FILL_NETS_MAX_EDGES
+        r = FillResultC()
+        self._ck(self.L.scan3d_voxel_surface_fill_holes(self.h, int(max_edges), C.byref(r)))
+        self._surface_counts = (r.vertices, r.faces)
+        self._components = 0
+        return self._fill_result(r)
+
+    def mesh_fill_holes_dev(self, xyz, faces, max_edges=FILL_MAX_EDGES):
+        """surface_fill_holes() for a triangle mesh on the ctx's GPU: xyz a CUDA float32 tensor [v][3], faces a CUDA
+        int32 tensor [f][3]; neither is changed.  torch's current stream is synchronised first, so data written there
+        is ready.  Returns (the added faces, a new CUDA int32 tensor [faces_added][3], the dict of
+        surface_fill_holes())."""
+        import torch
+
+        def ok(t, dtype):
+            return (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dtype and t.dim() == 2 and
+                    t.shape[1] == 3 and t.is_contiguous())
+        if not ok(xyz, torch.float32):
+            raise Scan3DError("xyz must be a contiguous CUDA float32 tensor of shape [v][3]")
+        if not ok(faces, torch.int32):
+            raise Scan3DError("faces must be a contiguous CUDA int32 tensor of shape [f][3]")
+        torch.cuda.current_stream(xyz.device).synchronize()
+        rows = faces.shape[0]
+        for attempt in range(2):
+            out = torch.empty((max(rows, 1), 3), dtype=torch.int32, device=xyz.device)
+            r = FillResultC()
+            rc = self.L.scan3d_mesh_fill_holes_dev(self.h, C.c_void_p(xyz.data_ptr()), xyz.shape[0],
+                                                   C.c_void_p(faces.data_ptr()), faces.shape[0], int(max_edges),
+                                                   C.c_void_p(out.data_ptr()), rows, C.byref(r))
+            if rc == -1 and attempt == 0 and r.faces_added > rows:   # SCAN3D_ERR_CONFIG
+                rows = r.faces_added                        # too small: once more with the reported size
+                continue
+            self._ck(rc)
+            return out[:r.faces_added], self._fill_result(r)
 
     # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
     @staticmethod

@@ -1505,6 +1505,100 @@ int scan3d_mesh_smooth_dev(scan3d_ctx* ctx, float* xyz_dev, float* normals_dev, 
 }
 
 // ------------------------------------------------------------------------------------------
+// hole filling of the voxel surface and of device meshes (include/scan3d.h and common/scan3d_fill_math.h have the
+// exact rules)
+// ------------------------------------------------------------------------------------------
+// finds the holes of the mesh (the first synchronisation) into *st; the faces the holes can add into *most
+static int fill_count(scan3d_ctx* ctx, const float* xyz, const int32_t* faces, int64_t nv, int64_t nf,
+                      int32_t max_edges, FillState* st, int64_t* most)
+{
+    if (6 * nf >= (1LL << 32)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than (2^32 - 1) / 6 faces");
+    CK(ctx->fill.count(xyz, faces, (uint32_t)nv, (uint32_t)nf, (uint32_t)max_edges, ctx->stream, &ctx->launches));
+    CK(cudaMemcpyAsync(st, ctx->fill.state, sizeof(*st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st->bad) return fail(ctx, SCAN3D_ERR_ARG, "a coordinate that is not finite or a face index outside [0, n_vertices)");
+    if (st->cells64 >= (1ULL << 32)) return fail(ctx, SCAN3D_ERR_CONFIG, "the holes need 2^32 DP cells or more");
+    *most = (int64_t)st->loop_edges - 2 * (int64_t)st->holes;
+    if (nf + *most >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "the filled mesh could have 2^31 faces or more");
+    return SCAN3D_OK;
+}
+
+// triangulates the holes found by fill_count and writes the added faces to faces_out unless there are more than
+// capacity (the second synchronisation); fills *out
+static int fill_finish(scan3d_ctx* ctx, const FillState& counts, const float* xyz, const int32_t* faces, int64_t nv,
+                       int64_t nf, int32_t* faces_out, int64_t capacity, scan3d_fill_result* out)
+{
+    CK(ctx->fill.fill(counts, xyz, faces, (uint32_t)nv, faces_out, (uint64_t)capacity, ctx->stream, &ctx->launches));
+    FillState st;
+    CK(cudaMemcpyAsync(&st, ctx->fill.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    const bool fits = st.added <= (uint64_t)capacity;
+    out->vertices = nv;
+    out->faces = nf + (fits ? st.added : 0);
+    out->boundary_edges = st.boundary;
+    out->holes = st.holes;
+    out->filled = st.filled;
+    out->faces_added = st.added;
+    // a filled hole of n edges adds n - 2 faces and closes its n hole edges
+    out->open_edges = (int64_t)st.boundary - (fits ? (int64_t)st.added + 2 * (int64_t)st.filled : 0);
+    if (!fits) return fail(ctx, SCAN3D_ERR_CONFIG, "more added faces than max_faces_out: call again with faces_added");
+    return SCAN3D_OK;
+}
+
+int scan3d_voxel_surface_fill_holes(scan3d_ctx* ctx, int32_t max_edges, scan3d_fill_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (!ctx->results.has(SURFACE))
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    // an unrefined surface stays decimatable only with holes of at most SCAN3D_FILL_NETS_MAX_EDGES edges
+    const bool refined = ctx->results.has(SIMPLIFIED) || ctx->results.has(SMOOTHED);
+    const int32_t cap = refined ? SCAN3D_FILL_MAX_EDGES : SCAN3D_FILL_NETS_MAX_EDGES;
+    if (max_edges < 3 || max_edges > cap)
+        return fail(ctx, SCAN3D_ERR_ARG, refined ? "max_edges must be in [3, 1024]"
+                                                 : "max_edges must be in [3, 22] on a surface that is neither "
+                                                   "simplified nor smoothed");
+    CK(cudaSetDevice(ctx->device));
+    SurfaceMesh &s = ctx->surface, &spare = ctx->spare;
+    const int64_t nv = s.vertices, nf = s.faces;
+    ctx->results.drop(COMPONENTS);
+    FillState counts;
+    int64_t most = 0;
+    int rc = fill_count(ctx, s.xyz, s.tri, nv, nf, max_edges, &counts, &most);
+    if (rc) return rc;
+    // the held faces, then the added ones, into the spare face set, which becomes the held one
+    CK(spare.tri.ensure(3 * (size_t)std::max<int64_t>(nf + most, 1)));
+    if (nf) CK(cudaMemcpyAsync(spare.tri, s.tri, (size_t)nf * 12, cudaMemcpyDeviceToDevice, ctx->stream));
+    rc = fill_finish(ctx, counts, s.xyz, s.tri, nv, nf, spare.tri.get() + 3 * nf, most, out);
+    if (rc) return rc;
+    std::swap(s.tri, spare.tri);
+    s.faces = out->faces;
+    return SCAN3D_OK;
+}
+
+int scan3d_mesh_fill_holes_dev(scan3d_ctx* ctx, const float* xyz_dev, int64_t n_vertices, const int32_t* faces_dev,
+                               int64_t n_faces, int32_t max_edges, int32_t* faces_out_dev, int64_t max_faces_out,
+                               scan3d_fill_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (max_edges < 3 || max_edges > SCAN3D_FILL_MAX_EDGES) return fail(ctx, SCAN3D_ERR_ARG, "max_edges must be in [3, 1024]");
+    if (n_faces < 0 || n_faces >= (1LL << 31) || n_vertices < 0 || n_vertices >= (1LL << 31) || max_faces_out < 0 ||
+        max_faces_out >= (1LL << 31))
+        return fail(ctx, SCAN3D_ERR_ARG, "n_vertices, n_faces and max_faces_out must be in [0, 2^31)");
+    if ((!xyz_dev && n_vertices > 0) || (!faces_dev && n_faces > 0) || (!faces_out_dev && max_faces_out > 0))
+        return fail(ctx, SCAN3D_ERR_ARG, "null device pointer");
+    if (((uintptr_t)xyz_dev & 3) || ((uintptr_t)faces_dev & 3) || ((uintptr_t)faces_out_dev & 3))
+        return fail(ctx, SCAN3D_ERR_ARG, "xyz_dev, faces_dev and faces_out_dev must be 4-byte aligned");
+    CK(cudaSetDevice(ctx->device));
+    FillState counts;
+    int64_t most = 0;
+    const int rc = fill_count(ctx, xyz_dev, faces_dev, n_vertices, n_faces, max_edges, &counts, &most);
+    if (rc) return rc;
+    return fill_finish(ctx, counts, xyz_dev, faces_dev, n_vertices, n_faces, faces_out_dev, max_faces_out, out);
+}
+
+// ------------------------------------------------------------------------------------------
 // stage 1: projector patterns on the device
 // ------------------------------------------------------------------------------------------
 int64_t scan3d_pattern_bytes(const scan3d_config* c, int dir)

@@ -1,8 +1,9 @@
 // scan3d_hash.cuh -- the open-addressing hash of 63-bit keys (s3v::pack_key) shared by the voxel-grid merge
 // (scan3d_voxel_kernels.cu), the alignment's cell index (scan3d_align_kernels.cu) and the surface's lattice table
-// (scan3d_surface_kernels.cu): linear probing over a 64-bit key array whose free slots hold s3v::EMPTY_KEY.  The
-// callers size their tables so that at most half the slots are taken, which keeps probe sequences short and makes them
-// end.  Also the nearest-model-point search of the cell index, shared by the alignment and the surface.
+// (scan3d_surface_kernels.cu), and the undirected-edge tables of the smoothing and the hole filling (edge_key): linear
+// probing over a 64-bit key array whose free slots hold s3v::EMPTY_KEY.  The callers size their tables so that at most
+// half the slots are taken, which keeps probe sequences short and makes them end.  Also the nearest-model-point search
+// of the cell index, shared by the alignment and the surface.
 #pragma once
 #include "scan3d_internal.h"
 #include "../common/scan3d_align_math.h"
@@ -23,6 +24,12 @@ __device__ __forceinline__ unsigned long long mix64(unsigned long long x)
 __device__ __forceinline__ uint32_t hash_home(unsigned long long key, uint32_t cap)
 {
     return (uint32_t)(((mix64(key) >> 32) * (unsigned long long)cap) >> 32);
+}
+
+// the key of the undirected edge {a, b}: (min << 32) | max (the smoothing's and the hole filling's edge tables)
+__device__ __forceinline__ unsigned long long edge_key(uint32_t a, uint32_t b)
+{
+    return a < b ? (unsigned long long)a << 32 | b : (unsigned long long)b << 32 | a;
 }
 
 // The key's slot, inserting it if absent.  At most cap probes, so a full table cannot hang the caller.

@@ -13,6 +13,10 @@
 
 #define S3D_PLANE_MASK_H 10   // internal: valid_map_horizontal when the stage API is used
 
+namespace s3h {
+struct Cell;                  // common/scan3d_fill_math.h
+}
+
 namespace s3d {
 // tensor maps of the last few capture stacks (a map depends on the stack's address and the tile size only)
 struct TensorMapCache {
@@ -257,6 +261,50 @@ struct SmoothWorkspace {
     cudaError_t run(const float* xyz, const float* nrm, const int32_t* faces, uint32_t n, uint32_t nf, int passes,
                     double lambda, double mu, float* xyz_out, float* nrm_out, cudaStream_t st, int64_t* launches);
 };
+
+// the hole filling (scan3d_fill_kernels.cu; common/scan3d_fill_math.h has the arithmetic); the undirected edges are
+// the smoothing's table of (min << 32 | max) keys
+struct FillState {
+    unsigned long long cells64;    // the DP cells of every hole, exact (the scan's 32-bit total may wrap)
+    uint32_t bad;                  // a coordinate not finite or a face index outside [0, vertices): SCAN3D_ERR_ARG
+    uint32_t boundary;             // hole edges (edges of count 1)
+    uint32_t holes, loop_edges, cells;   // the scans' totals: holes, their edges, their DP cells
+    uint32_t filled, added;        // holes filled, faces added (a scan total)
+    uint32_t pad;
+};
+struct FillBuffers;
+struct FillHole {
+    uint32_t v0, n;                // smallest vertex, edges
+    uint32_t vert;                 // first of its vertices (and stack entries)
+    uint32_t cell;                 // first of its DP cells
+};
+struct FillWorkspace {
+    DeviceBuffer<unsigned long long> keys;  // [6 faces] the edge table
+    DeviceBuffer<uint32_t> sides, face;     // [6 faces] sides per edge; the face of a side on it
+    DeviceBuffer<uint32_t> out_n, in_n;     // [vertices] hole edges leaving / entering the vertex
+    DeviceBuffer<uint32_t> next, rim;       // [vertices] head and rim face of the hole edge leaving the vertex
+    DeviceBuffer<uint32_t> len;             // [vertices] edges of the hole whose smallest vertex this is, else 0
+    DeviceBuffer<uint32_t> block_counts;    // [3][cdiv(vertices, POINT_BLOCK) + 1] holes, edges and cells per block
+    DeviceBuffer<FillHole> holes;           // [holes]
+    DeviceBuffer<uint32_t> hole_faces;      // [holes] faces the hole adds
+    DeviceBuffer<uint32_t> face_counts;     // [cdiv(holes, POINT_BLOCK) + 1] faces added per block of holes
+    DeviceBuffer<uint32_t> verts, stack;    // [loop edges] the holes' vertices; the emission's stacks
+    DeviceBuffer<s3h::Cell> cells;          // [cells]
+    DeviceBuffer<FillState> state;
+    uint32_t table = 0, stride = 0;         // the edge table's slots and block_counts' stride of the last count
+    FillBuffers view();
+    // 6 launches for n vertices and nf faces [nf][3], nf < 2^32 / 6, holes of at most max_edges edges: the sides into
+    // the edge table (with the face-index check), the hole edges per edge of count 1, the walk per vertex (with the
+    // finiteness check) that flags each hole's smallest vertex with the per-block sums, and k_scan over the holes, their
+    // edges and their cells; state->bad, boundary, holes, loop_edges and cells64 are then known
+    cudaError_t count(const float* xyz, const int32_t* faces, uint32_t n, uint32_t nf, uint32_t max_edges,
+                      cudaStream_t st, int64_t* launches);
+    // 4 launches after count and a synchronisation that read st: the holes and their vertices, the DP (one block per
+    // hole), k_scan over the faces added per block of holes (state->added), and the emission of the added faces into
+    // out, which writes nothing when state->added > capacity
+    cudaError_t fill(const FillState& counts, const float* xyz, const int32_t* faces, uint32_t n, int32_t* out,
+                     uint64_t capacity, cudaStream_t st, int64_t* launches);
+};
 }  // namespace s3d
 
 // Every device buffer the context owns is a DeviceBuffer: scan3d_destroy frees them all by deleting the context.
@@ -344,8 +392,9 @@ struct scan3d_ctx {
     s3d::ComponentsWorkspace cc;          // scan3d_voxel_surface_components, scan3d_mesh_components_dev
     s3d::DecimateWorkspace dec;           // scan3d_voxel_surface_decimate
     s3d::SmoothWorkspace smooth;          // scan3d_voxel_surface_smooth, scan3d_mesh_smooth_dev
+    s3d::FillWorkspace fill;              // scan3d_voxel_surface_fill_holes, scan3d_mesh_fill_holes_dev
 
-    // the held voxel surface, and the spare set that components, decimate and smooth write before they swap it in
+    // the held voxel surface, and the spare set that components, decimate, smooth and fill write before they swap it in
     s3d::SurfaceMesh surface, spare;
     int64_t cc_components = 0;
 

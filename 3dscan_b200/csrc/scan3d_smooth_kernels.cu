@@ -41,11 +41,6 @@ static_assert(POINT_BLOCK == 1024, "the row starts scan one degree per thread of
 
 unsigned grid(uint64_t n, int threads) { return n ? (unsigned)((n + threads - 1) / threads) : 1u; }
 
-__device__ __forceinline__ unsigned long long edge_key(uint32_t a, uint32_t b)
-{
-    return a < b ? (unsigned long long)a << 32 | b : (unsigned long long)b << 32 | a;
-}
-
 // the lanes of the warp whose v is the same take consecutive values of counter[v] (v == VOXEL_NO_SLOT: none); returns
 // this lane's.  Every lane of the warp calls it.
 __device__ __forceinline__ uint32_t take_per_warp(uint32_t* counter, uint32_t v)

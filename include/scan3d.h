@@ -631,6 +631,83 @@ int scan3d_mesh_smooth_dev(scan3d_ctx *ctx, float *xyz_dev, float *normals_dev, 
                            const int32_t *faces_dev, int64_t n_faces, const scan3d_smooth_params *p,
                            scan3d_smooth_result *out);
 
+/* ---- hole filling of the voxel surface and of device meshes: minimum-weight triangulation of boundary loops with
+ * Liepa's weight (Liepa 2003; Klincsek 1980; Barequet & Sharir 1995) ------------------------------------------------
+ * The result is a pure function of the mesh and max_edges: bit-reproducible, independent of scheduling, of the hash and
+ * of the SM count.  The exact operation order is in 3dscan_b200/common/scan3d_fill_math.h.
+ *
+ * Hole edges: each face (a, b, c) contributes its sides (a, b), (b, c), (c, a); a side with equal ends is skipped.  An
+ * undirected edge whose side count is 1 is a boundary edge; its hole edge is the reversed side b -> a, and its rim
+ * face is the one face that holds it.  A vertex is regular when exactly one hole edge leaves it and exactly one enters
+ * it.  The successor of a hole edge is the hole edge that leaves its head.
+ * Holes: a hole is a cycle of n hole edges, 3 <= n <= max_edges, through regular vertices only; v_0 is its smallest
+ * vertex index, v_{t+1} the head of the hole edge that leaves v_t, F_t the rim face of hole edge t (v_t -> v_{t+1}).
+ * Every loop of at most max_edges edges is a hole, the rim of a small open piece included.  Two kinds of boundary stay
+ * open and count in open_edges: chains through vertices that are not regular (non-manifold boundary, two holes sharing
+ * a vertex), and loops longer than max_edges.
+ * Triangle terms, in double from the float coordinates, each operation correctly rounded: cross = (p_b - p_a) x (p_c -
+ * p_a), l2 = (cx cx + cy cy) + cz cz, area = sqrt(l2) * 0.5, unit normal u = cross / sqrt(l2) when l2 > 0 (else none);
+ * cos(T1, T2) = (u1x u2x + u1y u2y) + u1z u2z, and -1 when either has no normal.
+ * Triangulation: for 0 <= i < j <= n - 1, cell (i, j) is the best triangulation of v_i ... v_j closed by v_j -> v_i.
+ * j - i = 1 is hole edge i: feasible with weight (+inf, 0) and the normal of F_i.  A cell with j - i >= 2 is infeasible
+ * when (i, j) != (0, n - 1) and {v_i, v_j} is already an edge of the mesh (so the output stays edge-manifold), or when
+ * it has no feasible candidate.  Candidates k = i + 1 ... j - 1 with both cells (i, k) and (k, j) feasible give T_k =
+ * (v_i, v_k, v_j), c_k = min(cos(T_k, N(i, k)), cos(T_k, N(k, j))) with N the triangle chosen for a cell (F_a for a hole
+ * edge), and for cell (0, n - 1) also min with cos(T_k, F_{n-1}); cmin = min(cmin(i, k), cmin(k, j), c_k), area =
+ * (area(i, k) + area(k, j)) + area(T_k).  The larger cmin wins, then the smaller area, then the smaller k.  When cell
+ * (0, n - 1) is infeasible the hole is unfillable and stays open.
+ * Output: a filled hole gets n - 2 faces (v_i, v_k, v_j) in preorder from cell (0, n - 1) (the cell's face, then cell
+ * (i, k), then cell (k, j)), wound like the rim faces, so a flat continuation has cos = +1.  Holes are emitted in
+ * ascending v_0, after the existing faces; vertices, their bytes and the existing faces do not change.  The patch has
+ * no interior vertices (Liepa's refinement and fairing are not done).
+ *
+ * scan3d_voxel_surface_fill_holes fills the held voxel surface in place: scan3d_get_voxel_surface,
+ * scan3d_write_voxel_surface_ply, components, smoothing and decimation then see the filled surface.  It needs a held
+ * surface (SCAN3D_ERR_STATE otherwise), makes the component table stale and changes no other state: a filled surface
+ * that was neither simplified nor smoothed can still be simplified.  For that, max_edges is capped at
+ * SCAN3D_FILL_NETS_MAX_EDGES on such a surface (the decimation's quadric bound, extended to the fill faces of holes of
+ * at most 22 surface-nets edges, is derived in the math header); on a simplified or smoothed surface, which decimation
+ * refuses anyway, the cap is SCAN3D_FILL_MAX_EDGES.  Recommended order: extract, components, then smooth or decimate,
+ * then fill; small pinholes can be filled right after extraction.  Smoothing after a fill is allowed, but a rim vertex
+ * is then free and its umbrella reaches across the patch, which has no interior vertices.  A second fill adds nothing
+ * unless max_edges grows.  A later begin, add or finish makes the surface stale as before.
+ * scan3d_mesh_fill_holes_dev fills any triangle mesh in device memory of the ctx's GPU (xyz_dev float [n_vertices][3],
+ * faces_dev int32 [n_faces][3]), capped at SCAN3D_FILL_MAX_EDGES: it writes only the added faces, int32 [faces_added][3],
+ * to faces_out_dev, ordered on the ctx stream, and leaves the mesh, the held surface and the component table alone.
+ * When more than max_faces_out faces are needed it writes nothing and returns SCAN3D_ERR_CONFIG with *out filled
+ * (faces_added the faces needed, faces = n_faces, open_edges = boundary_edges).  The ctx's camera-grid mesh
+ * (scan3d_device_points, scan3d_device_mesh_faces) is a valid input.
+ * Synchronisation: two per call: once the holes are known (to size the scratch and, in the surface route, the spare
+ * face set, into which the held faces are copied), and once after every launch.
+ * Launches: 10, an empty mesh included: the sides into the edge table, the hole edges, the loop walks with the per-block
+ * sums, k_scan over the holes, their edges and their DP cells; after the first synchronisation the holes and their
+ * vertices, the DP (one block per hole), k_scan over the faces added, and the emission.  6 when the first
+ * synchronisation finds an error.
+ * Memory (ctx-owned, allocated on first use, grown on demand): 20 B per vertex, 96 B per face (the edge table of 6 slots
+ * of 16 B), 8 B per hole edge of a hole, 20 B per hole, and 48 B per DP cell, n (n - 1) / 2 + 1 per hole of n edges
+ * (25 MB for a hole of 1024); the surface route also grows the spare face set to 12 B per face after the fill.
+ * Errors: SCAN3D_ERR_ARG for a null ctx or out; max_edges outside [3, cap]; in scan3d_mesh_fill_holes_dev n_vertices,
+ * n_faces or max_faces_out outside [0, 2^31), a NULL xyz_dev, faces_dev or faces_out_dev with a non-zero count, a pointer
+ * not 4-byte aligned, and, found on the device, a face index outside [0, n_vertices) or a coordinate that is not
+ * finite.  SCAN3D_ERR_CONFIG when 6 n_faces >= 2^32, when n_faces plus the n - 2 faces of every hole reaches 2^31, or
+ * when the holes' DP cells reach 2^32.
+ * An argument or state error launches nothing; on any error nothing is written and the held surface is unchanged. */
+#define SCAN3D_FILL_NETS_MAX_EDGES 22
+#define SCAN3D_FILL_MAX_EDGES 1024
+typedef struct {
+    int64_t vertices, faces;     /* of the mesh after the call */
+    int64_t boundary_edges;      /* hole edges before the call */
+    int64_t holes;               /* loops of 3 to max_edges edges through regular vertices */
+    int64_t filled;              /* holes closed; the others were unfillable */
+    int64_t faces_added;
+    int64_t open_edges;          /* hole edges after the call */
+} scan3d_fill_result;
+
+int scan3d_voxel_surface_fill_holes(scan3d_ctx *ctx, int32_t max_edges, scan3d_fill_result *out);
+int scan3d_mesh_fill_holes_dev(scan3d_ctx *ctx, const float *xyz_dev, int64_t n_vertices, const int32_t *faces_dev,
+                               int64_t n_faces, int32_t max_edges, int32_t *faces_out_dev, int64_t max_faces_out,
+                               scan3d_fill_result *out);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,
