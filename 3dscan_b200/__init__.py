@@ -125,6 +125,17 @@ FILL_NETS_MAX_EDGES = 22
 FILL_MAX_EDGES = 1024
 
 
+class RepairResultC(C.Structure):
+    _fields_ = [(name, C.c_int64) for name in (
+        "vertices", "faces", "degenerate_faces", "duplicate_faces", "nonmanifold_edges", "nonmanifold_faces",
+        "split_vertices", "vertices_added", "boundary_edges", "inconsistent_edges")]
+
+
+# the steps of scan3d_voxel_surface_repair and scan3d_mesh_repair_dev (include/scan3d.h)
+REPAIR_FACES = 1
+REPAIR_VERTICES = 2
+
+
 # voxel_surface's default max_points per merged voxel: the smallest power of two >= 1.5x the largest lattice points
 # per voxel measured on tools/bench_surface.py's workloads (29.2 on workload A, profiles/r3_bench_surface.json).  64 is
 # also the most a voxel can add (the 4 x 4 x 4 corners of its 27 cells), so the default never overflows; pass
@@ -262,6 +273,8 @@ def cuda_lib():
     L.scan3d_mesh_smooth_dev.argtypes = [vp, vp, vp, i64, vp, i64, C.POINTER(SmoothParams), C.POINTER(SmoothResultC)]
     L.scan3d_voxel_surface_fill_holes.argtypes = [vp, i32, C.POINTER(FillResultC)]
     L.scan3d_mesh_fill_holes_dev.argtypes = [vp, vp, i64, vp, i64, i32, vp, i64, C.POINTER(FillResultC)]
+    L.scan3d_voxel_surface_repair.argtypes = [vp, i32, C.POINTER(RepairResultC)]
+    L.scan3d_mesh_repair_dev.argtypes = [vp, vp, i64, vp, i64, i32, vp, vp, i64, C.POINTER(RepairResultC)]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -836,6 +849,54 @@ class Scan3D:
                 continue
             self._ck(rc)
             return out[:r.faces_added], self._fill_result(r)
+
+    # -- repair of non-manifold edges and vertices of the voxel surface and of device meshes (include/scan3d.h has the
+    # exact rules)
+    @staticmethod
+    def _repair_result(r):
+        return {name: getattr(r, name) for name, _ in RepairResultC._fields_}
+
+    @staticmethod
+    def _repair_flags(faces, vertices):
+        return (REPAIR_FACES if faces else 0) | (REPAIR_VERTICES if vertices else 0)
+
+    def surface_repair(self, faces=True, vertices=True):
+        """Repair, in place, the non-manifold edges (faces=True: duplicate faces and the extra faces of edges in more
+        than two, by area) and the non-manifold vertices (vertices=True: one new vertex per extra fan) of the held
+        voxel surface; degenerate faces always go.  Synchronises twice and returns a dict with the fields of
+        scan3d_repair_result.  voxel_surface_mesh() then returns the repaired surface; the component table goes
+        stale."""
+        r = RepairResultC()
+        self._ck(self.L.scan3d_voxel_surface_repair(self.h, self._repair_flags(faces, vertices), C.byref(r)))
+        self._surface_counts = (r.vertices, r.faces)
+        self._components = 0
+        return self._repair_result(r)
+
+    def mesh_repair_dev(self, xyz, faces, repair_faces=True, vertices=True):
+        """surface_repair() for a triangle mesh on the ctx's GPU (repair_faces is surface_repair's faces): xyz a CUDA
+        float32 tensor [v][3], faces a CUDA int32 tensor [f][3]; neither is changed.  torch's current stream is
+        synchronised first, so data written there is ready.  Returns (the repaired faces, a new CUDA int32 tensor
+        [faces][3]; the source vertex of each added vertex, a new CUDA int32 tensor [vertices_added], for extending
+        attribute arrays with a gather; the dict of surface_repair())."""
+        import torch
+
+        def ok(t, dtype):
+            return (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dtype and t.dim() == 2 and
+                    t.shape[1] == 3 and t.is_contiguous())
+        if not ok(xyz, torch.float32):
+            raise Scan3DError("xyz must be a contiguous CUDA float32 tensor of shape [v][3]")
+        if not ok(faces, torch.int32):
+            raise Scan3DError("faces must be a contiguous CUDA int32 tensor of shape [f][3]")
+        torch.cuda.current_stream(xyz.device).synchronize()
+        nf = faces.shape[0]
+        out = torch.empty((max(nf, 1), 3), dtype=torch.int32, device=xyz.device)
+        src = torch.empty(max(3 * nf, 1), dtype=torch.int32, device=xyz.device)   # a new vertex per corner at most
+        r = RepairResultC()
+        self._ck(self.L.scan3d_mesh_repair_dev(self.h, C.c_void_p(xyz.data_ptr()), xyz.shape[0],
+                                               C.c_void_p(faces.data_ptr()), nf,
+                                               self._repair_flags(repair_faces, vertices), C.c_void_p(out.data_ptr()),
+                                               C.c_void_p(src.data_ptr()), 3 * nf, C.byref(r)))
+        return out[:r.faces], src[:r.vertices_added], self._repair_result(r)
 
     # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
     @staticmethod

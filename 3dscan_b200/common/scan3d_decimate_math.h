@@ -34,6 +34,9 @@
 // its own cell (up to the float rounding of its coordinate), so a cluster holds the vertices of at most
 // floor(r) + 3 cells per axis.  Each cluster sum is therefore at most sum_bound(r) = (floor(r) + 3)^3 * 24 *
 // face_bound(r) in magnitude; with P = 40 and r in [1, 256] that is below 2^56.3 (r = 256), under 2^63.
+// The bound is per lattice cell, so it survives the non-manifold repair (scan3d_voxel_surface_repair): a split only
+// divides a cell's faces among copies at the same position, in the same cell, and dropped faces only lower the count,
+// so a repaired raw surface stays decimatable (common/scan3d_repair_math.h).
 #pragma once
 #include "scan3d_aux_math.h"
 #include "scan3d_voxel_math.h"

@@ -1246,6 +1246,7 @@ int scan3d_voxel_surface(scan3d_ctx* ctx, const scan3d_surface_params* p, scan3d
         return fail(ctx, SCAN3D_ERR_STATE, "no voxel outputs of the current adds to mesh: call scan3d_voxel_finish");
     CK(cudaSetDevice(ctx->device));
     ctx->results.drop(SURFACE);
+    ctx->srf_repaired = ctx->srf_filled_after_repair = false;
     AlignRun run{};                                      // the index only; T0 = I for the state it initialises
     run.T0[0] = run.T0[5] = run.T0[10] = 1.0;
     run.S = s3l::cell_edge(p->max_distance);
@@ -1403,6 +1404,9 @@ int scan3d_voxel_surface_decimate(scan3d_ctx* ctx, float cell_size, scan3d_decim
         return fail(ctx, SCAN3D_ERR_STATE, "the held surface is already simplified: extract it again first");
     if (ctx->results.has(SMOOTHED))
         return fail(ctx, SCAN3D_ERR_STATE, "the held surface is smoothed: extract it again to simplify it");
+    if (ctx->srf_filled_after_repair)
+        return fail(ctx, SCAN3D_ERR_STATE, "the held surface was filled after a repair changed it: extract it again to "
+                                           "simplify it");
     const int64_t nv = ctx->surface.vertices, nf = ctx->surface.faces;
     if (nf >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than 2^31 - 1 surface faces");
     CK(cudaSetDevice(ctx->device));
@@ -1573,6 +1577,7 @@ int scan3d_voxel_surface_fill_holes(scan3d_ctx* ctx, int32_t max_edges, scan3d_f
     if (rc) return rc;
     std::swap(s.tri, spare.tri);
     s.faces = out->faces;
+    if (out->faces_added && ctx->srf_repaired) ctx->srf_filled_after_repair = true;
     return SCAN3D_OK;
 }
 
@@ -1596,6 +1601,103 @@ int scan3d_mesh_fill_holes_dev(scan3d_ctx* ctx, const float* xyz_dev, int64_t n_
     const int rc = fill_count(ctx, xyz_dev, faces_dev, n_vertices, n_faces, max_edges, &counts, &most);
     if (rc) return rc;
     return fill_finish(ctx, counts, xyz_dev, faces_dev, n_vertices, n_faces, faces_out_dev, max_faces_out, out);
+}
+
+// ------------------------------------------------------------------------------------------
+// repair of the non-manifold edges and vertices of the voxel surface and of device meshes (include/scan3d.h and
+// common/scan3d_repair_math.h have the exact rules)
+// ------------------------------------------------------------------------------------------
+static int check_repair_flags(scan3d_ctx* ctx, int32_t flags, scan3d_repair_result* out)
+{
+    if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (flags <= 0 || (flags & ~(SCAN3D_REPAIR_FACES | SCAN3D_REPAIR_VERTICES)))
+        return fail(ctx, SCAN3D_ERR_ARG, "flags must be a non-empty combination of SCAN3D_REPAIR_FACES and "
+                                         "SCAN3D_REPAIR_VERTICES");
+    return SCAN3D_OK;
+}
+
+// finds the drops and the fans of the mesh (the first synchronisation) and fills *out
+static int repair_count(scan3d_ctx* ctx, const float* xyz, const int32_t* faces, int64_t nv, int64_t nf, int32_t flags,
+                        scan3d_repair_result* out)
+{
+    if (3 * nf >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "3 n_faces must be below 2^31");
+    CK(ctx->repair.count(xyz, faces, (uint32_t)nv, (uint32_t)nf, flags, ctx->stream, &ctx->launches));
+    RepairState st;
+    CK(cudaMemcpyAsync(&st, ctx->repair.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st.bad) return fail(ctx, SCAN3D_ERR_ARG, "a coordinate that is not finite or a face index outside [0, n_vertices)");
+    out->vertices = nv + st.added;
+    out->faces = st.faces;
+    out->degenerate_faces = st.degenerate;
+    out->duplicate_faces = st.duplicate;
+    out->nonmanifold_edges = st.nonmanifold_edges;
+    out->nonmanifold_faces = st.nonmanifold_faces;
+    out->split_vertices = st.split;
+    out->vertices_added = st.added;
+    out->boundary_edges = st.boundary;
+    out->inconsistent_edges = st.inconsistent;
+    if (out->vertices >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_CONFIG, "the repaired mesh would have 2^31 vertices or more");
+    return SCAN3D_OK;
+}
+
+int scan3d_voxel_surface_repair(scan3d_ctx* ctx, int32_t flags, scan3d_repair_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    int rc = check_repair_flags(ctx, flags, out);
+    if (rc) return rc;
+    if (!ctx->results.has(SURFACE))
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    CK(cudaSetDevice(ctx->device));
+    SurfaceMesh &s = ctx->surface, &spare = ctx->spare;
+    const int64_t nv = s.vertices, nf = s.faces;
+    ctx->results.drop(COMPONENTS);
+    rc = repair_count(ctx, s.xyz, s.tri, nv, nf, flags, out);
+    if (rc) return rc;
+    // the held vertices, the copies after them and the kept faces into the spare set, which becomes the held one
+    const int64_t added = out->vertices_added;
+    CK(spare.grow(std::max<int64_t>(nv + added, 1), std::max<int64_t>(out->faces, 1)));
+    CK(ctx->repair.source.ensure(std::max<int64_t>(added, 1)));
+    if (nv) {
+        CK(cudaMemcpyAsync(spare.xyz, s.xyz, (size_t)nv * 12, cudaMemcpyDeviceToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(spare.nrm, s.nrm, (size_t)nv * 12, cudaMemcpyDeviceToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(spare.rgb, s.rgb, (size_t)nv * 3, cudaMemcpyDeviceToDevice, ctx->stream));
+    }
+    CK(ctx->repair.emit(s.tri, (uint32_t)nv, (uint32_t)nf, flags, spare.tri, ctx->repair.source, s.xyz,
+                        s.nrm, s.rgb, spare.xyz, spare.nrm, spare.rgb, ctx->stream, &ctx->launches));
+    CK(cudaStreamSynchronize(ctx->stream));
+    std::swap(s, spare);
+    s.vertices = out->vertices;
+    s.faces = out->faces;
+    if (out->faces < nf || added) ctx->srf_repaired = true;
+    return SCAN3D_OK;
+}
+
+int scan3d_mesh_repair_dev(scan3d_ctx* ctx, const float* xyz_dev, int64_t n_vertices, const int32_t* faces_dev,
+                           int64_t n_faces, int32_t flags, int32_t* faces_out_dev, int32_t* source_out_dev,
+                           int64_t max_source_out, scan3d_repair_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    int rc = check_repair_flags(ctx, flags, out);
+    if (rc) return rc;
+    if (n_faces < 0 || n_faces >= (1LL << 31) || n_vertices < 0 || n_vertices >= (1LL << 31) || max_source_out < 0 ||
+        max_source_out >= (1LL << 31))
+        return fail(ctx, SCAN3D_ERR_ARG, "n_vertices, n_faces and max_source_out must be in [0, 2^31)");
+    if ((!xyz_dev && n_vertices > 0) || (!faces_dev && n_faces > 0) || (!faces_out_dev && n_faces > 0) ||
+        (!source_out_dev && max_source_out > 0))
+        return fail(ctx, SCAN3D_ERR_ARG, "null device pointer");
+    if (((uintptr_t)xyz_dev & 3) || ((uintptr_t)faces_dev & 3) || ((uintptr_t)faces_out_dev & 3) ||
+        ((uintptr_t)source_out_dev & 3))
+        return fail(ctx, SCAN3D_ERR_ARG, "xyz_dev, faces_dev, faces_out_dev and source_out_dev must be 4-byte aligned");
+    if (faces_out_dev && faces_out_dev == faces_dev) return fail(ctx, SCAN3D_ERR_ARG, "faces_out_dev must not be faces_dev");
+    CK(cudaSetDevice(ctx->device));
+    rc = repair_count(ctx, xyz_dev, faces_dev, n_vertices, n_faces, flags, out);
+    if (rc) return rc;
+    if (out->vertices_added > max_source_out)
+        return fail(ctx, SCAN3D_ERR_CONFIG, "more added vertices than max_source_out: call again with vertices_added");
+    CK(ctx->repair.emit(faces_dev, (uint32_t)n_vertices, (uint32_t)n_faces, flags, faces_out_dev, source_out_dev,
+                        nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, ctx->stream, &ctx->launches));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return SCAN3D_OK;
 }
 
 // ------------------------------------------------------------------------------------------

@@ -1,21 +1,16 @@
 // scan3d_components_kernels.cu -- connected components of a triangle mesh (scan3d_voxel_surface_components,
 // scan3d_mesh_components_dev) and the compaction of the held voxel surface to its kept components.
 //
-// Labels: a lock-free union-find over the vertices (ECL-CC, Jaiganesh & Burtscher, HPDC 2018).  Every face unites its
-// first vertex with the other two; a union links the larger of the two roots under the smaller with atomicCAS and
-// retries from the new roots when another thread linked first.  parent[x] <= x always holds, so each root is the
-// smallest vertex of its component whatever the interleaving, and the flags "v is a root" ranked by k_count + k_scan
-// give the ids (rank of the smallest vertex).  The unions' finds use path halving: a non-root's parent only ever moves
-// to another of its ancestors, and a CAS only ever targets a root, so the halving stores never race with a link.
-// parent is read with relaxed atomic loads, so a thread always sees the links other threads made.
+// Labels: the lock-free union-find of scan3d_union_find.cuh (ECL-CC) over the vertices.  Every face unites its first
+// vertex with the other two.  Each root is the smallest vertex of its component whatever the interleaving, and the
+// flags "v is a root" ranked by k_count + k_scan give the ids (rank of the smallest vertex).
 //
 // Selection: one block finds the threshold key K of the keep rule by a radix select over key(c) = faces << 32 |
 // (2^32 - 1 - c), which orders the components by faces descending and then by id ascending with no two keys equal.
 // The kept components are the eligible ones (faces >= min_faces) with key >= K.  Counts are integer atomics and the
 // selection works on integers only, so every output is a pure function of the mesh.
 #include "scan3d_internal.h"
-
-#include <cuda/atomic>
+#include "scan3d_union_find.cuh"
 
 namespace s3d {
 
@@ -25,46 +20,6 @@ constexpr int CT = 256;                                 // threads per block of 
 constexpr int SELECT_THREADS = 1024;
 constexpr unsigned FULL = 0xffffffffu;
 static_assert(POINT_BLOCK == 1024, "the emission kernels rank one flag per thread of a POINT_BLOCK block");
-
-__device__ __forceinline__ uint32_t load_parent(uint32_t* parent, uint32_t x)
-{
-    return cuda::atomic_ref<uint32_t, cuda::thread_scope_device>(parent[x]).load(cuda::memory_order_relaxed);
-}
-
-__device__ __forceinline__ void store_parent(uint32_t* parent, uint32_t x, uint32_t p)
-{
-    cuda::atomic_ref<uint32_t, cuda::thread_scope_device>(parent[x]).store(p, cuda::memory_order_relaxed);
-}
-
-// the root of x, halving the path on the way
-__device__ __forceinline__ uint32_t find(uint32_t* parent, uint32_t x)
-{
-    for (;;) {
-        const uint32_t p = load_parent(parent, x);
-        if (p == x) return x;
-        const uint32_t g = load_parent(parent, p);
-        if (g == p) return p;
-        store_parent(parent, x, g);
-        x = g;
-    }
-}
-
-__device__ __forceinline__ void unite(uint32_t* parent, uint32_t a, uint32_t b)
-{
-    a = find(parent, a);
-    b = find(parent, b);
-    while (a != b) {
-        if (a > b) {
-            const uint32_t t = a;
-            a = b;
-            b = t;
-        }
-        const uint32_t old = atomicCAS(&parent[b], b, a);
-        if (old == b) return;
-        a = find(parent, a);
-        b = find(parent, old);
-    }
-}
 
 __device__ __forceinline__ unsigned long long key_of(uint32_t faces, uint32_t c)
 {

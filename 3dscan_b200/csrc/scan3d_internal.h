@@ -305,6 +305,53 @@ struct FillWorkspace {
     cudaError_t fill(const FillState& counts, const float* xyz, const int32_t* faces, uint32_t n, int32_t* out,
                      uint64_t capacity, cudaStream_t st, int64_t* launches);
 };
+
+// the non-manifold repair (scan3d_repair_kernels.cu; common/scan3d_repair_math.h has the face key and the edge rule);
+// the undirected edges are the smoothing's table of (min << 32 | max) keys, the fans a union-find over face corners
+struct RepairState {
+    uint32_t bad;                  // a coordinate not finite or a face index outside [0, vertices): SCAN3D_ERR_ARG
+    uint32_t degenerate, duplicate;
+    uint32_t nonmanifold_edges, nonmanifold_faces;
+    uint32_t split;                // vertices with more than one fan
+    uint32_t added, faces;         // the scans' totals: new vertices, kept faces
+    uint32_t boundary, inconsistent;
+};
+struct RepairBuffers;
+struct RepairWorkspace {
+    DeviceBuffer<unsigned long long> keys;  // [6 faces] the edge table
+    DeviceBuffer<uint32_t> sides, kept_n;   // [6 faces] faces on each edge after steps 1-2; kept faces on it
+    DeviceBuffer<unsigned long long> best;  // [6 faces][3] largest face key per direction, largest other than f1
+    DeviceBuffer<uint32_t> pair;            // [6 faces][2] the kept faces of an edge with at most 2 of them
+    DeviceBuffer<uint32_t> triples;         // [2 faces] the duplicate table: face indices, VOXEL_NO_SLOT = free
+    DeviceBuffer<uint32_t> triple_slot;     // [faces] table slot of each face
+    DeviceBuffer<unsigned long long> key;   // [faces] K(f)
+    DeviceBuffer<uint32_t> side_slot;       // [faces][3] edge-table slot of each side
+    DeviceBuffer<uint8_t> status;           // [faces] 1 = survives steps 1-2
+    DeviceBuffer<uint8_t> keep;             // [faces] kept
+    DeviceBuffer<uint32_t> face_counts;     // [cdiv(faces, POINT_BLOCK) + 1]
+    DeviceBuffer<uint32_t> parent;          // [3 faces] union-find over corners, then each corner's root
+    DeviceBuffer<uint8_t> fresh;            // [3 faces] the corner is the smallest of a fan that gets a new vertex
+    DeviceBuffer<uint32_t> corner_counts;   // [cdiv(3 faces, POINT_BLOCK) + 1]
+    DeviceBuffer<uint32_t> new_id;          // [3 faces] the new vertex of a fan, at its smallest corner
+    DeviceBuffer<uint32_t> first, fans;     // [vertices] smallest kept corner; new fans
+    DeviceBuffer<int32_t> source;           // [added] the surface route's source vertices
+    DeviceBuffer<RepairState> state;
+    uint32_t table = 0, dup_table = 0;      // slots of the edge and duplicate tables of the last count
+    RepairBuffers view();
+    // 10 launches for n vertices and nf faces [nf][3], 3 nf < 2^31, flags SCAN3D_REPAIR_*: the finiteness check, the
+    // face-index check, the degenerate faces and the duplicate table; the surviving faces' keys and sides into the
+    // edge table; the largest key other than f1 per edge; the drop flags with the kept faces' sides and smallest
+    // corners; per edge the counts and the unions of the corners; the roots with the fresh flags; k_count + k_scan over
+    // the fresh flags (state->added) and over the keep flags (state->faces).  Every count of state is then known.
+    cudaError_t count(const float* xyz, const int32_t* faces, uint32_t n, uint32_t nf, int flags, cudaStream_t st,
+                      int64_t* launches);
+    // 2 launches after count and a synchronisation that read st: the new vertices (their sources into source_out and,
+    // when xyz_out is set, their xyz, normal and rgb bytes after the first n vertices of out), then the kept faces,
+    // remapped, into faces_out
+    cudaError_t emit(const int32_t* faces, uint32_t n, uint32_t nf, int flags, int32_t* faces_out, int32_t* source_out,
+                     const float* xyz, const float* nrm, const uint8_t* rgb, float* xyz_out, float* nrm_out,
+                     uint8_t* rgb_out, cudaStream_t st, int64_t* launches);
+};
 }  // namespace s3d
 
 // Every device buffer the context owns is a DeviceBuffer: scan3d_destroy frees them all by deleting the context.
@@ -393,10 +440,16 @@ struct scan3d_ctx {
     s3d::DecimateWorkspace dec;           // scan3d_voxel_surface_decimate
     s3d::SmoothWorkspace smooth;          // scan3d_voxel_surface_smooth, scan3d_mesh_smooth_dev
     s3d::FillWorkspace fill;              // scan3d_voxel_surface_fill_holes, scan3d_mesh_fill_holes_dev
+    s3d::RepairWorkspace repair;          // scan3d_voxel_surface_repair, scan3d_mesh_repair_dev
 
-    // the held voxel surface, and the spare set that components, decimate, smooth and fill write before they swap it in
+    // the held voxel surface, and the spare set that components, decimate, smooth, fill and repair write before they
+    // swap it in
     s3d::SurfaceMesh surface, spare;
     int64_t cc_components = 0;
+    // since the held surface was extracted: a repair dropped faces or split vertices; a fill added faces after that.
+    // The decimation's quadric bound needs one hole per cell, which holds unless both happened
+    // (common/scan3d_repair_math.h).
+    bool srf_repaired = false, srf_filled_after_repair = false;
 
     int cta_limit = 0;             // scan3d_set_cta_limit
 

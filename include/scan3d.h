@@ -708,6 +708,91 @@ int scan3d_mesh_fill_holes_dev(scan3d_ctx *ctx, const float *xyz_dev, int64_t n_
                                int64_t n_faces, int32_t max_edges, int32_t *faces_out_dev, int64_t max_faces_out,
                                scan3d_fill_result *out);
 
+/* ---- repair of the non-manifold edges and vertices of the voxel surface and of device meshes: MeshLab's "Repair non
+ * Manifold Edges" and "Repair non Manifold Vertices by splitting" (vcglib tri::Clean; Gueziec, Taubin, Lazarus & Horn
+ * 2001) ------------------------------------------------------------------------------------------------------------
+ * The result is a pure function of the mesh and the flags: bit-reproducible, independent of scheduling, of the hash and
+ * of the SM count.  The face key and the edge rule are in 3dscan_b200/common/scan3d_repair_math.h.
+ * Flags: any non-empty combination of SCAN3D_REPAIR_FACES and SCAN3D_REPAIR_VERTICES; 0 and unknown bits are
+ * SCAN3D_ERR_ARG.
+ *
+ * 1. Degenerate faces (always): a face with a repeated index is dropped (degenerate_faces).
+ * 2. Duplicate faces (FACES): of the faces with the same set of three vertices, in either winding, the one with the
+ *    smallest face index is kept and the others are dropped (duplicate_faces).  Unlike the simplification, opposite
+ *    windings are duplicates too: the aim is a manifold.
+ * 3. Non-manifold edges: the faces that survive steps 1-2 are counted on each undirected edge; an edge with more than 2
+ *    counts in nonmanifold_edges, with or without FACES.  With FACES: each face has the key K(f) =
+ *    (float_bits((float)area_f) << 32) | (0xFFFFFFFF - f), area_f the hole filling's triangle area (double, from the
+ *    float coordinates).  On such an edge, f1 is the face with the largest K; f2 the face with the largest K among the
+ *    faces whose side on the edge runs opposite to f1's, or, when none does, among the faces other than f1.  Every other
+ *    face on the edge is dropped by it, and a face is removed when any of its edges drops it (nonmanifold_faces).  Every
+ *    edge then has at most 2 faces.
+ * 4. Non-manifold vertices (VERTICES): a corner (f, k) is numbered 3 f + k with the input face index.  The corners of
+ *    vertex v in kept faces f and g are joined when f and g share an edge {v, w} that lies in exactly 2 kept faces; a
+ *    fan is a class of joined corners.  The fan that holds v's smallest corner keeps index v; every other fan gets a
+ *    new vertex, appended after the existing ones in ascending order of its smallest corner, with v's xyz, normal and
+ *    rgb bytes (a copy sits exactly on its source: no vertex moves).  split_vertices counts the vertices with more than
+ *    one fan, vertices_added the new vertices.
+ * 5. Kept faces keep their relative order and their rotation, their corners remapped to their fans' vertices.  The
+ *    input's vertices keep their index and bytes, those that no kept face uses included (components with min_faces = 1
+ *    removes them).
+ * With both flags no edge is in more than 2 faces and no vertex's faces form more than one fan; orientation is not
+ * changed.  boundary_edges (edges in 1 kept face) and inconsistent_edges (edges in 2 kept faces whose sides run the same
+ * way) are counted over the kept faces before the split; with FACES they equal the counts after the call.  A second
+ * repair with the same flags changes nothing.
+ *
+ * scan3d_voxel_surface_repair repairs the held voxel surface in place: scan3d_get_voxel_surface,
+ * scan3d_write_voxel_surface_ply and the later stages see the repaired surface.  It needs a held surface
+ * (SCAN3D_ERR_STATE otherwise) and makes the component table stale (the vertex count changes); whether the surface is
+ * simplified or smoothed does not change.  It is allowed before or after components, simplification, smoothing and
+ * filling, and again.  Recommended order: extract, components, repair, then smooth or decimate (repair again after
+ * decimating), then fill.  A repair never adds a face or moves a vertex, so a surface that could be simplified before
+ * it still can.  But after a repair that dropped a face or split a vertex, a cell of the lattice can hold more than
+ * one hole, which breaks the simplification's overflow bound for filled holes (derived in
+ * 3dscan_b200/common/scan3d_repair_math.h): a fill that adds faces to such a surface makes scan3d_voxel_surface_decimate
+ * return SCAN3D_ERR_STATE until the next scan3d_voxel_surface.  Repair before a fill of an unrefined surface only when
+ * it will not be simplified, or simplify first.  A later begin, add or finish makes the surface stale as before.
+ * scan3d_mesh_repair_dev repairs any triangle mesh in device memory of the ctx's GPU (xyz_dev float [n_vertices][3],
+ * faces_dev int32 [n_faces][3]): it writes the kept, remapped faces, int32 [faces][3], to faces_out_dev (n_faces rows
+ * always suffice; it must not be faces_dev), and the source vertex of each added vertex, int32 [vertices_added], to
+ * source_out_dev (3 n_faces entries always suffice), ordered on the ctx stream; the caller extends its own attribute arrays with a gather.  It leaves the
+ * inputs, the held surface and the component table alone.  When more than max_source_out vertices are needed it
+ * writes nothing and returns SCAN3D_ERR_CONFIG with *out filled.  The ctx's camera-grid mesh (scan3d_device_points,
+ * scan3d_device_mesh_faces) is a valid input.
+ * Synchronisation: two per call, once the counts are known (to size, in the surface route, the spare surface set, into
+ * which the held vertices are copied) and once after every launch.  On any error the held surface is unchanged.
+ * Launches: 12, an empty mesh included: the finiteness and face-index checks with the degenerate faces and the
+ * duplicate table, the keys and sides into the edge table, the largest key other than f1 per edge, the drop flags
+ * with the kept faces' sides, the edge counts with the unions of the corners, the fans' roots, k_count + k_scan over
+ * the new vertices and over the kept faces; after the first synchronisation the new vertices and the kept faces.  10
+ * when the first synchronisation finds an error or too small a max_source_out.
+ * Memory (ctx-owned, allocated on first use, grown on demand): 8 B per vertex and 353 B per face (an edge table of 6
+ * slots of 48 B, the duplicate table of 2 slots of 4 B, 41 B of per-face and per-corner scratch); the surface route
+ * also grows the spare surface set to 27 B per vertex and 12 B per face after the repair, and 4 B per added vertex.
+ * Errors: SCAN3D_ERR_ARG for a null ctx or out; bad flags; in scan3d_mesh_repair_dev n_vertices, n_faces or
+ * max_source_out outside [0, 2^31), a NULL xyz_dev, faces_dev, faces_out_dev or source_out_dev with a non-zero count,
+ * a pointer not 4-byte aligned, faces_out_dev equal to faces_dev, and, found on the device, a face index outside
+ * [0, n_vertices) or a coordinate that is not finite.  SCAN3D_ERR_CONFIG when 3 n_faces or the output vertex count
+ * reaches 2^31.  An argument or state error launches nothing; on any error nothing is written. */
+#define SCAN3D_REPAIR_FACES 1
+#define SCAN3D_REPAIR_VERTICES 2
+typedef struct {
+    int64_t vertices, faces;     /* of the mesh after the call */
+    int64_t degenerate_faces;    /* dropped: a repeated index */
+    int64_t duplicate_faces;     /* dropped: the same three vertices as a face of smaller index */
+    int64_t nonmanifold_edges;   /* edges in more than 2 faces after steps 1-2 */
+    int64_t nonmanifold_faces;   /* dropped by a non-manifold edge */
+    int64_t split_vertices;      /* vertices with more than one fan */
+    int64_t vertices_added;
+    int64_t boundary_edges;      /* edges in 1 kept face */
+    int64_t inconsistent_edges;  /* edges in 2 kept faces whose sides run the same way */
+} scan3d_repair_result;
+
+int scan3d_voxel_surface_repair(scan3d_ctx *ctx, int32_t flags, scan3d_repair_result *out);
+int scan3d_mesh_repair_dev(scan3d_ctx *ctx, const float *xyz_dev, int64_t n_vertices, const int32_t *faces_dev,
+                           int64_t n_faces, int32_t flags, int32_t *faces_out_dev, int32_t *source_out_dev,
+                           int64_t max_source_out, scan3d_repair_result *out);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,
