@@ -131,6 +131,20 @@ class RepairResultC(C.Structure):
         "split_vertices", "vertices_added", "boundary_edges", "inconsistent_edges")]
 
 
+class OrientResultC(C.Structure):
+    _fields_ = [(name, C.c_int64) for name in (
+        "vertices", "faces", "degenerate_faces", "patches", "closed_patches", "nonorientable_patches", "flipped_faces",
+        "flipped_normals", "inconsistent_edges_before", "inconsistent_edges")]
+
+
+class MeasureResultC(C.Structure):
+    _fields_ = [(name, C.c_int64) for name in (
+        "vertices", "faces", "degenerate_faces", "patches", "closed_patches", "nonorientable_patches",
+        "unreferenced_vertices", "edges", "boundary_edges", "nonmanifold_edges", "inconsistent_edges",
+        "euler_characteristic", "watertight")] + [
+        ("area", C.c_double), ("volume", C.c_double), ("bbox_min", C.c_float * 3), ("bbox_max", C.c_float * 3)]
+
+
 # the steps of scan3d_voxel_surface_repair and scan3d_mesh_repair_dev (include/scan3d.h)
 REPAIR_FACES = 1
 REPAIR_VERTICES = 2
@@ -275,6 +289,10 @@ def cuda_lib():
     L.scan3d_mesh_fill_holes_dev.argtypes = [vp, vp, i64, vp, i64, i32, vp, i64, C.POINTER(FillResultC)]
     L.scan3d_voxel_surface_repair.argtypes = [vp, i32, C.POINTER(RepairResultC)]
     L.scan3d_mesh_repair_dev.argtypes = [vp, vp, i64, vp, i64, i32, vp, vp, i64, C.POINTER(RepairResultC)]
+    L.scan3d_voxel_surface_orient.argtypes = [vp, C.POINTER(OrientResultC)]
+    L.scan3d_mesh_orient_dev.argtypes = [vp, vp, vp, i64, vp, i64, C.POINTER(OrientResultC)]
+    L.scan3d_voxel_surface_measure.argtypes = [vp, C.POINTER(MeasureResultC)]
+    L.scan3d_mesh_measure_dev.argtypes = [vp, vp, i64, vp, i64, C.POINTER(MeasureResultC)]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -897,6 +915,73 @@ class Scan3D:
                                                self._repair_flags(repair_faces, vertices), C.c_void_p(out.data_ptr()),
                                                C.c_void_p(src.data_ptr()), 3 * nf, C.byref(r)))
         return out[:r.faces], src[:r.vertices_added], self._repair_result(r)
+
+    # -- coherent orientation and measures of the voxel surface and of device meshes (include/scan3d.h has the exact
+    # rules)
+    @staticmethod
+    def _orient_result(r):
+        return {name: getattr(r, name) for name, _ in OrientResultC._fields_}
+
+    @staticmethod
+    def _measure_result(r):
+        out = {name: getattr(r, name) for name, _ in MeasureResultC._fields_}
+        out["watertight"] = bool(r.watertight)
+        out["bbox_min"], out["bbox_max"] = tuple(r.bbox_min), tuple(r.bbox_max)
+        return out
+
+    @staticmethod
+    def _mesh_tensors(xyz, faces, normals=None):
+        import torch
+
+        def ok(t, dtype, rows):
+            return (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dtype and t.dim() == 2 and
+                    t.shape[1] == 3 and t.is_contiguous() and (rows is None or t.shape[0] == rows))
+        if not ok(xyz, torch.float32, None):
+            raise Scan3DError("xyz must be a contiguous CUDA float32 tensor of shape [v][3]")
+        if not ok(faces, torch.int32, None):
+            raise Scan3DError("faces must be a contiguous CUDA int32 tensor of shape [f][3]")
+        if normals is not None and not ok(normals, torch.float32, xyz.shape[0]):
+            raise Scan3DError("normals must be None or a contiguous CUDA float32 tensor of the shape of xyz")
+        torch.cuda.current_stream(xyz.device).synchronize()
+
+    def surface_orient(self):
+        """Orient the faces of the held voxel surface coherently, in place: per patch of faces joined across edges of
+        two faces, the fewest flips that make it consistent, closed patches with their normals outward; a vertex all of
+        whose faces flipped has its normal negated.  Synchronises once and returns a dict with the fields of
+        scan3d_orient_result.  The component table stays current."""
+        r = OrientResultC()
+        self._ck(self.L.scan3d_voxel_surface_orient(self.h, C.byref(r)))
+        return self._orient_result(r)
+
+    def mesh_orient_dev(self, xyz, faces, normals=None):
+        """surface_orient() for a triangle mesh on the ctx's GPU, in place: xyz a CUDA float32 tensor [v][3] (read),
+        faces a CUDA int32 tensor [f][3] (the flips are written into it), normals None or a CUDA float32 tensor [v][3].
+        torch's current stream is synchronised first, so data written there is ready.  Returns the dict of
+        surface_orient()."""
+        self._mesh_tensors(xyz, faces, normals)
+        r = OrientResultC()
+        self._ck(self.L.scan3d_mesh_orient_dev(self.h, C.c_void_p(xyz.data_ptr()),
+                                               None if normals is None else C.c_void_p(normals.data_ptr()),
+                                               xyz.shape[0], C.c_void_p(faces.data_ptr()), faces.shape[0],
+                                               C.byref(r)))
+        return self._orient_result(r)
+
+    def surface_measure(self):
+        """The area, signed volume, bounding box and topology (edges by kind, patches, Euler characteristic, watertight)
+        of the held voxel surface: a dict with the fields of scan3d_measure_result (watertight a bool, the boxes
+        tuples).  Changes nothing; synchronises once."""
+        r = MeasureResultC()
+        self._ck(self.L.scan3d_voxel_surface_measure(self.h, C.byref(r)))
+        return self._measure_result(r)
+
+    def mesh_measure_dev(self, xyz, faces):
+        """surface_measure() for a triangle mesh on the ctx's GPU: xyz a CUDA float32 tensor [v][3], faces a CUDA int32
+        tensor [f][3]; neither is changed.  torch's current stream is synchronised first."""
+        self._mesh_tensors(xyz, faces)
+        r = MeasureResultC()
+        self._ck(self.L.scan3d_mesh_measure_dev(self.h, C.c_void_p(xyz.data_ptr()), xyz.shape[0],
+                                                C.c_void_p(faces.data_ptr()), faces.shape[0], C.byref(r)))
+        return self._measure_result(r)
 
     # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
     @staticmethod

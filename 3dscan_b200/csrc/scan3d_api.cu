@@ -16,6 +16,7 @@
 #include "../common/scan3d_align_math.h"
 #include "../common/scan3d_surface_math.h"
 #include "../common/scan3d_decimate_math.h"
+#include "../common/scan3d_orient_math.h"
 
 using namespace s3d;
 
@@ -1698,6 +1699,136 @@ int scan3d_mesh_repair_dev(scan3d_ctx* ctx, const float* xyz_dev, int64_t n_vert
                         nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, ctx->stream, &ctx->launches));
     CK(cudaStreamSynchronize(ctx->stream));
     return SCAN3D_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// coherent orientation and measures of the voxel surface and of device meshes (include/scan3d.h and
+// common/scan3d_orient_math.h have the exact rules)
+// ------------------------------------------------------------------------------------------
+static int check_mesh_args(scan3d_ctx* ctx, const float* xyz, const float* nrm, int64_t nv, const int32_t* faces,
+                           int64_t nf)
+{
+    if (nf < 0 || nf >= (1LL << 31) || nv < 0 || nv >= (1LL << 31))
+        return fail(ctx, SCAN3D_ERR_ARG, "n_vertices and n_faces must be in [0, 2^31)");
+    if ((!xyz && nv > 0) || (!faces && nf > 0)) return fail(ctx, SCAN3D_ERR_ARG, "null device pointer");
+    if (((uintptr_t)xyz & 3) || ((uintptr_t)nrm & 3) || ((uintptr_t)faces & 3))
+        return fail(ctx, SCAN3D_ERR_ARG, "xyz_dev, normals_dev and faces_dev must be 4-byte aligned");
+    return SCAN3D_OK;
+}
+
+// the counting pass over the mesh and, with apply, the flips into faces_out and nrm; one synchronisation
+static int orient_run(scan3d_ctx* ctx, const float* xyz, float* nrm, const int32_t* faces, bool apply,
+                      int32_t* faces_out, int64_t nv, int64_t nf, OrientState* st)
+{
+    if (6 * nf >= (1LL << 32)) return fail(ctx, SCAN3D_ERR_CONFIG, "more than (2^32 - 1) / 6 faces");
+    CK(ctx->orient.count(xyz, faces, (uint32_t)nv, (uint32_t)nf, ctx->stream, &ctx->launches));
+    if (apply) CK(ctx->orient.apply(faces_out, nrm, (uint32_t)nv, (uint32_t)nf, ctx->stream, &ctx->launches));
+    CK(cudaMemcpyAsync(st, ctx->orient.state, sizeof(*st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st->bad) return fail(ctx, SCAN3D_ERR_ARG, "a coordinate that is not finite or a face index outside [0, n_vertices)");
+    return SCAN3D_OK;
+}
+
+static int orient_mesh(scan3d_ctx* ctx, const float* xyz, float* nrm, int32_t* faces, int64_t nv, int64_t nf,
+                       scan3d_orient_result* out)
+{
+    OrientState st;
+    const int rc = orient_run(ctx, xyz, nrm, faces, true, faces, nv, nf, &st);
+    if (rc) return rc;
+    out->vertices = nv;
+    out->faces = nf;
+    out->degenerate_faces = st.degenerate;
+    out->patches = st.patches;
+    out->closed_patches = st.closed;
+    out->nonorientable_patches = st.nonorientable;
+    out->flipped_faces = st.flipped;
+    out->flipped_normals = st.flipped_normals;
+    out->inconsistent_edges_before = st.inconsistent;
+    out->inconsistent_edges = st.inconsistent_after;
+    return SCAN3D_OK;
+}
+
+static int measure_mesh(scan3d_ctx* ctx, const float* xyz, const int32_t* faces, int64_t nv, int64_t nf,
+                        scan3d_measure_result* out)
+{
+    OrientState st;
+    const int rc = orient_run(ctx, xyz, nullptr, faces, false, nullptr, nv, nf, &st);
+    if (rc) return rc;
+    const int64_t live = nf - (int64_t)st.degenerate;
+    out->vertices = nv;
+    out->faces = nf;
+    out->degenerate_faces = st.degenerate;
+    out->patches = st.patches;
+    out->closed_patches = st.closed;
+    out->nonorientable_patches = st.nonorientable;
+    out->unreferenced_vertices = nv - (int64_t)st.referenced;
+    out->edges = st.edges;
+    out->boundary_edges = st.boundary;
+    out->nonmanifold_edges = st.nonmanifold;
+    out->inconsistent_edges = st.inconsistent;
+    out->euler_characteristic = (int64_t)st.referenced - (int64_t)st.edges + live;
+    out->watertight = live > 0 && st.boundary == 0 && st.nonmanifold == 0 && st.inconsistent == 0;
+    const int E = s3o::exponent(st.exp_field);
+    out->area = s3o::area(st.area[0], st.area[1], E);
+    out->volume = s3o::volume(st.volume[0], st.volume[1], E);
+    for (int k = 0; k < 3; k++) {
+        uint32_t lo = 0, hi = 0;                         // +0.0f without a referenced vertex
+        if (st.referenced) {
+            lo = s3o::key_bits(st.box_lo[k]);
+            hi = s3o::key_bits(st.box_hi[k]);
+        }
+        memcpy(&out->bbox_min[k], &lo, 4);
+        memcpy(&out->bbox_max[k], &hi, 4);
+    }
+    return SCAN3D_OK;
+}
+
+int scan3d_voxel_surface_orient(scan3d_ctx* ctx, scan3d_orient_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (!ctx->results.has(SURFACE))
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    CK(cudaSetDevice(ctx->device));
+    SurfaceMesh& s = ctx->surface;
+    // faces and normals change in place; the vertex and face sets, and so every result, stay current
+    const int rc = orient_mesh(ctx, s.xyz, s.nrm, s.tri, s.vertices, s.faces, out);
+    if (rc) return rc;
+    if (out->flipped_faces) ctx->srf_repaired = true;
+    return SCAN3D_OK;
+}
+
+int scan3d_mesh_orient_dev(scan3d_ctx* ctx, const float* xyz_dev, float* normals_dev, int64_t n_vertices,
+                           int32_t* faces_dev, int64_t n_faces, scan3d_orient_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    const int rc = check_mesh_args(ctx, xyz_dev, normals_dev, n_vertices, faces_dev, n_faces);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    return orient_mesh(ctx, xyz_dev, normals_dev, faces_dev, n_vertices, n_faces, out);
+}
+
+int scan3d_voxel_surface_measure(scan3d_ctx* ctx, scan3d_measure_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (!ctx->results.has(SURFACE))
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    CK(cudaSetDevice(ctx->device));
+    const SurfaceMesh& s = ctx->surface;
+    return measure_mesh(ctx, s.xyz, s.tri, s.vertices, s.faces, out);
+}
+
+int scan3d_mesh_measure_dev(scan3d_ctx* ctx, const float* xyz_dev, int64_t n_vertices, const int32_t* faces_dev,
+                            int64_t n_faces, scan3d_measure_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    if (!out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    const int rc = check_mesh_args(ctx, xyz_dev, nullptr, n_vertices, faces_dev, n_faces);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    return measure_mesh(ctx, xyz_dev, faces_dev, n_vertices, n_faces, out);
 }
 
 // ------------------------------------------------------------------------------------------

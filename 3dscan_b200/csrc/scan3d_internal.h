@@ -352,6 +352,51 @@ struct RepairWorkspace {
                      const float* xyz, const float* nrm, const uint8_t* rgb, float* xyz_out, float* nrm_out,
                      uint8_t* rgb_out, cudaStream_t st, int64_t* launches);
 };
+
+// the coherent orientation and the measures (scan3d_orient_kernels.cu; common/scan3d_orient_math.h has the
+// arithmetic); the undirected edges are the smoothing's table of (min << 32 | max) keys, the 2-colouring a union-find
+// over the nodes 2 f (f as wound) and 2 f + 1 (f flipped)
+struct OrientState {
+    unsigned long long volume[2], area[2];   // int128 sums of the volume and area terms (low word, high word)
+    uint32_t box_lo[3], box_hi[3];           // s3o::order_key of the referenced vertices' bounding box
+    uint32_t exp_field;            // the largest double exponent field of an offset from the centre
+    uint32_t bad;                  // a coordinate not finite or a face index outside [0, vertices): SCAN3D_ERR_ARG
+    uint32_t degenerate, referenced;
+    uint32_t edges, boundary, nonmanifold, inconsistent;
+    uint32_t patches;              // a scan total
+    uint32_t closed, nonorientable, flipped, flipped_normals, inconsistent_after;
+};
+struct OrientBuffers;
+struct OrientWorkspace {
+    DeviceBuffer<unsigned long long> keys;  // [6 faces] the edge table
+    DeviceBuffer<uint32_t> sides;           // [6 faces] faces on each edge
+    DeviceBuffer<uint32_t> pair;            // [6 faces][2] the first two faces of each edge
+    DeviceBuffer<uint32_t> side_slot;       // [faces][3] edge-table slot of each side
+    DeviceBuffer<uint8_t> status;           // [faces] indices in range, not degenerate
+    DeviceBuffer<uint32_t> parent;          // [2 faces] union-find over the face nodes
+    DeviceBuffer<uint32_t> root;            // [faces] find(2 f)
+    DeviceBuffer<uint8_t> is_root;          // [faces] the smallest face of its patch
+    DeviceBuffer<uint32_t> face_counts;     // [cdiv(faces, POINT_BLOCK) + 1]
+    DeviceBuffer<uint32_t> size, npos;      // [faces] per patch (at its smallest face): faces, faces of sigma = +1
+    DeviceBuffer<unsigned long long> v0;    // [faces][2] per patch: int128 sum of sigma D
+    DeviceBuffer<uint8_t> open, nonorientable;   // [faces] per patch
+    DeviceBuffer<uint8_t> flip;             // [faces]
+    DeviceBuffer<uint8_t> ref, kept;        // [vertices] in a face that is not degenerate; in one that keeps its winding
+    DeviceBuffer<OrientState> state;
+    uint32_t table = 0;                     // slots of the edge table of the last count
+    OrientBuffers view();
+    // 7 launches for n vertices and nf faces [nf][3], 6 nf < 2^32: the face-index check with the degenerate faces, the
+    // referenced vertices and the sides into the edge table; the finiteness check with the bounding box; per edge the
+    // counts and the unions, per vertex the exponent of the offsets; per face the roots, the patch counters and the
+    // volume and area sums; k_count + k_scan over the roots (state->patches); per face the flips, per patch the closed
+    // and non-orientable counts, per edge the inconsistent edges left.  Every count of state but flipped_normals is
+    // then known.
+    cudaError_t count(const float* xyz, const int32_t* faces, uint32_t n, uint32_t nf, cudaStream_t st,
+                      int64_t* launches);
+    // 1 launch after count on the same stream: the flips into faces and, when nrm is set, the negated normals
+    // (state->flipped_normals); nothing is written when state->bad is set
+    cudaError_t apply(int32_t* faces, float* nrm, uint32_t n, uint32_t nf, cudaStream_t st, int64_t* launches);
+};
 }  // namespace s3d
 
 // Every device buffer the context owns is a DeviceBuffer: scan3d_destroy frees them all by deleting the context.
@@ -441,14 +486,15 @@ struct scan3d_ctx {
     s3d::SmoothWorkspace smooth;          // scan3d_voxel_surface_smooth, scan3d_mesh_smooth_dev
     s3d::FillWorkspace fill;              // scan3d_voxel_surface_fill_holes, scan3d_mesh_fill_holes_dev
     s3d::RepairWorkspace repair;          // scan3d_voxel_surface_repair, scan3d_mesh_repair_dev
+    s3d::OrientWorkspace orient;          // scan3d_voxel_surface_orient / _measure, scan3d_mesh_orient_dev / _measure_dev
 
     // the held voxel surface, and the spare set that components, decimate, smooth, fill and repair write before they
     // swap it in
     s3d::SurfaceMesh surface, spare;
     int64_t cc_components = 0;
-    // since the held surface was extracted: a repair dropped faces or split vertices; a fill added faces after that.
-    // The decimation's quadric bound needs one hole per cell, which holds unless both happened
-    // (common/scan3d_repair_math.h).
+    // since the held surface was extracted: a repair dropped faces or split vertices, or an orientation flipped faces;
+    // a fill added faces after that.  The decimation's quadric bound needs one hole per cell, which holds unless both
+    // happened (common/scan3d_repair_math.h, common/scan3d_orient_math.h).
     bool srf_repaired = false, srf_filled_after_repair = false;
 
     int cta_limit = 0;             // scan3d_set_cta_limit

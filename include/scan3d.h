@@ -793,6 +793,93 @@ int scan3d_mesh_repair_dev(scan3d_ctx *ctx, const float *xyz_dev, int64_t n_vert
                            int64_t n_faces, int32_t flags, int32_t *faces_out_dev, int32_t *source_out_dev,
                            int64_t max_source_out, scan3d_repair_result *out);
 
+/* ---- coherent orientation and measures of the voxel surface and of device meshes: MeshLab's "Re-Orient all faces
+ * coherently" (vcglib tri::Clean::OrientCoherentlyMesh), "Compute Geometric Measures" and "Compute Topological
+ * Measures" ------------------------------------------------------------------------------------------------------
+ * Every result is a pure function of the mesh: bit-reproducible, independent of scheduling, of the hash and of the SM
+ * count.  The arithmetic is in 3dscan_b200/common/scan3d_orient_math.h.
+ *
+ * Definitions.
+ * - A face (a, b, c) has the sides a->b, b->c and c->a.  A face with a repeated index is degenerate: it is in no
+ *   patch, has no edges, is never flipped and adds no area or volume (degenerate_faces).  A vertex is referenced when a
+ *   face that is not degenerate uses it (unreferenced_vertices counts the others).
+ * - The count of an undirected edge is the number of non-degenerate faces with a side on it.  Count 1: a boundary
+ *   edge; 3 or more: non-manifold; 2: inconsistent when its two sides run the same way.  On the same faces these are
+ *   the repair's boundary_edges, nonmanifold_edges and inconsistent_edges.
+ * - A patch is a maximal set of non-degenerate faces joined across edges of count exactly 2.  It is closed when none of
+ *   its faces has a boundary or non-manifold edge, and orientable when some choice of flips makes every joining edge
+ *   consistent.
+ * - Orientation rule.  f0 is the smallest face index of an orientable patch P; sigma(f) = +1 when f keeps its winding
+ *   if f0 keeps its own, else -1; n+ counts the faces with sigma = +1 and V0 = sum sigma(f) D(f) (D below, exact).  A
+ *   closed patch with V0 != 0 keeps f0's winding exactly when V0 > 0, so its normals point outward.  Any other patch
+ *   keeps f0's winding exactly when 2 n+ >= |P|: the fewest faces flip, a tie keeps f0.  A flip turns (a, b, c) into
+ *   (a, c, b).  Non-orientable (Moebius-like) patches are left unchanged and counted.  Face order, vertex order, xyz
+ *   and rgb never change.  A referenced vertex all of whose non-degenerate faces were flipped has its normal negated
+ *   (the sign bit of each component; flipped_normals counts these vertices, with or without normals); every other
+ *   normal keeps its bytes.  A second orientation flips nothing.
+ * - Volume and area.  c is the midpoint of the exact float bounding box of the referenced vertices, rounded to float.
+ *   D(f) = det(p_a - c, p_b - c, p_c - c), six times the signed volume of the tetrahedron (c, f), in double from the
+ *   float coordinates in a fixed order; area(f) is the hole filling's triangle area sqrt(l2) * 0.5.  Each term is
+ *   rounded to an int64 fixed point whose scale comes from E, the exponent of the largest |p - c| of a referenced
+ *   vertex (2^(59 - 3E) for D, 2^(59 - 2E) for the area), and the terms are summed exactly in int128; volume = sum D /
+ *   6 and area = sum area, scaled back.  The volume is signed, with the current windings: positive for a closed
+ *   surface whose normals point outward.
+ * - euler_characteristic = referenced vertices - edges + non-degenerate faces.  For a closed, consistent mesh without
+ *   non-manifold vertices (after a repair with SCAN3D_REPAIR_VERTICES), each patch is a closed orientable surface and
+ *   genus = patches - euler_characteristic / 2; with non-manifold vertices no genus follows, so none is reported.
+ * - watertight = (faces - degenerate_faces > 0) && boundary_edges == nonmanifold_edges == inconsistent_edges == 0.
+ *
+ * scan3d_voxel_surface_orient orients the held voxel surface in place (faces and normals); the component table stays
+ * current and whether the surface is simplified or smoothed does not change.  The decimation's quadric does not depend
+ * on the winding, so an oriented raw surface can still be simplified; but an orientation that flipped a face counts as
+ * a repair that changed the surface: a fill that adds faces after it makes scan3d_voxel_surface_decimate return
+ * SCAN3D_ERR_STATE until the next scan3d_voxel_surface (3dscan_b200/common/scan3d_orient_math.h).
+ * scan3d_mesh_orient_dev orients any triangle mesh in device memory of the ctx's GPU in place (xyz_dev float
+ * [n_vertices][3], read; normals_dev float [n_vertices][3] or NULL; faces_dev int32 [n_faces][3]), ordered on the ctx
+ * stream.  The ctx's camera-grid mesh (scan3d_device_points, scan3d_device_mesh_faces) is a valid input.
+ * scan3d_voxel_surface_measure and scan3d_mesh_measure_dev only read; they change no state.
+ * Recommended order: extract, components, repair, orient, smooth or decimate, fill, measure.
+ * Synchronisation: one per call, after every launch.  Launches: 8 per orientation and 7 per measure, an empty mesh
+ * and an error found on the device included: the face-index check with the degenerate faces and the sides into the
+ * edge table, the finiteness check with the bounding box, the edge counts with the unions and the exponent, the
+ * roots with the patch sums, k_count + k_scan over the patches' smallest faces, the flips; the orientation then
+ * writes the flips.
+ * Memory (ctx-owned, allocated on first use, grown on demand, shared by both calls): 2 B per vertex and 173 B per face
+ * (an edge table of 6 slots of 20 B, 53 B of per-face scratch).
+ * Errors: SCAN3D_ERR_ARG for a null ctx or out; in the dev routes n_vertices or n_faces outside [0, 2^31), a NULL
+ * xyz_dev or faces_dev with a non-zero count, a pointer not 4-byte aligned, and, found on the device, a face index
+ * outside [0, n_vertices) or a coordinate that is not finite (of any vertex).  SCAN3D_ERR_CONFIG when 6 n_faces
+ * reaches 2^32.  SCAN3D_ERR_STATE for the surface routes without a held surface.  An argument or state error
+ * launches nothing; on any error nothing is written. */
+typedef struct {
+    int64_t vertices, faces;
+    int64_t degenerate_faces;
+    int64_t patches, closed_patches, nonorientable_patches;
+    int64_t flipped_faces;
+    int64_t flipped_normals;            /* referenced vertices all of whose faces were flipped */
+    int64_t inconsistent_edges_before;
+    int64_t inconsistent_edges;         /* after the call: those inside non-orientable patches */
+} scan3d_orient_result;
+
+typedef struct {
+    int64_t vertices, faces;
+    int64_t degenerate_faces;
+    int64_t patches, closed_patches, nonorientable_patches;
+    int64_t unreferenced_vertices;
+    int64_t edges, boundary_edges, nonmanifold_edges, inconsistent_edges;
+    int64_t euler_characteristic;
+    int64_t watertight;                 /* 1 or 0 */
+    double area, volume;                /* volume signed, with the current windings */
+    float bbox_min[3], bbox_max[3];     /* of the referenced vertices; zeros when there are none */
+} scan3d_measure_result;
+
+int scan3d_voxel_surface_orient(scan3d_ctx *ctx, scan3d_orient_result *out);
+int scan3d_mesh_orient_dev(scan3d_ctx *ctx, const float *xyz_dev, float *normals_dev, int64_t n_vertices,
+                           int32_t *faces_dev, int64_t n_faces, scan3d_orient_result *out);
+int scan3d_voxel_surface_measure(scan3d_ctx *ctx, scan3d_measure_result *out);
+int scan3d_mesh_measure_dev(scan3d_ctx *ctx, const float *xyz_dev, int64_t n_vertices, const int32_t *faces_dev,
+                            int64_t n_faces, scan3d_measure_result *out);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,
