@@ -145,6 +145,16 @@ class MeasureResultC(C.Structure):
         ("area", C.c_double), ("volume", C.c_double), ("bbox_min", C.c_float * 3), ("bbox_max", C.c_float * 3)]
 
 
+class DistanceParams(C.Structure):
+    _fields_ = [("max_distance", C.c_float)]
+
+
+class DistanceResultC(C.Structure):
+    _fields_ = [(name, C.c_int64) for name in ("samples", "matched", "invalid", "inside", "max_sample")] + [
+        ("max", C.c_double), ("mean", C.c_double), ("rms", C.c_double), ("min_signed", C.c_float),
+        ("max_signed", C.c_float), ("entries", C.c_int64)]
+
+
 # the steps of scan3d_voxel_surface_repair and scan3d_mesh_repair_dev (include/scan3d.h)
 REPAIR_FACES = 1
 REPAIR_VERTICES = 2
@@ -293,6 +303,11 @@ def cuda_lib():
     L.scan3d_mesh_orient_dev.argtypes = [vp, vp, vp, i64, vp, i64, C.POINTER(OrientResultC)]
     L.scan3d_voxel_surface_measure.argtypes = [vp, C.POINTER(MeasureResultC)]
     L.scan3d_mesh_measure_dev.argtypes = [vp, vp, i64, vp, i64, C.POINTER(MeasureResultC)]
+    L.scan3d_voxel_surface_distance.argtypes = [vp, C.POINTER(DistanceParams), vp, vp, C.POINTER(DistanceResultC)]
+    L.scan3d_voxel_surface_distance_dev.argtypes = [vp, vp, i64, C.POINTER(DistanceParams), vp, vp,
+                                                    C.POINTER(DistanceResultC)]
+    L.scan3d_mesh_distance_dev.argtypes = [vp, vp, i64, vp, i64, vp, i64, C.POINTER(DistanceParams), vp, vp,
+                                           C.POINTER(DistanceResultC)]
     L.scan3d_debug_atan2.argtypes = [vp, vp, vp, vp, i32, i32]
     L.scan3d_debug_divcheck.argtypes = [vp, C.POINTER(C.c_uint64)]
     _cuda = L
@@ -982,6 +997,76 @@ class Scan3D:
         self._ck(self.L.scan3d_mesh_measure_dev(self.h, C.c_void_p(xyz.data_ptr()), xyz.shape[0],
                                                 C.c_void_p(faces.data_ptr()), faces.shape[0], C.byref(r)))
         return self._measure_result(r)
+
+    # -- distances of samples from a triangle surface within a radius (include/scan3d.h has the exact rules)
+    @staticmethod
+    def _distance_result(r):
+        return {name: getattr(r, name) for name, _ in DistanceResultC._fields_}
+
+    @staticmethod
+    def _distance_outputs(samples, n):
+        import torch
+        dev = samples.device
+        return (torch.empty(n, dtype=torch.float32, device=dev), torch.empty(n, dtype=torch.int32, device=dev))
+
+    @staticmethod
+    def _samples_tensor(samples):
+        import torch
+        if not (isinstance(samples, torch.Tensor) and samples.is_cuda and samples.dtype == torch.float32 and
+                samples.dim() == 2 and samples.shape[1] == 3 and samples.is_contiguous()):
+            raise Scan3DError("samples must be a contiguous CUDA float32 tensor of shape [n][3]")
+        torch.cuda.current_stream(samples.device).synchronize()
+
+    def surface_distance(self, max_distance, per_sample=False):
+        """The distances of the merge's model (the voxel outputs with a non-zero normal) from the held voxel surface,
+        each to its nearest face within max_distance, signed by that face's normal (negative inside an outward
+        surface).  Returns a dict with the fields of scan3d_distance_result (max is the one-sided Hausdorff distance
+        within max_distance); with per_sample=True, (dist, face, dict): CUDA tensors indexed by voxel ordinal, NaN and
+        -1 for a voxel that is not matched or not in the model.  Changes nothing; synchronises twice."""
+        import torch
+        p = DistanceParams(max_distance)
+        r = DistanceResultC()
+        if not per_sample:
+            self._ck(self.L.scan3d_voxel_surface_distance(self.h, C.byref(p), None, None, C.byref(r)))
+            return self._distance_result(r)
+        n = self.voxel_count()[0]                       # the outputs of the last finish: no SURFACE without them
+        dev = torch.device("cuda", torch.cuda.current_device())
+        dist = torch.empty(n, dtype=torch.float32, device=dev)
+        face = torch.empty(n, dtype=torch.int32, device=dev)
+        torch.cuda.current_stream(dev).synchronize()
+        self._ck(self.L.scan3d_voxel_surface_distance(self.h, C.byref(p), C.c_void_p(dist.data_ptr()) if n else None,
+                                                      C.c_void_p(face.data_ptr()) if n else None, C.byref(r)))
+        return dist, face, self._distance_result(r)
+
+    def surface_distance_dev(self, samples, max_distance):
+        """surface_distance() for samples of the caller: a CUDA float32 tensor [n][3] on the ctx's GPU (a view's
+        device_points(), for instance) against the held voxel surface.  torch's current stream is synchronised first.
+        Returns (dist, face, dict): dist float32 [n] signed, NaN when invalid or unmatched; face int32 [n], -1 then."""
+        self._samples_tensor(samples)
+        n = samples.shape[0]
+        dist, face = self._distance_outputs(samples, n)
+        p = DistanceParams(max_distance)
+        r = DistanceResultC()
+        self._ck(self.L.scan3d_voxel_surface_distance_dev(self.h, C.c_void_p(samples.data_ptr()), n, C.byref(p),
+                                                          C.c_void_p(dist.data_ptr()), C.c_void_p(face.data_ptr()),
+                                                          C.byref(r)))
+        return dist, face, self._distance_result(r)
+
+    def mesh_distance_dev(self, samples, xyz, faces, max_distance):
+        """surface_distance_dev() against any triangle mesh on the ctx's GPU: xyz a CUDA float32 tensor [v][3], faces
+        a CUDA int32 tensor [f][3] (the camera-grid mesh included); nothing is changed."""
+        self._samples_tensor(samples)
+        self._mesh_tensors(xyz, faces)
+        n = samples.shape[0]
+        dist, face = self._distance_outputs(samples, n)
+        p = DistanceParams(max_distance)
+        r = DistanceResultC()
+        self._ck(self.L.scan3d_mesh_distance_dev(self.h, C.c_void_p(samples.data_ptr()), n,
+                                                 C.c_void_p(xyz.data_ptr()), xyz.shape[0],
+                                                 C.c_void_p(faces.data_ptr()), faces.shape[0], C.byref(p),
+                                                 C.c_void_p(dist.data_ptr()), C.c_void_p(face.data_ptr()),
+                                                 C.byref(r)))
+        return dist, face, self._distance_result(r)
 
     # -- scan-to-model alignment against the voxel outputs (include/scan3d.h has the exact rules)
     @staticmethod

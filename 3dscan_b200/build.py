@@ -30,7 +30,8 @@ CU_SOURCES = ["scan3d_api.cu", "scan3d_stage_kernels.cu", "scan3d_worklist.cu", 
               "scan3d_aux_kernels.cu", "scan3d_aux_api.cu", "scan3d_shard.cu", "scan3d_mesh_kernels.cu",
               "scan3d_voxel_kernels.cu", "scan3d_align_kernels.cu", "scan3d_surface_kernels.cu",
               "scan3d_components_kernels.cu", "scan3d_decimate_kernels.cu", "scan3d_smooth_kernels.cu",
-              "scan3d_fill_kernels.cu", "scan3d_repair_kernels.cu", "scan3d_orient_kernels.cu"]
+              "scan3d_fill_kernels.cu", "scan3d_repair_kernels.cu", "scan3d_orient_kernels.cu",
+              "scan3d_distance_kernels.cu"]
 HOST_SOURCES = ["scan3d_io.cpp", "scan3d_synth.cpp"]
 COMPAT_SOURCES = ["scan3d_stages.cpp"]
 

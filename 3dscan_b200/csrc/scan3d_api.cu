@@ -1832,6 +1832,109 @@ int scan3d_mesh_measure_dev(scan3d_ctx* ctx, const float* xyz_dev, int64_t n_ver
 }
 
 // ------------------------------------------------------------------------------------------
+// sample-to-surface distances (include/scan3d.h and common/scan3d_distance_math.h have the exact rules)
+// ------------------------------------------------------------------------------------------
+static int check_distance_args(scan3d_ctx* ctx, const scan3d_distance_params* p, const float* dist, const int32_t* face,
+                               scan3d_distance_result* out)
+{
+    if (!p || !out) return fail(ctx, SCAN3D_ERR_ARG, "null argument");
+    if (!(p->max_distance > 0.0f && p->max_distance - p->max_distance == 0.0f))
+        return fail(ctx, SCAN3D_ERR_ARG, "max_distance must be finite and > 0");
+    if (((uintptr_t)dist & 3) || ((uintptr_t)face & 3))
+        return fail(ctx, SCAN3D_ERR_ARG, "dist_dev and face_dev must be 4-byte aligned");
+    return SCAN3D_OK;
+}
+
+static int check_samples(scan3d_ctx* ctx, const float* samples, int64_t n)
+{
+    if (n < 0 || n >= (1LL << 31)) return fail(ctx, SCAN3D_ERR_ARG, "n must be in [0, 2^31)");
+    if (!samples && n > 0) return fail(ctx, SCAN3D_ERR_ARG, "null samples_dev");
+    if ((uintptr_t)samples & 3) return fail(ctx, SCAN3D_ERR_ARG, "samples_dev must be 4-byte aligned");
+    return SCAN3D_OK;
+}
+
+// the whole call: the count, the first synchronisation (errors; on the surface route also the voxel count, n_vox set),
+// the index and the query, the second synchronisation
+static int distance_run(scan3d_ctx* ctx, const float* samples, const float* nrm, int64_t n, const uint32_t* n_vox,
+                        const float* xyz, int64_t nv, const int32_t* faces, int64_t nf, const scan3d_distance_params* p,
+                        float* dist, int32_t* face, scan3d_distance_result* out)
+{
+    CK(cudaSetDevice(ctx->device));
+    const double S = s3l::cell_edge(p->max_distance);
+    const double r2 = (double)p->max_distance * (double)p->max_distance;   // host TU: -ffp-contract=off
+    CK(ctx->dist.count(xyz, faces, (uint32_t)nv, (uint32_t)nf, S, ctx->stream, &ctx->launches));
+    DistanceState st;
+    uint32_t total = 0;
+    CK(cudaMemcpyAsync(&st, ctx->dist.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    if (n_vox) CK(cudaMemcpyAsync(&total, n_vox, sizeof(total), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (st.bad) return fail(ctx, SCAN3D_ERR_ARG, "a coordinate that is not finite or a face index outside [0, n_vertices)");
+    if (st.range) return fail(ctx, SCAN3D_ERR_CONFIG, "a face vertex whose cell (edge max_distance) is outside [-2^20, 2^20)");
+    if (st.entries >= (1ull << 32))
+        return fail(ctx, SCAN3D_ERR_CONFIG, "2^32 or more face-cell entries: choose a larger max_distance");
+    if (n_vox) n = std::min<int64_t>(total, n);
+    CK(ctx->dist.query(xyz, faces, (uint32_t)nf, (uint32_t)st.entries, S, r2, samples, nrm, (uint32_t)n, dist, face,
+                       ctx->stream, &ctx->launches));
+    CK(cudaMemcpyAsync(&st, ctx->dist.state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    out->samples = (int64_t)st.samples;
+    out->matched = (int64_t)st.matched;
+    out->invalid = (int64_t)st.invalid;
+    out->inside = (int64_t)st.inside;
+    out->max_sample = st.max_sample;
+    out->max = st.max_d;
+    out->mean = st.matched ? st.sum_d / (double)st.matched : 0.0;
+    out->rms = st.matched ? sqrt(st.sum_d2 / (double)st.matched) : 0.0;
+    out->min_signed = st.min_signed;
+    out->max_signed = st.max_signed;
+    out->entries = (int64_t)st.entries;
+    return SCAN3D_OK;
+}
+
+int scan3d_voxel_surface_distance(scan3d_ctx* ctx, const scan3d_distance_params* p, float* dist_dev, int32_t* face_dev,
+                                  scan3d_distance_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    const int rc = check_distance_args(ctx, p, dist_dev, face_dev, out);
+    if (rc) return rc;
+    if (!ctx->results.has(SURFACE))
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    const SurfaceMesh& s = ctx->surface;
+    const uint32_t* total = &ctx->vox.state.get()->total[ctx->vox_chunks & 1];
+    return distance_run(ctx, ctx->vox_xyz, ctx->vox_nrm, ctx->vox.view.max_voxels, total, s.xyz, s.vertices, s.tri,
+                        s.faces, p, dist_dev, face_dev, out);
+}
+
+int scan3d_voxel_surface_distance_dev(scan3d_ctx* ctx, const float* samples_dev, int64_t n,
+                                      const scan3d_distance_params* p, float* dist_dev, int32_t* face_dev,
+                                      scan3d_distance_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    int rc = check_distance_args(ctx, p, dist_dev, face_dev, out);
+    if (rc == SCAN3D_OK) rc = check_samples(ctx, samples_dev, n);
+    if (rc) return rc;
+    if (!ctx->results.has(SURFACE))
+        return fail(ctx, SCAN3D_ERR_STATE, "no surface of the current voxel outputs: call scan3d_voxel_surface");
+    const SurfaceMesh& s = ctx->surface;
+    return distance_run(ctx, samples_dev, nullptr, n, nullptr, s.xyz, s.vertices, s.tri, s.faces, p, dist_dev,
+                        face_dev, out);
+}
+
+int scan3d_mesh_distance_dev(scan3d_ctx* ctx, const float* samples_dev, int64_t n, const float* xyz_dev,
+                             int64_t n_vertices, const int32_t* faces_dev, int64_t n_faces,
+                             const scan3d_distance_params* p, float* dist_dev, int32_t* face_dev,
+                             scan3d_distance_result* out)
+{
+    if (!ctx) return SCAN3D_ERR_ARG;
+    int rc = check_distance_args(ctx, p, dist_dev, face_dev, out);
+    if (rc == SCAN3D_OK) rc = check_samples(ctx, samples_dev, n);
+    if (rc == SCAN3D_OK) rc = check_mesh_args(ctx, xyz_dev, nullptr, n_vertices, faces_dev, n_faces);
+    if (rc) return rc;
+    return distance_run(ctx, samples_dev, nullptr, n, nullptr, xyz_dev, n_vertices, faces_dev, n_faces, p, dist_dev,
+                        face_dev, out);
+}
+
+// ------------------------------------------------------------------------------------------
 // stage 1: projector patterns on the device
 // ------------------------------------------------------------------------------------------
 int64_t scan3d_pattern_bytes(const scan3d_config* c, int dir)

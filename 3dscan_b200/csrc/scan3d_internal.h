@@ -397,6 +397,48 @@ struct OrientWorkspace {
     // (state->flipped_normals); nothing is written when state->bad is set
     cudaError_t apply(int32_t* faces, float* nrm, uint32_t n, uint32_t nf, cudaStream_t st, int64_t* launches);
 };
+
+// the sample-to-surface distances (scan3d_distance_kernels.cu; common/scan3d_distance_math.h has the arithmetic and
+// the index rule): a cell index over the faces, queried by one sample per thread
+struct DistanceState {
+    unsigned long long entries;    // sum of the clamped face entry counts
+    double sum_d, sum_d2, max_d;   // the sums of sqrt(d2) and d2, and the largest sqrt(d2), over the matched samples
+    long long max_sample;          // -1 when nothing matched
+    unsigned long long samples, matched, invalid, inside;
+    float min_signed, max_signed;
+    uint32_t bad;                  // a face index outside [0, vertices) or a coordinate not finite: SCAN3D_ERR_ARG
+    uint32_t range;                // a face vertex's cell outside the key range: SCAN3D_ERR_CONFIG
+    uint32_t entries32;            // the 32-bit scan total (equal to entries when entries < 2^32)
+    uint32_t pad;
+};
+// the statistics of one block of samples
+struct DistancePartial {
+    double sum_d, sum_d2, max_d;
+    long long max_sample;
+    uint32_t samples, matched, invalid, inside;
+    float min_signed, max_signed;
+};
+struct DistanceWorkspace {
+    DeviceBuffer<uint32_t> face_counts;        // [cdiv(faces, POINT_BLOCK)] entries per block of faces, then offsets
+    DeviceBuffer<unsigned long long> keys;     // [2 entries] the cell table
+    DeviceBuffer<uint2> cells;                 // [2 entries] (faces in the cell, end of its range)
+    DeviceBuffer<uint32_t> entry_slot, entry_face;   // [entries] per (face, cell) entry: its table slot, its face
+    DeviceBuffer<uint32_t> ids;                // [entries] face ids by cell
+    DeviceBuffer<uint32_t> cursor;             // [1]
+    DeviceBuffer<DistancePartial> partials;    // [cdiv(samples, s3p::BLOCK)]
+    DeviceBuffer<DistanceState> state;
+    uint32_t table = 0;                        // slots of the cell table of the last build
+    // 2 launches for the faces [nf][3] of n vertices: per face the index and finiteness checks, the cell box and the
+    // entry count (state->bad, range, entries), k_scan over the per-block counts
+    cudaError_t count(const float* xyz, const int32_t* faces, uint32_t n, uint32_t nf, double S, cudaStream_t st,
+                      int64_t* launches);
+    // 5 launches after a count without an error that found entries < 2^32: the cells into the table, their ranges, the
+    // face-id scatter, the query of samples [ns][3] (nrm set: a sample is a point with a non-zero normal) into dist /
+    // face (either may be null), the statistics into state
+    cudaError_t query(const float* xyz, const int32_t* faces, uint32_t nf, uint32_t entries, double S, double r2,
+                      const float* samples, const float* nrm, uint32_t ns, float* dist, int32_t* face, cudaStream_t st,
+                      int64_t* launches);
+};
 }  // namespace s3d
 
 // Every device buffer the context owns is a DeviceBuffer: scan3d_destroy frees them all by deleting the context.
@@ -487,6 +529,7 @@ struct scan3d_ctx {
     s3d::FillWorkspace fill;              // scan3d_voxel_surface_fill_holes, scan3d_mesh_fill_holes_dev
     s3d::RepairWorkspace repair;          // scan3d_voxel_surface_repair, scan3d_mesh_repair_dev
     s3d::OrientWorkspace orient;          // scan3d_voxel_surface_orient / _measure, scan3d_mesh_orient_dev / _measure_dev
+    s3d::DistanceWorkspace dist;          // scan3d_voxel_surface_distance / _distance_dev, scan3d_mesh_distance_dev
 
     // the held voxel surface, and the spare set that components, decimate, smooth, fill and repair write before they
     // swap it in

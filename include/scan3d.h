@@ -880,6 +880,86 @@ int scan3d_voxel_surface_measure(scan3d_ctx *ctx, scan3d_measure_result *out);
 int scan3d_mesh_measure_dev(scan3d_ctx *ctx, const float *xyz_dev, int64_t n_vertices, const int32_t *faces_dev,
                             int64_t n_faces, scan3d_measure_result *out);
 
+/* ---- distances of samples from a triangle surface: MeshLab's "Hausdorff Distance" (Metro, Cignoni, Rocchini &
+ * Scopigno 1998), one-sided and within a radius --------------------------------------------------------------------
+ * For every sample, the nearest face of a triangle mesh within R = (double)max_distance, the exact distance to it and
+ * its side; and the one-sided Hausdorff distance, the mean and the RMS over the matched samples.  A symmetric Hausdorff
+ * distance between two meshes is two calls with the roles swapped.  Every result is a pure function of the samples,
+ * the mesh and R: bit-reproducible, independent of the hash, of scheduling, of the order of the faces in a cell and of
+ * the SM count.  The arithmetic is in 3dscan_b200/common/scan3d_distance_math.h.
+ *
+ * Rules.
+ * - A face with a repeated index is degenerate and never matched.
+ * - q is the closest point of a face (a, b, c) to the sample p (float coordinates as doubles): Ericson's
+ *   ClosestPtPointTriangle (Real-Time Collision Detection, 5.1.5), his Voronoi-region tests in his order, every double
+ *   operation one correctly rounded IEEE operation in a fixed order without FMA.  A face of zero area (l2 == 0 in the
+ *   hole filling's triangle terms), and a region whose divisor is not > 0, take the closest point of the segments ab,
+ *   bc, ca instead (the smaller d2, a tie the first segment; a zero-length segment gives its start).  No NaN arises
+ *   from finite inputs.
+ * - d2 = (dx dx + dy dy) + dz dz with d = p - q.  The candidate faces of p are those whose cell box (below) meets the
+ *   3 x 3 x 3 cells around p's cell; every face whose exact distance from p is at most R is one.  A candidate
+ *   qualifies when d2 <= R R; the nearest face has the smallest d2, a tie the smaller face index.  p is matched when
+ *   a face qualifies.
+ * - s = (p - q) . N with N = (b - a) x (c - a) in double; the signed distance is (float)(-sqrt(d2)) when s < 0, else
+ *   (float)sqrt(d2).  With outward windings (an extraction, scan3d_voxel_surface_orient) negative means inside.  At a
+ *   saddle vertex or edge the sign of the nearest face's normal can be wrong (Baerentzen & Aanaes 2005); the
+ *   angle-weighted pseudonormal that fixes it is not used.
+ * - A sample with a coordinate that is not finite is invalid; one whose cell is outside the key range is unmatched.
+ * - The index: cell edge S = max_distance (1 + 2^-20) (the alignment's); a face is registered in every cell of the box
+ *   [floor(lo / S), floor(hi / S)] per axis, lo and hi the float bounding box of its corners; a face has
+ *   prod (floor(hi / S) - floor(lo / S) + 1) entries.
+ * - Outputs per sample, both optional (NULL), in device memory of the ctx's GPU: dist_dev float, the signed distance,
+ *   NaN when invalid or unmatched; face_dev int32, the nearest face, -1 when invalid or unmatched.
+ * - Statistics over the matched samples: max = the largest sqrt(d2) in double (the one-sided Hausdorff distance within
+ *   R), max_sample its sample (a tie the smaller index, -1 when nothing matched), mean = sum sqrt(d2) / matched,
+ *   rms = sqrt(sum d2 / matched) (0 when nothing matched), min_signed and max_signed the extreme signed distances (0
+ *   when nothing matched); inside counts the matched samples of negative sign.  The two sums follow the alignment's
+ *   scheme: a grid fixed by the sample count (256 samples per block), a fixed tree in each block and one block summing
+ *   the partials in a fixed order.
+ *
+ * scan3d_voxel_surface_distance: the samples are the merge's model, the outputs of the last scan3d_voxel_finish with a
+ * non-zero normal (the alignment's model); the target is the held voxel surface.  dist_dev and face_dev are indexed by
+ * voxel ordinal, min(total, max_voxels) of them (scan3d_voxel_count); a voxel that is not in the model is no sample and
+ * gets NaN / -1.  scan3d_voxel_surface_distance_dev: n samples xyz float [n][3] in device memory (scan3d_device_points,
+ * for instance: one view against the model) against the held voxel surface.  scan3d_mesh_distance_dev: any samples
+ * against any triangle mesh in device memory of the ctx's GPU (xyz_dev float [n_vertices][3], faces_dev int32
+ * [n_faces][3]), the camera-grid mesh (scan3d_device_mesh_faces) included.
+ * State: the surface routes need a held surface (SCAN3D_ERR_STATE otherwise).  All three only read: they change no
+ * result, no byte of the held surface, of the component table or of the accumulator, and no decimation flag.
+ * Synchronisation: two per call, one after the per-face entry counts (to size the index), one after every launch.
+ * Launches: 7 per call, an empty mesh and an empty sample set included: the per-face checks, cell boxes and entry
+ * counts, k_scan over them, the cells into the table, the cell ranges, the face-id scatter, the query, the statistics.
+ * When the first synchronisation finds an error the call has made 2.
+ * Memory (ctx-owned, allocated on first use, grown on demand, shared by the three calls): 44 B per entry (a cell table
+ * of 2 slots of 16 B, 12 B of entry scratch), 4 B per 1024 faces and 56 B per 256 samples.
+ * Errors: SCAN3D_ERR_ARG for a null ctx, params or out; max_distance not finite or <= 0; n, n_vertices or n_faces
+ * outside [0, 2^31); a NULL samples_dev, xyz_dev or faces_dev with a non-zero count; a pointer not 4-byte aligned;
+ * and, found on the device, a face index outside [0, n_vertices) or a vertex coordinate that is not finite.
+ * SCAN3D_ERR_CONFIG when a vertex of a face (indices in range) has its cell outside [-2^20, 2^20) on some axis, or the
+ * mesh has 2^32 or more entries (a larger max_distance needs fewer).  SCAN3D_ERR_STATE for the surface routes without
+ * a held surface.  An argument or state error launches nothing; on any error nothing is written. */
+typedef struct {
+    float max_distance;                 /* R: finite, > 0 */
+} scan3d_distance_params;
+
+typedef struct {
+    int64_t samples, matched, invalid, inside;
+    int64_t max_sample;                 /* -1 when nothing matched */
+    double max, mean, rms;              /* unsigned, over the matched samples */
+    float min_signed, max_signed;
+    int64_t entries;                    /* face-cell entries of the index (to size memory, choose R) */
+} scan3d_distance_result;
+
+int scan3d_voxel_surface_distance(scan3d_ctx *ctx, const scan3d_distance_params *p, float *dist_dev,
+                                  int32_t *face_dev, scan3d_distance_result *out);
+int scan3d_voxel_surface_distance_dev(scan3d_ctx *ctx, const float *samples_dev, int64_t n,
+                                      const scan3d_distance_params *p, float *dist_dev, int32_t *face_dev,
+                                      scan3d_distance_result *out);
+int scan3d_mesh_distance_dev(scan3d_ctx *ctx, const float *samples_dev, int64_t n, const float *xyz_dev,
+                             int64_t n_vertices, const int32_t *faces_dev, int64_t n_faces,
+                             const scan3d_distance_params *p, float *dist_dev, int32_t *face_dev,
+                             scan3d_distance_result *out);
+
 /* ---- either side of the path (SURVEY.md 8 f2 / f4) --------------------------------------- */
 /* cvUndistort2(cap, undist_cap, K, d) as the capture loop applies it to every captured camera frame
  * and every projected pattern (2/project_pattern.cpp:220,234,372-427): OpenCV 2.4's cv::undistort,
